@@ -2,6 +2,7 @@
 """bench.py — Mistral-7B batch-1 decode throughput on N B200s (BASELINE.json metric), with roofline and CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--shape m7] [--wtype q8_0] [--ctx 4096]
+                    [--dump-outputs DIR]
 
 A "step" is one decoded token: one pass of the hot path (embed -> 32 x [norm+QKV+rope+KV, attention, Wo+residual,
 norm+W1|W3+GLU, W2+residual] -> norm+classifier).  The workload is BASELINE config[1]: Mistral-7B-v0.2 architecture,
@@ -17,6 +18,11 @@ streams them from HBM; no L2 flush is needed between steps.
 `--impl reference` : the reference's CPU path (oracle/ restatement; the reference C++ does not build on x86, DESIGN.md)
            on all host cores, same model, one token per step.
 N > 1    : tensor parallel over N GPUs (one process per GPU, strong scaling: same model, sharded).
+`--dump-outputs DIR` : after the timed steps, rank 0 writes what the timed path computed in its last step, as float32 .npy
+           files: the decode workload and every --impl reference run write DIR/logits.npy, the vocab_size logits of the last
+           timed token; the perplexity workload on the GPU writes DIR/logits_sample.npy, the logits of a fixed, seeded
+           sample of at most 128 of its positions (perplexity_sample_rows).  Weights, tokens and positions depend only on the arguments, so two builds run with the
+           same arguments can be compared output for output.  bench_outputs/ in the repository is git-ignored for this.
 """
 from __future__ import annotations
 
@@ -102,6 +108,32 @@ def positions_for(steps: int, ctx: int) -> list:
     return [int(round(i * (ctx - 1) / (steps - 1))) for i in range(steps)]
 
 
+def decode_inputs(steps: int, warmup: int, ctx: int, vocab_size: int) -> tuple:
+    """(tokens, positions, warm-up steps, timed steps) of the decode workload, a fixed function of the arguments; each step
+    is a (token, position) pair."""
+    pos_list = positions_for(steps, ctx)
+    toks = [int(t) for t in np.random.default_rng(123).integers(3, vocab_size, size=steps + warmup)]
+    warm = [(toks[i], pos_list[min(i, len(pos_list) - 1)]) for i in range(warmup)]
+    timed = [(toks[warmup + i], pos_list[i]) for i in range(steps)]
+    return toks, pos_list, warm, timed
+
+
+def perplexity_tokens(n_tok: int, vocab_size: int) -> np.ndarray:
+    """The perplexity workload's input: n_tok tokens and the target after the last one, a fixed function of the arguments."""
+    return np.random.default_rng(321).integers(3, vocab_size, size=n_tok + 1).astype(np.int32)
+
+
+def perplexity_sample_rows(n_tok: int) -> np.ndarray:
+    """The positions whose logits --dump-outputs keeps for the perplexity workload: a fixed, seeded sample (<= 64 MB at m7)."""
+    return np.sort(np.random.default_rng(0).choice(n_tok, size=min(128, n_tok), replace=False))
+
+
+def dump_outputs(d: str, **arrays):
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), np.asarray(a, dtype=np.float32))
+
+
 def build_model_streaming(cfg_full: dict, cfg: dict, wtype, seed: int, keep_host: bool, std: float = 0.02, **cuda_kw):
     """Generate the synthetic checkpoint tensor by tensor and upload each as it is made (peak host RAM = one tensor
     unless keep_host, which the CPU baseline needs)."""
@@ -170,6 +202,8 @@ def run_reference(args):
         lg = om.forward(tok, pos_list[i], 1)
         tok = oracle.sample_argmax(lg)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, logits=lg)
     tps = args.steps / dt
     sample = (f"{args.steps} tokens at positions spread uniformly over [0, {cfg['max_seq_len']}) — the GPU arm's positions — of the same "
               f"{args.shape} {args.wtype} model (full depth), wall clock")
@@ -218,8 +252,7 @@ def perplexity_summary(model, cfg, capi, n_tok: int) -> dict:
     the decode kernels, on the model bench.py already holds.  Full line: `bench.py --workload perplexity`."""
     import torch
     from xalm_b200.model import InferenceState
-    rng = np.random.default_rng(321)
-    toks = rng.integers(3, cfg["vocab_size"], size=n_tok + 1).astype(np.int32)
+    toks = perplexity_tokens(n_tok, cfg["vocab_size"])
     out = {"tokens_per_step": n_tok, "metric": "perplexity_tokens_per_s"}
     st = InferenceState(cfg).cuda()
     for split, name in ((3, "precise_hi_lo_fp16"), (1, "plain_fp16")):
@@ -263,8 +296,7 @@ def run_perplexity_workload(args):
     cfg = X.parse_config(synth.metadata_strings(cfg_full), args.ctx)
     wtype = T.parse(args.wtype)
     n_tok = min(args.tokens, cfg["max_seq_len"])
-    rng = np.random.default_rng(321)
-    toks = rng.integers(3, cfg["vocab_size"], size=n_tok + 1).astype(np.int32)
+    toks = perplexity_tokens(n_tok, cfg["vocab_size"])
     config = {"workload": f"{args.shape} ({'Mistral-7B-v0.2' if args.shape == 'm7' else args.shape} architecture) random-init {args.wtype}, "
                           f"perplexity mode over a {n_tok}-token synthetic input (batched prefill, dequantised weights on tcgen05 GEMMs)",
               "shape": args.shape, "weight_format": args.wtype, "tokens_per_step": n_tok, "context": cfg["max_seq_len"],
@@ -286,6 +318,8 @@ def run_perplexity_workload(args):
             lg = om.forward(int(toks[i]), i, 1)
             s += float(np.log(oracle.sample_prob(lg, int(toks[i + 1]))))
         dt = time.perf_counter() - t0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, logits=lg)
         tps = n / dt
         sample = f"positions 0..{n - 1} of the same input, one Model::forward + sample_prob each (main.cpp:244-254), wall clock"
         print(json.dumps({"impl": "reference", "metric": "perplexity_tokens_per_s", "value": tps, "unit": "tok/s", "n_gpus": args.gpus,
@@ -343,6 +377,9 @@ def run_perplexity_workload(args):
     # accuracy of this mode against the token-at-a-time decode kernels on the same KV prefix (last 4 positions)
     from xalm_b200.model import InferenceState
     lg_all = model.prefill(toks[:-1], 0, want_logits=2)
+    if args.dump_outputs:
+        # the timed step is a pure function of (weights, tokens, position 0): this pass recomputes exactly its logits
+        dump_outputs(args.dump_outputs, logits_sample=lg_all[perplexity_sample_rows(n_tok)])
     st = InferenceState(cfg).cuda()
     worst = 0.0
     for pos in range(n_tok - 4, n_tok):
@@ -403,7 +440,11 @@ def main():
                     help="decode = BASELINE config[1] (the headline metric); perplexity = config[2]: batched prefill of a 4k-token input")
     ap.add_argument("--tokens", type=int, default=4096, help="perplexity workload: tokens per step")
     ap.add_argument("--split", type=int, default=0, help="perplexity workload: operand precision (0 = library default 3; 1 = plain fp16)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/*.npy (float32; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
 
     if args.workload == "perplexity":
@@ -462,24 +503,25 @@ def main():
                                                 tp_size=world, comm_id=comm_id, stream=stream, ipc_exchange=ipc_exchange)
     gen_s = time.time() - t0
     ctx = cfg["max_seq_len"]
-    pos_list = positions_for(args.steps, ctx)
-    rng = np.random.default_rng(123)
-    toks = [int(t) for t in rng.integers(3, cfg["vocab_size"], size=args.steps + args.warmup)]
+    toks, pos_list, warm_steps, timed_steps = decode_inputs(args.steps, args.warmup, ctx, cfg["vocab_size"])
 
     # ---- device-timed: weights and KV resident, logits stay on the device ----
-    for i in range(args.warmup):
-        model.forward_async(toks[i], pos_list[min(i, len(pos_list) - 1)], 1)
+    for tok, pos in warm_steps:
+        model.forward_async(tok, pos, 1)
     model.sync()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(local_rank) as clocks:
         barrier()
         e0.record()
-        for i in range(args.steps):
-            model.forward_async(toks[args.warmup + i], pos_list[i], 1)
+        for tok, pos in timed_steps:
+            model.forward_async(tok, pos, 1)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
         launches = model.last_launch_count() * args.steps
+        if args.dump_outputs and rank == 0:
+            # read now: the end-to-end loops below overwrite the device logits
+            dump_outputs(args.dump_outputs, logits=model.read_state(capi.S_LOGITS, cfg["vocab_size"]))
         # ---- end to end through the public API: host token in, host logits out, host sampler ----
         state = InferenceState(cfg).cuda()
         sampler = Sampler(cfg)

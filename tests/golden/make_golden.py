@@ -17,7 +17,8 @@ executable pins there are):
   tiny_<type>.xalm   complete checkpoints written by /root/reference/convert.py from a synthetic HF
                      directory (config.json + tokenizer.json + model.safetensors), for
                      f16 / bf16 / q8_0 / q4_0 / f8_e4m3.
-  tiny_src.npz       the fp32 source weights those files were converted from.
+                     Their fp32 source weights are not stored: torch.Generator seed 1234 regenerates them
+                     bit for bit (make_tiny_checkpoints).
 """
 import json
 import os
@@ -148,7 +149,6 @@ def make_tiny_checkpoints():
             w[p + "mlp.down_proj.weight"] = rnd(d, h, std=0.1)
         w = {k: v.contiguous() for k, v in w.items()}
         save_file(w, os.path.join(tmp, "model.safetensors"))
-        np.savez_compressed(os.path.join(HERE, "tiny_src.npz"), **{k: v.numpy() for k, v in w.items()})
         for t in ["f16", "bf16", "q8_0", "q4_0", "f8_e4m3"]:
             out = os.path.join(HERE, f"tiny_{t}.xalm")
             r = subprocess.run([sys.executable, os.path.join(REF, "convert.py"), "--input", tmp, "--type", t, "--output", out],

@@ -125,7 +125,7 @@ def test_cuda_reproduces_the_reference(name, tmp_path):
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libxalm_ref.so")
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref/libxalm_ref.so not built (needs /root/reference: make -f oracle/Makefile.ref)")
+@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref/libxalm_ref.so not built (build() builds it when XALM_REFERENCE names the reference's sources)")
 def test_oracle_against_the_live_reference(tmp_path):
     """A checkpoint no fixture covers (bf16 weights, 3 kv heads' worth of GQA, window 20 with the prompt running past it)."""
     path = str(tmp_path / "live.xalm")
