@@ -129,7 +129,7 @@ int xalm_cuda_forward_async(xalm_cuda_model* m, int token, int pos, int mode);
 int xalm_cuda_sync(xalm_cuda_model* m);
 /* ---- batched prefill: the loops of main.cpp:94-100 (prompt hydrate) and :244-254 (perplexity), which call
  *      Model::forward once per position, as ONE pass over the weights on the tcgen05 tensor-core path ---------- */
-/* Positions pos0 .. pos0+n-1 (pos0 + n <= max_seq_len: no ring wrap; past that use xalm_cuda_forward).  Fills the KV
+/* Positions pos0 .. pos0+n-1 (pos0 + n <= max_seq_len: no ring wrap; past that use xalm_cuda_prefill_window).  Fills the KV
  * cache exactly as n forward calls would (fp16-operand rounding aside).  want_logits: 0 = none (HYDRATE_KV_CACHE for
  * every position), 1 = logits of the last position -> logits_host[vocab], 2 = every position -> logits_host[n*vocab].
  * targets/probs_host (n entries each, or NULL; needs want_logits 2): probs_host[i] = Sampler::sample_prob(targets[i])
@@ -140,6 +140,16 @@ int xalm_cuda_sync(xalm_cuda_model* m);
  * for activations only, 1 = plain fp16 (fastest; ~4e-2 at that depth).  North star tolerance: 1e-2. */
 int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
                       const int* targets, float* probs_host);
+/* The same batched pass past the context window, where the KV cache is a ring: positions pos0 .. pos0+n-1 with
+ * pos0 >= max_seq_len and 1 <= n <= max_seq_len - 2 (each ring slot is written at most once per call; longer runs go in
+ * chunks).  Leaves the KV cache as n xalm_cuda_forward calls would: each new row in its ring slot 2 + (pos - 2) % (max_seq_len - 2),
+ * and the two attention-sink keys in slots 0 and 1 re-rotated n more times (bit-identical to the token loop).  Each
+ * position attends to the two sinks and the max_seq_len - 2 latest positions, itself included.  want_logits, logits_host,
+ * targets, probs_host and the "prefill_split" knob mean what they mean for xalm_cuda_prefill.  Anything else — positions
+ * below the window, n too large, a token out of range — is XALM_ERR_INVALID before anything runs (the cache is untouched);
+ * tensor-parallel handles get XALM_ERR_UNSUPPORTED.  Synchronous. */
+int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
+                             const int* targets, float* probs_host);
 /* Enqueue only (no read-back, no host sync) — bench.py's device-timed leg. */
 int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits);
 /* Pinned host buffer the logits are copied into by xalm_cuda_forward (alias it as InferenceState::_logits). */

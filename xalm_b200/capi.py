@@ -77,6 +77,7 @@ SYMBOLS = {
     "xalm_cuda_mega_timeline": (_i, [_vp, _vp, C.c_size_t, C.POINTER(_i), C.POINTER(_i)]),
     "xalm_cuda_bench_matvec": (_i, [_i, _i, _i, _i, _i, _i, _i, _fp]),
     "xalm_cuda_prefill": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
+    "xalm_cuda_prefill_window": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "xalm_cuda_prefill_async": (_i, [_vp, _vp, _i, _i, _i]),
     "xalm_cuda_gemm": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i]),
     "xalm_cuda_bench_gemm": (_i, [_i, _i, _i, _i, _i, _fp]),

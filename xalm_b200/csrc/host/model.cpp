@@ -398,17 +398,30 @@ void Model::forward(const InferenceState& s, const int token, const int pos, con
 
 bool Model::prefill(const InferenceState& s, const int* tokens, const int n, const int pos0, const InferenceMode mode, const int* targets,
                     float* probs) const {
+	if (n <= 0 || pos0 < 0 || (long long) pos0 + n > config.max_seq_len) return false;
+	return prefill_call(false, s, tokens, n, pos0, mode, targets, probs);
+}
+
+bool Model::prefill_window(const InferenceState& s, const int* tokens, const int n, const int pos0, const InferenceMode mode, const int* targets,
+                           float* probs) const {
+	if (n <= 0 || pos0 < config.max_seq_len || n > config.max_seq_len - 2) return false;
+	return prefill_call(true, s, tokens, n, pos0, mode, targets, probs);
+}
+
+bool Model::prefill_call(const bool window, const InferenceState& s, const int* tokens, const int n, const int pos0, const InferenceMode mode,
+                         const int* targets, float* probs) const {
 	if (device != Device::CUDA || !handle_)
 		throw std::runtime_error("Model::prefill: model is not on a CUDA device (call model.cuda()); this backend has no CPU path");
-	if (n <= 0 || pos0 < 0 || (long long) pos0 + n > config.max_seq_len || tp_size_ > 1) return false;
+	if (tp_size_ > 1) return false;
 	if (!s.logits_ptr_ && s.device == Device::CUDA) s.logits_ptr_ = xalm_cuda_logits_host(handle_);
+	auto call = window ? xalm_cuda_prefill_window : xalm_cuda_prefill;
 	int rc;
-	if (targets && probs) rc = xalm_cuda_prefill(handle_, tokens, n, pos0, 2, nullptr, targets, probs);
-	else if (mode == InferenceMode::OUTPUT_LOGITS) rc = xalm_cuda_prefill(handle_, tokens, n, pos0, 1, s.logits(), nullptr, nullptr);
-	else rc = xalm_cuda_prefill(handle_, tokens, n, pos0, 0, nullptr, nullptr, nullptr);
+	if (targets && probs) rc = call(handle_, tokens, n, pos0, 2, nullptr, targets, probs);
+	else if (mode == InferenceMode::OUTPUT_LOGITS) rc = call(handle_, tokens, n, pos0, 1, s.logits(), nullptr, nullptr);
+	else rc = call(handle_, tokens, n, pos0, 0, nullptr, nullptr, nullptr);
 	if (rc == XALM_ERR_UNSUPPORTED) return false; // e.g. a head_dim the batched attention kernel does not take
 	if (rc != XALM_OK) {
-		std::fprintf(stderr, "Model::prefill: %s\n", xalm_cuda_last_error());
+		std::fprintf(stderr, "Model::%s: %s\n", window ? "prefill_window" : "prefill", xalm_cuda_last_error());
 		std::abort();
 	}
 	return true;

@@ -160,9 +160,16 @@ struct Model {
 	// when the batch cannot take this path (ring-buffer wrap past max_seq_len, tensor-parallel shard): callers fall back to forward().
 	bool prefill(const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode = InferenceMode::OUTPUT_LOGITS,
 	             const int* targets = nullptr, float* probs = nullptr) const;
+	// The same past the context window, where the KV cache is a ring with two attention sinks (xalm_cuda_prefill_window):
+	// pos0 >= max_seq_len and n <= max_seq_len - 2 (longer runs go in chunks).  Leaves the cache as n forward() calls would.
+	// Returns false — and does nothing — when the batch cannot take this path (positions outside that range, tensor-parallel shard).
+	bool prefill_window(const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode = InferenceMode::OUTPUT_LOGITS,
+	                    const int* targets = nullptr, float* probs = nullptr) const;
 
 private:
 	explicit Model(const Config& c) : config(c) {}
+	bool prefill_call(bool window, const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode, const int* targets,
+	                  float* probs) const;
 	std::map<std::string, Tensor> host_; // until cuda()
 	std::map<std::string, Type> types_;  // kept for active_bytes after the host copies are gone
 	const Xalm::file_info* deferred_ = nullptr; // defer_load: where cuda() reads the tensors from

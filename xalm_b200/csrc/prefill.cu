@@ -14,6 +14,8 @@
 //   x --rmsnorm_rows--> xb;  xb . (W1|W3)^T --gemm, GLU epilogue act(g)*u--> hb [A tiles]
 //   hb . W2^T      --gemm, residual epilogue--> x += .
 // then final rmsnorm, classifier GEMM -> logits fp32 (rows, vocab), and softmax-at-target for perplexity.
+// Past the context window (window mode) the same loop runs over the KV ring with its two attention sinks: see
+// gather_ring_kernel / sink_versions_kernel and the window-mode notes of the attention kernels.
 //
 // Operand layout ("A tiles"/"B tiles"): 128 (A) or 256 (B) rows x 64 K-elements of fp16, stored as the exact
 // shared-memory image tcgen05.mma wants for a K-major SWIZZLE_128B operand (8-row x 128-byte atoms, 16-byte chunks
@@ -31,6 +33,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <float.h>
+#include <limits.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -407,8 +410,12 @@ struct GemmArgs {
 	int n_kb_total;     // 128-key blocks per kv head in kt / vt
 	__half* k_cache;
 	__half* v_cache;
+	int ring;           // window mode: the KV cache is a ring of this many data slots after 2 sinks (cache row 2 + (pos - 2) % ring); 0 = linear
+	__half* k_stage;    // window mode: K / V rows also go to these linear staging buffers, row stage_row0 + m (attention reads them)
+	__half* v_stage;
+	int stage_row0;
 	const float2* rope_cs; // (T, head_dim/2): {cos, sin}(pos * freq) per row, from rope_table_kernel
-	int q_dim, kv_dim, head_dim, pos0;
+	int q_dim, kv_dim, head_dim, pos0; // pos0: position of row 0 (the cache row in linear mode)
 	float qkv_clip;
 	// GLU
 	ATiles o;
@@ -540,6 +547,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const GemmArgs
 				// 16 columns = 8 rotation pairs at a time; q_dim, kv_dim and head_dim are multiples of 16, so a chunk never straddles
 				// the q | k | v regions or a head, and leaves as two 16-byte stores
 				const int pos = g.pos0 + m;
+				const int crow = g.ring ? 2 + (pos - 2) % g.ring : pos; // KV cache row of this position
 				const float2* cs_row = g.rope_cs + (size_t) (mrow ? m : 0) * (g.head_dim / 2);
 				for (int c = 0; c < GB_N; c += 16) {
 					float v[16];
@@ -582,9 +590,14 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_tc_kernel(const GemmArgs
 						continue;
 					}
 					__half* dst = region == 0 ? g.q_out + (size_t) m * g.q_dim + j0
-					            : region == 1 ? g.k_cache + (size_t) pos * g.kv_dim + j0 : g.v_cache + (size_t) pos * g.kv_dim + j0;
+					            : region == 1 ? g.k_cache + (size_t) crow * g.kv_dim + j0 : g.v_cache + (size_t) crow * g.kv_dim + j0;
 					reinterpret_cast<uint4*>(dst)[0] = reinterpret_cast<const uint4*>(h)[0];
 					reinterpret_cast<uint4*>(dst)[1] = reinterpret_cast<const uint4*>(h)[1];
+					if (region > 0 && g.k_stage) {
+						__half* sd = (region == 1 ? g.k_stage : g.v_stage) + (size_t) (g.stage_row0 + m) * g.kv_dim + j0;
+						reinterpret_cast<uint4*>(sd)[0] = reinterpret_cast<const uint4*>(h)[0];
+						reinterpret_cast<uint4*>(sd)[1] = reinterpret_cast<const uint4*>(h)[1];
+					}
 					if (region > 0 && g.kt) { // the same values as operand tiles (key = pos: this path is only taken with pos0 == 0)
 						const int kvh = j0 >> 7, hc = j0 & 127;
 						const size_t blk = (size_t) (kvh * g.n_kb_total + (pos >> 7)) * 2;
@@ -765,6 +778,9 @@ __global__ void target_prob_kernel(const float* __restrict__ logits, int vocab, 
 // causal attention over the fp16 KV cache for a block of 64 query rows of one head (attn + softmax, infer.cpp:325-359,
 // 280-297, for T rows at once).  Flash-style: S = Q K^T and O += P V on mma.sync m16n8k16 tiles (fp16 in, fp32 out),
 // online softmax in fp32 with expf.  Query row i (position pos0+i) sees cache rows [0, pos0+i].
+// Window mode (win > 0, past the context window): k/v point at a linear staging copy of the ring, query row i sees only the
+// band of rows (pos0+i-win, pos0+i], plus two attention-sink keys of its own (sink_k row i) scored in fp32; the sink scores
+// seed the running maximum and enter the sum and the output at the end.
 // Not a tcgen05 kernel: attention is ~7 % of the prefill flops at 4k; the GEMMs above are where the tensor time goes.
 // ------------------------------------------------------------------------------------------------------------------
 struct AttnPArgs {
@@ -774,7 +790,31 @@ struct AttnPArgs {
 	const __half* v_cache;
 	ATiles o;              // xb2
 	int T, pos0, q_dim, kv_dim, n_heads, n_kv_heads, n_qt;
+	int win;               // window mode: keys per query in the band; 0 = linear (causal over [0, pos0+i])
+	const __half* sink_k;  // window mode: (T, 2, kv_dim) the sink keys as query row i sees them
+	const __half* sink_v;  // window mode: (2, kv_dim) the sink values
 };
+
+// window mode: the two sink scores of query row `row`, q.k in fp32 over head_dim from the (hi + lo) q held in global memory,
+// split over the 4 lanes of a quad (each lane: HD/4 elements), reduced over the quad
+template <int HD>
+__device__ __forceinline__ void sink_scores_quad(const AttnPArgs& a, int row, int h, int kvh, int lane, float (&sc)[2]) {
+	const int r = min(row, a.T - 1);
+	const __half* qh = a.q + (size_t) r * a.q_dim + h * HD;
+	const __half* ql = a.q_lo ? a.q_lo + (size_t) r * a.q_dim + h * HD : nullptr;
+#pragma unroll
+	for (int s = 0; s < 2; s++) {
+		const __half* kp = a.sink_k + ((size_t) r * 2 + s) * a.kv_dim + kvh * HD;
+		float acc = 0.f;
+		for (int d = (lane & 3) * (HD / 4); d < (lane & 3) * (HD / 4) + HD / 4; d++) {
+			const float qv = __half2float(qh[d]) + (ql ? __half2float(ql[d]) : 0.f);
+			acc = fmaf(qv, __half2float(kp[d]), acc);
+		}
+		acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+		acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+		sc[s] = acc;
+	}
+}
 
 __device__ __forceinline__ void ldsm4(uint32_t (&r)[4], uint32_t saddr) {
 	asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(saddr));
@@ -815,6 +855,7 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 	const int q_last = min(q0 + BQ, a.T) - 1;
 	const int kv_total = a.pos0 + q_last + 1;  // cache rows any row of this tile may see
 	const int n_kb = (kv_total + BKV - 1) / BKV;
+	const int kb0 = a.win ? max(0, a.pos0 + q0 - a.win + 1) / BKV : 0; // window mode: blocks wholly below the band are skipped
 	// chunk (r, c) lives at r*ROWB + ((c ^ (r & 7)) * 16): conflict-free for ldmatrix (8 rows x 16 bytes per phase)
 	auto soff = [](int r, int c) { return (uint32_t) (r * ROWB + ((c ^ (r & 7)) << 4)); };
 
@@ -835,7 +876,7 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 			cp_async16(s_u32(sV) + buf * BKV * ROWB + soff(r, c), a.v_cache + g, ok);
 		}
 	};
-	load_kv(0, 0);
+	load_kv(kb0, 0);
 	asm volatile("cp.async.commit_group;" ::: "memory");
 
 	float o_acc[HD / 8][4];
@@ -849,9 +890,18 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 	const float scale = 1.0f / sqrtf((float) HD);
 	const int row_a = q0 + warp * 16 + (lane >> 2); // this thread's two query rows: row_a and row_a + 8
 	bool q_loaded = false;
+	float sink_s[2][2]; // [row_a, row_a + 8][sink], scaled
+	if (a.win) {
+#pragma unroll
+		for (int r = 0; r < 2; r++) {
+			sink_scores_quad<HD>(a, row_a + 8 * r, h, kvh, lane, sink_s[r]);
+			sink_s[r][0] *= scale; sink_s[r][1] *= scale;
+			m_run[r] = fmaxf(sink_s[r][0], sink_s[r][1]); // every row has a finite maximum even where a block masks all its keys
+		}
+	}
 
-	for (int kb = 0; kb < n_kb; kb++) {
-		const int buf = kb & 1;
+	for (int kb = kb0; kb < n_kb; kb++) {
+		const int buf = (kb - kb0) & 1;
 		if (kb + 1 < n_kb) load_kv(kb + 1, buf ^ 1);
 		asm volatile("cp.async.commit_group;" ::: "memory");
 		asm volatile("cp.async.wait_group 1;" ::: "memory");
@@ -886,7 +936,8 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 			}
 		}
 		// ---- scale, causal mask, online softmax ----
-		const bool need_mask = kb * BKV + BKV - 1 > a.pos0 + q0 + warp * 16; // some key of this block is beyond the warp's first row
+		const bool need_mask = kb * BKV + BKV - 1 > a.pos0 + q0 + warp * 16  // some key of this block is beyond the warp's first row
+		                    || (a.win && kb * BKV < a.pos0 + q0 + warp * 16 + 15 - a.win + 1); // or below the band of its last row
 		float mx[2] = {-INFINITY, -INFINITY};
 #pragma unroll
 		for (int i = 0; i < BKV / 8; i++) {
@@ -896,7 +947,7 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 				if (need_mask) {
 					const int key = kb * BKV + i * 8 + 2 * (lane & 3) + (j & 1);
 					const int row = row_a + (j >> 1) * 8;
-					if (key > a.pos0 + row) v = -INFINITY;
+					if (key > a.pos0 + row || (a.win && key <= a.pos0 + row - a.win)) v = -INFINITY;
 				}
 				s[i][j] = v;
 				mx[j >> 1] = fmaxf(mx[j >> 1], v);
@@ -963,6 +1014,15 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 		l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 1);
 		l_run[r] += __shfl_xor_sync(0xffffffffu, l_run[r], 2);
 	}
+	float sink_p[2][2] = {{0.f, 0.f}, {0.f, 0.f}};
+	if (a.win) {
+#pragma unroll
+		for (int r = 0; r < 2; r++) {
+			sink_p[r][0] = expf(sink_s[r][0] - m_run[r]);
+			sink_p[r][1] = expf(sink_s[r][1] - m_run[r]);
+			l_run[r] += sink_p[r][0] + sink_p[r][1];
+		}
+	}
 #pragma unroll
 	for (int r = 0; r < 2; r++) {
 		const int row = row_a + r * 8;
@@ -970,7 +1030,15 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 		const float inv = 1.0f / l_run[r];
 #pragma unroll
 		for (int i = 0; i < HD / 8; i++) {
-			const float v0 = o_acc[i][2 * r] * inv, v1 = o_acc[i][2 * r + 1] * inv;
+			float o0 = o_acc[i][2 * r], o1 = o_acc[i][2 * r + 1];
+			if (a.win) {
+				const int d = kvh * HD + i * 8 + 2 * (lane & 3);
+				const float2 v0s = __half22float2(*reinterpret_cast<const __half2*>(a.sink_v + d));
+				const float2 v1s = __half22float2(*reinterpret_cast<const __half2*>(a.sink_v + a.kv_dim + d));
+				o0 += sink_p[r][0] * v0s.x + sink_p[r][1] * v1s.x;
+				o1 += sink_p[r][0] * v0s.y + sink_p[r][1] * v1s.y;
+			}
+			const float v0 = o0 * inv, v1 = o1 * inv;
 			const int col = h * HD + i * 8 + 2 * (lane & 3);
 			const size_t off = a_off(row, col, a.o.KT);
 			const __half2 hh = __floats2half2_rn(v0, v1);
@@ -993,6 +1061,9 @@ __global__ void __launch_bounds__(128) attn_prefill_kernel(const AttnPArgs a) {
 // it waits for P of block j (S is double-buffered in TMEM).  warps 2-5: softmax, thread = query row: two passes over S in
 // TMEM (row max, then exp), P as fp16 (hi, lo) into a shared-memory operand tile, running (max, sum) and the fp32 output
 // row in registers; O_blk comes back from TMEM one block later and is folded in with the rescale.
+// Window mode (win > 0): the tiles hold a linear staging copy of the ring, query row i sees the band (pos0+i-win, pos0+i] —
+// key blocks wholly below a tile's band are not loaded — plus two sink keys of its own whose fp32 scores seed the running
+// maximum and are added to the sum and the output row at the end.
 // ------------------------------------------------------------------------------------------------------------------
 struct AttnTcArgs {
 	const uint8_t* qt_hi;
@@ -1001,6 +1072,10 @@ struct AttnTcArgs {
 	const uint8_t* vt;   // V^T tiles
 	ATiles o;            // xb2
 	int T, pos0, n_heads, n_kv_heads, n_qb, n_kb_total;
+	int win;              // window mode: keys per query in the band; 0 = linear
+	const __half* sink_k; // window mode: (T, 2, kv_dim) the sink keys as query row i sees them
+	const __half* sink_v; // window mode: (2, kv_dim)
+	int kv_dim;
 	int dbg; // timing knock-outs (XALM_ATTN_DBG, results are then meaningless): 1 = no QK MMAs, 2 = no PV MMAs, 4 = no softmax math / P stores
 };
 
@@ -1085,6 +1160,8 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 	const int q0 = qb * 128;
 	const int q_last = min(q0 + 128, a.T) - 1;
 	const int n_kb = (a.pos0 + q_last) / ATT_BKV + 1; // 64-key blocks any row of this tile sees
+	const int kb0 = a.win ? max(0, a.pos0 + q0 - a.win + 1) / ATT_BKV : 0; // window mode: first block inside the tile's band
+	const int n_it = n_kb - kb0;                       // blocks this tile visits; the rings below count visits, not block indices
 
 	if (threadIdx.x == 0) {
 		mb_init(q_full, 1);
@@ -1108,8 +1185,9 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 			mb_expect_tx(q_full, Cfg::Q_BYTES);
 			bulk_load(sQ, a.qt_hi + qoff, 2 * A_TILE_BYTES, q_full);
 			if (PRECISE) bulk_load(sQ + 2 * A_TILE_BYTES, a.qt_lo + qoff, 2 * A_TILE_BYTES, q_full);
-			for (int j = 0; j < n_kb; j++) {
-				const int slot = j % NKV, use = j / NKV; // use-th fill of this slot
+			for (int it = 0; it < n_it; it++) {
+				const int j = kb0 + it;
+				const int slot = it % NKV, use = it / NKV; // use-th fill of this slot
 				// the retiled cache holds 128-key tiles; block j is rows [64 (j & 1), +64) of K tile (kvh, j / 2, hd half) — a contiguous
 				// 8 KB run of whole 8-row atoms — and V^T tile (kvh, j / 2, j & 1)
 				const uint8_t* ksrc = a.kt + ((size_t) (kvh * a.n_kb_total + (j >> 1)) * 2) * A_TILE_BYTES + (size_t) (j & 1) * (A_TILE_BYTES / 2);
@@ -1165,9 +1243,9 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 			__syncwarp();
 		};
 		mb_wait(q_full, 0);
-		for (int j = 0; j < LA && j < n_kb; j++) issue_qk(j);
-		for (int j = 0; j < n_kb; j++) {
-			if (j + LA < n_kb) issue_qk(j + LA); // the tensor pipe works on later scores while the softmax warps turn these into P
+		for (int j = 0; j < LA && j < n_it; j++) issue_qk(j);
+		for (int j = 0; j < n_it; j++) {
+			if (j + LA < n_it) issue_qk(j + LA); // the tensor pipe works on later scores while the softmax warps turn these into P
 			const int b = j & 1, slot = j % NKV, use = j / NKV;
 			mb_wait(&p_full[b], (j >> 1) & 1);
 			mb_wait(&v_full[slot], use & 1);
@@ -1202,12 +1280,39 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 		// (in natural-log units: exp(8) = 2981 still fits fp16 comfortably) over the maximum its probabilities are expressed against.
 		const float TAU_RAW = 8.0f * sqrtf(128.0f);
 		float m_run = -INFINITY, l_run = 0.f; // m_run: maximum of the raw scores
-		for (int j = 0; j < n_kb; j++) {
-			const int b = j & 1, sb = j & 3;
-			mb_wait(&s_full[sb], (j >> 2) & 1);
+		float sink_s[2] = {-INFINITY, -INFINITY};
+		if (a.win) { // q row r from the Q tiles in shared memory (hi + lo in the precise mode) . this row's sink keys, fp32
+			mb_wait(q_full, 0);
+			const int rr = min(row, a.T - 1);
+#pragma unroll
+			for (int s = 0; s < 2; s++) {
+				const __half* kp = a.sink_k + ((size_t) rr * 2 + s) * a.kv_dim + kvh * 128;
+				float acc = 0.f;
+				for (int c8 = 0; c8 < 16; c8++) { // 8 hd values = one 16-byte chunk of a Q tile row
+					const size_t off = (size_t) (c8 >> 3) * A_TILE_BYTES + tile_inner_off(r, (c8 & 7) * 8);
+					const uint4 qh4 = *reinterpret_cast<const uint4*>(sQ + off);
+					const uint4 k4 = *reinterpret_cast<const uint4*>(kp + c8 * 8);
+					const __half* qh = reinterpret_cast<const __half*>(&qh4);
+					const __half* kh = reinterpret_cast<const __half*>(&k4);
+					uint4 ql4 = make_uint4(0, 0, 0, 0);
+					if (PRECISE) ql4 = *reinterpret_cast<const uint4*>(sQ + 2 * A_TILE_BYTES + off);
+					const __half* ql = reinterpret_cast<const __half*>(&ql4);
+#pragma unroll
+					for (int i = 0; i < 8; i++) acc = fmaf(__half2float(qh[i]) + (PRECISE ? __half2float(ql[i]) : 0.f), __half2float(kh[i]), acc);
+				}
+				sink_s[s] = acc;
+			}
+			m_run = fmaxf(sink_s[0], sink_s[1]); // finite for every row, even where a block masks all of its keys
+		}
+		for (int it = 0; it < n_it; it++) {
+			const int j = kb0 + it;            // key block
+			const int b = it & 1, sb = it & 3; // ring positions
+			mb_wait(&s_full[sb], (it >> 2) & 1);
 			tc_fence_after();
-			const bool need_mask = j * ATT_BKV + ATT_BKV - 1 > a.pos0 + q0; // some key of this block is beyond the tile's first row
+			const bool need_mask = j * ATT_BKV + ATT_BKV - 1 > a.pos0 + q0   // some key of this block is beyond the tile's first row
+			                    || (a.win && j * ATT_BKV < a.pos0 + q_last - a.win + 1); // or below the band of its last row
 			const int lim = a.pos0 + row - j * ATT_BKV;                      // keys with index (inside the block) > lim are masked
+			const int lo = a.win ? lim - a.win + 1 : INT_MIN;                // window mode: and those < lo
 			float sv[ATT_BKV];
 			__syncwarp();
 #pragma unroll
@@ -1217,7 +1322,7 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 			if (need_mask) {
 #pragma unroll
 				for (int i = 0; i < ATT_BKV; i++) {
-					if (i > lim) sv[i] = -INFINITY;
+					if (i > lim || i < lo) sv[i] = -INFINITY;
 					mx = fmaxf(mx, sv[i]);
 				}
 			} else {
@@ -1225,12 +1330,12 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 				for (int i = 0; i < ATT_BKV; i++) mx = fmaxf(mx, sv[i]);
 			}
 			// this P buffer was last read by the P V of block j-2: it must have completed (it has, long ago, in steady state)
-			if (j >= 2) mb_wait(&o_full[b], ((j >> 1) - 1) & 1);
+			if (it >= 2) mb_wait(&o_full[b], ((it >> 1) - 1) & 1);
 			const bool grow = mx > m_run + TAU_RAW;   // block 0: m_run = -inf -> true, but there is nothing to rescale yet
-			if (j == 0) m_run = mx;
+			if (it == 0) m_run = fmaxf(m_run, mx);    // (window mode: m_run holds the sink maximum)
 			else if (__any_sync(0xffffffffu, grow)) {
 				// rare: O must be quiescent, i.e. the P V of block j-1 (the last one issued) has completed
-				mb_wait(&o_full[(j - 1) & 1], ((j - 1) >> 1) & 1);
+				mb_wait(&o_full[(it - 1) & 1], ((it - 1) >> 1) & 1);
 				const float m_new = grow ? mx : m_run;
 				const float corr = ex2((m_run - m_new) * c1); // 1 for the rows that keep their maximum
 				tc_fence_after();
@@ -1277,15 +1382,27 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 			}
 		}
 		{ // the last P V (and with it every earlier one: MMAs complete in order)
-			const int jl = n_kb - 1;
+			const int jl = n_it - 1;
 			mb_wait(&o_full[jl & 1], (jl >> 1) & 1);
 		}
 		tc_fence_after();
+		float sp0 = 0.f, sp1 = 0.f;
+		if (a.win) {
+			sp0 = ex2((sink_s[0] - m_run) * c1);
+			sp1 = ex2((sink_s[1] - m_run) * c1);
+			l_run += sp0 + sp1;
+		}
 		const float inv = 1.0f / l_run;
 #pragma unroll
 		for (int c = 0; c < 4; c++) {
 			float v[32];
 			tmem_ld32(TM_O + lane_addr + 32 * c, v);
+			if (a.win) { // + the sinks' share of the output row
+				const __half* v0 = a.sink_v + kvh * 128 + 32 * c;
+				const __half* v1 = v0 + a.kv_dim;
+#pragma unroll
+				for (int i = 0; i < 32; i++) v[i] += sp0 * __half2float(v0[i]) + sp1 * __half2float(v1[i]);
+			}
 			if (row < a.T) {
 #pragma unroll
 				for (int g8 = 0; g8 < 4; g8++) {
@@ -1303,6 +1420,46 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attn_tc_kernel(const AttnTcArg
 		tc_fence_after();
 		tmem_dealloc(tmem_base, 512);
 	}
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// window mode (positions pos0 .. pos0+T-1, all >= max_seq_len): the KV cache is a ring, slot 2 + (p - 2) % S of S = max_seq_len - 2
+// data slots after two attention sinks (infer.cpp:608-613).  The batch's own K/V rows overwrite ring rows that its earlier
+// queries still need, so attention reads a linear staging copy instead: rows [0, S-1) = positions pos0-S+1 .. pos0-1
+// (gathered from the ring before the QKV GEMM), rows [S-1, S-1+T) = the new rows (QKV epilogue).
+// ------------------------------------------------------------------------------------------------------------------
+__global__ void gather_ring_kernel(const __half* __restrict__ k_cache, const __half* __restrict__ v_cache, int kv_dim, int S, int pos0,
+                                   __half* __restrict__ k_stage, __half* __restrict__ v_stage) {
+	const int cpr = kv_dim / 8; // 16-byte chunks per row
+	const size_t total = (size_t) (S - 1) * cpr;
+	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < total; i += (size_t) gridDim.x * blockDim.x) {
+		const int r = (int) (i / cpr), c = (int) (i % cpr);
+		const int p = pos0 - S + 1 + r;  // >= 3: below the window its slot is p itself, which the same formula gives
+		const size_t src = (size_t) (2 + (p - 2) % S) * kv_dim + c * 8, dst = (size_t) r * kv_dim + c * 8;
+		*reinterpret_cast<uint4*>(k_stage + dst) = *reinterpret_cast<const uint4*>(k_cache + src);
+		*reinterpret_cast<uint4*>(v_stage + dst) = *reinterpret_cast<const uint4*>(v_cache + src);
+	}
+}
+
+// The sink keys (cache rows 0 and 1) as each query of the batch sees them: the token-at-a-time path re-rotates them by one
+// position per token before that token's attention (rotate_sinks, matvec.cuh), so query i sees them i+1 rotations on from the
+// state before the call.  One thread per rotation pair walks the T steps with the same expression, rounding through fp16 each
+// step (bit-identical to T forwards); version i -> sink_k row i, the last one goes back to the cache.
+__global__ void sink_versions_kernel(__half* __restrict__ k_cache, int kv_dim, int head_dim, const float* __restrict__ rope_freq, int T,
+                                     __half* __restrict__ sink_k) {
+	const int pairs = kv_dim / 2;
+	const int i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= 2 * pairs) return;
+	const int r = i / pairs, p = i % pairs;
+	__half2* kp = reinterpret_cast<__half2*>(k_cache + (size_t) r * kv_dim) + p;
+	__half2 h = *kp;
+	for (int t = 0; t < T; t++) {
+		float2 v = __half22float2(h);
+		rope_pair(v.x, v.y, (2 * p) % head_dim, 1, rope_freq);
+		h = __floats2half2_rn(v.x, v.y);
+		reinterpret_cast<__half2*>(sink_k + ((size_t) t * 2 + r) * kv_dim)[p] = h;
+	}
+	*kp = h;
 }
 
 // fp32 row-major (T, K) -> A tiles (op-level hook and tests)
@@ -1354,7 +1511,8 @@ struct DevBuf {
 };
 
 struct PrefillScratch {
-	DevBuf x, xb_hi, xb_lo, xb2_hi, xb2_lo, hb_hi, hb_lo, q, q_lo, wt[2], wt_lo[2], logits, tokens, targets, probs, rope, qt_hi, qt_lo, kt, vt;
+	DevBuf x, xb_hi, xb_lo, xb2_hi, xb2_lo, hb_hi, hb_lo, q, q_lo, wt[2], wt_lo[2], logits, tokens, targets, probs, rope, qt_hi, qt_lo, kt, vt,
+	    k_stage, v_stage, sink_k; // window mode
 	int logits_rows = 0;
 	cudaStream_t side = nullptr;          // dequantises the NEXT GEMM's weights while the current GEMM runs
 	cudaEvent_t ev_start = nullptr, ev_deq[2] = {nullptr, nullptr}, ev_gemm[2] = {nullptr, nullptr};
@@ -1363,7 +1521,8 @@ struct PrefillScratch {
 void prefill_free(PrefillScratch* s) {
 	if (!s) return;
 	DevBuf* all[] = {&s->x, &s->xb_hi, &s->xb_lo, &s->xb2_hi, &s->xb2_lo, &s->hb_hi, &s->hb_lo, &s->q, &s->q_lo, &s->wt[0], &s->wt[1],
-	                 &s->wt_lo[0], &s->wt_lo[1], &s->logits, &s->tokens, &s->targets, &s->probs, &s->rope, &s->qt_hi, &s->qt_lo, &s->kt, &s->vt};
+	                 &s->wt_lo[0], &s->wt_lo[1], &s->logits, &s->tokens, &s->targets, &s->probs, &s->rope, &s->qt_hi, &s->qt_lo, &s->kt, &s->vt,
+	                 &s->k_stage, &s->v_stage, &s->sink_k};
 	for (DevBuf* b : all) b->release();
 	if (s->side) cudaStreamDestroy(s->side);
 	if (s->ev_start) cudaEventDestroy(s->ev_start);
@@ -1454,12 +1613,20 @@ static int launch_attn_p(const AttnPArgs& a, cudaStream_t s) {
 }
 
 int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
-                const int* targets, float* probs_host, int split, int* n_launches) {
+                const int* targets, float* probs_host, int split, int* n_launches, bool window) {
 	const xalm_config& c = pm.c;
 	if (n <= 0) return set_error(XALM_ERR_INVALID, "prefill: n = %d", n);
-	if (pos0 < 0 || (long long) pos0 + n > c.max_seq_len)
-		return set_error(XALM_ERR_INVALID, "prefill: positions [%d, %d) do not fit the %d-slot KV cache without wrapping (use forward)", pos0,
+	if (!window && (pos0 < 0 || (long long) pos0 + n > c.max_seq_len))
+		return set_error(XALM_ERR_INVALID,
+		                 "prefill: positions [%d, %d) do not fit the %d-slot KV cache without wrapping (use xalm_cuda_prefill_window past it)", pos0,
 		                 pos0 + n, c.max_seq_len);
+	if (window && pos0 < c.max_seq_len)
+		return set_error(XALM_ERR_INVALID, "prefill_window: pos0 %d is inside the %d-position window (use xalm_cuda_prefill below it)", pos0,
+		                 c.max_seq_len);
+	if (window && n > c.max_seq_len - 2)
+		return set_error(XALM_ERR_INVALID, "prefill_window: n = %d exceeds the %d ring slots (split it into chunks of at most that many)", n,
+		                 c.max_seq_len - 2);
+	if (window && (long long) pos0 + n > INT_MAX) return set_error(XALM_ERR_INVALID, "prefill_window: positions overflow");
 	if (c.head_dim != 64 && c.head_dim != 128) return set_error(XALM_ERR_UNSUPPORTED, "prefill: head_dim %d (64 or 128)", c.head_dim);
 	if (c.dim % 16 || c.hidden_dim % 16 || pm.q_dim % 16 || pm.kv_dim % 16) return set_error(XALM_ERR_UNSUPPORTED, "prefill: dims must be multiples of 16");
 	if (targets && want_logits != 2) return set_error(XALM_ERR_INVALID, "prefill: target probabilities need the logits of every position");
@@ -1519,7 +1686,15 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 	}
 	// head_dim 128: attention on tcgen05 (attn_tc_kernel); otherwise the mma.sync kernel on row-major q
 	const bool attn_tc = c.head_dim == 128 && getenv("XALM_ATTN_MMA_SYNC") == nullptr;
-	const int n_qb = MT, n_kb_total = cdiv(pos0 + T, 128);
+	// window mode: attention reads the staging copy, rows [0, S-1+T), as if it were a cache prefix of S-1 rows (pos0 of the kernels)
+	const int S = c.max_seq_len - 2;
+	const int attn_pos0 = window ? S - 1 : pos0;
+	const int n_qb = MT, n_kb_total = cdiv(attn_pos0 + T, 128);
+	if (window) {
+		XALM_TRY(sc.k_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
+		XALM_TRY(sc.v_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
+		XALM_TRY(sc.sink_k.ensure((size_t) T * 2 * pm.kv_dim * 2, false, s));
+	}
 	if (attn_tc) {
 		XALM_TRY(sc.qt_hi.ensure((size_t) c.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
 		if (precise) XALM_TRY(sc.qt_lo.ensure((size_t) c.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
@@ -1599,6 +1774,17 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		t_begin("rmsnorm");
 		rmsnorm_rows_kernel<<<norm_grid, 128, 0, s>>>(x, T, c.dim, P.rms_att, P.rms_att_type, c.norm_eps, xb);
 		t_end();
+		__half* k_stage = reinterpret_cast<__half*>(sc.k_stage.p);
+		__half* v_stage = reinterpret_cast<__half*>(sc.v_stage.p);
+		__half* sink_k = reinterpret_cast<__half*>(sc.sink_k.p);
+		if (window) { // before the QKV epilogue overwrites the ring slots of positions pos0-S .. pos0+T-1-S
+			t_begin("ring");
+			gather_ring_kernel<<<std::min(cdiv((S - 1) * (pm.kv_dim / 8), 256), sm_count() * 8), 256, 0, s>>>(P.k_cache, P.v_cache, pm.kv_dim, S, pos0,
+			                                                                                                   k_stage, v_stage);
+			sink_versions_kernel<<<cdiv(pm.kv_dim, 128), 128, 0, s>>>(P.k_cache, pm.kv_dim, c.head_dim, pm.rope_freq, T, sink_k);
+			t_end();
+			launches += 2;
+		}
 		XALM_TRY(prep(P.wo, false, 0, c.dim, pm.q_dim, NT_dim, KT_q));
 		GemmArgs g = {};
 		g.a_hi = xb.hi; g.a_lo = xb.lo;
@@ -1606,19 +1792,24 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		g.q_out = q; g.q_lo = q_lo; g.k_cache = P.k_cache; g.v_cache = P.v_cache; g.rope_cs = rope_cs;
 		g.q_dim = pm.q_dim; g.kv_dim = pm.kv_dim; g.head_dim = c.head_dim; g.pos0 = pos0; g.qkv_clip = c.qkv_clip;
 		if (attn_tc) { g.qt_hi = sc.qt_hi.p; g.qt_lo = precise ? sc.qt_lo.p : nullptr; g.n_qb = n_qb; }
-		const bool tiles_from_epilogue = attn_tc && pos0 == 0 && getenv("XALM_ATTN_RETILE") == nullptr; // later chunks re-tile the whole cache prefix
+		if (window) { g.ring = S; g.k_stage = k_stage; g.v_stage = v_stage; g.stage_row0 = S - 1; }
+		// later chunks (and the window mode) re-tile the whole cache prefix / staging copy
+		const bool tiles_from_epilogue = attn_tc && !window && pos0 == 0 && getenv("XALM_ATTN_RETILE") == nullptr;
 		if (tiles_from_epilogue) { g.kt = sc.kt.p; g.vt = sc.vt.p; g.n_kb_total = n_kb_total; }
 		XALM_TRY(run(g, P.wqkv));
 		t_begin("attention");
 		if (attn_tc) {
 			if (!tiles_from_epilogue)
-				retile_kv_kernel<<<dim3(2 * n_kb_total, c.n_kv_heads), 256, 0, s>>>(P.k_cache, P.v_cache, pm.kv_dim, pos0 + T, n_kb_total, sc.kt.p, sc.vt.p);
-			AttnTcArgs at = {sc.qt_hi.p, precise ? sc.qt_lo.p : nullptr, sc.kt.p, sc.vt.p, xb2, T, pos0, c.n_heads, c.n_kv_heads, n_qb, n_kb_total,
+				retile_kv_kernel<<<dim3(2 * n_kb_total, c.n_kv_heads), 256, 0, s>>>(window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, pm.kv_dim,
+				                                                                    attn_pos0 + T, n_kb_total, sc.kt.p, sc.vt.p);
+			AttnTcArgs at = {sc.qt_hi.p, precise ? sc.qt_lo.p : nullptr, sc.kt.p, sc.vt.p, xb2, T, attn_pos0, c.n_heads, c.n_kv_heads, n_qb, n_kb_total,
+			                 window ? S : 0, window ? sink_k : nullptr, window ? P.v_cache : nullptr, pm.kv_dim,
 			                 getenv("XALM_ATTN_DBG") ? atoi(getenv("XALM_ATTN_DBG")) : 0};
 			XALM_TRY(precise ? launch_attn_tc<true>(at, s) : launch_attn_tc<false>(at, s));
 			launches++;
 		} else {
-			AttnPArgs at = {q, q_lo, P.k_cache, P.v_cache, xb2, T, pos0, pm.q_dim, pm.kv_dim, c.n_heads, c.n_kv_heads, cdiv(T, 64)};
+			AttnPArgs at = {q, q_lo, window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, xb2, T, attn_pos0, pm.q_dim, pm.kv_dim, c.n_heads,
+			                c.n_kv_heads, cdiv(T, 64), window ? S : 0, window ? sink_k : nullptr, window ? P.v_cache : nullptr};
 			if (c.head_dim == 128) XALM_TRY(precise ? (launch_attn_p<128, true>(at, s)) : (launch_attn_p<128, false>(at, s)));
 			else XALM_TRY(precise ? (launch_attn_p<64, true>(at, s)) : (launch_attn_p<64, false>(at, s)));
 		}

@@ -42,8 +42,11 @@ struct PrefillScratch; // device scratch + pinned staging, grown on demand; owne
 // logits_host: NULL, or vocab floats (want 1) / n*vocab floats (want 2).  targets/probs_host: NULL, or n entries —
 // probs_host[i] = softmax(logits_i)[targets[i]] as Sampler::sample_prob computes it (needs want 2).
 // split: 1 = activations as one fp16 operand, 2 = hi+lo fp16 pair (two MMAs per weight tile, ~fp32 activations).
+// window = false: the linear regime, pos0 + n <= max_seq_len.  window = true: the ring regime past the context window,
+// pos0 >= max_seq_len and n <= max_seq_len - 2 (each ring slot written at most once); new rows go to their ring slots and the
+// two sink keys are re-rotated n times, as n token-at-a-time forwards would leave the cache.
 int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tokens, int n, int pos0, int want_logits,
-                float* logits_host, const int* targets, float* probs_host, int split, int* n_launches);
+                float* logits_host, const int* targets, float* probs_host, int split, int* n_launches, bool window = false);
 void prefill_free(PrefillScratch* s);
 // device pointer of the logits of the last prefill (rows x vocab) — bench / tests
 const float* prefill_logits_dev(const PrefillScratch* s, int* rows);

@@ -2051,6 +2051,24 @@ int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, in
 	return XALM_OK;
 }
 
+// past the context window: the ring regime (prefill_run's window mode)
+int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host, const int* targets,
+                             float* probs_host) {
+	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
+	if (m->tp_size > 1) return set_error(XALM_ERR_UNSUPPORTED, "prefill_window: tensor-parallel models take the token-at-a-time path");
+	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill_window: want_logits = %d", want_logits);
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	PrefillModel pm;
+	fill_prefill_model(m, pm);
+	const int split = tune("prefill_split");
+	XALM_TRY(prefill_run(pm, &m->prefill, tokens, n, pos0, want_logits, logits_host, targets, probs_host, split, &m->last_prefill_launches, true));
+	cudaError_t e = cudaStreamSynchronize(m->stream);
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "prefill_window failed: %s", cudaGetErrorString(e));
+	m->last_launches = m->last_prefill_launches;
+	return XALM_OK;
+}
+
 int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits) {
 	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
 	// same as xalm_cuda_prefill without the host synchronisation and read-back (bench.py's device-timed leg)

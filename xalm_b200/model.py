@@ -175,8 +175,17 @@ class Model:
         position (vocab,); 2: all positions (n, vocab).  With `targets` returns (logits, probs) where probs[i] is
         Sampler.sample_prob(targets[i]) at position pos0+i; fetch_logits=False leaves the logits on the device (perplexity
         mode needs only the probabilities)."""
+        return self._prefill_call("prefill", tokens, pos0, want_logits, targets, fetch_logits)
+
+    def prefill_window(self, tokens, pos0: int, want_logits: int = 1, targets=None, fetch_logits: bool = True):
+        """prefill past the context window, where the KV cache is a ring with two attention sinks: positions
+        pos0..pos0+len(tokens)-1 with pos0 >= max_seq_len and len(tokens) <= max_seq_len - 2 (longer runs go in chunks).
+        Leaves the KV cache as that many forward() calls would.  Arguments and results as for prefill()."""
+        return self._prefill_call("prefill_window", tokens, pos0, want_logits, targets, fetch_logits)
+
+    def _prefill_call(self, which: str, tokens, pos0: int, want_logits: int, targets, fetch_logits: bool):
         if self._h is None:
-            raise RuntimeError("Model.prefill: the model is not on a CUDA device (call model.cuda()); this backend has no CPU path")
+            raise RuntimeError(f"Model.{which}: the model is not on a CUDA device (call model.cuda()); this backend has no CPU path")
         tok = np.ascontiguousarray(tokens, dtype=np.int32)
         n = int(tok.size)
         V = self.config["vocab_size"]
@@ -186,7 +195,8 @@ class Model:
             tg = np.ascontiguousarray(targets, dtype=np.int32)
             pr = np.empty(n, dtype=np.float32)
         vp = lambda a: a.ctypes.data_as(C.c_void_p) if a is not None else None
-        capi.check(capi.lib().xalm_cuda_prefill(self._h, vp(tok), n, pos0, want_logits, vp(lg), vp(tg), vp(pr)))
+        fn = getattr(capi.lib(), "xalm_cuda_" + which)
+        capi.check(fn(self._h, vp(tok), n, pos0, want_logits, vp(lg), vp(tg), vp(pr)))
         return (lg, pr) if targets is not None else lg
 
     def prefill_async(self, tokens: np.ndarray, pos0: int = 0, want_logits: int = 2) -> None:
