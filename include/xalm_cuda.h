@@ -137,7 +137,11 @@ int xalm_cuda_sync(xalm_cuda_model* m);
  * logits_host may be NULL.  Synchronous.  Tensor-core operands are fp16 with fp32 accumulation; the "prefill_split"
  * knob (xalm_cuda_tune) picks how fp32 values enter them: 3 (default) = hi+lo fp16 pairs for activations, weights and the
  * attention operands (3 MMAs per product; 32-layer 4k-token logits within ~1e-3 of the token-at-a-time path), 2 = pairs
- * for activations only, 1 = plain fp16 (fastest; ~4e-2 at that depth).  North star tolerance: 1e-2. */
+ * for activations only, 1 = plain fp16 (fastest; ~4e-2 at that depth).  North star tolerance: 1e-2.
+ * Tensor-parallel handles: a collective.  Every rank of the group calls it with the same arguments, in the same order; each
+ * fills its own KV-cache shard (its kv heads) and receives the FULL logits and probabilities, as xalm_cuda_forward returns
+ * full logits on every rank.  A refusal (bad argument, or a scratch allocation that failed on any one rank) is the same
+ * error on every rank and leaves every rank's cache untouched. */
 int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
                       const int* targets, float* probs_host);
 /* The same batched pass past the context window, where the KV cache is a ring: positions pos0 .. pos0+n-1 with
@@ -146,11 +150,12 @@ int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, in
  * and the two attention-sink keys in slots 0 and 1 re-rotated n more times (bit-identical to the token loop).  Each
  * position attends to the two sinks and the max_seq_len - 2 latest positions, itself included.  want_logits, logits_host,
  * targets, probs_host and the "prefill_split" knob mean what they mean for xalm_cuda_prefill.  Anything else — positions
- * below the window, n too large, a token out of range — is XALM_ERR_INVALID before anything runs (the cache is untouched);
- * tensor-parallel handles get XALM_ERR_UNSUPPORTED.  Synchronous. */
+ * below the window, n too large, a token out of range — is XALM_ERR_INVALID before anything runs (the cache is untouched).
+ * Synchronous.  A collective on tensor-parallel handles, with the same per-rank results and refusals as xalm_cuda_prefill. */
 int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
                              const int* targets, float* probs_host);
-/* Enqueue only (no read-back, no host sync) — bench.py's device-timed leg. */
+/* Enqueue only (no read-back, no host sync) — bench.py's device-timed leg.  A collective on tensor-parallel handles; a
+ * refusal there is agreed between the ranks, which takes one host synchronisation before the pass is enqueued. */
 int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits);
 /* Pinned host buffer the logits are copied into by xalm_cuda_forward (alias it as InferenceState::_logits). */
 float* xalm_cuda_logits_host(xalm_cuda_model* m);

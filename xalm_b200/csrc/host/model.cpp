@@ -269,7 +269,7 @@ xalm_config Config::to_c() const {
 InferenceState::InferenceState(const Config& config) : own_logits_((size_t) config.vocab_size, 0.f) {}
 
 // ---- Model -------------------------------------------------------------------------------------------------------
-Model::Model(Model&& o) noexcept : config(o.config), device(o.device), host_(std::move(o.host_)), types_(std::move(o.types_)), handle_(o.handle_), tp_size_(o.tp_size_) {
+Model::Model(Model&& o) noexcept : config(o.config), device(o.device), host_(std::move(o.host_)), types_(std::move(o.types_)), handle_(o.handle_) {
 	o.handle_ = nullptr;
 }
 Model::~Model() {
@@ -319,7 +319,6 @@ void Model::cuda(int device_index, int tp_rank, int tp_size, const void* comm_id
 	if (handle_) return;
 	const xalm_config c = config.to_c();
 	if (xalm_cuda_create(&c, device_index, tp_rank, tp_size, &handle_) != XALM_OK) xalm_throw_last("model.cuda()");
-	tp_size_ = tp_size;
 	if (tp_size > 1) {
 		if (!comm_id) throw std::invalid_argument("model.cuda(): tensor parallel needs a communicator id");
 		if (xalm_cuda_comm_init(handle_, comm_id) != XALM_OK) xalm_throw_last("model.cuda()");
@@ -412,7 +411,6 @@ bool Model::prefill_call(const bool window, const InferenceState& s, const int* 
                          const int* targets, float* probs) const {
 	if (device != Device::CUDA || !handle_)
 		throw std::runtime_error("Model::prefill: model is not on a CUDA device (call model.cuda()); this backend has no CPU path");
-	if (tp_size_ > 1) return false;
 	if (!s.logits_ptr_ && s.device == Device::CUDA) s.logits_ptr_ = xalm_cuda_logits_host(handle_);
 	auto call = window ? xalm_cuda_prefill_window : xalm_cuda_prefill;
 	int rc;

@@ -157,12 +157,14 @@ struct Model {
 	// The per-position loops of main.cpp:94-100 / :244-254 as one batched pass on the tensor cores (xalm_cuda_prefill).
 	// Positions pos0 .. pos0+n-1; mode OUTPUT_LOGITS leaves the LAST position's logits in s.logits().  With `targets` and
 	// `probs` (n entries) also returns Sampler::sample_prob(targets[i]) at every position.  Returns false — and does nothing —
-	// when the batch cannot take this path (ring-buffer wrap past max_seq_len, tensor-parallel shard): callers fall back to forward().
+	// when the batch cannot take this path (ring-buffer wrap past max_seq_len): callers fall back to forward().  Under tensor
+	// parallelism it is a collective: every rank calls it with the same arguments and gets the full logits.
 	bool prefill(const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode = InferenceMode::OUTPUT_LOGITS,
 	             const int* targets = nullptr, float* probs = nullptr) const;
 	// The same past the context window, where the KV cache is a ring with two attention sinks (xalm_cuda_prefill_window):
 	// pos0 >= max_seq_len and n <= max_seq_len - 2 (longer runs go in chunks).  Leaves the cache as n forward() calls would.
-	// Returns false — and does nothing — when the batch cannot take this path (positions outside that range, tensor-parallel shard).
+	// Returns false — and does nothing — when the batch cannot take this path (positions outside that range).  Collective under
+	// tensor parallelism, as prefill().
 	bool prefill_window(const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode = InferenceMode::OUTPUT_LOGITS,
 	                    const int* targets = nullptr, float* probs = nullptr) const;
 
@@ -174,7 +176,6 @@ private:
 	std::map<std::string, Type> types_;  // kept for active_bytes after the host copies are gone
 	const Xalm::file_info* deferred_ = nullptr; // defer_load: where cuda() reads the tensors from
 	xalm_cuda_model* handle_ = nullptr;
-	int tp_size_ = 1;
 };
 
 // ---- Sampler (sampler.h / sampler.cpp): host-side, unchanged semantics incl. the FLT_MIN seed (SURVEY.md §0.8) ---

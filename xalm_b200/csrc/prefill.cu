@@ -44,6 +44,7 @@
 
 #include "matvec.cuh"
 #include "frag_layout.cuh"
+#include "nccl_api.h"
 #include "prefill.h"
 
 namespace xalm {
@@ -1474,6 +1475,18 @@ __global__ void pack_a_kernel(const float* __restrict__ a, int T, int K, ATiles 
 	}
 }
 
+// tensor parallel: the all-gathered classifier shards (P, rows, vocab_l) -> (rows, P * vocab_l), the one-GPU layout
+__global__ void unshard_logits_kernel(const float* __restrict__ shards, int P, int rows, int vocab_l, float* __restrict__ out) {
+	const int q = vocab_l / 4; // float4 per shard row (vocab_l % 32 == 0)
+	const size_t total = (size_t) P * rows * q;
+	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < total; i += (size_t) gridDim.x * blockDim.x) {
+		const int j = (int) (i % q);
+		const size_t pr = i / q;
+		const int r = (int) (pr % rows), p = (int) (pr / rows);
+		reinterpret_cast<float4*>(out + (size_t) r * P * vocab_l + (size_t) p * vocab_l)[j] = reinterpret_cast<const float4*>(shards)[i];
+	}
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------------------------
@@ -1512,7 +1525,8 @@ struct DevBuf {
 
 struct PrefillScratch {
 	DevBuf x, xb_hi, xb_lo, xb2_hi, xb2_lo, hb_hi, hb_lo, q, q_lo, wt[2], wt_lo[2], logits, tokens, targets, probs, rope, qt_hi, qt_lo, kt, vt,
-	    k_stage, v_stage, sink_k; // window mode
+	    k_stage, v_stage, sink_k, // window mode
+	    part, logits_tp;          // tensor parallel: this rank's partial sums of Wo / W2; the all-gathered classifier shards
 	int logits_rows = 0;
 	cudaStream_t side = nullptr;          // dequantises the NEXT GEMM's weights while the current GEMM runs
 	cudaEvent_t ev_start = nullptr, ev_deq[2] = {nullptr, nullptr}, ev_gemm[2] = {nullptr, nullptr};
@@ -1522,7 +1536,7 @@ void prefill_free(PrefillScratch* s) {
 	if (!s) return;
 	DevBuf* all[] = {&s->x, &s->xb_hi, &s->xb_lo, &s->xb2_hi, &s->xb2_lo, &s->hb_hi, &s->hb_lo, &s->q, &s->q_lo, &s->wt[0], &s->wt[1],
 	                 &s->wt_lo[0], &s->wt_lo[1], &s->logits, &s->tokens, &s->targets, &s->probs, &s->rope, &s->qt_hi, &s->qt_lo, &s->kt, &s->vt,
-	                 &s->k_stage, &s->v_stage, &s->sink_k};
+	                 &s->k_stage, &s->v_stage, &s->sink_k, &s->part, &s->logits_tp};
 	for (DevBuf* b : all) b->release();
 	if (s->side) cudaStreamDestroy(s->side);
 	if (s->ev_start) cudaEventDestroy(s->ev_start);
@@ -1612,6 +1626,18 @@ static int launch_attn_p(const AttnPArgs& a, cudaStream_t s) {
 	return XALM_OK;
 }
 
+// Tensor parallel: every rank learns the worst status of the group (XALM_OK = 0, errors > 0) before anything touches a cache.  A
+// scratch allocation can fail on one rank only; then every rank returns an error and none is left waiting in a collective.
+static int agree_status(const PrefillModel& pm, int rc) {
+	int v = rc;
+	XALM_CUDA_CHECK(cudaMemcpyAsync(pm.status_dev, &v, sizeof v, cudaMemcpyHostToDevice, pm.stream));
+	XALM_NCCL_CHECK(g_nccl.AllReduce(pm.status_dev, pm.status_dev, 1, ncclInt32, ncclMax, pm.comm, pm.stream));
+	XALM_CUDA_CHECK(cudaMemcpyAsync(&v, pm.status_dev, sizeof v, cudaMemcpyDeviceToHost, pm.stream));
+	XALM_CUDA_CHECK(cudaStreamSynchronize(pm.stream));
+	if (v == XALM_OK || rc != XALM_OK) return rc; // a rank that failed keeps its own message
+	return set_error(v, "prefill: another rank of the tensor-parallel group failed (status %d)", v);
+}
+
 int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
                 const int* targets, float* probs_host, int split, int* n_launches, bool window) {
 	const xalm_config& c = pm.c;
@@ -1628,7 +1654,8 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		                 c.max_seq_len - 2);
 	if (window && (long long) pos0 + n > INT_MAX) return set_error(XALM_ERR_INVALID, "prefill_window: positions overflow");
 	if (c.head_dim != 64 && c.head_dim != 128) return set_error(XALM_ERR_UNSUPPORTED, "prefill: head_dim %d (64 or 128)", c.head_dim);
-	if (c.dim % 16 || c.hidden_dim % 16 || pm.q_dim % 16 || pm.kv_dim % 16) return set_error(XALM_ERR_UNSUPPORTED, "prefill: dims must be multiples of 16");
+	if (c.dim % 16 || pm.hidden % 16 || pm.q_dim % 16 || pm.kv_dim % 16) return set_error(XALM_ERR_UNSUPPORTED, "prefill: dims must be multiples of 16");
+	if (pm.tp_size > 1 && (!pm.comm || !pm.status_dev)) return set_error(XALM_ERR_STATE, "prefill: tensor-parallel model without a communicator");
 	if (targets && want_logits != 2) return set_error(XALM_ERR_INVALID, "prefill: target probabilities need the logits of every position");
 	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill: want_logits = %d", want_logits);
 	for (int i = 0; i < n; i++)
@@ -1645,20 +1672,85 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 	// split: 1 = fp16 x fp16; 2 = hi+lo activations; 3 = hi+lo activations AND weights AND attention operands (fp32-grade)
 	const int na = split >= 2 ? 2 : 1;
 	const bool precise = split >= 3;
+	const bool tp = pm.tp_size > 1;
 	cudaStream_t s = pm.stream;
+	const int T = n, MT = cdiv(T, GB_M), Tp = MT * GB_M;
+	const int KT_dim = cdiv(c.dim, GB_K), KT_q = cdiv(pm.q_dim, GB_K), KT_h = cdiv(pm.hidden, GB_K);
+	const int n_qkv = pm.q_dim + 2 * pm.kv_dim;
+	const int NT_qkv = cdiv(n_qkv, GB_N), NT_dim = cdiv(c.dim, GB_N), NT_glu = cdiv(pm.hidden, GB_N / 2), NT_cls = cdiv(pm.vocab, GB_N);
+	// tensor parallel: the Wo / W2 partial sums are reduce-scattered in blocks of Tr / P rows of x (Tr = T rounded up to a multiple of
+	// P); rows [T, Tr) carry values nothing reads
+	const int Tr = cdiv(T, pm.tp_size) * pm.tp_size;
+	// head_dim 128: attention on tcgen05 (attn_tc_kernel); otherwise the mma.sync kernel on row-major q
+	const bool attn_tc = c.head_dim == 128 && getenv("XALM_ATTN_MMA_SYNC") == nullptr;
+	// window mode: attention reads the staging copy, rows [0, S-1+T), as if it were a cache prefix of S-1 rows (pos0 of the kernels)
+	const int S = c.max_seq_len - 2;
+	const int attn_pos0 = window ? S - 1 : pos0;
+	const int n_qb = MT, n_kb_total = cdiv(attn_pos0 + T, 128);
+	size_t wt_tiles = std::max({(size_t) NT_qkv * KT_dim, (size_t) NT_dim * KT_q, (size_t) NT_glu * KT_dim, (size_t) NT_dim * KT_h});
+	if (want_logits) wt_tiles = std::max(wt_tiles, (size_t) NT_cls * KT_dim);
+	// want 1: only the last M tile goes through the classifier; its valid rows are stored, the last one is the answer
+	const int logit_row0 = want_logits == 1 ? (MT - 1) * GB_M : 0;
+	const int logit_rows = want_logits ? T - logit_row0 : 0;
 	if (!*scratch) *scratch = new PrefillScratch();
 	PrefillScratch& sc = **scratch;
-	if (!sc.side) {
-		XALM_CUDA_CHECK(cudaStreamCreateWithFlags(&sc.side, cudaStreamNonBlocking));
-		XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_start, cudaEventDisableTiming));
-		for (int i = 0; i < 2; i++) {
-			XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_deq[i], cudaEventDisableTiming));
-			XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_gemm[i], cudaEventDisableTiming));
+	// ---- scratch (grown on demand; (re)allocation synchronises, steady state does not) ----
+	auto grow = [&]() -> int {
+		if (!sc.side) {
+			XALM_CUDA_CHECK(cudaStreamCreateWithFlags(&sc.side, cudaStreamNonBlocking));
+			XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_start, cudaEventDisableTiming));
+			for (int i = 0; i < 2; i++) {
+				XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_deq[i], cudaEventDisableTiming));
+				XALM_CUDA_CHECK(cudaEventCreateWithFlags(&sc.ev_gemm[i], cudaEventDisableTiming));
+			}
 		}
-	}
+		XALM_TRY(sc.x.ensure((size_t) std::max(Tp, Tr) * c.dim * 4, true, s));
+		XALM_TRY(sc.xb_hi.ensure((size_t) MT * KT_dim * A_TILE_BYTES, true, s));
+		XALM_TRY(sc.xb2_hi.ensure((size_t) MT * KT_q * A_TILE_BYTES, true, s));
+		XALM_TRY(sc.hb_hi.ensure((size_t) MT * KT_h * A_TILE_BYTES, true, s));
+		if (na == 2) {
+			XALM_TRY(sc.xb_lo.ensure((size_t) MT * KT_dim * A_TILE_BYTES, true, s));
+			XALM_TRY(sc.xb2_lo.ensure((size_t) MT * KT_q * A_TILE_BYTES, true, s));
+			XALM_TRY(sc.hb_lo.ensure((size_t) MT * KT_h * A_TILE_BYTES, true, s));
+		}
+		if (window) {
+			XALM_TRY(sc.k_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
+			XALM_TRY(sc.v_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
+			XALM_TRY(sc.sink_k.ensure((size_t) T * 2 * pm.kv_dim * 2, false, s));
+		}
+		if (attn_tc) {
+			XALM_TRY(sc.qt_hi.ensure((size_t) pm.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
+			if (precise) XALM_TRY(sc.qt_lo.ensure((size_t) pm.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
+			XALM_TRY(sc.kt.ensure((size_t) pm.n_kv_heads * n_kb_total * 2 * A_TILE_BYTES, true, s)); // zeroed: tail keys of the last tile must stay finite
+			XALM_TRY(sc.vt.ensure((size_t) pm.n_kv_heads * n_kb_total * 2 * A_TILE_BYTES, true, s));
+		} else {
+			XALM_TRY(sc.q.ensure((size_t) Tp * pm.q_dim * 2, true, s));
+			if (precise) XALM_TRY(sc.q_lo.ensure((size_t) Tp * pm.q_dim * 2, true, s));
+		}
+		XALM_TRY(sc.rope.ensure((size_t) T * (c.head_dim / 2) * sizeof(float2), false, s));
+		for (int i = 0; i < 2; i++) {
+			XALM_TRY(sc.wt[i].ensure(wt_tiles * B_TILE_BYTES, false, s));
+			if (precise) XALM_TRY(sc.wt_lo[i].ensure(wt_tiles * B_TILE_BYTES, false, s));
+		}
+		XALM_TRY(sc.tokens.ensure((size_t) T * 4, false, s));
+		if (logit_rows) XALM_TRY(sc.logits.ensure((size_t) logit_rows * c.vocab_size * 4, false, s));
+		if (want_logits && targets && probs_host) {
+			XALM_TRY(sc.targets.ensure((size_t) T * 4, false, s));
+			XALM_TRY(sc.probs.ensure((size_t) T * 4, false, s));
+		}
+		if (tp) {
+			XALM_TRY(sc.part.ensure((size_t) Tr * c.dim * 4, true, s));
+			if (logit_rows) XALM_TRY(sc.logits_tp.ensure((size_t) logit_rows * c.vocab_size * 4, false, s));
+		}
+		return XALM_OK;
+	};
+	int rc = grow();
+	if (tp) rc = agree_status(pm, rc);
+	if (rc != XALM_OK) return rc;
+	sc.logits_rows = logit_rows;
 	const bool timing = getenv("XALM_PREFILL_TIMING") != nullptr; // per-category CUDA-event timing, everything on one stream
 	cudaStream_t ds = timing ? s : sc.side;
-	int launches = 0;
+	int launches = tp ? 1 : 0; // the status vote
 	struct Span { const char* what; cudaEvent_t a, b; };
 	std::vector<Span> spans;
 	auto t_begin = [&](const char* what) {
@@ -1669,54 +1761,6 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		spans.push_back(sp);
 	};
 	auto t_end = [&]() { if (timing) cudaEventRecord(spans.back().b, s); };
-
-	const int T = n, MT = cdiv(T, GB_M), Tp = MT * GB_M;
-	const int KT_dim = cdiv(c.dim, GB_K), KT_q = cdiv(pm.q_dim, GB_K), KT_h = cdiv(c.hidden_dim, GB_K);
-	const int n_qkv = pm.q_dim + 2 * pm.kv_dim;
-	const int NT_qkv = cdiv(n_qkv, GB_N), NT_dim = cdiv(c.dim, GB_N), NT_glu = cdiv(c.hidden_dim, GB_N / 2), NT_cls = cdiv(c.vocab_size, GB_N);
-	// ---- scratch (grown on demand; (re)allocation synchronises, steady state does not) ----
-	XALM_TRY(sc.x.ensure((size_t) Tp * c.dim * 4, true, s));
-	XALM_TRY(sc.xb_hi.ensure((size_t) MT * KT_dim * A_TILE_BYTES, true, s));
-	XALM_TRY(sc.xb2_hi.ensure((size_t) MT * KT_q * A_TILE_BYTES, true, s));
-	XALM_TRY(sc.hb_hi.ensure((size_t) MT * KT_h * A_TILE_BYTES, true, s));
-	if (na == 2) {
-		XALM_TRY(sc.xb_lo.ensure((size_t) MT * KT_dim * A_TILE_BYTES, true, s));
-		XALM_TRY(sc.xb2_lo.ensure((size_t) MT * KT_q * A_TILE_BYTES, true, s));
-		XALM_TRY(sc.hb_lo.ensure((size_t) MT * KT_h * A_TILE_BYTES, true, s));
-	}
-	// head_dim 128: attention on tcgen05 (attn_tc_kernel); otherwise the mma.sync kernel on row-major q
-	const bool attn_tc = c.head_dim == 128 && getenv("XALM_ATTN_MMA_SYNC") == nullptr;
-	// window mode: attention reads the staging copy, rows [0, S-1+T), as if it were a cache prefix of S-1 rows (pos0 of the kernels)
-	const int S = c.max_seq_len - 2;
-	const int attn_pos0 = window ? S - 1 : pos0;
-	const int n_qb = MT, n_kb_total = cdiv(attn_pos0 + T, 128);
-	if (window) {
-		XALM_TRY(sc.k_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
-		XALM_TRY(sc.v_stage.ensure((size_t) (S - 1 + T) * pm.kv_dim * 2, false, s));
-		XALM_TRY(sc.sink_k.ensure((size_t) T * 2 * pm.kv_dim * 2, false, s));
-	}
-	if (attn_tc) {
-		XALM_TRY(sc.qt_hi.ensure((size_t) c.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
-		if (precise) XALM_TRY(sc.qt_lo.ensure((size_t) c.n_heads * n_qb * 2 * A_TILE_BYTES, true, s));
-		XALM_TRY(sc.kt.ensure((size_t) c.n_kv_heads * n_kb_total * 2 * A_TILE_BYTES, true, s)); // zeroed: tail keys of the last tile must stay finite
-		XALM_TRY(sc.vt.ensure((size_t) c.n_kv_heads * n_kb_total * 2 * A_TILE_BYTES, true, s));
-	} else {
-		XALM_TRY(sc.q.ensure((size_t) Tp * pm.q_dim * 2, true, s));
-		if (precise) XALM_TRY(sc.q_lo.ensure((size_t) Tp * pm.q_dim * 2, true, s));
-	}
-	XALM_TRY(sc.rope.ensure((size_t) T * (c.head_dim / 2) * sizeof(float2), false, s));
-	size_t wt_tiles = std::max({(size_t) NT_qkv * KT_dim, (size_t) NT_dim * KT_q, (size_t) NT_glu * KT_dim, (size_t) NT_dim * KT_h});
-	if (want_logits) wt_tiles = std::max(wt_tiles, (size_t) NT_cls * KT_dim);
-	for (int i = 0; i < 2; i++) {
-		XALM_TRY(sc.wt[i].ensure(wt_tiles * B_TILE_BYTES, false, s));
-		if (precise) XALM_TRY(sc.wt_lo[i].ensure(wt_tiles * B_TILE_BYTES, false, s));
-	}
-	XALM_TRY(sc.tokens.ensure((size_t) T * 4, false, s));
-	// want 1: only the last M tile goes through the classifier; its valid rows are stored, the last one is the answer
-	const int logit_row0 = want_logits == 1 ? (MT - 1) * GB_M : 0;
-	const int logit_rows = want_logits ? T - logit_row0 : 0;
-	if (logit_rows) XALM_TRY(sc.logits.ensure((size_t) logit_rows * c.vocab_size * 4, false, s));
-	sc.logits_rows = logit_rows;
 
 	ATiles xb{sc.xb_hi.p, na == 2 ? sc.xb_lo.p : nullptr, KT_dim};
 	ATiles xb2{sc.xb2_hi.p, na == 2 ? sc.xb2_lo.p : nullptr, KT_q};
@@ -1743,17 +1787,36 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		launches++;
 		return XALM_OK;
 	};
-	auto run = [&](GemmArgs& g, const WMat& w) -> int {
+	auto run = [&](GemmArgs& g, const WMat& w, const char* what) -> int {
 		const int b = job & 1;
 		g.b = sc.wt[b].p;
 		g.b_lo = sc.wt_lo[b].p;
 		XALM_CUDA_CHECK(cudaStreamWaitEvent(s, sc.ev_deq[b], 0));
-		t_begin(g.epi == GEPI_QKV ? "gemm_qkv" : g.epi == GEPI_GLU ? "gemm_w13" : g.epi == GEPI_STORE ? "gemm_cls" : g.KT == KT_q ? "gemm_wo" : "gemm_w2");
+		t_begin(what);
 		XALM_TRY(launch_gemm(g, na, nb_of(w), s));
 		t_end();
 		XALM_CUDA_CHECK(cudaEventRecord(sc.ev_gemm[b], s));
 		job++;
 		launches++;
+		return XALM_OK;
+	};
+	// Wo / W2 under tensor parallelism: each rank holds a slice of the input axis, so its GEMM gives a partial (T, dim) sum.  Rank 0
+	// adds it to x (residual epilogue), the others store it to `part`; a reduce-scatter sums the P contributions of each row block
+	// into the owning rank's rows of x, and an in-place all-gather copies every block to every rank.  Each element is summed once,
+	// by one rank, so x stays bit-identical on every rank.  One GPU: the residual epilogue alone.
+	float* part = reinterpret_cast<float*>(sc.part.p);
+	auto row_split = [&](GemmArgs& g, const WMat& w, const char* what) -> int {
+		const bool partial = tp && pm.tp_rank != 0;
+		g.epi = partial ? GEPI_STORE : GEPI_RESID; g.out = partial ? part : x; g.ldo = c.dim;
+		XALM_TRY(run(g, w, what));
+		if (!tp) return XALM_OK;
+		t_begin("exchange");
+		const size_t cnt = (size_t) (Tr / pm.tp_size) * c.dim;
+		float* mine = x + (size_t) pm.tp_rank * cnt;
+		XALM_NCCL_CHECK(g_nccl.ReduceScatter(partial ? part : x, mine, cnt, ncclFloat32, ncclSum, pm.comm, s));
+		XALM_NCCL_CHECK(g_nccl.AllGather(mine, x, cnt, ncclFloat32, pm.comm, s));
+		t_end();
+		launches += 2;
 		return XALM_OK;
 	};
 	const size_t L = pm.layers.size();
@@ -1796,61 +1859,70 @@ int prefill_run(const PrefillModel& pm, PrefillScratch** scratch, const int* tok
 		// later chunks (and the window mode) re-tile the whole cache prefix / staging copy
 		const bool tiles_from_epilogue = attn_tc && !window && pos0 == 0 && getenv("XALM_ATTN_RETILE") == nullptr;
 		if (tiles_from_epilogue) { g.kt = sc.kt.p; g.vt = sc.vt.p; g.n_kb_total = n_kb_total; }
-		XALM_TRY(run(g, P.wqkv));
+		XALM_TRY(run(g, P.wqkv, "gemm_qkv"));
 		t_begin("attention");
 		if (attn_tc) {
 			if (!tiles_from_epilogue)
-				retile_kv_kernel<<<dim3(2 * n_kb_total, c.n_kv_heads), 256, 0, s>>>(window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, pm.kv_dim,
+				retile_kv_kernel<<<dim3(2 * n_kb_total, pm.n_kv_heads), 256, 0, s>>>(window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, pm.kv_dim,
 				                                                                    attn_pos0 + T, n_kb_total, sc.kt.p, sc.vt.p);
-			AttnTcArgs at = {sc.qt_hi.p, precise ? sc.qt_lo.p : nullptr, sc.kt.p, sc.vt.p, xb2, T, attn_pos0, c.n_heads, c.n_kv_heads, n_qb, n_kb_total,
+			AttnTcArgs at = {sc.qt_hi.p, precise ? sc.qt_lo.p : nullptr, sc.kt.p, sc.vt.p, xb2, T, attn_pos0, pm.n_heads, pm.n_kv_heads, n_qb, n_kb_total,
 			                 window ? S : 0, window ? sink_k : nullptr, window ? P.v_cache : nullptr, pm.kv_dim,
 			                 getenv("XALM_ATTN_DBG") ? atoi(getenv("XALM_ATTN_DBG")) : 0};
 			XALM_TRY(precise ? launch_attn_tc<true>(at, s) : launch_attn_tc<false>(at, s));
 			launches++;
 		} else {
-			AttnPArgs at = {q, q_lo, window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, xb2, T, attn_pos0, pm.q_dim, pm.kv_dim, c.n_heads,
-			                c.n_kv_heads, cdiv(T, 64), window ? S : 0, window ? sink_k : nullptr, window ? P.v_cache : nullptr};
+			AttnPArgs at = {q, q_lo, window ? k_stage : P.k_cache, window ? v_stage : P.v_cache, xb2, T, attn_pos0, pm.q_dim, pm.kv_dim, pm.n_heads,
+			                pm.n_kv_heads, cdiv(T, 64), window ? S : 0, window ? sink_k : nullptr, window ? P.v_cache : nullptr};
 			if (c.head_dim == 128) XALM_TRY(precise ? (launch_attn_p<128, true>(at, s)) : (launch_attn_p<128, false>(at, s)));
 			else XALM_TRY(precise ? (launch_attn_p<64, true>(at, s)) : (launch_attn_p<64, false>(at, s)));
 		}
 		t_end();
-		XALM_TRY(prep(P.w13, true, P.glu_off, c.hidden_dim, c.dim, NT_glu, KT_dim));
+		XALM_TRY(prep(P.w13, true, P.glu_off, pm.hidden, c.dim, NT_glu, KT_dim));
 		g = {};
 		g.a_hi = xb2.hi; g.a_lo = xb2.lo;
-		g.MT = MT; g.NT = NT_dim; g.KT = KT_q; g.M = T; g.N = c.dim; g.epi = GEPI_RESID; g.out = x; g.ldo = c.dim;
-		XALM_TRY(run(g, P.wo));
+		g.MT = MT; g.NT = NT_dim; g.KT = KT_q; g.M = T; g.N = c.dim;
+		XALM_TRY(row_split(g, P.wo, "gemm_wo"));
 		// ---- feed-forward half ----
 		t_begin("rmsnorm");
 		rmsnorm_rows_kernel<<<norm_grid, 128, 0, s>>>(x, T, c.dim, P.rms_ffn, P.rms_ffn_type, c.norm_eps, xb);
 		t_end();
-		XALM_TRY(prep(P.w2, false, 0, c.dim, c.hidden_dim, NT_dim, KT_h));
+		XALM_TRY(prep(P.w2, false, 0, c.dim, pm.hidden, NT_dim, KT_h));
 		g = {};
 		g.a_hi = xb.hi; g.a_lo = xb.lo;
-		g.MT = MT; g.NT = NT_glu; g.KT = KT_dim; g.M = T; g.N = c.hidden_dim; g.epi = GEPI_GLU; g.o = hb; g.act = c.act;
-		XALM_TRY(run(g, P.w13));
+		g.MT = MT; g.NT = NT_glu; g.KT = KT_dim; g.M = T; g.N = pm.hidden; g.epi = GEPI_GLU; g.o = hb; g.act = c.act;
+		XALM_TRY(run(g, P.w13, "gemm_w13"));
 		if (l + 1 < L) XALM_TRY(prep_qkv(l + 1));
-		else if (want_logits) XALM_TRY(prep(pm.wcls, false, 0, c.vocab_size, c.dim, NT_cls, KT_dim));
+		else if (want_logits) XALM_TRY(prep(pm.wcls, false, 0, pm.vocab, c.dim, NT_cls, KT_dim));
 		g = {};
 		g.a_hi = hb.hi; g.a_lo = hb.lo;
-		g.MT = MT; g.NT = NT_dim; g.KT = KT_h; g.M = T; g.N = c.dim; g.epi = GEPI_RESID; g.out = x; g.ldo = c.dim;
-		XALM_TRY(run(g, P.w2));
+		g.MT = MT; g.NT = NT_dim; g.KT = KT_h; g.M = T; g.N = c.dim;
+		XALM_TRY(row_split(g, P.w2, "gemm_w2"));
 		launches += 3;
 	}
 	if (want_logits) {
-		if (!L) XALM_TRY(prep(pm.wcls, false, 0, c.vocab_size, c.dim, NT_cls, KT_dim));
+		if (!L) XALM_TRY(prep(pm.wcls, false, 0, pm.vocab, c.dim, NT_cls, KT_dim));
 		rmsnorm_rows_kernel<<<norm_grid, 128, 0, s>>>(x, T, c.dim, pm.rms_final, pm.rms_final_type, c.norm_eps, xb);
 		GemmArgs g = {};
 		g.a_hi = xb.hi; g.a_lo = xb.lo;
-		g.NT = NT_cls; g.KT = KT_dim; g.M = T; g.N = c.vocab_size; g.epi = GEPI_STORE;
-		g.out = reinterpret_cast<float*>(sc.logits.p); g.ldo = c.vocab_size;
+		g.NT = NT_cls; g.KT = KT_dim; g.M = T; g.N = pm.vocab; g.epi = GEPI_STORE;
+		// tensor parallel: this rank's (rows, vocab_l) block of the all-gathered shards, then back to the one-GPU layout
+		float* logits_tp = reinterpret_cast<float*>(sc.logits_tp.p);
+		const size_t shard = (size_t) logit_rows * pm.vocab;
+		g.out = tp ? logits_tp + pm.tp_rank * shard : reinterpret_cast<float*>(sc.logits.p); g.ldo = pm.vocab;
 		g.mt0 = want_logits == 1 ? MT - 1 : 0;
 		g.MT = want_logits == 1 ? 1 : MT;
 		g.out_row0 = logit_row0;
-		XALM_TRY(run(g, pm.wcls));
+		XALM_TRY(run(g, pm.wcls, "gemm_cls"));
 		launches++;
+		if (tp) {
+			t_begin("exchange");
+			XALM_NCCL_CHECK(g_nccl.AllGather(logits_tp + pm.tp_rank * shard, logits_tp, shard, ncclFloat32, pm.comm, s));
+			t_end();
+			unshard_logits_kernel<<<(int) std::min<size_t>((logit_rows * (size_t) c.vocab_size / 4 + 255) / 256, (size_t) sm_count() * 8), 256, 0, s>>>(
+			    logits_tp, pm.tp_size, logit_rows, pm.vocab, reinterpret_cast<float*>(sc.logits.p));
+			launches += 2;
+		}
 		if (targets && probs_host) {
-			XALM_TRY(sc.targets.ensure((size_t) T * 4, false, s));
-			XALM_TRY(sc.probs.ensure((size_t) T * 4, false, s));
 			for (int i = 0; i < T; i++)
 				if (targets[i] < 0 || targets[i] >= c.vocab_size) return set_error(XALM_ERR_INVALID, "prefill: target %d out of range", targets[i]);
 			XALM_CUDA_CHECK(cudaMemcpyAsync(sc.targets.p, targets, (size_t) T * 4, cudaMemcpyHostToDevice, s));

@@ -4,6 +4,7 @@
 #pragma once
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
+#include <nccl.h>
 
 #include <vector>
 
@@ -23,7 +24,12 @@ struct PrefillLayer {
 
 struct PrefillModel {
 	xalm_config c;
-	int q_dim = 0, kv_dim = 0;
+	// this rank's shard of the sharded dimensions (one GPU: the full sizes; tensor parallel: SURVEY.md 8e)
+	int q_dim = 0, kv_dim = 0, n_heads = 0, n_kv_heads = 0, hidden = 0, vocab = 0;
+	// tensor parallel (tp_size > 1): the pass is a collective over `comm`; status_dev: one device int for the status vote
+	int tp_rank = 0, tp_size = 1;
+	ncclComm_t comm = nullptr;
+	int* status_dev = nullptr;
 	const uint8_t* embed_raw = nullptr; // on-disk rows
 	int embed_type = 0;
 	size_t embed_row_bytes = 0;
@@ -42,6 +48,8 @@ struct PrefillScratch; // device scratch + pinned staging, grown on demand; owne
 // logits_host: NULL, or vocab floats (want 1) / n*vocab floats (want 2).  targets/probs_host: NULL, or n entries —
 // probs_host[i] = softmax(logits_i)[targets[i]] as Sampler::sample_prob computes it (needs want 2).
 // split: 1 = activations as one fp16 operand, 2 = hi+lo fp16 pair (two MMAs per weight tile, ~fp32 activations).
+// Tensor parallel (pm.tp_size > 1): every rank calls it with the same arguments; each fills its KV-cache shard and receives the
+// full logits / probabilities.  A refusal is the same on every rank and leaves every cache untouched.
 // window = false: the linear regime, pos0 + n <= max_seq_len.  window = true: the ring regime past the context window,
 // pos0 >= max_seq_len and n <= max_seq_len - 2 (each ring slot written at most once); new rows go to their ring slots and the
 // two sink keys are re-rotated n times, as n token-at-a-time forwards would leave the cache.

@@ -13,7 +13,6 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 #include <math.h>
-#include <nccl.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -30,6 +29,7 @@
 #include "matvec_idp.cuh"
 #include "matvec_mma.cuh"
 #include "decode_mega.h"
+#include "nccl_api.h"
 #include "prefill.h"
 
 namespace xalm {
@@ -814,20 +814,10 @@ static int upload_piece(WMat& m, int dst_row, int type, const uint8_t* host, int
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// NCCL, loaded lazily: single-GPU users need no libnccl at all, and inside a torch process the already-loaded
-// libnccl.so.2 is the one dlopen returns.
+// NCCL, loaded lazily (nccl_api.h)
 // ---------------------------------------------------------------------------------------------------------
-struct NcclApi {
-	void* h = nullptr;
-	ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
-	ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
-	ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-	ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-	ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
-	const char* (*GetErrorString)(ncclResult_t) = nullptr;
-};
-static NcclApi g_nccl;
-static int nccl_load() {
+NcclApi g_nccl;
+int nccl_load() {
 	if (g_nccl.h) return XALM_OK;
 	const char* names[] = {"libnccl.so.2", "libnccl.so"};
 	for (const char* n : names)
@@ -842,16 +832,12 @@ static int nccl_load() {
 	XALM_NCCL_SYM(CommInitRank, "ncclCommInitRank");
 	XALM_NCCL_SYM(AllReduce, "ncclAllReduce");
 	XALM_NCCL_SYM(AllGather, "ncclAllGather");
+	XALM_NCCL_SYM(ReduceScatter, "ncclReduceScatter");
 	XALM_NCCL_SYM(CommDestroy, "ncclCommDestroy");
 	XALM_NCCL_SYM(GetErrorString, "ncclGetErrorString");
 #undef XALM_NCCL_SYM
 	return XALM_OK;
 }
-#define XALM_NCCL_CHECK(expr)                                                                                     \
-	do {                                                                                                          \
-		ncclResult_t _r = (expr);                                                                                 \
-		if (_r != ncclSuccess) return set_error(XALM_ERR_COMM, "%s failed: %s", #expr, g_nccl.GetErrorString(_r)); \
-	} while (0)
 
 } // namespace xalm
 
@@ -932,6 +918,7 @@ struct xalm_cuda_model {
 	// batched prefill (prefill.cu)
 	PrefillScratch* prefill = nullptr;
 	int last_prefill_launches = 0;
+	int* prefill_status = nullptr;    // tensor parallel: the one int the ranks' status vote reduces (allocated by finalize)
 };
 
 static int parse_tensor_name(const char* name, int n_layers, int* layer, int* piece) {
@@ -1634,8 +1621,12 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 			ok = ok && takes(L.wqkv.m, c.dim) && takes(L.wo.m, m->q_dim_l) && takes(L.w13.m, c.dim) && takes(L.w2.m, m->hidden_l);
 		m->tp_fused = ok;
 	}
-	if (m->tp_size > 1) XALM_TRY(fzero(&m->logits_full, c.vocab_size));
-	else m->logits_full = m->logits;
+	if (m->tp_size > 1) {
+		XALM_TRY(fzero(&m->logits_full, c.vocab_size));
+		XALM_TRY(m->da.alloc((void**) &m->prefill_status, sizeof(int)));
+	} else {
+		m->logits_full = m->logits;
+	}
 	const size_t kv_elems = (size_t) c.max_seq_len * m->kv_dim_l;
 	for (auto& L : m->layers) {
 		XALM_TRY(m->da.alloc((void**) &L.k_cache, kv_elems * sizeof(__half)));
@@ -2018,7 +2009,9 @@ int xalm_cuda_ffn(float* xout, const float* x, const void* w1, const void* w2, c
 
 static void fill_prefill_model(xalm_cuda_model* m, PrefillModel& pm) {
 	pm.c = m->c;
-	pm.q_dim = m->q_dim; pm.kv_dim = m->kv_dim;
+	pm.q_dim = m->q_dim_l; pm.kv_dim = m->kv_dim_l; pm.n_heads = m->n_heads_l; pm.n_kv_heads = m->n_kv_heads_l;
+	pm.hidden = m->hidden_l; pm.vocab = m->vocab_l;
+	pm.tp_rank = m->tp_rank; pm.tp_size = m->tp_size; pm.comm = m->comm; pm.status_dev = m->prefill_status;
 	pm.embed_raw = m->embed_raw; pm.embed_type = m->embed_type; pm.embed_row_bytes = m->embed_row_bytes;
 	pm.wcls = m->wcls.m; pm.rms_final = m->rms_final; pm.rms_final_type = m->rms_final_type;
 	pm.rope_freq = m->rope_freq;
@@ -2033,12 +2026,11 @@ static void fill_prefill_model(xalm_cuda_model* m, PrefillModel& pm) {
 	}
 }
 
-// ---- batched prefill / perplexity on the tensor-core path (prefill.cu) ----------------------------------------------------
+// ---- batched prefill / perplexity on the tensor-core path (prefill.cu); a collective under tensor parallelism --------------
 int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host, const int* targets,
                       float* probs_host) {
 	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
 	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	if (m->tp_size > 1) return set_error(XALM_ERR_UNSUPPORTED, "prefill: tensor-parallel models take the token-at-a-time path");
 	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill: want_logits = %d", want_logits);
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
 	PrefillModel pm;
@@ -2056,7 +2048,6 @@ int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int p
                              float* probs_host) {
 	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
 	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	if (m->tp_size > 1) return set_error(XALM_ERR_UNSUPPORTED, "prefill_window: tensor-parallel models take the token-at-a-time path");
 	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill_window: want_logits = %d", want_logits);
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
 	PrefillModel pm;
@@ -2073,7 +2064,6 @@ int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int po
 	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
 	// same as xalm_cuda_prefill without the host synchronisation and read-back (bench.py's device-timed leg)
 	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	if (m->tp_size > 1) return set_error(XALM_ERR_UNSUPPORTED, "prefill: tensor-parallel models take the token-at-a-time path");
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
 	PrefillModel pm;
 	fill_prefill_model(m, pm);

@@ -174,13 +174,15 @@ class Model:
         """Positions pos0..pos0+len(tokens)-1 at once.  want_logits 0: hydrate only -> None; 1: logits of the last
         position (vocab,); 2: all positions (n, vocab).  With `targets` returns (logits, probs) where probs[i] is
         Sampler.sample_prob(targets[i]) at position pos0+i; fetch_logits=False leaves the logits on the device (perplexity
-        mode needs only the probabilities)."""
+        mode needs only the probabilities).  On a tensor-parallel model this is a collective: every rank calls it with the
+        same arguments and gets the full logits and probabilities; a refusal raises the same error on every rank."""
         return self._prefill_call("prefill", tokens, pos0, want_logits, targets, fetch_logits)
 
     def prefill_window(self, tokens, pos0: int, want_logits: int = 1, targets=None, fetch_logits: bool = True):
         """prefill past the context window, where the KV cache is a ring with two attention sinks: positions
         pos0..pos0+len(tokens)-1 with pos0 >= max_seq_len and len(tokens) <= max_seq_len - 2 (longer runs go in chunks).
-        Leaves the KV cache as that many forward() calls would.  Arguments and results as for prefill()."""
+        Leaves the KV cache as that many forward() calls would.  Arguments, results and the tensor-parallel collective as for
+        prefill()."""
         return self._prefill_call("prefill_window", tokens, pos0, want_logits, targets, fetch_logits)
 
     def _prefill_call(self, which: str, tokens, pos0: int, want_logits: int, targets, fetch_logits: bool):
