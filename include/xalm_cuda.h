@@ -189,10 +189,10 @@ int xalm_cuda_rope(float* vec, int d, int head_dim, int pos, float theta, int ro
 int xalm_cuda_ffn(float* xout, const float* x, const void* w1, const void* w2, const void* w3, int type_id,
                   int hidden_dim, int dim, int act);
 
-/* Integer tuning knobs by name ("pdl", "graph", "attn_splits", "attn_min_split", "mv_cfg_rows", "prefill_split", "idp", "mma", "mega",
+/* Integer tuning knobs by name ("pdl", "graph", "attn_splits", "attn_min_split", "prefill_split", "idp", "mma",
  * "tail_prefetch_mb", ...); an XALM_<KEY> environment variable overrides the stored value.  Takes effect for graphs captured
  * afterwards; "mma" (which matvec kernel and device layout the integer formats take: 0 = dp4a + unit layout, 1 = tensor-core mma +
- * fragment tiles, 2 = default: mma for the 4/5-bit formats and, under tensor parallelism, the 8-bit ones) and "mega" are read when a
+ * fragment tiles, 2 = default: mma for the 4/5-bit formats and, under tensor parallelism, the 8-bit ones) is read when a
  * matrix is uploaded. */
 int xalm_cuda_tune(const char* key, int value);
 
@@ -200,10 +200,6 @@ int xalm_cuda_tune(const char* key, int value);
  * stop and fetch the records — 4 x u64 each: kernel id (100+epi = TMA matvec, 200+epi = LDG matvec, 300 = attention),
  * %globaltimer (ns) of block 0 at entry, after the dependency wait, at exit. */
 int xalm_cuda_timeline(int n_records, unsigned long long* out, int* n_out);
-/* Same idea for the one-kernel-per-token decode path (decode_mega.cu; tune "mega_timeline" = 1 before the first forward):
- * out receives n_phases x 8 u64 of CTA 0 (phase entry, hand-off done, activations staged, phase done, four finer marks) followed by
- * n_phases x grid arrival stamps of every CTA.  With out == NULL only n_phases / grid are returned (0 = token kernel not in use). */
-int xalm_cuda_mega_timeline(xalm_cuda_model* m, unsigned long long* out, size_t cap_words, int* n_phases, int* grid);
 
 /* ---- kernel micro-benchmark hook (bench.py roofline leg; README.md:62-84 `-k matmul`) ------------------- */
 /* Times `iters` back-to-back launches of the matvec kernel on resident weights of `type_id` (random bytes), rotating

@@ -50,7 +50,7 @@ for kn in configs:
         model.sync()
         tl = capi.timeline_stop(800).astype(np.int64)
         t0 = tl[:, 1].min()
-        names = {400: "mega", 410: "mk_store", 411: "mk_resid", 412: "mk_glu", 413: "mk_qkv", 419: "mk_attn", 100: "tma_store", 101: "tma_resid", 102: "tma_glu", 103: "tma_qkv", 200: "ldg_store", 201: "ldg_resid", 202: "ldg_glu", 203: "ldg_qkv", 300: "attn"}
+        names = {100: "tma_store", 101: "tma_resid", 102: "tma_glu", 103: "tma_qkv", 200: "ldg_store", 201: "ldg_resid", 202: "ldg_glu", 203: "ldg_qkv", 300: "attn"}
         order = np.argsort(tl[:, 1])
         prev_end = None
         rows = []

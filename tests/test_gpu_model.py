@@ -69,8 +69,8 @@ def test_hydrate_mode_and_state_buffers():
     gm.forward(state, 5, len(PROMPT), 1)
     assert np.max(np.abs(state.logits() - lg_o)) <= LOGIT_TOL
     assert np.array_equal(gm.read_state(capi.S_LOGITS, config["vocab_size"]), state.logits())
-    # launches per token: embed + 5 fused kernels per layer + classifier, or embed + the token kernel
-    assert gm.last_launch_count() in (1 + 5 * config["n_layers"] + 1, 2)
+    # launches per token: embed + 5 fused kernels per layer + classifier
+    assert gm.last_launch_count() == 1 + 5 * config["n_layers"] + 1
     gm.close(); om.close()
 
 
@@ -115,49 +115,6 @@ def test_finite_qkv_clip():
     gm2.forward(st, PROMPT[0], 0, 1)
     assert np.max(np.abs(gm2.read_state(capi.S_Q, config2["n_heads"] * config2["head_dim"]))) > 0.75
     gm2.close(); om2.close()
-
-
-# ---- the one-kernel-per-token path (decode_mega.cu, opt-in: tune "mega" = 1): same contract as the kernel-per-op path ----
-@pytest.fixture
-def token_kernel():
-    capi.tune("mega", 1)
-    yield
-    capi.tune("mega", 0)
-
-
-@pytest.mark.parametrize("shape,std,steps", [("tiny", 0.06, 24), ("small", 0.03, 16)])
-@pytest.mark.parametrize("wtype", ["q8_0", "q4_0", "q4_1", "q5_0", "q5_1", "q8"])
-def test_token_kernel_every_integer_format(token_kernel, wtype, shape, std, steps):
-    config, om, gm = synth_pair(shape, wtype, seed=2, std=std)
-    otoks, gtoks, maxdiff, margin = greedy_compare(config, om, gm, PROMPT, steps)
-    assert gm.last_launch_count() == 2, "embed + the token kernel"
-    assert maxdiff <= LOGIT_TOL, f"{wtype}: logits differ by {maxdiff}"
-    assert otoks == gtoks, f"{wtype}: greedy tokens diverge (min margin {margin})"
-    gm.close(); om.close()
-
-
-def test_token_kernel_ring_sinks_hydrate_and_long_context(token_kernel, golden_dir):
-    # ring buffer + re-rotated sinks (-T 6)
-    config, om, gm = synth_pair("tiny", "q8_0", seed=5, std=0.06, context=6)
-    assert config["max_seq_len"] == 6
-    otoks, gtoks, maxdiff, _ = greedy_compare(config, om, gm, [1, 266, 267], 30)
-    assert gm.last_launch_count() == 2 and maxdiff <= LOGIT_TOL and otoks == gtoks
-    gm.close(); om.close()
-    # multi-split attention (200 positions, GQA 8:2, head_dim 128) after a HYDRATE-only prompt
-    config, om, gm = synth_pair("small", "q8_0", seed=1, std=0.03)
-    prompt = [int(t) for t in np.random.default_rng(0).integers(3, config["vocab_size"], size=180)]
-    otoks, gtoks, maxdiff, margin = greedy_compare(config, om, gm, prompt, 24)
-    assert gm.last_launch_count() == 2 and maxdiff <= LOGIT_TOL
-    assert otoks == gtoks, f"min margin {margin}"
-    gm.close(); om.close()
-
-
-def test_token_kernel_falls_back_for_float_formats(token_kernel):
-    config, om, gm = synth_pair("tiny", "f16", seed=2, std=0.06)
-    otoks, gtoks, maxdiff, _ = greedy_compare(config, om, gm, PROMPT, 8)
-    assert gm.last_launch_count() == 1 + 5 * config["n_layers"] + 1       # kernel-per-op path
-    assert maxdiff <= LOGIT_TOL and otoks == gtoks
-    gm.close(); om.close()
 
 
 def test_small_model_longer_context():

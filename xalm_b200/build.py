@@ -39,7 +39,7 @@ def _sources(d, exts):
     return out
 
 
-CUDA_TUS = ["xalm_cuda.cu", "prefill.cu", "decode_mega.cu"]   # translation units of libxalm_cuda.so (objects cached under csrc/.obj)
+CUDA_TUS = ["xalm_cuda.cu", "prefill.cu"]   # translation units of libxalm_cuda.so (objects cached under csrc/.obj)
 
 
 def build_cuda(force: bool = False, verbose: bool = False, extra=()) -> str:

@@ -74,7 +74,6 @@ SYMBOLS = {
     "xalm_cuda_ffn": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i]),
     "xalm_cuda_tune": (_i, [C.c_char_p, _i]),
     "xalm_cuda_timeline": (_i, [_i, _vp, C.POINTER(_i)]),
-    "xalm_cuda_mega_timeline": (_i, [_vp, _vp, C.c_size_t, C.POINTER(_i), C.POINTER(_i)]),
     "xalm_cuda_bench_matvec": (_i, [_i, _i, _i, _i, _i, _i, _i, _fp]),
     "xalm_cuda_prefill": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "xalm_cuda_prefill_window": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
@@ -182,19 +181,6 @@ def timeline_stop(n_records: int) -> np.ndarray:
     n = C.c_int(0)
     check(lib().xalm_cuda_timeline(n_records, _p(out), C.byref(n)))
     return out[: n.value]
-
-
-def mega_timeline(handle):
-    """(stamps of CTA 0 [n_phases, 8], arrival stamps of every CTA [n_phases, grid]) of the last token kernel, in ns;
-    (None, None) when the one-kernel-per-token path is not in use.  Needs tune("mega_timeline", 1) before the first forward."""
-    n_ph, grid = C.c_int(0), C.c_int(0)
-    check(lib().xalm_cuda_mega_timeline(handle, None, 0, C.byref(n_ph), C.byref(grid)))
-    if not n_ph.value:
-        return None, None
-    words = n_ph.value * (8 + grid.value)
-    out = np.zeros(words, dtype=np.uint64)
-    check(lib().xalm_cuda_mega_timeline(handle, _p(out), words, C.byref(n_ph), C.byref(grid)))
-    return out[: 8 * n_ph.value].reshape(n_ph.value, 8), out[8 * n_ph.value:].reshape(n_ph.value, grid.value)
 
 
 def bench_matvec(type_id: int, n: int, d: int, n_buffers: int, iters: int, epi: int = 0, with_norm: bool = False) -> float:

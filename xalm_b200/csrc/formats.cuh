@@ -36,7 +36,7 @@ __host__ __device__ inline bool type_info(int t, TypeInfo* ti) {
 	return false;
 }
 
-// bytes of one 256-element "unit" of the unit-interleaved device layout (matvec_tma.cuh, decode_mega.cu); 0 = not a unit format
+// bytes of one 256-element "unit" of the unit-interleaved device layout (matvec_tma.cuh, matvec_idp.cuh); 0 = not a unit format
 __host__ __device__ inline int unit_bytes(int t) {
 	switch (t) {
 		case XALM_F32: return 1024;

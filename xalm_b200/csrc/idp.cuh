@@ -34,57 +34,20 @@ struct XqView {
 __host__ __device__ inline size_t xq_bytes(int n) { return (size_t) 3 * n + (size_t) (n / 32) * 16; }
 __device__ __forceinline__ XqView xq_view(uint8_t* base, int n) { return {base, reinterpret_cast<int4*>(base + (size_t) 3 * n), n}; }
 
-// One thread quantises one 32-element block held in registers: no cross-lane traffic at all (an earlier version split a block
-// over 8 lanes and spent 12 shuffles per 4 elements — the staging of a 14336-long vector cost 4 us per layer).
-__device__ __forceinline__ void xq_store_block(const XqView& v, int blk, const float (&x)[32]) {
-	uint32_t mb = 0; // block maximum of |x| (non-negative floats order like their bit patterns)
-#pragma unroll
-	for (int e = 0; e < 32; e++) mb = max(mb, __float_as_uint(x[e]) & 0x7fffffffu);
-	const int eb = (int) (mb >> 23);                 // biased exponent of the maximum: max < 2^(eb-126)
-	const bool live = eb >= 40 && eb < 255;          // blocks below 2^-87 contribute nothing; non-finite blocks are dropped
-	const float sc = live ? __uint_as_float((uint32_t) (276 - eb) << 23) : 0.f;  // 2^(149-eb): |x*sc| < 2^23
-	const float dx = live ? __uint_as_float((uint32_t) (eb - 22) << 23) : 0.f;   // 2^(eb-149)
-	uint32_t w[3][8];
-	int s0 = 0, s1 = 0, s2 = 0;
-#pragma unroll
-	for (int q = 0; q < 8; q++) {
-		int X[4];
-#pragma unroll
-		for (int e = 0; e < 4; e++) X[e] = min(__float2int_rn(x[4 * q + e] * sc), 8388607);
-		// byte k of X[0..3] -> word k (limb 2 = low byte, limb 0 = signed high byte)
-#pragma unroll
-		for (int k = 0; k < 3; k++) {
-			const uint32_t sel = (uint32_t) k | ((uint32_t) (4 + k) << 4);
-			const uint32_t lo = prmt((uint32_t) X[0], (uint32_t) X[1], sel), hi = prmt((uint32_t) X[2], (uint32_t) X[3], sel);
-			w[2 - k][q] = prmt(lo, hi, 0x5410u);
-		}
-		asm("dp4a.s32.u32 %0, %1, %2, %0;" : "+r"(s0) : "r"(w[0][q]), "r"(0x01010101u));
-		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s1) : "r"(w[1][q]), "r"(0x01010101u));
-		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s2) : "r"(w[2][q]), "r"(0x01010101u));
-	}
-#pragma unroll
-	for (int k = 0; k < 3; k++) {
-		uint8_t* p = v.q + (size_t) k * v.n + (size_t) blk * 32;
-		*reinterpret_cast<uint4*>(p) = make_uint4(w[k][0], w[k][1], w[k][2], w[k][3]);
-		*reinterpret_cast<uint4*>(p + 16) = make_uint4(w[k][4], w[k][5], w[k][6], w[k][7]);
-	}
-	v.meta[blk] = make_int4(s0, s1, s2, (int) __float_as_uint(dx));
-}
-
-// The staging used by the kernels: EIGHT consecutive elements per lane, the four lanes 4k..4k+3 of a warp share a block (call with
-// all lanes of the warp).  Loads are coalesced (32 bytes per lane, 1 KB per warp instruction) and every thread of the CTA works;
-// the thread-per-block version above left half the CTA idle behind 32 line-strided loads per lane and took 7 us of a 25 us
-// kernel (profiles/r2_decode_timeline.md).  Same image in shared memory, bit for bit.
+// The staging: EIGHT consecutive elements per lane, the four lanes 4k..4k+3 of a warp share a block (call with all lanes of the
+// warp).  Loads are coalesced (32 bytes per lane, 1 KB per warp instruction) and every thread of the CTA works; a thread-per-block
+// staging left half the CTA idle behind 32 line-strided loads per lane and took 7 us of a 25 us kernel
+// (profiles/r2_decode_timeline.md).
 __device__ __forceinline__ void xq_store_group8(const XqView& v, int grp, const float (&x)[8]) {
-	uint32_t mb = 0;
+	uint32_t mb = 0; // block maximum of |x| (non-negative floats order like their bit patterns)
 #pragma unroll
 	for (int e = 0; e < 8; e++) mb = max(mb, __float_as_uint(x[e]) & 0x7fffffffu);
 	mb = max(mb, __shfl_xor_sync(0xffffffffu, mb, 1));
 	mb = max(mb, __shfl_xor_sync(0xffffffffu, mb, 2));
-	const int eb = (int) (mb >> 23);
-	const bool live = eb >= 40 && eb < 255;
-	const float sc = live ? __uint_as_float((uint32_t) (276 - eb) << 23) : 0.f;
-	const float dx = live ? __uint_as_float((uint32_t) (eb - 22) << 23) : 0.f;
+	const int eb = (int) (mb >> 23);                 // biased exponent of the maximum: max < 2^(eb-126)
+	const bool live = eb >= 40 && eb < 255;          // blocks below 2^-87 contribute nothing; non-finite blocks are dropped
+	const float sc = live ? __uint_as_float((uint32_t) (276 - eb) << 23) : 0.f;  // 2^(149-eb): |x*sc| < 2^23
+	const float dx = live ? __uint_as_float((uint32_t) (eb - 22) << 23) : 0.f;   // 2^(eb-149)
 	uint32_t w[3][2];
 	int s0 = 0;
 	uint32_t s1 = 0, s2 = 0;
@@ -93,6 +56,7 @@ __device__ __forceinline__ void xq_store_group8(const XqView& v, int grp, const 
 		int X[4];
 #pragma unroll
 		for (int e = 0; e < 4; e++) X[e] = min(__float2int_rn(x[4 * q + e] * sc), 8388607);
+		// byte k of X[0..3] -> word k (limb 2 = low byte, limb 0 = signed high byte)
 #pragma unroll
 		for (int k = 0; k < 3; k++) {
 			const uint32_t sel = (uint32_t) k | ((uint32_t) (4 + k) << 4);
