@@ -79,7 +79,7 @@ def build_host(force: bool = False) -> str:
     main_src = os.path.join(hdir, "main.cpp")
     if os.path.exists(main_src) and (force or not _newer(MAIN, deps + [LIB])):
         build_cuda()
-        subprocess.check_call([*common, "-o", MAIN, main_src, os.path.join(hdir, "model.cpp"), quant, "-L", HERE, "-lxalm_cuda",
+        subprocess.check_call([*common, "-o", MAIN, main_src, os.path.join(hdir, "launch.cpp"), os.path.join(hdir, "model.cpp"), quant, "-L", HERE, "-lxalm_cuda",
                                "-Wl,-rpath,$ORIGIN"])
     return HOSTLIB
 

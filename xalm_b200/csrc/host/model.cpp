@@ -315,13 +315,21 @@ Model Model::from_xalm(Xalm::file_info& xalm, const int context, const bool defe
 	return m;
 }
 
-void Model::cuda(int device_index, int tp_rank, int tp_size, const void* comm_id) {
+void Model::cuda(int device_index, int tp_rank, int tp_size, const void* comm_id, const IpcExchange& ipc_exchange) {
 	if (handle_) return;
 	const xalm_config c = config.to_c();
 	if (xalm_cuda_create(&c, device_index, tp_rank, tp_size, &handle_) != XALM_OK) xalm_throw_last("model.cuda()");
 	if (tp_size > 1) {
 		if (!comm_id) throw std::invalid_argument("model.cuda(): tensor parallel needs a communicator id");
 		if (xalm_cuda_comm_init(handle_, comm_id) != XALM_OK) xalm_throw_last("model.cuda()");
+		if (ipc_exchange) {
+			std::vector<uint8_t> mine(XALM_IPC_HANDLE_BYTES);
+			if (xalm_cuda_ipc_export(handle_, mine.data()) != XALM_OK) xalm_throw_last("model.cuda()");
+			const std::vector<uint8_t> table = ipc_exchange(mine);
+			if (table.size() != (size_t) tp_size * XALM_IPC_HANDLE_BYTES)
+				throw std::invalid_argument("model.cuda(): the IPC exchange must return tp_size x 64 bytes");
+			if (xalm_cuda_ipc_import(handle_, table.data()) != XALM_OK) xalm_throw_last("model.cuda()");
+		}
 	}
 	if (deferred_) {
 		// disk -> pinned staging -> device, one tensor at a time; row-sharded tensors read only this rank's rows
@@ -381,6 +389,12 @@ size_t Model::active_bytes(const size_t pos) const {
 		bytes += 2 * kv_len * kv_dim * sizeof(uint16_t);
 	}
 	return bytes;
+}
+
+int Model::last_launch_count() const {
+	int n = 0;
+	if (!handle_ || xalm_cuda_last_launch_count(handle_, &n) != XALM_OK) return 0;
+	return n;
 }
 
 void Model::forward(const InferenceState& s, const int token, const int pos, const InferenceMode mode) const {

@@ -12,6 +12,7 @@
 #include <cfloat>
 #include <cstdint>
 #include <cstring>
+#include <functional>
 #include <map>
 #include <memory>
 #include <stdexcept>
@@ -136,6 +137,9 @@ private:
 
 enum class InferenceMode { HYDRATE_KV_CACHE, OUTPUT_LOGITS };
 
+// Tensor parallel over peer memory: gets this rank's XALM_IPC_HANDLE_BYTES handle, returns every rank's, in rank order.
+using IpcExchange = std::function<std::vector<uint8_t>(const std::vector<uint8_t>& mine)>;
+
 // ---- Model (model.h:254-284) ------------------------------------------------------------------------------------
 struct Model {
 	// defer_load: do not read the weights into host memory now — model.cuda() then streams each tensor disk -> pinned staging
@@ -150,9 +154,13 @@ struct Model {
 	Config config;
 	Device device = Device::CPU;
 
-	// model.cuda(): upload every tensor (sharded for tp_size > 1), release the host copies, finalize.
-	void cuda(int device_index = 0, int tp_rank = 0, int tp_size = 1, const void* comm_id = nullptr);
+	// model.cuda(): upload every tensor (sharded for tp_size > 1), release the host copies, finalize.  With tp_size > 1 and an
+	// ipc_exchange, the ranks also swap CUDA IPC handles (after the communicator, before the uploads), which enables the fused
+	// peer-memory exchange; without one the decode exchange is ncclAllReduce.
+	void cuda(int device_index = 0, int tp_rank = 0, int tp_size = 1, const void* comm_id = nullptr, const IpcExchange& ipc_exchange = {});
 	[[nodiscard]] size_t active_bytes(size_t pos) const;
+	// Kernels launched by the last forward / prefill call (xalm_cuda_last_launch_count).
+	[[nodiscard]] int last_launch_count() const;
 	void forward(const InferenceState& s, int token, int pos, InferenceMode mode = InferenceMode::OUTPUT_LOGITS) const;
 	// The per-position loops of main.cpp:94-100 / :244-254 as one batched pass on the tensor cores (xalm_cuda_prefill).
 	// Positions pos0 .. pos0+n-1; mode OUTPUT_LOGITS leaves the LAST position's logits in s.logits().  With `targets` and
