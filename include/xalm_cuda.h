@@ -157,6 +157,27 @@ int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int p
 /* Enqueue only (no read-back, no host sync) — bench.py's device-timed leg.  A collective on tensor-parallel handles; a
  * refusal there is agreed between the ranks, which takes one host synchronisation before the pass is enqueued. */
 int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits);
+/* ---- batched decode: several independent sequences per pass over the weights (one GPU) ---------------------------------
+ * xalm_cuda_set_batch: call after create and before the first upload; 1 <= max_seqs <= 8.  Allocates max_seqs sequence slots,
+ * each with its own KV cache, and puts every matrix in the tensor-core matvec's layout: an upload of a matrix that kernel cannot
+ * take (float formats, TQ1_0, QI8, rows not a multiple of 16 or too long for it, a classifier tied to such an embedding) is
+ * XALM_ERR_UNSUPPORTED naming the tensor; the embedding table itself may be in any format.  XALM_ERR_UNSUPPORTED with
+ * tp_size > 1, XALM_ERR_STATE after an upload.
+ * xalm_cuda_forward_batch: one step of n sequences: slot seqs[i] takes tokens[i] at position pos[i] (positions are independent:
+ * each slot has its own ring and attention sinks past the window).  With XALM_OUTPUT_LOGITS, logits_host (may be NULL) receives
+ * n x vocab_size floats, row i for seqs[i].  Synchronous.  Slots not named are untouched.  Each sequence's logits and cache are
+ * bit-identical to decoding it alone on a batch-1 handle with the tensor-core matvec (xalm_cuda_tune("mma", 1)), whatever else
+ * shares the step.  n outside [1, max_seqs], a slot out of range or named twice, a token out of range, a negative position or a
+ * bad mode are XALM_ERR_INVALID before anything is enqueued.
+ * xalm_cuda_forward_batch_argmax: forward_batch + Sampler::sample_argmax per row on the device; next_tokens[i] for seqs[i].
+ * xalm_cuda_forward_batch_async: enqueue only (pair with xalm_cuda_sync).
+ * xalm_cuda_select_seq: the slot the single-sequence calls (forward*, prefill*, read_kv, read_state) work on; default 0.  A prompt
+ * is hydrated into a slot with select_seq + prefill / prefill_window. */
+int xalm_cuda_set_batch(xalm_cuda_model* m, int max_seqs);
+int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, float* logits_host);
+int xalm_cuda_forward_batch_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens);
+int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode);
+int xalm_cuda_select_seq(xalm_cuda_model* m, int seq);
 /* Pinned host buffer the logits are copied into by xalm_cuda_forward (alias it as InferenceState::_logits). */
 float* xalm_cuda_logits_host(xalm_cuda_model* m);
 /* Model::active_bytes(pos) (model.cpp:12-35), 64-bit, per-format bytes; this rank's shard only. */
@@ -207,6 +228,10 @@ int xalm_cuda_timeline(int n_records, unsigned long long* out, int* n_out);
  * 2 = the fused gate|up kernel (2d rows -> d outputs through act*gate); with_norm: fuse the rmsnorm prologue.  Returns
  * mean milliseconds per launch (CUDA events on the launch stream). */
 int xalm_cuda_bench_matvec(int type_id, int n, int d, int epi, int with_norm, int n_buffers, int iters, float* ms_per_launch);
+/* The same for the batched tensor-core matvec of batched handles at n_seqs sequences (1..8): each iteration is the activation
+ * quantiser and the matvec, as in a batched step.  Integer block formats only (else XALM_ERR_UNSUPPORTED). */
+int xalm_cuda_bench_matvec_batch(int type_id, int n, int d, int epi, int with_norm, int n_seqs, int n_buffers, int iters,
+                                 float* ms_per_launch);
 
 /* Times `iters` launches of the tcgen05 GEMM kernel alone on resident fp16 tiles (T x K activations, N x K weights);
  * mean milliseconds per launch.  2*T*N*K flops per launch. */

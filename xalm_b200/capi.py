@@ -80,6 +80,12 @@ SYMBOLS = {
     "xalm_cuda_prefill_async": (_i, [_vp, _vp, _i, _i, _i]),
     "xalm_cuda_gemm": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i]),
     "xalm_cuda_bench_gemm": (_i, [_i, _i, _i, _i, _i, _fp]),
+    "xalm_cuda_set_batch": (_i, [_vp, _i]),
+    "xalm_cuda_forward_batch": (_i, [_vp, _i, _vp, _vp, _vp, _i, _vp]),
+    "xalm_cuda_forward_batch_argmax": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "xalm_cuda_forward_batch_async": (_i, [_vp, _i, _vp, _vp, _vp, _i]),
+    "xalm_cuda_select_seq": (_i, [_vp, _i]),
+    "xalm_cuda_bench_matvec_batch": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _fp]),
 }
 
 _LIB = None
@@ -186,6 +192,13 @@ def timeline_stop(n_records: int) -> np.ndarray:
 def bench_matvec(type_id: int, n: int, d: int, n_buffers: int, iters: int, epi: int = 0, with_norm: bool = False) -> float:
     ms = C.c_float(0)
     check(lib().xalm_cuda_bench_matvec(type_id, n, d, epi, int(with_norm), n_buffers, iters, C.byref(ms)))
+    return ms.value
+
+
+def bench_matvec_batch(type_id: int, n: int, d: int, n_seqs: int, n_buffers: int, iters: int, epi: int = 0, with_norm: bool = False) -> float:
+    """bench_matvec for the batched tensor-core matvec (activation quantiser + matvec) at n_seqs sequences."""
+    ms = C.c_float(0)
+    check(lib().xalm_cuda_bench_matvec_batch(type_id, n, d, epi, int(with_norm), n_seqs, n_buffers, iters, C.byref(ms)))
     return ms.value
 
 

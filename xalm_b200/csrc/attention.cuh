@@ -35,6 +35,10 @@ struct AttnArgs {
 	unsigned int* tickets; // (n_kv_heads,) zero-initialised, self-resetting
 	const uint8_t* pf_ptr; // first bytes of the next kernel's weights (Wo), pulled into L2 before this kernel waits for q
 	unsigned long long pf_bytes;
+	// batched decode (BATCH = true, blockIdx.z = sequence): step is the step's StepParams array, k_cache / v_cache are slot 0's
+	// caches, and q, out, the split partials and the tickets hold one block per sequence
+	int q_stride;          // floats between two sequences' q (and out)
+	size_t kv_slot;        // elements between two slots' caches
 };
 
 // K/V rows: coherent L2 loads (ld.global.cg).  NOT the read-only path: row kv_pos and the sink rows are written by the QKV
@@ -48,7 +52,7 @@ __host__ __device__ inline int attn_split_len(int kv_len, int n_splits, int min_
 	return len;
 }
 
-template <int HD, int G, int NW>
+template <int HD, int G, int NW, bool BATCH = false>
 __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) {
 	constexpr int LPR = HD / 8;       // lanes per K/V row
 	constexpr int RPW = 32 / LPR;     // rows per warp request
@@ -68,9 +72,17 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	// step parameters were written before the graph was launched) and the first batch of K/V rows — only the row being written
 	// this step (kv_pos) and the re-rotated sink rows are fetched again afterwards.
 	const int kvh = blockIdx.y, split = blockIdx.x;
-	const int kv_len = a.kv_len_fixed >= 0 ? a.kv_len_fixed : a.step->kv_len;
-	const int kv_pos = a.kv_len_fixed >= 0 ? -1 : a.step->kv_pos;
-	const int kv_sink = a.kv_len_fixed >= 0 ? 0 : a.step->kv_sink;
+	const int z = BATCH ? (int) blockIdx.z : 0;
+	const StepParams* step = a.step + z;
+	const float* q = a.q + (size_t) z * a.q_stride;
+	float* out = a.out + (size_t) z * a.q_stride;
+	const size_t kv_off = BATCH ? (size_t) step->slot * a.kv_slot : 0;
+	float* part_acc = a.part_acc + (size_t) z * a.n_kv_heads * a.n_splits * G * HD;
+	float* part_ml = a.part_ml + (size_t) z * a.n_kv_heads * a.n_splits * G * 2;
+	unsigned int* tickets = a.tickets + z * a.n_kv_heads;
+	const int kv_len = a.kv_len_fixed >= 0 ? a.kv_len_fixed : step->kv_len;
+	const int kv_pos = a.kv_len_fixed >= 0 ? -1 : step->kv_pos;
+	const int kv_sink = a.kv_len_fixed >= 0 ? 0 : step->kv_sink;
 	const int slen = attn_split_len(kv_len, a.n_splits, a.min_split);
 	const int n_active = (kv_len + slen - 1) / slen;
 	const int t0 = split * slen, t1 = min(kv_len, t0 + slen);
@@ -79,8 +91,8 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	const int sub = lane / LPR, li = lane % LPR; // which row of the request, which 8-dim slice
 	const int kv_stride = a.n_kv_heads * HD;
 	const float inv_sqrt = 1.0f / sqrtf((float) HD);
-	const __half* kbase = a.k_cache + (size_t) kvh * HD + li * 8;
-	const __half* vbase = a.v_cache + (size_t) kvh * HD + li * 8;
+	const __half* kbase = a.k_cache + kv_off + (size_t) kvh * HD + li * 8;
+	const __half* vbase = a.v_cache + kv_off + (size_t) kvh * HD + li * 8;
 
 	uint4 kn[TB], vn[TB]; // next batch, requested one iteration ahead
 	auto fetch = [&](int tb) {
@@ -104,7 +116,7 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	float qf[G][8];
 #pragma unroll
 	for (int g = 0; g < G; g++) {
-		const float* qp = a.q + (size_t) (kvh * G + g) * HD + li * 8;
+		const float* qp = q + (size_t) (kvh * G + g) * HD + li * 8;
 		const float4 u = ld_act4(qp), v = ld_act4(qp + 4);
 		qf[g][0] = u.x; qf[g][1] = u.y; qf[g][2] = u.z; qf[g][3] = u.w;
 		qf[g][4] = v.x; qf[g][5] = v.y; qf[g][6] = v.z; qf[g][7] = v.w;
@@ -214,8 +226,8 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 		}
 	}
 	__syncthreads();
-	float* pacc = a.part_acc + ((size_t) kvh * a.n_splits + split) * G * HD;
-	float* pml = a.part_ml + ((size_t) kvh * a.n_splits + split) * G * 2;
+	float* pacc = part_acc + ((size_t) kvh * a.n_splits + split) * G * HD;
+	float* pml = part_ml + ((size_t) kvh * a.n_splits + split) * G * 2;
 	if (n_active == 1) {
 		// the whole sequence fit in one split: normalise and write the output directly (no partial round trip, no ticket)
 		for (int i = threadIdx.x; i < G * HD; i += NW * 32) {
@@ -224,7 +236,7 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 #pragma unroll
 			for (int w = 0; w < NW; w++) v += s_acc[w][g][dpos];
 			for (int k = 0; k < NGRP; k++) L += s_l[k][g] * s_scale[k][g];
-			a.out[(size_t) kvh * G * HD + i] = v / L;
+			out[(size_t) kvh * G * HD + i] = v / L;
 		}
 		tl_mark(tl, 3);
 		return;
@@ -251,16 +263,16 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	__threadfence();
 	__syncthreads();
 	if (threadIdx.x == 0) {
-		const unsigned int ticket = atomicAdd(&a.tickets[kvh], 1u);
+		const unsigned int ticket = atomicAdd(&tickets[kvh], 1u);
 		s_last = ticket == (unsigned int) (n_active - 1);
-		if (s_last) a.tickets[kvh] = 0; // ready for the next launch
+		if (s_last) tickets[kvh] = 0; // ready for the next launch
 	}
 	__syncthreads();
 	tl_mark(tl, 3);
 	if (!s_last) return;
 	__threadfence();
-	const float* bacc = a.part_acc + (size_t) kvh * a.n_splits * G * HD;
-	const float* bml = a.part_ml + (size_t) kvh * a.n_splits * G * 2;
+	const float* bacc = part_acc + (size_t) kvh * a.n_splits * G * HD;
+	const float* bml = part_ml + (size_t) kvh * a.n_splits * G * 2;
 	// every partial of this thread's first four outputs is requested BEFORE the scales are computed: one L2 round trip for up
 	// to 16 splits, overlapped with the (m, l) pass, instead of a chain of dependent ones after it
 	constexpr int MB = 16;
@@ -304,7 +316,7 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 			}
 		}
 		const float den = s_den[g];
-		*reinterpret_cast<float4*>(a.out + (size_t) kvh * G * HD + i4) = make_float4(num.x / den, num.y / den, num.z / den, num.w / den);
+		*reinterpret_cast<float4*>(out + (size_t) kvh * G * HD + i4) = make_float4(num.x / den, num.y / den, num.z / den, num.w / den);
 	}
 }
 

@@ -37,7 +37,7 @@ struct StepParams {
 	int kv_len;  // infer.cpp:613
 	int mode;
 	unsigned int ar_base; // peer allreduce sequence base of this token (same on every rank)
-	int pad;
+	int slot;    // batched decode: the sequence slot (KV cache) this entry drives
 };
 
 // ---- loads ---------------------------------------------------------------------------------------------

@@ -1,6 +1,6 @@
 // main.cpp — the reference's CLI surface (src/main.cpp:417-547) on top of the CUDA backend.
 //
-//   xalm_main <checkpoint.xalm> [-d cuda] [-m completion|passkey|perplexity] [-T ctx] [-i prompt | -f file] [-n steps] [-l pos] [-g gpus]
+//   xalm_main <checkpoint.xalm> [-d cuda] [-m completion|passkey|perplexity|batch] [-T ctx] [-i prompt | -f file] [-n steps] [-l pos] [-g gpus] [-b seqs]
 //
 // Same flags, same prefix matching for -m/-d, same defaults (mode completion, -n 128, the default prompt), same stats
 // block, plus the roofline fraction.  Differences, on purpose:
@@ -37,12 +37,14 @@ namespace {
 	fprintf(stderr, "Options:\n");
 	fprintf(stderr, "  -h Display this help message\n");
 	fprintf(stderr, "  -d [cuda] which device to use (default - cuda; this build has no cpu path)\n");
-	fprintf(stderr, "  -m [completion,passkey,perplexity] which mode to run in (default - completion)\n");
+	fprintf(stderr, "  -m [completion,passkey,perplexity,batch] which mode to run in (default - completion)\n");
 	fprintf(stderr, "  -T <int> sliding window context length (0 - max)\n");
 	fprintf(stderr, "  -g <int> number of GPUs to run tensor-parallel on (default - 1; not with -m verify)\n");
 	fprintf(stderr, "\nPerplexity mode options:\n  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
 	fprintf(stderr, "Completion mode options:\n  -n <int>    number of steps to run for in completion mode, default 128. 0 = max_seq_len, -1 = infinite\n");
 	fprintf(stderr, "  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
+	fprintf(stderr, "Batch mode options (one GPU; integer block formats):\n  -f <filepath> prompts, one per non-empty line\n"
+	                "  -b <int>    sequences decoded together (1..8, default 8)\n  -n <int>    tokens per prompt, default 128. 0 = max_seq_len\n");
 	fprintf(stderr, "Passkey mode options:\n  -n <int>    number of junk lines to insert (default - 250)\n  -l <int>    passkey position (-1 - random)\n");
 	exit(1);
 }
@@ -61,6 +63,39 @@ void to_device(Model& model, const TpRank& tp) { model.cuda(tp.device, tp.rank, 
 // Under tensor parallelism: which GPUs, and how many kernels one decode token takes (this shows which exchange path runs).
 void print_tp_stats(const TpRank& tp, int launches) {
 	if (tp.size > 1) printf("  tensor parallel: %d GPUs, %d launches/token\n", tp.size, launches);
+}
+
+// Hydrate the KV cache with a prompt (main.cpp:94-100) and leave the last position's logits in `state`.  The reference walks the
+// prompt token by token; here the part of the prompt that fits the cache without wrapping goes through ONE batched pass (tcgen05
+// GEMMs), the part past the context window through batched passes over the KV ring, and whatever those refuse (e.g. a head_dim
+// the batched attention does not take) through the same loop.  The chunk sizes depend on the prompt and the config only, and a
+// refusal is agreed between the ranks (xalm_cuda.h), so under -g every rank makes the same calls and falls back at the same
+// position.  Returns the bytes the calls streamed (Model::active_bytes per pass).
+size_t hydrate(const Model& model, const InferenceState& state, const std::vector<int>& encoding) {
+	size_t read_bytes = 0;
+	size_t pos = 0;
+	if (getenv("XALM_NO_PREFILL") == nullptr && encoding.size() > 1) {
+		const size_t W = (size_t) model.config.max_seq_len;
+		const size_t n = std::min(encoding.size(), W);
+		const InferenceMode mode = n == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
+		if (model.prefill(state, encoding.data(), (int) n, 0, mode)) {
+			read_bytes += model.active_bytes(n - 1); // the weights are streamed once for the whole batch
+			pos = n;
+		}
+		while (pos >= W && pos < encoding.size()) {
+			const size_t c = std::min({encoding.size() - pos, W - 2, (size_t) 4096});
+			const InferenceMode cmode = pos + c == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
+			if (!model.prefill_window(state, encoding.data() + pos, (int) c, (int) pos, cmode)) break;
+			read_bytes += model.active_bytes(pos + c - 1);
+			pos += c;
+		}
+	}
+	for (; pos < encoding.size(); pos++) {
+		const InferenceMode mode = pos + 1 == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
+		model.forward(state, encoding[pos], (int) pos, mode);
+		read_bytes += model.active_bytes(pos);
+	}
+	return read_bytes;
 }
 
 void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps) {
@@ -86,34 +121,7 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	       encoding.size() / enc_s, enc_s / encoding.size(), enc_s);
 
 	t0 = now_s();
-	size_t read_bytes = 0;
-	// hydrate the KV cache (main.cpp:94-100).  The reference walks the prompt token by token; here the part of the prompt
-	// that fits the cache without wrapping goes through ONE batched pass (tcgen05 GEMMs), the part past the context window
-	// through batched passes over the KV ring, and whatever those refuse (e.g. a head_dim the batched attention does not take)
-	// through the same loop.  The chunk sizes depend on the prompt and the config only, and a refusal is agreed between the
-	// ranks (xalm_cuda.h), so under -g every rank makes the same calls and falls back at the same position.
-	size_t pos = 0;
-	if (getenv("XALM_NO_PREFILL") == nullptr && encoding.size() > 1) {
-		const size_t W = (size_t) model.config.max_seq_len;
-		const size_t n = std::min(encoding.size(), W);
-		const InferenceMode mode = n == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
-		if (model.prefill(state, encoding.data(), (int) n, 0, mode)) {
-			read_bytes += model.active_bytes(n - 1); // the weights are streamed once for the whole batch
-			pos = n;
-		}
-		while (pos >= W && pos < encoding.size()) {
-			const size_t c = std::min({encoding.size() - pos, W - 2, (size_t) 4096});
-			const InferenceMode cmode = pos + c == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
-			if (!model.prefill_window(state, encoding.data() + pos, (int) c, (int) pos, cmode)) break;
-			read_bytes += model.active_bytes(pos + c - 1);
-			pos += c;
-		}
-	}
-	for (; pos < encoding.size(); pos++) {
-		const InferenceMode mode = pos + 1 == encoding.size() ? InferenceMode::OUTPUT_LOGITS : InferenceMode::HYDRATE_KV_CACHE;
-		model.forward(state, encoding[pos], (int) pos, mode);
-		read_bytes += model.active_bytes(pos);
-	}
+	size_t read_bytes = hydrate(model, state, encoding);
 	const double hydrate_s = now_s() - t0;
 	for (int i = 0; i < num_steps || num_steps == -1; i++) { // main.cpp:105-115
 		// the logits are all-gathered under -g, so every rank picks the same token and stops at the same step
@@ -132,6 +140,88 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	       "  roofline: %.1f%% of %.0f GB/s HBM\n  total: %.5gs\n",
 	       encoding.size(), encoding.size() / elapsed_s, elapsed_s / encoding.size(), hydrate_s, gbs, 100.0 * gbs / peak, peak, elapsed_s);
 	print_tp_stats(tp, launches);
+}
+
+// -m batch: every non-empty line of the prompt file is one prompt; up to `max_batch` of them decode together on one batched handle,
+// greedy, with continuous batching: when a sequence ends (eos / eot or num_steps tokens) the next prompt is hydrated into its slot
+// (select_seq + the completion mode's hydrate) and joins the following step.  Each sequence's tokens are what -m completion
+// produces for that prompt (the batched matvec is bit-identical to the single-sequence tensor-core kernel).
+void run_batch(const std::string& checkpoint_path, const std::vector<std::string>& prompts, int context, int num_steps, int max_batch) {
+	auto model_data = Xalm::load(checkpoint_path);
+	std::cout << "loading model " << checkpoint_path << std::endl;
+	Model model = Model::from_xalm(model_data, context, /*defer_load=*/true);
+	const int B = std::max(1, std::min(max_batch, (int) prompts.size()));
+	std::cout << "Using CUDA, " << B << " sequence slots" << std::endl;
+	model.cuda(0, 0, 1, nullptr, {}, std::max(B, 2)); // a batched handle even when one slot is enough
+	InferenceState state(model.config);
+	state.cuda();
+	Sampler sampler(model.config);
+	Tokenizer tokenizer(model_data);
+	if (num_steps == 0) num_steps = model.config.max_seq_len;
+	// bytes of one cached position (K and V of every layer) and of the weights alone, for the bandwidth figure
+	const size_t kv_row = model.config.max_seq_len > 1 ? model.active_bytes(1) - model.active_bytes(0) : 0;
+	const size_t weights = model.active_bytes(0) - kv_row;
+
+	struct Seq {
+		int prompt = -1;  // -1: slot idle
+		std::vector<int> enc;
+		int generated = 0;
+	};
+	std::vector<Seq> slot(B);
+	std::vector<std::string> text(prompts.size());
+	size_t next_prompt = 0, generated = 0, read_bytes = 0, steps = 0, seq_steps = 0;
+	double hydrate_s = 0.0;
+	const double t0 = now_s();
+	// emit the sequence's next token (as run_completion prints it); true when the sequence has ended
+	auto emit = [&](Seq& q, int token) {
+		text[q.prompt] += tokenizer.decode_one(q.enc.back(), token);
+		q.enc.push_back(token);
+		q.generated++;
+		generated++;
+		return token == tokenizer.eos_id || token == tokenizer.eot_id || q.generated == num_steps;
+	};
+	// hydrate the next prompt into slot s and emit its first token; prompts that end at once free the slot for the next one
+	auto start = [&](int s) {
+		slot[s].prompt = -1;
+		while (next_prompt < prompts.size()) {
+			Seq& q = slot[s];
+			q = Seq{(int) next_prompt, tokenizer.encode(prompts[next_prompt], true), 0};
+			next_prompt++;
+			const double h0 = now_s();
+			model.select_seq(s);
+			read_bytes += hydrate(model, state, q.enc);
+			hydrate_s += now_s() - h0;
+			if (!emit(q, sampler.sample_argmax(state))) return;
+			q.prompt = -1;
+		}
+	};
+	for (int s = 0; s < B; s++) start(s);
+	std::vector<int> seqs, toks, pos, nxt(B);
+	for (;;) {
+		seqs.clear(); toks.clear(); pos.clear();
+		for (int s = 0; s < B; s++)
+			if (slot[s].prompt >= 0) {
+				seqs.push_back(s);
+				toks.push_back(slot[s].enc.back());
+				pos.push_back((int) slot[s].enc.size() - 1);
+			}
+		if (seqs.empty()) break;
+		const int n = (int) seqs.size();
+		model.forward_batch_argmax(n, seqs.data(), toks.data(), pos.data(), nxt.data());
+		steps++;
+		seq_steps += n;
+		read_bytes += weights;
+		for (int i = 0; i < n; i++) read_bytes += std::min((size_t) pos[i] + 1, (size_t) model.config.max_seq_len) * kv_row;
+		for (int i = 0; i < n; i++)
+			if (emit(slot[seqs[i]], nxt[i])) start(seqs[i]);
+	}
+	const double elapsed_s = now_s() - t0;
+	for (size_t i = 0; i < prompts.size(); i++) printf("[prompt %zu]\n%s\n", i, text[i].c_str());
+	const double gbs = (double) read_bytes / 1e9 / elapsed_s;
+	printf("\nBatch stats:\n  %zu prompts\n  %zu generated tokens\n  throughput: %.5gtok/s\n  hydrate: %.5gs\n  mean sequences per step: %.3g\n"
+	       "  bandwidth: %.5gGB/s\n  roofline: %.1f%% of %.0f GB/s HBM\n  total: %.5gs\n",
+	       prompts.size(), generated, generated / elapsed_s, hydrate_s, steps ? (double) seq_steps / steps : 0.0, gbs, 100.0 * gbs / hbm_peak_gbs(),
+	       hbm_peak_gbs(), elapsed_s);
 }
 
 void run_perplexity(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context) {
@@ -279,7 +369,7 @@ int main(int argc, char* argv[]) {
 	std::string prompt = "Q: What is the meaning of life? A:"; // main.cpp:421
 	std::string prompt_path;
 	std::string convert_type;
-	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1;
+	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8;
 	if (argc >= 2) checkpoint_path = argv[1];
 	else error_usage();
 	for (int i = 2; i < argc;) { // main.cpp:435-512
@@ -291,6 +381,7 @@ int main(int argc, char* argv[]) {
 			else if (is_prefix_of("passkey", v)) mode = "passkey";
 			else if (is_prefix_of("perplexity", v)) mode = "perplexity";
 			else if (is_prefix_of("verify", v)) mode = "verify";
+			else if (is_prefix_of("batch", v)) mode = "batch";
 			else error_usage();
 		} else if (f == 'd') {
 			if (is_prefix_of("cpu", v)) device = "cpu";
@@ -302,6 +393,10 @@ int main(int argc, char* argv[]) {
 		else if (f == 't') convert_type = v;
 		else if (f == 'l') passkey_pos = std::stoi(v);
 		else if (f == 'g') gpus = parse_gpus(v);
+		else if (f == 'b') {
+			max_batch = parse_gpus(v);
+			if (max_batch > 8) error_usage();
+		}
 		else if (f == 'n') { num_steps = std::stoi(v); n_junk = num_steps; }
 		else error_usage();
 		i += 2;
@@ -321,6 +416,25 @@ int main(int argc, char* argv[]) {
 	if (device != "cuda") {
 		fprintf(stderr, "Error: this binary is the CUDA backend; it carries no CPU forward pass (use the reference for -d cpu)\n");
 		return 1;
+	}
+	if (mode == "batch") {
+		if (gpus != 1 || num_steps < 0 || prompt_path.empty()) {
+			fprintf(stderr, "Error: -m batch runs on one GPU (no -g), needs -f <prompts> and -n >= 0\n");
+			error_usage();
+		}
+		std::ifstream file(prompt_path);
+		if (!file.is_open()) { std::cerr << "Error: could not open file " << prompt_path << std::endl; return 1; }
+		std::vector<std::string> prompts;
+		for (std::string line; std::getline(file, line);)
+			if (!line.empty()) prompts.push_back(line);
+		if (prompts.empty()) { std::cerr << "Error: no prompts in " << prompt_path << std::endl; return 1; }
+		try {
+			run_batch(checkpoint_path, prompts, context, num_steps, max_batch);
+		} catch (const std::exception& e) {
+			fprintf(stderr, "error: %s\n", e.what());
+			return 1;
+		}
+		return 0;
 	}
 	if (mode == "completion" || mode == "perplexity") {
 		if (!prompt_path.empty()) { // the reference's default prompt makes `-f` alone an error (main.cpp:513-517); -f simply wins here

@@ -315,10 +315,11 @@ Model Model::from_xalm(Xalm::file_info& xalm, const int context, const bool defe
 	return m;
 }
 
-void Model::cuda(int device_index, int tp_rank, int tp_size, const void* comm_id, const IpcExchange& ipc_exchange) {
+void Model::cuda(int device_index, int tp_rank, int tp_size, const void* comm_id, const IpcExchange& ipc_exchange, int max_seqs) {
 	if (handle_) return;
 	const xalm_config c = config.to_c();
 	if (xalm_cuda_create(&c, device_index, tp_rank, tp_size, &handle_) != XALM_OK) xalm_throw_last("model.cuda()");
+	if (max_seqs != 1 && xalm_cuda_set_batch(handle_, max_seqs) != XALM_OK) xalm_throw_last("model.cuda()");
 	if (tp_size > 1) {
 		if (!comm_id) throw std::invalid_argument("model.cuda(): tensor parallel needs a communicator id");
 		if (xalm_cuda_comm_init(handle_, comm_id) != XALM_OK) xalm_throw_last("model.cuda()");
@@ -437,6 +438,22 @@ bool Model::prefill_call(const bool window, const InferenceState& s, const int* 
 		std::abort();
 	}
 	return true;
+}
+
+void Model::forward_batch(const int n, const int* seqs, const int* tokens, const int* pos, const InferenceMode mode, float* logits) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_batch: model is not on a CUDA device (call model.cuda())");
+	const int m = mode == InferenceMode::OUTPUT_LOGITS ? XALM_OUTPUT_LOGITS : XALM_HYDRATE_KV_CACHE;
+	if (xalm_cuda_forward_batch(handle_, n, seqs, tokens, pos, m, logits) != XALM_OK) xalm_throw_last("Model::forward_batch");
+}
+
+void Model::forward_batch_argmax(const int n, const int* seqs, const int* tokens, const int* pos, int* next) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_batch_argmax: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_forward_batch_argmax(handle_, n, seqs, tokens, pos, next) != XALM_OK) xalm_throw_last("Model::forward_batch_argmax");
+}
+
+void Model::select_seq(const int seq) const {
+	if (!handle_) throw std::runtime_error("Model::select_seq: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_select_seq(handle_, seq) != XALM_OK) xalm_throw_last("Model::select_seq");
 }
 
 // ---- Sampler (sampler.cpp:3-30) ----------------------------------------------------------------------------------

@@ -157,7 +157,9 @@ struct Model {
 	// model.cuda(): upload every tensor (sharded for tp_size > 1), release the host copies, finalize.  With tp_size > 1 and an
 	// ipc_exchange, the ranks also swap CUDA IPC handles (after the communicator, before the uploads), which enables the fused
 	// peer-memory exchange; without one the decode exchange is ncclAllReduce.
-	void cuda(int device_index = 0, int tp_rank = 0, int tp_size = 1, const void* comm_id = nullptr, const IpcExchange& ipc_exchange = {});
+	// max_seqs > 1: a batched handle with that many sequence slots (xalm_cuda_set_batch; one GPU, integer block formats only).
+	void cuda(int device_index = 0, int tp_rank = 0, int tp_size = 1, const void* comm_id = nullptr, const IpcExchange& ipc_exchange = {},
+	          int max_seqs = 1);
 	[[nodiscard]] size_t active_bytes(size_t pos) const;
 	// Kernels launched by the last forward / prefill call (xalm_cuda_last_launch_count).
 	[[nodiscard]] int last_launch_count() const;
@@ -175,6 +177,14 @@ struct Model {
 	// tensor parallelism, as prefill().
 	bool prefill_window(const InferenceState& s, const int* tokens, int n, int pos0, InferenceMode mode = InferenceMode::OUTPUT_LOGITS,
 	                    const int* targets = nullptr, float* probs = nullptr) const;
+
+	// Batched decode on a max_seqs > 1 handle: one step of n sequences, slot seqs[i] takes tokens[i] at pos[i]
+	// (xalm_cuda_forward_batch).  OUTPUT_LOGITS fills logits with n x vocab_size floats (may be null).  A refused call throws.
+	void forward_batch(int n, const int* seqs, const int* tokens, const int* pos, InferenceMode mode, float* logits) const;
+	// forward_batch + Sampler::sample_argmax of every row on the device: next[i] for seqs[i].
+	void forward_batch_argmax(int n, const int* seqs, const int* tokens, const int* pos, int* next) const;
+	// The slot forward / prefill / prefill_window work on (default 0): how a prompt is hydrated into a slot.
+	void select_seq(int seq) const;
 
 private:
 	explicit Model(const Config& c) : config(c) {}

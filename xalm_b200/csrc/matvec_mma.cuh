@@ -45,10 +45,16 @@ struct XmView {
 __host__ __device__ inline size_t xm_bytes(int n) { return ((size_t) 3 * (n + 16) + (size_t) (n / 32) * 64 + 127) / 128 * 128; }
 __device__ __forceinline__ XmView xm_view(uint8_t* base, int n) { return {base, reinterpret_cast<int4*>(base + (size_t) 3 * (n + 16)), n + 16}; }
 
+// one group of eight elements quantised: the three limb words of each half, the block's limb sums (s0 = low limb, u = mid | high
+// << 16, summed over the four lanes of the block) and the block exponent dx
+struct XmGroup {
+	uint32_t w[3][2];
+	uint32_t s0, u;
+	float dx;
+};
+
 // eight consecutive elements per lane, the four lanes 4k .. 4k+3 of a warp share a block (call with all lanes of the warp)
-// (lanes past the end of the vector pass valid = false and take part in the shuffles only)
-template <int BIAS>
-__device__ __forceinline__ void xm_store_group8(const XmView& v, int grp, const float (&x)[8], bool valid = true) {
+__device__ __forceinline__ void xm_quant_group8(const float (&x)[8], XmGroup& o) {
 	uint32_t mb = 0;
 #pragma unroll
 	for (int e = 0; e < 8; e++) mb = max(mb, __float_as_uint(x[e]) & 0x7fffffffu);
@@ -58,7 +64,6 @@ __device__ __forceinline__ void xm_store_group8(const XmView& v, int grp, const 
 	const bool live = eb >= 40 && eb < 255; // as idp.cuh: blocks below 2^-87 contribute nothing, non-finite blocks are dropped
 	const float sc = live ? __uint_as_float((uint32_t) (276 - eb) << 23) : 0.f;
 	const float dx = live ? __uint_as_float((uint32_t) (eb - 22) << 23) : 0.f;
-	uint32_t w[3][2];
 	uint32_t s0 = 0, s1 = 0, s2 = 0;
 #pragma unroll
 	for (int q = 0; q < 2; q++) {
@@ -69,18 +74,31 @@ __device__ __forceinline__ void xm_store_group8(const XmView& v, int grp, const 
 		for (int k = 0; k < 3; k++) {
 			const uint32_t sel = (uint32_t) k | ((uint32_t) (4 + k) << 4);
 			const uint32_t lo = prmt((uint32_t) X[0], (uint32_t) X[1], sel), hi = prmt((uint32_t) X[2], (uint32_t) X[3], sel);
-			w[2 - k][q] = prmt(lo, hi, 0x5410u);
+			o.w[2 - k][q] = prmt(lo, hi, 0x5410u);
 		}
-		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s0) : "r"(w[0][q]), "r"(0x01010101u));
-		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s1) : "r"(w[1][q]), "r"(0x01010101u));
-		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s2) : "r"(w[2][q]), "r"(0x01010101u));
+		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s0) : "r"(o.w[0][q]), "r"(0x01010101u));
+		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s1) : "r"(o.w[1][q]), "r"(0x01010101u));
+		asm("dp4a.u32.u32 %0, %1, %2, %0;" : "+r"(s2) : "r"(o.w[2][q]), "r"(0x01010101u));
 	}
 	uint32_t u = s1 | (s2 << 16); // block totals <= 32 * 255 < 2^16
 	u += __shfl_xor_sync(0xffffffffu, u, 1);
 	u += __shfl_xor_sync(0xffffffffu, u, 2);
 	s0 += __shfl_xor_sync(0xffffffffu, s0, 1);
 	s0 += __shfl_xor_sync(0xffffffffu, s0, 2);
+	o.s0 = s0;
+	o.u = u;
+	o.dx = dx;
+}
+
+// (lanes past the end of the vector pass valid = false and take part in the shuffles only)
+template <int BIAS>
+__device__ __forceinline__ void xm_store_group8(const XmView& v, int grp, const float (&x)[8], bool valid = true) {
+	XmGroup o;
+	xm_quant_group8(x, o);
 	if (!valid) return;
+	const uint32_t(&w)[3][2] = o.w;
+	const uint32_t s0 = o.s0, u = o.u;
+	const float dx = o.dx;
 #pragma unroll
 	for (int k = 0; k < 3; k++) *reinterpret_cast<uint2*>(v.q + (size_t) k * v.ps + (size_t) grp * 8) = make_uint2(w[k][0], w[k][1]);
 	if ((grp & 3) == 0) {
@@ -381,6 +399,8 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_kernel(const
 		}
 	}
 	// ---- stage activations: quantise(NORM ? x * g : x); the scalar 1/rms is applied to the row sums (y = scale * sum w (x g)) ----
+	//      xq_batch_kernel repeats this loop (thread -> group map, norm-weight decode, sum-of-squares order) and the epilogue warp's
+	//      1/rms expression: batched decode is bit-identical to this kernel only while the two stay the same ----
 	const XmView xv = xm_view(smem, n);
 	float ss = 0.f;
 	{
@@ -522,6 +542,383 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_kernel(const
 		if (lane == 0) mbar_arrive(&pbar[pb]); // (release: this warp's partial sums are visible to whoever completes the wait)
 	}
 	tl_mark(tl, 3);
+}
+
+// =============================================================================================================================
+// Batched decode: up to 8 independent sequences per pass over the weights.
+//
+// Column packing.  The B operand has 8 columns and one sequence needs 4 (three limbs and the ones column), so a PAIR of sequences
+// shares one mma: sequence 2p in columns 0-3, sequence 2p+1 in columns 4-7.  The lanes with tig 0, 1 then accumulate sequence 2p
+// and the lanes with tig 2, 3 sequence 2p+1, each exactly as tig 0, 1 do in matvec_mma_kernel (same records in the same per-lane
+// order, same c-init values, same float operations).  The quad reduction adds the two lanes of a sequence (xor 1) and then +0,
+// which is what the batch-1 kernel's second shuffle adds from its zero columns; the epilogue warp adds the 16 warps' partial
+// sums in the same order.  So each sequence's outputs are bit-identical to the batch-1 kernel's, whatever shares the step.
+//
+// Activation staging.  One CTA cannot hold eight staged copies of a 14336-element row (5 bytes per element each).  Instead
+// xq_batch_kernel quantises every sequence ONCE per matvec into an image in global memory (it stays in L2), laid out by block and
+// pair: MMB_PAIR bytes per (32-element block, pair) = the three limb planes of each of the two sequences (32 bytes each) and the
+// four 16-byte table entries of the pair's lanes tig 0-3.  The producer bulk-copies a stage's slice of the image into the ring
+// next to the stage's weight records, so shared memory no longer grows with n.  The same kernel computes each sequence's 1/rms
+// with the batch-1 kernel's reduction order (512 threads, the same thread -> group map, warp shuffles, 16 warp sums in order).
+// =============================================================================================================================
+constexpr int MMB_PAIR = 256; // image bytes per (block, pair)
+constexpr int MMB_SB = 32;    // records per ring stage (any multiple of MMA_NCW keeps each lane's record order)
+constexpr int MMB_MAX_SEQS = 8;
+
+struct XqArgs {
+	const float* x;         // (nseq, x_stride) activations
+	int x_stride, n, nseq, np; // np = pairs in the image
+	const uint8_t* norm_w;  // nullptr = no norm
+	int norm_type;
+	float norm_eps;
+	uint8_t* img;           // (n / 32, np, MMB_PAIR)
+	float* nscale;          // (nseq,) 1/rms per sequence (norm only)
+};
+
+// One CTA of MMA_NT threads per sequence.  The staging loop below (thread -> group map, norm-weight decode, the order of the sum of
+// squares) and the 1/rms expression are those of matvec_mma_kernel's staging and epilogue warp: each sequence's image and 1/rms
+// are then bit-identical to what the batch-1 kernel stages.  Edit both together.
+template <int BIAS, bool NORM>
+__global__ void __launch_bounds__(MMA_NT) xq_batch_kernel(const XqArgs q) {
+	constexpr int NT = MMA_NT, MP = MMA_MP;
+	__shared__ float s_red[MMA_NCW];
+	pdl_launch_dependents();
+	pdl_wait();
+	const int s = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+	const int n = q.n, ngrp = n / 8;
+	const float* x = q.x + (size_t) s * q.x_stride;
+	uint8_t* mine = q.img + (size_t) (s >> 1) * MMB_PAIR + (s & 1) * 96; // this sequence's limb planes inside a (block, pair) record
+	float ss = 0.f;
+	for (int base = 0; base < ngrp; base += MP * NT) {
+		float xr[MP][8];
+		uint4 gw[MP][2];
+#pragma unroll
+		for (int p = 0; p < MP; p++) {
+			const int grp = base + p * NT + tid;
+			if (grp < ngrp) {
+				const float4 q0 = ld_act4(x + grp * 8), q1 = ld_act4(x + grp * 8 + 4);
+				xr[p][0] = q0.x; xr[p][1] = q0.y; xr[p][2] = q0.z; xr[p][3] = q0.w;
+				xr[p][4] = q1.x; xr[p][5] = q1.y; xr[p][6] = q1.z; xr[p][7] = q1.w;
+				if (NORM) {
+					if (q.norm_type == XALM_F32) {
+						gw[p][0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(q.norm_w) + grp * 8);
+						gw[p][1] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(q.norm_w) + grp * 8 + 4);
+					} else {
+						gw[p][0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(q.norm_w) + grp * 8);
+					}
+				}
+			} else {
+#pragma unroll
+				for (int e = 0; e < 8; e++) xr[p][e] = 0.f;
+			}
+		}
+#pragma unroll
+		for (int p = 0; p < MP; p++) {
+			const int grp = base + p * NT + tid;
+			if (base + p * NT + warp * 32 < ngrp) { // warp-uniform: the quantiser shuffles within quads of lanes
+				const bool valid = grp < ngrp;
+				if (NORM && valid) {
+#pragma unroll
+					for (int e = 0; e < 8; e++) {
+						ss += xr[p][e] * xr[p][e];
+						float g;
+						if (q.norm_type == XALM_F32) {
+							const uint4 w = gw[p][e >> 2];
+							g = __uint_as_float((e & 3) == 0 ? w.x : (e & 3) == 1 ? w.y : (e & 3) == 2 ? w.z : w.w);
+						} else {
+							const uint4 w = gw[p][0];
+							const int h = e >> 1;
+							const uint32_t u = h == 0 ? w.x : h == 1 ? w.y : h == 2 ? w.z : w.w;
+							g = __uint_as_float((e & 1) ? (u & 0xFFFF0000u) : (u << 16));
+						}
+						xr[p][e] = xr[p][e] * g;
+					}
+				}
+				XmGroup o;
+				xm_quant_group8(xr[p], o);
+				if (valid) {
+					uint8_t* rec = mine + (size_t) (grp >> 2) * q.np * MMB_PAIR;
+#pragma unroll
+					for (int k = 0; k < 3; k++) *reinterpret_cast<uint2*>(rec + k * 32 + (grp & 3) * 8) = make_uint2(o.w[k][0], o.w[k][1]);
+					if ((grp & 3) == 0) { // this sequence's two table entries (lanes tig 0, 1 of its half of the pair)
+						const int S0 = (int) o.s0, S1 = (int) (o.u & 0xFFFFu), S2 = (int) (o.u >> 16);
+						const int tot = (S0 - 4096) * 65536 + S1 * 256 + S2;
+						const float sx = __int2float_rn(tot) * o.dx;
+						int4* e = reinterpret_cast<int4*>(rec - (s & 1) * 96 + 192 + (s & 1) * 32);
+						e[0] = make_int4(-BIAS * S2, -BIAS * S1, (int) __float_as_uint(o.dx), (int) __float_as_uint(sx));
+						e[1] = make_int4(-BIAS * (S0 - 4096), 0, (int) __float_as_uint(o.dx * 65536.f), 0);
+					}
+				}
+			}
+		}
+	}
+	if (NORM) {
+		ss = warp_sum(ss);
+		if (lane == 0) s_red[warp] = ss;
+		__syncthreads();
+		if (tid == 0) {
+			float tot = 0.f;
+#pragma unroll
+			for (int i = 0; i < MMA_NCW; i++) tot += s_red[i];
+			q.nscale[s] = 1.0f / sqrtf(tot / (float) n + q.norm_eps); // infer.cpp:229-232
+		}
+	}
+}
+
+__host__ __device__ inline size_t mmb_stage_bytes(int type, int np) { return (size_t) MMB_SB * (frag_record_bytes(type) + (size_t) np * MMB_PAIR); }
+__host__ __device__ inline size_t mmb_smem_bytes(int type, int np, int NS) {
+	size_t s = (size_t) NS * mmb_stage_bytes(type, np);
+	s += (size_t) mma_pb(NS) * MMA_NCW * (2 * np) * MMA_RC * sizeof(float);
+	s += (2 * (size_t) NS + 2 * mma_pb(NS)) * sizeof(uint64_t);
+	return s + 128;
+}
+
+struct MmbArgs {
+	MatvecArgs a;          // a.step = the step's StepParams array (one per sequence), a.k_cache / a.v_cache = slot 0's caches
+	int NS, n_tiles, nseq;
+	const uint8_t* img;    // xq_batch_kernel's image of the input activations
+	const float* nscale;   // per-sequence 1/rms, or nullptr
+	int out_stride;        // floats between two sequences' outputs
+	size_t kv_slot;        // elements between two slots' caches
+};
+
+template <int TYPE, int NP>
+__global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_batch_kernel(const MmbArgs ta) {
+	using F = MmaFmt<TYPE>;
+	constexpr int RC = MMA_RC, SB = MMB_SB, NCW = MMA_NCW, NT = MMA_NT, RB = F::RB, NS2 = 2 * NP;
+	constexpr int WB = SB * RB, XB = SB * NP * MMB_PAIR, STAGE = WB + XB;
+	const MatvecArgs& a = ta.a;
+	const int NS = ta.NS, PB = mma_pb(ta.NS), nseq = ta.nseq;
+	const int n = a.n, nb = n / 32;
+	const int kranges = (nb + SB - 1) / SB;
+
+	extern __shared__ __align__(128) uint8_t smem[];
+	uint8_t* ring = smem;
+	float* part = reinterpret_cast<float*>(ring + (size_t) NS * STAGE); // [PB][NCW][NS2][RC]
+	uint64_t* full = reinterpret_cast<uint64_t*>(part + PB * NCW * NS2 * RC);
+	uint64_t* empty = full + NS;
+	uint64_t* pbar = empty + NS;
+	uint64_t* pfree = pbar + PB;
+
+	const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+	if (threadIdx.x == 0) {
+		for (int s = 0; s < NS; s++) {
+			mbar_init(&full[s], 1);
+			mbar_init(&empty[s], NCW);
+		}
+		for (int s = 0; s < PB; s++) {
+			mbar_init(&pbar[s], NCW);
+			mbar_init(&pfree[s], 1);
+		}
+		asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+	}
+	__syncthreads();
+	pdl_launch_dependents();
+
+	const int my_tiles = ((int) blockIdx.x < ta.n_tiles) ? (ta.n_tiles - 1 - (int) blockIdx.x) / (int) gridDim.x + 1 : 0;
+
+	if (warp == NCW) {
+		// ===================== producer: the first stages' weights before the dependency wait, the image slices after it =========
+		if (lane == 0) {
+			const int total = my_tiles * kranges;
+			auto wsrc = [&](int i, uint32_t* wbytes, uint32_t* xbytes, uint32_t* xoff) {
+				const int tt = i / kranges, kr = i % kranges;
+				const int nbs = min(SB, nb - kr * SB);
+				*wbytes = (uint32_t) nbs * RB;
+				*xbytes = (uint32_t) nbs * NP * MMB_PAIR;
+				*xoff = (uint32_t) kr * XB;
+				return a.w.p0 + (size_t) ((int) blockIdx.x + tt * (int) gridDim.x) * a.w.s0 + (size_t) kr * WB;
+			};
+			const int pre = min(NS, total);
+			for (int i = 0; i < pre; i++) {
+				uint32_t wb, xb, xo;
+				const uint8_t* src = wsrc(i, &wb, &xb, &xo);
+				mbar_expect_tx(&full[i], wb + xb);
+				bulk_g2s(ring + (size_t) i * STAGE, src, wb, &full[i]);
+			}
+			pdl_wait(); // the image is written by the kernel before this one
+			for (int i = 0; i < pre; i++) {
+				uint32_t wb, xb, xo;
+				wsrc(i, &wb, &xb, &xo);
+				bulk_g2s(ring + (size_t) i * STAGE + WB, ta.img + xo, xb, &full[i]);
+			}
+			for (int i = pre; i < total; i++) {
+				const int slot = i % NS, phase = (i / NS) & 1;
+				uint32_t wb, xb, xo;
+				const uint8_t* src = wsrc(i, &wb, &xb, &xo);
+				mbar_wait(&empty[slot], phase ^ 1);
+				mbar_expect_tx(&full[slot], wb + xb);
+				bulk_g2s(ring + (size_t) slot * STAGE, src, wb, &full[slot]);
+				bulk_g2s(ring + (size_t) slot * STAGE + WB, ta.img + xo, xb, &full[slot]);
+			}
+			l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
+		}
+		return;
+	}
+
+	if (warp == NCW + 1) {
+		// ===================== epilogue warp: two sequences per pass, lanes 0-15 and 16-31 each take the 16 rows of one =============
+		pdl_wait();
+		const int r = lane & (RC - 1);
+		int pb = 0, pph = 0;
+		for (int tt = 0; tt < my_tiles; tt++) {
+			const int row0 = ((int) blockIdx.x + tt * (int) gridDim.x) * RC;
+			float xold[NP];
+#pragma unroll
+			for (int ps = 0; ps < NP; ps++) {
+				const int s = 2 * ps + (lane >> 4);
+				xold[ps] = 0.f;
+				if (a.epi == EPI_RESIDUAL && s < nseq && row0 + r < a.d) xold[ps] = a.out[(size_t) s * ta.out_stride + row0 + r];
+			}
+			mbar_wait(&pbar[pb], pph);
+			const float* pt = part + pb * NCW * NS2 * RC;
+#pragma unroll
+			for (int ps = 0; ps < NP; ps++) {
+				const int s = 2 * ps + (lane >> 4);
+				const bool live = s < nseq;
+				float yv = 0.f;
+				if (live) {
+#pragma unroll
+					for (int w = 0; w < NCW; w++) yv += pt[(w * NS2 + s) * RC + r];
+					if (ta.nscale) yv *= ta.nscale[s];
+				}
+				const float ynext = __shfl_down_sync(0xffffffffu, yv, 1);
+				const float ypart = __shfl_down_sync(0xffffffffu, yv, RC / 2);
+				if (!live) continue;
+				float* out = a.out + (size_t) s * ta.out_stride;
+				const int row = row0 + r;
+				if (a.epi == EPI_RESIDUAL) {
+					if (row < a.d) out[row] = xold[ps] + yv;
+				} else if (a.epi == EPI_STORE) {
+					if (row < a.d) out[row] = yv;
+				} else if (a.epi == EPI_GLU) {
+					const int o = row0 / 2 + r;
+					if (r < RC / 2 && o < a.d) {
+						const float gt = a.act == XALM_SILU ? act_silu(yv) : act_gelu(yv);
+						out[o] = gt * ypart;
+					}
+				} else if ((r & 1) == 0 && row < a.d) { // EPI_QKV, as epilogue<2>: clip -> RoPE -> q fp32 / k, v fp16 into this slot's ring
+					const StepParams& sp = a.step[s];
+					const int pos = sp.pos, kv_pos = sp.kv_pos;
+					float v0 = clipf(yv, a.qkv_clip), v1 = clipf(ynext, a.qkv_clip);
+					if (row < a.q_dim) {
+						rope_pair(v0, v1, row % a.head_dim, pos, a.rope_freq);
+						out[row] = v0;
+						out[row + 1] = v1;
+					} else if (row < a.q_dim + a.kv_dim) {
+						const int i = row - a.q_dim;
+						rope_pair(v0, v1, i % a.head_dim, pos, a.rope_freq);
+						__half* kc = a.k_cache + (size_t) sp.slot * ta.kv_slot;
+						*reinterpret_cast<__half2*>(kc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
+					} else {
+						const int i = row - a.q_dim - a.kv_dim;
+						__half* vc = a.v_cache + (size_t) sp.slot * ta.kv_slot;
+						*reinterpret_cast<__half2*>(vc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
+					}
+				}
+			}
+			__syncwarp();
+			if (lane == 0) mbar_arrive(&pfree[pb]);
+			if (++pb == PB) { pb = 0; pph ^= 1; }
+		}
+		return;
+	}
+
+	// ===================== consumers =====================
+	pdl_wait();
+	if (a.epi == EPI_QKV && blockIdx.x == 0) { // re-rotate the attention sinks of every sequence past its window (infer.cpp:393-399)
+		const int pairs = a.kv_dim / 2;
+		for (int s = 0; s < nseq; s++) {
+			const int kv_sink = a.step[s].kv_sink;
+			__half* kc = a.k_cache + (size_t) a.step[s].slot * ta.kv_slot;
+			for (int i = threadIdx.x; i < kv_sink * pairs; i += NT) {
+				const int rr = i / pairs, p = i % pairs;
+				__half2* kp = reinterpret_cast<__half2*>(kc + (size_t) rr * a.kv_dim) + p;
+				float2 v = __half22float2(*kp);
+				rope_pair(v.x, v.y, (2 * p) % a.head_dim, 1, a.rope_freq);
+				*kp = __floats2half2_rn(v.x, v.y);
+			}
+		}
+	}
+
+	// this lane's place in the mma fragments: column g of the B operand is limb plane (2 - g) of sequence 2p (g < 3), the ones column
+	// (g = 3, 7) or limb plane (6 - g) of sequence 2p + 1 (4 <= g < 7); accumulator columns 2 tig, 2 tig + 1
+	const int g = lane >> 2, tig = lane & 3;
+	const int vmul = (tig & 1) ? -128 : 256;
+	const bool ones = (g & 3) == 3;
+	const int boff = (g < 4 ? (2 - g) * 32 : 96 + (6 - g) * 32) + tig * 4;
+	const int toff = 192 + tig * 16;
+
+	int slot = 0, phase = 0;
+	int pb_next = 0, pph_next = 0;
+	for (int tt = 0; tt < my_tiles; tt++) {
+		const int pb = pb_next, pph = pph_next;
+		if (++pb_next == PB) { pb_next = 0; pph_next ^= 1; }
+		float y0[NP], y1[NP]; // rows g and g + 8 of the tile, this lane's sequence of each pair
+#pragma unroll
+		for (int p = 0; p < NP; p++) y0[p] = y1[p] = 0.f;
+		for (int kr = 0; kr < kranges; kr++) {
+			const int nbs = min(SB, nb - kr * SB);
+			const uint8_t* st = ring + (size_t) slot * STAGE;
+			mbar_wait(&full[slot], phase);
+			auto record = [&](int j) {
+				const uint8_t* rec = st + (size_t) j * RB;
+				const uint8_t* xr = st + WB + (size_t) j * NP * MMB_PAIR;
+				uint32_t A[4];
+				float d0, d1, m0 = 0.f, m1 = 0.f;
+				F::load(rec, lane, g, A, d0, d1, m0, m1);
+#pragma unroll
+				for (int p = 0; p < NP; p++) {
+					const uint8_t* xp = xr + p * MMB_PAIR;
+					uint32_t B0 = 0x01010101u, B1 = 0x01010101u;
+					if (!ones) {
+						B0 = *reinterpret_cast<const uint32_t*>(xp + boff);
+						B1 = *reinterpret_cast<const uint32_t*>(xp + boff + 16);
+					}
+					const int4 tb = *reinterpret_cast<const int4*>(xp + toff);
+					int c[4];
+					mma_u8(c, A, B0, B1, tb.x, tb.y);
+					const int v0 = c[1] * vmul + c[0], v1 = c[3] * vmul + c[2];
+					const float dxl = __int_as_float(tb.z);
+					y0[p] = fmaf(__int2float_rn(v0), d0 * dxl, y0[p]);
+					y1[p] = fmaf(__int2float_rn(v1), d1 * dxl, y1[p]);
+					if (F::HAS_MIN) {
+						const float sxl = __int_as_float(tb.w);
+						y0[p] = fmaf(m0, sxl, y0[p]);
+						y1[p] = fmaf(m1, sxl, y1[p]);
+					}
+				}
+			};
+			if (nbs == SB) {
+#pragma unroll
+				for (int i = 0; i < SB / NCW; i++) record(warp + i * NCW);
+			} else {
+				for (int j = warp; j < nbs; j += NCW) record(j);
+			}
+			__syncwarp();
+			if (lane == 0) mbar_arrive(&empty[slot]);
+			if (++slot == NS) { slot = 0; phase ^= 1; }
+		}
+		// ---- the two lanes of a sequence -> one sum per row (+0: the batch-1 kernel's zero-column lanes), warps -> shared memory ----
+#pragma unroll
+		for (int p = 0; p < NP; p++) {
+			y0[p] += __shfl_xor_sync(0xffffffffu, y0[p], 1);
+			y1[p] += __shfl_xor_sync(0xffffffffu, y1[p], 1);
+			y0[p] = __fadd_rn(y0[p], 0.f);
+			y1[p] = __fadd_rn(y1[p], 0.f);
+		}
+		if (tt >= PB) mbar_wait(&pfree[pb], pph ^ 1);
+		if ((tig & 1) == 0) {
+#pragma unroll
+			for (int p = 0; p < NP; p++) {
+				float* pt = part + ((pb * NCW + warp) * NS2 + 2 * p + (tig >> 1)) * RC;
+				pt[g] = y0[p];
+				pt[g + 8] = y1[p];
+			}
+		}
+		__syncwarp();
+		if (lane == 0) mbar_arrive(&pbar[pb]);
+	}
 }
 
 } // namespace xalm

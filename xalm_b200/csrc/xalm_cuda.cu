@@ -412,6 +412,76 @@ static int launch_matvec_mma(const MatvecArgs& a, cudaStream_t s, bool pdl) {
 	return XALM_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// batched tensor-core matvec (matvec_mma.cuh): xq_batch_kernel quantises the nseq input rows once, then one pass over the weights
+// serves them all.  a.x / a.out hold one row per sequence (x_stride / out_stride floats apart), a.step the step's StepParams array.
+// ---------------------------------------------------------------------------------------------------------
+struct BatchIo {
+	int nseq, x_stride, out_stride;
+	uint8_t* img;       // activation image, (n / 32) x ceil(nseq / 2) x MMB_PAIR bytes
+	float* nscale;      // (nseq,) 1/rms
+	size_t kv_slot;
+};
+template <int BIAS>
+static cudaError_t launch_xq(const XqArgs& q, bool norm, cudaStream_t s, bool pdl) {
+	return norm ? launch(xq_batch_kernel<BIAS, true>, dim3(q.nseq), dim3(MMA_NT), s, pdl, q)
+	            : launch(xq_batch_kernel<BIAS, false>, dim3(q.nseq), dim3(MMA_NT), s, pdl, q);
+}
+template <int TYPE, int NP>
+static cudaError_t launch_mmb_inst(const MmbArgs& ta, size_t smem, cudaStream_t s, bool pdl) {
+	auto kern = matvec_mma_batch_kernel<TYPE, NP>;
+	cudaError_t e = ensure_smem_attr(kern, 227 * 1024);
+	if (e != cudaSuccess) return e;
+	int grid = num_sms();
+	if (grid > ta.n_tiles) grid = ta.n_tiles;
+	return launch_smem(kern, dim3(grid), dim3((MMA_NCW + 2) * 32), smem, s, pdl, ta);
+}
+template <int TYPE>
+static cudaError_t launch_mmb_typed(const MatvecArgs& a, const BatchIo& io, cudaStream_t s, bool pdl) {
+	const int np = (io.nseq + 1) / 2;
+	const int vrows = a.epi == EPI_GLU ? 2 * a.d : a.d;
+	XqArgs q = {};
+	q.x = a.x; q.x_stride = io.x_stride; q.n = a.n; q.nseq = io.nseq; q.np = np;
+	q.norm_w = a.norm_w; q.norm_type = a.norm_type; q.norm_eps = a.norm_eps; q.img = io.img; q.nscale = io.nscale;
+	cudaError_t e = launch_xq<MmaFmt<TYPE>::BIAS>(q, a.norm_w != nullptr, s, pdl);
+	if (e != cudaSuccess) return e;
+	int NS = 0;
+	for (int ns = 8; ns >= 2; ns--)
+		if (mmb_smem_bytes(TYPE, np, ns) <= 226 * 1024) { NS = ns; break; }
+	MmbArgs ta;
+	ta.a = a; ta.NS = NS; ta.n_tiles = vrows / MMA_RC; ta.nseq = io.nseq;
+	ta.img = io.img; ta.nscale = a.norm_w ? io.nscale : nullptr; ta.out_stride = io.out_stride; ta.kv_slot = io.kv_slot;
+	const size_t smem = mmb_smem_bytes(TYPE, np, NS);
+	switch (np) {
+		case 1: return launch_mmb_inst<TYPE, 1>(ta, smem, s, pdl);
+		case 2: return launch_mmb_inst<TYPE, 2>(ta, smem, s, pdl);
+		case 3: return launch_mmb_inst<TYPE, 3>(ta, smem, s, pdl);
+		case 4: return launch_mmb_inst<TYPE, 4>(ta, smem, s, pdl);
+	}
+	return cudaErrorInvalidValue;
+}
+// two launches: the quantiser and the matvec
+static int launch_matvec_batch(const MatvecArgs& a, const BatchIo& io, cudaStream_t s, bool pdl) {
+	const int t = a.w.type;
+	const int vrows = a.epi == EPI_GLU ? 2 * a.d : a.d;
+	if (!a.w.layout_frag || a.n % 32 || vrows % MMA_RC || vrows != a.w.rows || io.nseq < 1 || io.nseq > MMB_MAX_SEQS)
+		return set_error(XALM_ERR_STATE, "batched matvec: matrix not in fragment layout or bad shape (type=%d n=%d rows=%d nseq=%d)", t, a.n, vrows, io.nseq);
+	if (a.norm_w && a.norm_type != XALM_F32 && a.norm_type != XALM_BF16)
+		return set_error(XALM_ERR_UNSUPPORTED, "rmsnorm: unsupported data type %d", a.norm_type);
+	cudaError_t e;
+	switch (t) {
+		case XALM_Q8_0: e = launch_mmb_typed<XALM_Q8_0>(a, io, s, pdl); break;
+		case XALM_Q8: e = launch_mmb_typed<XALM_Q8>(a, io, s, pdl); break;
+		case XALM_Q4_0: e = launch_mmb_typed<XALM_Q4_0>(a, io, s, pdl); break;
+		case XALM_Q4_1: e = launch_mmb_typed<XALM_Q4_1>(a, io, s, pdl); break;
+		case XALM_Q5_0: e = launch_mmb_typed<XALM_Q5_0>(a, io, s, pdl); break;
+		case XALM_Q5_1: e = launch_mmb_typed<XALM_Q5_1>(a, io, s, pdl); break;
+		default: return set_error(XALM_ERR_STATE, "batched matvec: fragment layout with type %d", t);
+	}
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "batched matvec launch failed: %s", cudaGetErrorString(e));
+	return XALM_OK;
+}
+
 static int launch_matvec(MatvecArgs a, cudaStream_t s, bool pdl) {
 	const bool norm = a.norm_w != nullptr;
 	if (norm && a.norm_type != XALM_F32 && a.norm_type != XALM_BF16)
@@ -484,14 +554,24 @@ __global__ void embed_kernel(int type, const uint8_t* __restrict__ table, size_t
 	for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < dim; i += gridDim.x * blockDim.x) x[i] = decode_disk_elem(type, row, i);
 }
 
+// batched decode: one row per sequence (blockIdx.y), x is (nseq, dim)
+__global__ void embed_batch_kernel(int type, const uint8_t* __restrict__ table, size_t row_bytes, int dim, const StepParams* steps,
+                                   float* __restrict__ x) {
+	pdl_launch_dependents();
+	pdl_wait();
+	const uint8_t* row = table + (size_t) steps[blockIdx.y].token * row_bytes;
+	float* xs = x + (size_t) blockIdx.y * dim;
+	for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < dim; i += gridDim.x * blockDim.x) xs[i] = decode_disk_elem(type, row, i);
+}
+
 __global__ void dequant_kernel(int type, const uint8_t* __restrict__ src, size_t n, float* __restrict__ dst) {
 	for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < n; i += (size_t) gridDim.x * blockDim.x)
 		dst[i] = decode_disk_elem(type, src, i);
 }
 
 // Sampler::sample_argmax (sampler.cpp:3-16) on the device: running maximum seeded with FLT_MIN (the reference's quirk: with no
-// logit above 1.18e-38 the answer is 0), strict '>' so the FIRST maximum wins.  One CTA.
-__global__ void argmax_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) {
+// logit above 1.18e-38 the answer is 0), strict '>' so the FIRST maximum wins.  One CTA per row.
+__device__ __forceinline__ void argmax_row(const float* __restrict__ logits, int n, int* __restrict__ out) {
 	__shared__ float s_v[32];
 	__shared__ int s_i[32];
 	float best = 1.17549435e-38f; // numeric_limits<float>::min()
@@ -521,6 +601,11 @@ __global__ void argmax_kernel(const float* __restrict__ logits, int n, int* __re
 		}
 		if (threadIdx.x == 0) *out = bi >= n ? 0 : bi;
 	}
+}
+__global__ void argmax_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) { argmax_row(logits, n, out); }
+// batched decode: row b of (rows, n) logits -> out[b]
+__global__ void argmax_rows_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) {
+	argmax_row(logits + (size_t) blockIdx.x * n, n, out + blockIdx.x);
 }
 
 __global__ void residual_add_kernel(float* __restrict__ x, const float* __restrict__ y, int n) {
@@ -627,25 +712,28 @@ static std::vector<float> rope_freq_table(int head_dim, int rotary_dim, float th
 // ---------------------------------------------------------------------------------------------------------
 // attention dispatch
 // ---------------------------------------------------------------------------------------------------------
-template <int HD>
-static cudaError_t launch_attn_hd(const AttnArgs& a, int G, cudaStream_t s, bool pdl) {
-	dim3 grid(a.n_splits, a.n_kv_heads), block(256);
+template <int HD, bool BATCH>
+static cudaError_t launch_attn_hd(const AttnArgs& a, int G, int nseq, cudaStream_t s, bool pdl) {
+	dim3 grid(a.n_splits, a.n_kv_heads, nseq), block(256);
 	constexpr int NW8 = HD >= 256 ? 4 : 8; // 8 query heads x 256 dims: keep the per-warp partials within 48 KB of static smem
 	switch (G) {
-		case 1: return launch(attn_decode_kernel<HD, 1, 8>, grid, block, s, pdl, a);
-		case 2: return launch(attn_decode_kernel<HD, 2, 8>, grid, block, s, pdl, a);
-		case 4: return launch(attn_decode_kernel<HD, 4, 8>, grid, block, s, pdl, a);
-		case 8: return launch(attn_decode_kernel<HD, 8, NW8>, grid, dim3(NW8 * 32), s, pdl, a);
+		case 1: return launch(attn_decode_kernel<HD, 1, 8, BATCH>, grid, block, s, pdl, a);
+		case 2: return launch(attn_decode_kernel<HD, 2, 8, BATCH>, grid, block, s, pdl, a);
+		case 4: return launch(attn_decode_kernel<HD, 4, 8, BATCH>, grid, block, s, pdl, a);
+		case 8: return launch(attn_decode_kernel<HD, 8, NW8, BATCH>, grid, dim3(NW8 * 32), s, pdl, a);
 	}
 	return cudaErrorInvalidValue;
 }
-static int launch_attn(const AttnArgs& a, int head_dim, int G, cudaStream_t s, bool pdl) {
+// nseq > 0: the batched kernel, one grid layer per sequence (AttnArgs' batched fields); 0: one sequence
+static int launch_attn(const AttnArgs& a, int head_dim, int G, cudaStream_t s, bool pdl, int nseq = 0) {
 	cudaError_t e;
+	const bool b = nseq > 0;
+	const int z = b ? nseq : 1;
 	switch (head_dim) {
-		case 32: e = launch_attn_hd<32>(a, G, s, pdl); break;
-		case 64: e = launch_attn_hd<64>(a, G, s, pdl); break;
-		case 128: e = launch_attn_hd<128>(a, G, s, pdl); break;
-		case 256: e = launch_attn_hd<256>(a, G, s, pdl); break;
+		case 32: e = b ? launch_attn_hd<32, true>(a, G, z, s, pdl) : launch_attn_hd<32, false>(a, G, z, s, pdl); break;
+		case 64: e = b ? launch_attn_hd<64, true>(a, G, z, s, pdl) : launch_attn_hd<64, false>(a, G, z, s, pdl); break;
+		case 128: e = b ? launch_attn_hd<128, true>(a, G, z, s, pdl) : launch_attn_hd<128, false>(a, G, z, s, pdl); break;
+		case 256: e = b ? launch_attn_hd<256, true>(a, G, z, s, pdl) : launch_attn_hd<256, false>(a, G, z, s, pdl); break;
 		default: return set_error(XALM_ERR_UNSUPPORTED, "attention: head_dim %d not in {32,64,128,256}", head_dim);
 	}
 	if (e == cudaErrorInvalidValue && (G != 1 && G != 2 && G != 4 && G != 8))
@@ -692,15 +780,20 @@ struct WSlot {
 	bool allocated = false;
 };
 
-static int alloc_wmat(DevAlloc& da, WMat& m, int type, int rows, int n, int glu_half = 0, bool sharded = false) {
+// can the tensor-core matvec take this matrix (batch 1: its activations staged whole in shared memory)?
+static bool mma_takes(int type, int rows, int n, int glu_half) {
+	return mma_supported(type) && n % 32 == 0 && rows % MMA_RC == 0 && glu_half % 8 == 0 && mma_smem_bytes(type, n, 2) <= 226 * 1024;
+}
+
+// batched: the matrix goes to fragment tiles whatever the knobs say (the caller has checked mma_takes)
+static int alloc_wmat(DevAlloc& da, WMat& m, int type, int rows, int n, int glu_half = 0, bool sharded = false, bool batched = false) {
 	m.type = type; m.rows = rows; m.n = n; m.flags = 0; m.layout_units = 0; m.layout_frag = 0; m.glu_half = 0;
 	TypeInfo tinfo;
 	type_info(type, &tinfo);
 	// 2 (default): the 4/5-bit formats always; the 8-bit ones under tensor parallelism, where the per-rank rows are short (the dp4a kernel
 	// maps one 32-element block to a lane: rows of 512 elements keep 16 of its 256 lanes busy) — TP2 611 -> 637 tok/s
 	const bool mma_on = tune("mma") == 1 || (tune("mma") == 2 && (sharded || (type != XALM_Q8_0 && type != XALM_Q8)));
-	if (mma_supported(type) && n % 32 == 0 && rows % MMA_RC == 0 && glu_half % 8 == 0 && mma_on && tune("tma") &&
-	    mma_smem_bytes(type, n, 2) <= 226 * 1024) {
+	if (mma_takes(type, rows, n, glu_half) && (batched || (mma_on && tune("tma")))) {
 		// integer formats on the tensor-core path: fragment tiles (frag_layout.cuh); same byte count as on disk
 		m.layout_frag = 1;
 		m.glu_half = glu_half;
@@ -823,6 +916,16 @@ enum { P_ATT_NORM = 0, P_FFN_NORM, P_Q, P_K, P_V, P_O, P_GATE, P_DOWN, P_UP };
 struct xalm_cuda_model {
 	xalm_config c;
 	int device = 0, tp_rank = 0, tp_size = 1;
+	// batched decode (xalm_cuda_set_batch): max_seqs sequence slots, each with its own KV cache, slot_stride elements apart
+	int max_seqs = 1;
+	bool batched = false;
+	bool uploaded = false;
+	int cur_seq = 0;                  // the slot the single-sequence calls use (xalm_cuda_select_seq)
+	size_t kv_slot = 0;
+	uint8_t* ximg = nullptr;          // activation image of the batched matvec
+	float* nscale = nullptr;          // (max_seqs,) 1/rms of the batched matvec's norm prologue
+	std::map<int, cudaGraphExec_t> bgraph; // (mode, n) -> captured batched step
+	std::map<int, int> bgraph_launches;
 	// local (per-rank) sizes
 	int q_dim = 0, kv_dim = 0, q_dim_l = 0, kv_dim_l = 0, n_heads_l = 0, n_kv_heads_l = 0, hidden_l = 0, vocab_l = 0;
 	DevAlloc da;
@@ -966,6 +1069,7 @@ void xalm_cuda_destroy(xalm_cuda_model* m) {
 	cudaStreamSynchronize(m->stream);
 	for (int i = 0; i < 2; i++)
 		if (m->graph[i]) cudaGraphExecDestroy(m->graph[i]);
+	for (auto& kv : m->bgraph) cudaGraphExecDestroy(kv.second);
 	if (m->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(m->comm);
 	for (int i = 0; i < 64; i++)
 		if (m->h_step_ev_used[i]) cudaEventDestroy(m->h_step_ev[i]);
@@ -1154,6 +1258,7 @@ static int upload_impl(xalm_cuda_model* m, const char* name, int type_id, const 
 		elems = (size_t) (sr1 - sr0) * (sc1 - sc0);
 	}
 	if (nbytes != elems / ti.block * ti.bytes) return set_error(XALM_ERR_INVALID, "buffer size mismatch for %s: %zu vs %zu", name, nbytes, elems / ti.block * ti.bytes);
+	m->uploaded = true;
 	const uint8_t* host = (const uint8_t*) data;
 	// geometry of `host`: its rows are (sc1 - sc0) elements long and its first row / column is (sr0, sc0) of the tensor
 	auto put = [&](WMat& w, int dst_row, int r0, int r1, int c0, int c1) -> int {
@@ -1179,7 +1284,11 @@ static int upload_impl(xalm_cuda_model* m, const char* name, int type_id, const 
 			if (slot.m.type != type_id) return set_error(XALM_ERR_UNSUPPORTED, "%s: tensors fused into one matrix must share a type (%d vs %d)", name, type_id, slot.m.type);
 			return XALM_OK;
 		}
-		XALM_TRY(alloc_wmat(m->da, slot.m, type_id, rows, n, glu_half, m->tp_size > 1));
+		if (m->batched && !mma_takes(type_id, rows, n, glu_half))
+			return set_error(XALM_ERR_UNSUPPORTED, "%s%s: a batched handle takes only matrices the tensor-core matvec can (the six integer block "
+			                 "formats, rows a multiple of 16, input rows that fit the batch-1 kernel's shared memory); type %d, %d x %d", name,
+			                 piece == 100 ? " (tied classifier)" : "", type_id, rows, n);
+		XALM_TRY(alloc_wmat(m->da, slot.m, type_id, rows, n, glu_half, m->tp_size > 1, m->batched));
 		slot.total_rows = rows;
 		slot.allocated = true;
 		return XALM_OK;
@@ -1248,17 +1357,19 @@ static void fill_layer_args(xalm_cuda_model* m, int l, MatvecArgs* qkv, AttnArgs
 	const xalm_config& c = m->c;
 	LayerDev& L = m->layers[l];
 	const bool tp = m->tp_size > 1;
+	__half* k_cache = L.k_cache + (size_t) m->cur_seq * m->kv_slot;
+	__half* v_cache = L.v_cache + (size_t) m->cur_seq * m->kv_slot;
 	{ // attention pre-norm + q,k,v + clip + rope + KV write (+ sinks)
 		MatvecArgs a = {};
 		a.w = L.wqkv.m; a.x = m->x; a.n = c.dim; a.d = m->q_dim_l + 2 * m->kv_dim_l; a.epi = EPI_QKV;
 		a.norm_w = L.rms_att; a.norm_type = L.rms_att_type; a.norm_eps = c.norm_eps;
-		a.out = m->q; a.step = m->d_step; a.k_cache = L.k_cache; a.v_cache = L.v_cache; a.rope_freq = m->rope_freq;
+		a.out = m->q; a.step = m->d_step; a.k_cache = k_cache; a.v_cache = v_cache; a.rope_freq = m->rope_freq;
 		a.q_dim = m->q_dim_l; a.kv_dim = m->kv_dim_l; a.head_dim = c.head_dim; a.qkv_clip = c.qkv_clip;
 		*qkv = a;
 	}
 	{
 		AttnArgs a = {};
-		a.q = m->q; a.k_cache = L.k_cache; a.v_cache = L.v_cache; a.out = m->xb2; a.step = m->d_step; a.kv_len_fixed = -1;
+		a.q = m->q; a.k_cache = k_cache; a.v_cache = v_cache; a.out = m->xb2; a.step = m->d_step; a.kv_len_fixed = -1;
 		a.n_kv_heads = m->n_kv_heads_l; a.n_splits = m->attn_splits; a.min_split = tune("attn_min_split");
 		a.part_acc = m->attn_acc; a.part_ml = m->attn_ml; a.tickets = m->tickets;
 		*at = a;
@@ -1440,11 +1551,19 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 		XALM_CUDA_CHECK(cudaMemset(*p, 0, n * sizeof(float)));
 		return XALM_OK;
 	};
-	XALM_TRY(fzero(&m->x, c.dim));
-	XALM_TRY(fzero(&m->xb2, m->q_dim_l));
-	XALM_TRY(fzero(&m->hb, m->hidden_l));
-	XALM_TRY(fzero(&m->q, m->q_dim_l));
-	XALM_TRY(fzero(&m->logits, m->vocab_l));
+	// one row per sequence slot (the single-sequence calls use row 0)
+	const int S = m->max_seqs;
+	XALM_TRY(fzero(&m->x, (size_t) S * c.dim));
+	XALM_TRY(fzero(&m->xb2, (size_t) S * m->q_dim_l));
+	XALM_TRY(fzero(&m->hb, (size_t) S * m->hidden_l));
+	XALM_TRY(fzero(&m->q, (size_t) S * m->q_dim_l));
+	XALM_TRY(fzero(&m->logits, (size_t) S * m->vocab_l));
+	if (m->batched) {
+		const int nmax = std::max(c.dim, std::max(m->q_dim_l, m->hidden_l));
+		XALM_TRY(m->da.alloc((void**) &m->ximg, (size_t) nmax / 32 * ((S + 1) / 2) * MMB_PAIR));
+		XALM_CUDA_CHECK(cudaMemset(m->ximg, 0, (size_t) nmax / 32 * ((S + 1) / 2) * MMB_PAIR));
+		XALM_TRY(fzero(&m->nscale, S));
+	}
 	XALM_TRY(fzero(&m->part, c.dim));
 	XALM_TRY(fzero(&m->x_alt, c.dim));
 	XALM_TRY(m->da.alloc((void**) &m->xl, (size_t) 2 * c.dim * sizeof(uint2)));
@@ -1462,7 +1581,8 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 	} else {
 		m->logits_full = m->logits;
 	}
-	const size_t kv_elems = (size_t) c.max_seq_len * m->kv_dim_l;
+	m->kv_slot = (size_t) c.max_seq_len * m->kv_dim_l;
+	const size_t kv_elems = m->kv_slot * S;
 	for (auto& L : m->layers) {
 		XALM_TRY(m->da.alloc((void**) &L.k_cache, kv_elems * sizeof(__half)));
 		XALM_TRY(m->da.alloc((void**) &L.v_cache, kv_elems * sizeof(__half)));
@@ -1476,13 +1596,14 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 	m->attn_splits = attn_auto_splits(m->n_kv_heads_l);
 	// the last-CTA merge parks 3 floats per (split, head) in the 8 x G x head_dim floats of the per-warp partial area (attention.cuh)
 	if (m->attn_splits > 8 * c.head_dim / 3) m->attn_splits = 8 * c.head_dim / 3;
-	XALM_TRY(fzero(&m->attn_acc, (size_t) m->n_kv_heads_l * m->attn_splits * G * c.head_dim));
-	XALM_TRY(fzero(&m->attn_ml, (size_t) m->n_kv_heads_l * m->attn_splits * G * 2));
-	XALM_TRY(m->da.alloc((void**) &m->tickets, m->n_kv_heads_l * sizeof(unsigned int)));
-	XALM_CUDA_CHECK(cudaMemset(m->tickets, 0, m->n_kv_heads_l * sizeof(unsigned int)));
-	XALM_TRY(m->da.alloc((void**) &m->d_step, sizeof(StepParams)));
-	XALM_CUDA_CHECK(cudaMallocHost((void**) &m->h_step, 64 * sizeof(StepParams)));
-	XALM_CUDA_CHECK(cudaMallocHost((void**) &m->h_logits, (size_t) c.vocab_size * sizeof(float)));
+	XALM_TRY(fzero(&m->attn_acc, (size_t) S * m->n_kv_heads_l * m->attn_splits * G * c.head_dim));
+	XALM_TRY(fzero(&m->attn_ml, (size_t) S * m->n_kv_heads_l * m->attn_splits * G * 2));
+	XALM_TRY(m->da.alloc((void**) &m->tickets, S * m->n_kv_heads_l * sizeof(unsigned int)));
+	XALM_CUDA_CHECK(cudaMemset(m->tickets, 0, S * m->n_kv_heads_l * sizeof(unsigned int)));
+	XALM_TRY(m->da.alloc((void**) &m->d_step, S * sizeof(StepParams)));
+	XALM_CUDA_CHECK(cudaMallocHost((void**) &m->h_step, 64 * S * sizeof(StepParams)));
+	XALM_CUDA_CHECK(cudaMemset(m->d_step, 0, S * sizeof(StepParams)));
+	XALM_CUDA_CHECK(cudaMallocHost((void**) &m->h_logits, (size_t) S * c.vocab_size * sizeof(float)));
 	XALM_CUDA_CHECK(cudaMallocHost((void**) &m->h_err, 64));
 	memset(m->h_err, 0, 64);
 	XALM_TRY(m->da.alloc((void**) &m->d_argmax, 64));
@@ -1524,7 +1645,7 @@ int xalm_cuda_forward_async(xalm_cuda_model* m, int token, int pos, int mode) {
 	m->step_slot = (slot + 1) % 64;
 	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
 	else { XALM_CUDA_CHECK(cudaEventCreateWithFlags(&m->h_step_ev[slot], cudaEventDisableTiming)); m->h_step_ev_used[slot] = true; }
-	StepParams& sp = m->h_step[slot];
+	StepParams& sp = m->h_step[(size_t) slot * m->max_seqs];
 	sp.token = token; sp.pos = pos;
 	sp.kv_sink = pos >= c.max_seq_len ? 2 : 0;
 	sp.kv_pos = sp.kv_sink + (pos - sp.kv_sink) % (c.max_seq_len - sp.kv_sink);
@@ -1580,6 +1701,165 @@ int xalm_cuda_forward_argmax(xalm_cuda_model* m, int token, int pos, int* next_t
 	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
 	XALM_TRY(check_tp_error(m));
 	*next_token = *m->h_argmax;
+	return XALM_OK;
+}
+
+// ---- batched decode: several sequence slots, one pass over the weights per step ------------------------------------------
+int xalm_cuda_set_batch(xalm_cuda_model* m, int max_seqs) {
+	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
+	if (m->tp_size > 1) return set_error(XALM_ERR_UNSUPPORTED, "set_batch: batched decode runs on one GPU (tp_size %d)", m->tp_size);
+	if (m->uploaded || m->finalized) return set_error(XALM_ERR_STATE, "set_batch must precede the first upload");
+	if (max_seqs < 1 || max_seqs > MMB_MAX_SEQS) return set_error(XALM_ERR_INVALID, "set_batch: max_seqs %d not in [1, %d]", max_seqs, MMB_MAX_SEQS);
+	m->max_seqs = max_seqs;
+	m->batched = true;
+	return XALM_OK;
+}
+
+int xalm_cuda_select_seq(xalm_cuda_model* m, int seq) {
+	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
+	if (seq < 0 || seq >= m->max_seqs) return set_error(XALM_ERR_INVALID, "select_seq: slot %d not in [0, %d)", seq, m->max_seqs);
+	if (seq == m->cur_seq) return XALM_OK;
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+	for (int i = 0; i < 2; i++) // the single-sequence graphs hold the previous slot's cache pointers
+		if (m->graph[i]) { cudaGraphExecDestroy(m->graph[i]); m->graph[i] = nullptr; }
+	m->cur_seq = seq;
+	return XALM_OK;
+}
+
+static int enqueue_batch(xalm_cuda_model* m, int mode, int n, cudaStream_t s, int* n_launches) {
+	const xalm_config& c = m->c;
+	const bool pdl = tune("pdl") != 0;
+	const int G = c.n_heads / c.n_kv_heads;
+	int nl = 0;
+	cudaError_t e = launch(embed_batch_kernel, dim3(4, n), dim3(256), s, false, m->embed_type, (const uint8_t*) m->embed_raw, m->embed_row_bytes,
+	                       c.dim, (const StepParams*) m->d_step, m->x);
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "embed launch failed: %s", cudaGetErrorString(e));
+	nl++;
+	auto io = [&](int x_stride, int out_stride) { return BatchIo{n, x_stride, out_stride, m->ximg, m->nscale, m->kv_slot}; };
+	for (int l = 0; l < c.n_layers; l++) {
+		LayerDev& L = m->layers[l];
+		MatvecArgs a_qkv, a_wo, a_w13, a_w2;
+		AttnArgs a_at;
+		fill_layer_args(m, l, &a_qkv, &a_at, &a_wo, &a_w13, &a_w2);
+		a_qkv.k_cache = L.k_cache; a_qkv.v_cache = L.v_cache; // slot 0: the kernels add step[i].slot * kv_slot
+		a_at.k_cache = L.k_cache; a_at.v_cache = L.v_cache;
+		a_at.q_stride = m->q_dim_l; a_at.kv_slot = m->kv_slot;
+		if (const int pf_mb = tune("tail_prefetch_mb")) {
+			auto head = [&](const WMat& w, const uint8_t** ptr, unsigned long long* bytes) {
+				*ptr = w.p0;
+				*bytes = std::min<unsigned long long>((unsigned long long) w.s0 * (w.rows / MMA_RC), (unsigned long long) pf_mb << 20);
+			};
+			head(a_wo.w, &a_at.pf_ptr, &a_at.pf_bytes);
+			head(a_w13.w, &a_wo.pf_ptr, &a_wo.pf_bytes);
+			head(a_w2.w, &a_w13.pf_ptr, &a_w13.pf_bytes);
+			if (l + 1 < c.n_layers) head(m->layers[l + 1].wqkv.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
+			else if (mode == XALM_OUTPUT_LOGITS) head(m->wcls.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
+		}
+		XALM_TRY(launch_matvec_batch(a_qkv, io(c.dim, m->q_dim_l), s, pdl));
+		XALM_TRY(launch_attn(a_at, c.head_dim, G, s, pdl, n));
+		XALM_TRY(launch_matvec_batch(a_wo, io(m->q_dim_l, c.dim), s, pdl));
+		XALM_TRY(launch_matvec_batch(a_w13, io(c.dim, m->hidden_l), s, pdl));
+		XALM_TRY(launch_matvec_batch(a_w2, io(m->hidden_l, c.dim), s, pdl));
+		nl += 9;
+	}
+	if (mode == XALM_OUTPUT_LOGITS) {
+		MatvecArgs a = {};
+		a.w = m->wcls.m; a.x = m->x; a.n = c.dim; a.d = m->vocab_l; a.epi = EPI_STORE;
+		a.norm_w = m->rms_final; a.norm_type = m->rms_final_type; a.norm_eps = c.norm_eps; a.out = m->logits;
+		XALM_TRY(launch_matvec_batch(a, io(c.dim, m->vocab_l), s, pdl));
+		nl += 2;
+	}
+	if (n_launches) *n_launches = nl;
+	return XALM_OK;
+}
+
+static int ensure_bgraph(xalm_cuda_model* m, int mode, int n) {
+	const int key = mode * 16 + n;
+	if (m->bgraph.count(key)) return XALM_OK;
+	cudaStream_t s = m->stream;
+	cudaGraph_t g = nullptr;
+	XALM_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+	int nl = 0;
+	int rc = enqueue_batch(m, mode, n, s, &nl);
+	cudaError_t e = cudaStreamEndCapture(s, &g);
+	if (rc != XALM_OK) { if (g) cudaGraphDestroy(g); return rc; }
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(e));
+	cudaGraphExec_t ge = nullptr;
+	e = cudaGraphInstantiate(&ge, g, 0);
+	cudaGraphDestroy(g);
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
+	m->bgraph[key] = ge;
+	m->bgraph_launches[key] = nl;
+	return XALM_OK;
+}
+
+int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode) {
+	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "forward_batch before finalize");
+	if (!m->batched) return set_error(XALM_ERR_STATE, "forward_batch on a handle without xalm_cuda_set_batch");
+	if (mode != XALM_HYDRATE_KV_CACHE && mode != XALM_OUTPUT_LOGITS) return set_error(XALM_ERR_INVALID, "bad mode %d", mode);
+	if (n < 1 || n > m->max_seqs) return set_error(XALM_ERR_INVALID, "forward_batch: n = %d not in [1, %d]", n, m->max_seqs);
+	if (!seqs || !tokens || !pos) return set_error(XALM_ERR_INVALID, "NULL argument");
+	const xalm_config& c = m->c;
+	unsigned int seen = 0;
+	for (int i = 0; i < n; i++) {
+		if (seqs[i] < 0 || seqs[i] >= m->max_seqs) return set_error(XALM_ERR_INVALID, "forward_batch: slot %d not in [0, %d)", seqs[i], m->max_seqs);
+		if (seen & (1u << seqs[i])) return set_error(XALM_ERR_INVALID, "forward_batch: slot %d named twice", seqs[i]);
+		seen |= 1u << seqs[i];
+		if (tokens[i] < 0 || tokens[i] >= c.vocab_size) return set_error(XALM_ERR_INVALID, "token %d out of range [0,%d)", tokens[i], c.vocab_size);
+		if (pos[i] < 0) return set_error(XALM_ERR_INVALID, "negative position");
+	}
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	cudaStream_t s = m->stream;
+	const int slot = m->step_slot;
+	m->step_slot = (slot + 1) % 64;
+	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
+	else { XALM_CUDA_CHECK(cudaEventCreateWithFlags(&m->h_step_ev[slot], cudaEventDisableTiming)); m->h_step_ev_used[slot] = true; }
+	StepParams* sp = m->h_step + (size_t) slot * m->max_seqs;
+	for (int i = 0; i < n; i++) { // ring / sink index math per sequence: infer.cpp:611-613, KV_SINKS = 2 (model.h:10)
+		StepParams& p = sp[i];
+		p.token = tokens[i]; p.pos = pos[i];
+		p.kv_sink = pos[i] >= c.max_seq_len ? 2 : 0;
+		p.kv_pos = p.kv_sink + (pos[i] - p.kv_sink) % (c.max_seq_len - p.kv_sink);
+		p.kv_len = pos[i] >= c.max_seq_len ? c.max_seq_len : pos[i] + 1;
+		p.mode = mode;
+		p.ar_base = 0;
+		p.slot = seqs[i];
+	}
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, sp, (size_t) n * sizeof(StepParams), cudaMemcpyHostToDevice, s));
+	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], s));
+	if (tune("graph")) {
+		XALM_TRY(ensure_bgraph(m, mode, n));
+		XALM_CUDA_CHECK(cudaGraphLaunch(m->bgraph[mode * 16 + n], s));
+		m->last_launches = m->bgraph_launches[mode * 16 + n];
+	} else {
+		XALM_TRY(enqueue_batch(m, mode, n, s, &m->last_launches));
+	}
+	return XALM_OK;
+}
+
+int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, float* logits_host) {
+	XALM_TRY(xalm_cuda_forward_batch_async(m, n, seqs, tokens, pos, mode));
+	const size_t bytes = (size_t) n * m->c.vocab_size * sizeof(float);
+	if (mode == XALM_OUTPUT_LOGITS && logits_host) {
+		XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_logits, m->logits, bytes, cudaMemcpyDeviceToHost, m->stream));
+		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+		memcpy(logits_host, m->h_logits, bytes);
+	} else {
+		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+	}
+	return XALM_OK;
+}
+
+int xalm_cuda_forward_batch_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens) {
+	if (!next_tokens) return set_error(XALM_ERR_INVALID, "next_tokens is NULL");
+	XALM_TRY(xalm_cuda_forward_batch_async(m, n, seqs, tokens, pos, XALM_OUTPUT_LOGITS));
+	argmax_rows_kernel<<<n, 1024, 0, m->stream>>>(m->logits, m->c.vocab_size, m->d_argmax);
+	XALM_CUDA_CHECK(cudaGetLastError());
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, (size_t) n * sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+	memcpy(next_tokens, m->h_argmax, (size_t) n * sizeof(int));
 	return XALM_OK;
 }
 
@@ -1645,7 +1925,8 @@ int xalm_cuda_read_kv(xalm_cuda_model* m, int layer, int which, uint16_t* dst, s
 	if (n_elems > cap) return set_error(XALM_ERR_INVALID, "read_kv: %zu > %zu", n_elems, cap);
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
 	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-	XALM_CUDA_CHECK(cudaMemcpy(dst, which == 0 ? m->layers[layer].k_cache : m->layers[layer].v_cache, n_elems * sizeof(uint16_t), cudaMemcpyDeviceToHost));
+	const __half* src = (which == 0 ? m->layers[layer].k_cache : m->layers[layer].v_cache) + (size_t) m->cur_seq * m->kv_slot;
+	XALM_CUDA_CHECK(cudaMemcpy(dst, src, n_elems * sizeof(uint16_t), cudaMemcpyDeviceToHost));
 	return XALM_OK;
 }
 
@@ -1843,7 +2124,7 @@ static void fill_prefill_model(xalm_cuda_model* m, PrefillModel& pm) {
 		PrefillLayer& P = pm.layers[l];
 		P.wqkv = L.wqkv.m; P.wo = L.wo.m; P.w13 = L.w13.m; P.w2 = L.w2.m; P.glu_off = m->hidden_l;
 		P.rms_att = L.rms_att; P.rms_ffn = L.rms_ffn; P.rms_att_type = L.rms_att_type; P.rms_ffn_type = L.rms_ffn_type;
-		P.k_cache = L.k_cache; P.v_cache = L.v_cache;
+		P.k_cache = L.k_cache + (size_t) m->cur_seq * m->kv_slot; P.v_cache = L.v_cache + (size_t) m->cur_seq * m->kv_slot;
 	}
 }
 
@@ -1992,6 +2273,72 @@ int xalm_cuda_bench_matvec(int type_id, int n, int d, int epi, int with_norm, in
 			a.glu_off = d; a.act = XALM_SILU;
 			if (with_norm) { a.norm_w = (const uint8_t*) dg; a.norm_type = XALM_F32; a.norm_eps = 1e-5f; }
 			rc = launch_matvec(a, s, pdl);
+		}
+		cudaEventRecord(e1, s);
+		cudaError_t e = cudaStreamSynchronize(s);
+		if (rc == XALM_OK && e != cudaSuccess) rc = set_error(XALM_ERR_CUDA, "bench failed: %s", cudaGetErrorString(e));
+		float ms = 0.f;
+		cudaEventElapsedTime(&ms, e0, e1);
+		*ms_per_launch = ms / iters;
+		cudaEventDestroy(e0); cudaEventDestroy(e1); cudaStreamDestroy(s);
+	}
+	if (sg.p) cudaFree(sg.p);
+	if (sg.flag) cudaFree(sg.flag);
+	da.free_all();
+	return rc;
+}
+
+int xalm_cuda_bench_matvec_batch(int type_id, int n, int d, int epi, int with_norm, int n_seqs, int n_buffers, int iters, float* ms_per_launch) {
+	if (!ms_per_launch || n <= 0 || d <= 0 || n % 32 || d % 32 || n_buffers <= 0 || iters <= 0 || n_seqs < 1 || n_seqs > MMB_MAX_SEQS)
+		return set_error(XALM_ERR_INVALID, "bad argument");
+	if (epi != EPI_STORE && epi != EPI_GLU && epi != EPI_RESIDUAL) return set_error(XALM_ERR_INVALID, "bench epi must be 0 (store), 1 (residual) or 2 (glu)");
+	TypeInfo ti;
+	if (!type_info(type_id, &ti)) return set_error(XALM_ERR_INVALID, "invalid type: %d", type_id);
+	const int rows = epi == EPI_GLU ? 2 * d : d;
+	if (!mma_takes(type_id, rows, n, epi == EPI_GLU ? d : 0)) return set_error(XALM_ERR_UNSUPPORTED, "the batched matvec cannot take type %d, %d x %d", type_id, rows, n);
+	XALM_TRY(need_device());
+	DevAlloc da;
+	std::vector<WMat> ws(n_buffers);
+	const size_t raw_bytes = (size_t) rows * n / ti.block * ti.bytes;
+	std::vector<uint8_t> host(raw_bytes);
+	uint32_t st = 12345;
+	for (size_t i = 0; i < raw_bytes; i++) { st = st * 1664525u + 1013904223u; host[i] = (uint8_t) ((st >> 24) & 0x3F); }
+	int rc = XALM_OK;
+	Staging sg;
+	for (int b = 0; b < n_buffers && rc == XALM_OK; b++) {
+		rc = alloc_wmat(da, ws[b], type_id, rows, n, epi == EPI_GLU ? d : 0, false, true);
+		if (rc == XALM_OK) rc = upload_piece(ws[b], 0, type_id, host.data(), n, 0, rows, 0, n, sg, 0);
+	}
+	float *dx = nullptr, *dy = nullptr, *dg = nullptr, *dsc = nullptr;
+	uint8_t* img = nullptr;
+	if (rc == XALM_OK && with_norm) {
+		rc = da.alloc((void**) &dg, (size_t) n * sizeof(float));
+		if (rc == XALM_OK) {
+			std::vector<float> hg(n, 1.0f);
+			cudaMemcpy(dg, hg.data(), (size_t) n * sizeof(float), cudaMemcpyHostToDevice);
+		}
+	}
+	if (rc == XALM_OK) rc = da.alloc((void**) &dx, (size_t) n_seqs * n * sizeof(float));
+	if (rc == XALM_OK) rc = da.alloc((void**) &dy, (size_t) n_seqs * d * sizeof(float));
+	if (rc == XALM_OK) rc = da.alloc((void**) &dsc, (size_t) n_seqs * sizeof(float));
+	if (rc == XALM_OK) rc = da.alloc((void**) &img, (size_t) n / 32 * ((n_seqs + 1) / 2) * MMB_PAIR);
+	if (rc == XALM_OK) {
+		std::vector<float> hx((size_t) n_seqs * n, 0.01f);
+		cudaMemcpy(dx, hx.data(), hx.size() * sizeof(float), cudaMemcpyHostToDevice);
+		cudaMemset(dy, 0, (size_t) n_seqs * d * sizeof(float));
+		cudaEvent_t e0, e1;
+		cudaEventCreate(&e0); cudaEventCreate(&e1);
+		cudaStream_t s;
+		cudaStreamCreate(&s);
+		const bool pdl = tune("pdl") != 0;
+		const BatchIo io = {n_seqs, n, d, img, dsc, 0};
+		for (int it = -3 * n_buffers; it < iters && rc == XALM_OK; it++) {
+			if (it == 0) cudaEventRecord(e0, s);
+			MatvecArgs a = {};
+			a.w = ws[((it % n_buffers) + n_buffers) % n_buffers]; a.x = dx; a.n = n; a.d = d; a.epi = epi; a.out = dy;
+			a.glu_off = d; a.act = XALM_SILU;
+			if (with_norm) { a.norm_w = (const uint8_t*) dg; a.norm_type = XALM_F32; a.norm_eps = 1e-5f; }
+			rc = launch_matvec_batch(a, io, s, pdl);
 		}
 		cudaEventRecord(e1, s);
 		cudaError_t e = cudaStreamSynchronize(s);

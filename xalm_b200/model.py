@@ -88,14 +88,18 @@ class Model:
 
     # ---- model.cuda() -----------------------------------------------------------------------------------------
     def cuda(self, device: int = 0, tp_rank: int = 0, tp_size: int = 1, comm_id: bytes | None = None, stream: int | None = None,
-             release_host: bool = False, ipc_exchange=None) -> "Model":
+             release_host: bool = False, ipc_exchange=None, max_seqs: int = 1) -> "Model":
+        """max_seqs > 1: a batched handle with that many sequence slots (forward_batch*, select_seq)."""
         L = capi.lib()
         h = C.c_void_p()
         cfg = capi.XalmConfig.from_dict(self.config)
         capi.check(L.xalm_cuda_create(C.byref(cfg), device, tp_rank, tp_size, C.byref(h)))
         self._h = h
         self.tp_rank, self.tp_size = tp_rank, tp_size
+        self.max_seqs = max_seqs
         try:
+            if max_seqs != 1:
+                capi.check(L.xalm_cuda_set_batch(h, max_seqs))
             if stream is not None:
                 capi.check(L.xalm_cuda_set_stream(h, C.c_void_p(stream)))
             if tp_size > 1:
@@ -168,6 +172,37 @@ class Model:
 
     def sync(self):
         capi.check(capi.lib().xalm_cuda_sync(self._h))
+
+    # ---- batched decode: one step of several independent sequences (slots of a max_seqs > 1 handle) ---------------------
+    @staticmethod
+    def _batch_args(seqs, tokens, pos):
+        arrs = [np.ascontiguousarray(v, dtype=np.int32).reshape(-1) for v in (seqs, tokens, pos)]
+        if not arrs[0].size == arrs[1].size == arrs[2].size:
+            raise ValueError("seqs, tokens and pos must have the same length")
+        return arrs, [a.ctypes.data_as(C.c_void_p) for a in arrs]
+
+    def forward_batch(self, seqs, tokens, pos, mode: int = InferenceMode.OUTPUT_LOGITS):
+        """Slot seqs[i] takes tokens[i] at position pos[i].  OUTPUT_LOGITS -> (n, vocab) logits, row i for seqs[i]; else None."""
+        arrs, ptrs = self._batch_args(seqs, tokens, pos)
+        n = arrs[0].size
+        lg = np.empty((n, self.config["vocab_size"]), dtype=np.float32) if mode == InferenceMode.OUTPUT_LOGITS else None
+        capi.check(capi.lib().xalm_cuda_forward_batch(self._h, n, *ptrs, mode, lg.ctypes.data_as(C.c_void_p) if lg is not None else None))
+        return lg
+
+    def forward_batch_argmax(self, seqs, tokens, pos) -> list:
+        """forward_batch + Sampler.sample_argmax of each row on the device."""
+        arrs, ptrs = self._batch_args(seqs, tokens, pos)
+        out = np.empty(arrs[0].size, dtype=np.int32)
+        capi.check(capi.lib().xalm_cuda_forward_batch_argmax(self._h, arrs[0].size, *ptrs, out.ctypes.data_as(C.c_void_p)))
+        return [int(v) for v in out]
+
+    def forward_batch_async(self, seqs, tokens, pos, mode: int = InferenceMode.OUTPUT_LOGITS) -> None:
+        arrs, ptrs = self._batch_args(seqs, tokens, pos)
+        capi.check(capi.lib().xalm_cuda_forward_batch_async(self._h, arrs[0].size, *ptrs, mode))
+
+    def select_seq(self, seq: int) -> None:
+        """The slot forward*, prefill*, read_kv and read_state work on (default 0)."""
+        capi.check(capi.lib().xalm_cuda_select_seq(self._h, seq))
 
     # ---- batched prefill: the per-position loops of main.cpp:94-100 / :244-254 in one pass (tcgen05 GEMMs) ----
     def prefill(self, tokens, pos0: int = 0, want_logits: int = 1, targets=None, fetch_logits: bool = True):
