@@ -178,6 +178,21 @@ int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const in
 int xalm_cuda_forward_batch_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens);
 int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode);
 int xalm_cuda_select_seq(xalm_cuda_model* m, int seq);
+/* ---- spans: several consecutive positions of one sequence in one step (speculative decoding) -------------------------------
+ * xalm_cuda_forward_spans: forward_batch with XALM_OUTPUT_LOGITS on a batched handle, where a slot may appear several times.  The
+ * entries of one slot, in the order given, must have consecutive positions p, p+1, ...; when a slot has more than one entry, all
+ * of its positions must be < max_seq_len (a span never touches the ring or the attention sinks).  A slot that appears once keeps
+ * forward_batch's rules, positions past the window included.  Entry i at position p+j attends to the slot's rows 0 .. p+j, the
+ * rows p .. p+j-1 written by the earlier entries of the same step included, so its logits (logits_host row i, may be NULL) and
+ * the rows it writes are bit-identical to decoding tokens[i] at pos[i] after the previous entries one step at a time.
+ * Non-consecutive or repeated positions, a span reaching max_seq_len, and everything forward_batch refuses are XALM_ERR_INVALID
+ * before anything is enqueued, with every cache untouched; XALM_ERR_STATE on a handle without xalm_cuda_set_batch.
+ * Rejected drafts need no rollback: the KV rows written for entries whose tokens are then thrown away stay in the cache, and a
+ * later step (forward, forward_batch or another span) rewrites position q before any entry reads it, since an entry at q reads
+ * rows 0 .. q only.  So a caller continues from the last accepted position as if the rejected entries had never run.
+ * xalm_cuda_forward_spans_argmax: the same + Sampler::sample_argmax per row on the device; next_tokens[i] for entry i.  Synchronous. */
+int xalm_cuda_forward_spans(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, float* logits_host);
+int xalm_cuda_forward_spans_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens);
 /* Pinned host buffer the logits are copied into by xalm_cuda_forward (alias it as InferenceState::_logits). */
 float* xalm_cuda_logits_host(xalm_cuda_model* m);
 /* Model::active_bytes(pos) (model.cpp:12-35), 64-bit, per-format bytes; this rank's shard only. */

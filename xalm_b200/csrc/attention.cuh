@@ -41,7 +41,7 @@ struct AttnArgs {
 	size_t kv_slot;        // elements between two slots' caches
 };
 
-// K/V rows: coherent L2 loads (ld.global.cg).  NOT the read-only path: row kv_pos and the sink rows are written by the QKV
+// K/V rows: coherent L2 loads (ld.global.cg).  NOT the read-only path: rows kv_fresh .. kv_pos and the sink rows are written by the QKV
 // kernel that may still be running when this kernel's early batch is requested (PDL), and ld.global.nc is only defined for data
 // that nobody writes during the kernel's lifetime.
 __device__ __forceinline__ uint4 ld_kv16(const __half* p) { return __ldcg(reinterpret_cast<const uint4*>(p)); }
@@ -69,8 +69,9 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	if (threadIdx.x == 0) l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) (blockIdx.y * gridDim.x + blockIdx.x), (int) (gridDim.x * gridDim.y));
 
 	// Everything that does not depend on the QKV kernel still running is done BEFORE the dependency wait: the split bounds (the
-	// step parameters were written before the graph was launched) and the first batch of K/V rows — only the row being written
-	// this step (kv_pos) and the re-rotated sink rows are fetched again afterwards.
+	// step parameters were written before the graph was launched) and the first batch of K/V rows — only the rows being written
+	// this step (kv_fresh .. kv_pos: one row, or the rows of every entry of a span up to this one) and the re-rotated sink rows
+	// are fetched again afterwards.
 	const int kvh = blockIdx.y, split = blockIdx.x;
 	const int z = BATCH ? (int) blockIdx.z : 0;
 	const StepParams* step = a.step + z;
@@ -83,6 +84,7 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	const int kv_len = a.kv_len_fixed >= 0 ? a.kv_len_fixed : step->kv_len;
 	const int kv_pos = a.kv_len_fixed >= 0 ? -1 : step->kv_pos;
 	const int kv_sink = a.kv_len_fixed >= 0 ? 0 : step->kv_sink;
+	const int kv_fresh = a.kv_len_fixed >= 0 ? -1 : step->kv_fresh;
 	const int slen = attn_split_len(kv_len, a.n_splits, a.min_split);
 	const int n_active = (kv_len + slen - 1) / slen;
 	const int t0 = split * slen, t1 = min(kv_len, t0 + slen);
@@ -132,7 +134,7 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 #pragma unroll
 		for (int j = 0; j < TB; j++) {
 			const int t = tb_first + j * RPW + sub;
-			if (t < t1 && (t == kv_pos || t < kv_sink)) {
+			if (t < t1 && ((t >= kv_fresh && t <= kv_pos) || t < kv_sink)) {
 				kn[j] = ld_kv16(kbase + (size_t) t * kv_stride);
 				vn[j] = ld_kv16(vbase + (size_t) t * kv_stride);
 			}

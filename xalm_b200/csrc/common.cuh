@@ -38,6 +38,8 @@ struct StepParams {
 	int mode;
 	unsigned int ar_base; // peer allreduce sequence base of this token (same on every rank)
 	int slot;    // batched decode: the sequence slot (KV cache) this entry drives
+	int kv_fresh; // first ring row of this entry's slot written in this step: kv_pos, or the span's first row when the slot has
+	              // several entries (consecutive positions, xalm_cuda_forward_spans); rows kv_fresh .. kv_pos are written by the QKV kernel
 };
 
 // ---- loads ---------------------------------------------------------------------------------------------

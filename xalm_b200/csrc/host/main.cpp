@@ -1,6 +1,7 @@
 // main.cpp — the reference's CLI surface (src/main.cpp:417-547) on top of the CUDA backend.
 //
 //   xalm_main <checkpoint.xalm> [-d cuda] [-m completion|passkey|perplexity|batch] [-T ctx] [-i prompt | -f file] [-n steps] [-l pos] [-g gpus] [-b seqs]
+//             [-s draft]
 //
 // Same flags, same prefix matching for -m/-d, same defaults (mode completion, -n 128, the default prompt), same stats
 // block, plus the roofline fraction.  Differences, on purpose:
@@ -42,6 +43,8 @@ namespace {
 	fprintf(stderr, "  -g <int> number of GPUs to run tensor-parallel on (default - 1; not with -m verify)\n");
 	fprintf(stderr, "\nPerplexity mode options:\n  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
 	fprintf(stderr, "Completion mode options:\n  -n <int>    number of steps to run for in completion mode, default 128. 0 = max_seq_len, -1 = infinite\n");
+	fprintf(stderr, "  -s <int>    speculative decoding: verify up to this many prompt-lookup draft tokens per pass (1..7; one GPU,\n"
+	                "              integer block formats; same output as without -s)\n");
 	fprintf(stderr, "  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
 	fprintf(stderr, "Batch mode options (one GPU; integer block formats):\n  -f <filepath> prompts, one per non-empty line\n"
 	                "  -b <int>    sequences decoded together (1..8, default 8)\n  -n <int>    tokens per prompt, default 128. 0 = max_seq_len\n");
@@ -98,13 +101,88 @@ size_t hydrate(const Model& model, const InferenceState& state, const std::vecto
 	return read_bytes;
 }
 
-void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps) {
+// Prompt lookup: up to k tokens that followed the most recent earlier occurrence of the sequence's last 3 tokens (else its last 2;
+// a single token is too weak a match to be worth a wider pass).  Empty when neither suffix occurred before.
+std::vector<int> draft_lookup(const std::vector<int>& seq, int k) {
+	const size_t N = seq.size();
+	for (size_t n = 3; n >= 2; n--) {
+		if (N <= n) continue;
+		for (size_t s = N - n; s-- > 0;) // occurrences starting before the suffix itself, latest first
+			if (std::equal(seq.begin() + s, seq.begin() + s + n, seq.end() - n)) {
+				const size_t from = s + n, len = std::min((size_t) k, N - from);
+				return std::vector<int>(seq.begin() + from, seq.begin() + from + len);
+			}
+	}
+	return {};
+}
+
+struct SpecStats {
+	size_t passes = 0, drafted = 0, accepted = 0, decoded = 0; // decoded: tokens the passes produced (accepted + one per pass)
+};
+
+// The generation loop of -m completion -s k: the same greedy tokens, fewer passes over the weights.  Each step drafts up to k
+// tokens by prompt lookup and verifies them with the last token in ONE span (Model::forward_spans_argmax): entry j's greedy
+// token is what a plain step would produce after the entries before it, so the longest prefix of the draft that matches those
+// tokens is accepted, plus the model's own token after it.  Rows written for rejected drafts need no cleanup (xalm_cuda.h).
+// Without a draft, or past the context window where spans are refused, the step is a plain forward on slot 0.  Prints the tokens
+// as run_completion does; returns the bytes read.
+size_t generate_speculative(const Model& model, const InferenceState& state, const Sampler& sampler, const Tokenizer& tokenizer,
+                            std::vector<int>& encoding, int num_steps, int k, SpecStats& st) {
+	const size_t W = (size_t) model.config.max_seq_len;
+	const size_t kv_row = W > 1 ? model.active_bytes(1) - model.active_bytes(0) : 0, weights = model.active_bytes(0) - kv_row;
+	size_t read_bytes = 0;
+	std::vector<int> pending = {sampler.sample_argmax(state)}; // greedy tokens known but not printed yet
+	std::vector<int> seqs, toks, pos, out;
+	for (int i = 0;;) {
+		bool stop = false;
+		for (const int token_id : pending) {
+			if (!(i < num_steps || num_steps == -1)) { stop = true; break; }
+			std::cout << tokenizer.decode_one(encoding.back(), token_id) << std::flush;
+			encoding.push_back(token_id);
+			i++;
+			if (token_id == tokenizer.eos_id || token_id == tokenizer.eot_id) { stop = true; break; }
+		}
+		if (stop || !(i < num_steps || num_steps == -1)) break;
+		const size_t P = encoding.size() - 1;            // position of the last token, not yet decoded
+		const size_t room = P + 1 < W ? W - 1 - P : 0;    // draft positions P+1 .. P+len stay inside the window
+		const std::vector<int> draft = room ? draft_lookup(encoding, (int) std::min(room, (size_t) k)) : std::vector<int>{};
+		st.passes++;
+		if (draft.empty()) {
+			model.forward(state, encoding.back(), (int) P);
+			read_bytes += model.active_bytes(P);
+			pending = {sampler.sample_argmax(state)};
+			st.decoded++;
+			continue;
+		}
+		const int n = (int) draft.size() + 1;
+		seqs.assign(n, 0);
+		toks.assign(1, encoding.back());
+		toks.insert(toks.end(), draft.begin(), draft.end());
+		pos.resize(n);
+		out.resize(n);
+		for (int j = 0; j < n; j++) pos[j] = (int) P + j;
+		model.forward_spans_argmax(n, seqs.data(), toks.data(), pos.data(), out.data());
+		read_bytes += weights;
+		for (int j = 0; j < n; j++) read_bytes += (P + j + 1) * kv_row;
+		int a = 0;
+		while (a < n - 1 && out[a] == draft[a]) a++;
+		pending.assign(draft.begin(), draft.begin() + a);
+		pending.push_back(out[a]);
+		st.drafted += draft.size();
+		st.accepted += a;
+		st.decoded += a + 1;
+	}
+	return read_bytes;
+}
+
+void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps, int spec) {
 	auto model_data = Xalm::load(checkpoint_path);
 	std::cout << "loading model " << checkpoint_path << std::endl;
 	Model model = Model::from_xalm(model_data, context, /*defer_load=*/true); // weights go disk -> pinned -> device in model.cuda()
 	printf("Model active bytes(m): %zu\n", model.active_bytes(model.config.max_seq_len) / (1024 * 1024));
 	std::cout << "Using CUDA" << std::endl;
-	to_device(model, tp);
+	if (spec) model.cuda(0, 0, 1, nullptr, {}, spec + 1); // -s k: a batched handle wide enough for a span of k drafts + the last token
+	else to_device(model, tp);
 	InferenceState state(model.config);
 	state.cuda();
 	Sampler sampler(model.config);
@@ -123,7 +201,9 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	t0 = now_s();
 	size_t read_bytes = hydrate(model, state, encoding);
 	const double hydrate_s = now_s() - t0;
-	for (int i = 0; i < num_steps || num_steps == -1; i++) { // main.cpp:105-115
+	SpecStats spec_stats;
+	if (spec) read_bytes += generate_speculative(model, state, sampler, tokenizer, encoding, num_steps, spec, spec_stats);
+	else for (int i = 0; i < num_steps || num_steps == -1; i++) { // main.cpp:105-115
 		// the logits are all-gathered under -g, so every rank picks the same token and stops at the same step
 		const int token_id = sampler.sample_argmax(state);
 		std::cout << tokenizer.decode_one(encoding.back(), token_id) << std::flush;
@@ -140,6 +220,9 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	       "  roofline: %.1f%% of %.0f GB/s HBM\n  total: %.5gs\n",
 	       encoding.size(), encoding.size() / elapsed_s, elapsed_s / encoding.size(), hydrate_s, gbs, 100.0 * gbs / peak, peak, elapsed_s);
 	print_tp_stats(tp, launches);
+	if (spec)
+		printf("  speculative: %zu passes, %zu drafted, %zu accepted, %.3g tokens/pass\n", spec_stats.passes, spec_stats.drafted, spec_stats.accepted,
+		       spec_stats.passes ? (double) spec_stats.decoded / spec_stats.passes : 0.0);
 }
 
 // -m batch: every non-empty line of the prompt file is one prompt; up to `max_batch` of them decode together on one batched handle,
@@ -369,7 +452,7 @@ int main(int argc, char* argv[]) {
 	std::string prompt = "Q: What is the meaning of life? A:"; // main.cpp:421
 	std::string prompt_path;
 	std::string convert_type;
-	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8;
+	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8, spec = 0;
 	if (argc >= 2) checkpoint_path = argv[1];
 	else error_usage();
 	for (int i = 2; i < argc;) { // main.cpp:435-512
@@ -397,9 +480,17 @@ int main(int argc, char* argv[]) {
 			max_batch = parse_gpus(v);
 			if (max_batch > 8) error_usage();
 		}
+		else if (f == 's') {
+			spec = parse_gpus(v);
+			if (spec > 7) error_usage();
+		}
 		else if (f == 'n') { num_steps = std::stoi(v); n_junk = num_steps; }
 		else error_usage();
 		i += 2;
+	}
+	if (spec && (mode != "completion" || gpus != 1)) {
+		fprintf(stderr, "Error: -s runs -m completion on one GPU (no -g)\n");
+		error_usage();
 	}
 	if (mode == "verify") {
 		if (gpus != 1) {
@@ -450,7 +541,7 @@ int main(int argc, char* argv[]) {
 	}
 	auto run = [&](const TpRank& tp) {
 		try {
-			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps);
+			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps, spec);
 			else if (mode == "passkey") run_passkey(tp, checkpoint_path, context, n_junk, passkey_pos);
 			else run_perplexity(tp, checkpoint_path, prompt, context);
 		} catch (const std::exception& e) {

@@ -451,6 +451,11 @@ void Model::forward_batch_argmax(const int n, const int* seqs, const int* tokens
 	if (xalm_cuda_forward_batch_argmax(handle_, n, seqs, tokens, pos, next) != XALM_OK) xalm_throw_last("Model::forward_batch_argmax");
 }
 
+void Model::forward_spans_argmax(const int n, const int* seqs, const int* tokens, const int* pos, int* next) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_spans_argmax: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_forward_spans_argmax(handle_, n, seqs, tokens, pos, next) != XALM_OK) xalm_throw_last("Model::forward_spans_argmax");
+}
+
 void Model::select_seq(const int seq) const {
 	if (!handle_) throw std::runtime_error("Model::select_seq: model is not on a CUDA device (call model.cuda())");
 	if (xalm_cuda_select_seq(handle_, seq) != XALM_OK) xalm_throw_last("Model::select_seq");

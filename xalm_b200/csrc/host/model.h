@@ -183,6 +183,9 @@ struct Model {
 	void forward_batch(int n, const int* seqs, const int* tokens, const int* pos, InferenceMode mode, float* logits) const;
 	// forward_batch + Sampler::sample_argmax of every row on the device: next[i] for seqs[i].
 	void forward_batch_argmax(int n, const int* seqs, const int* tokens, const int* pos, int* next) const;
+	// forward_batch_argmax where a slot may take several consecutive positions in one step (xalm_cuda_forward_spans_argmax):
+	// how drafted tokens are verified in one pass over the weights.  next[i] is the greedy token after entry i.  A refused call throws.
+	void forward_spans_argmax(int n, const int* seqs, const int* tokens, const int* pos, int* next) const;
 	// The slot forward / prefill / prefill_window work on (default 0): how a prompt is hydrated into a slot.
 	void select_seq(int seq) const;
 

@@ -1650,6 +1650,7 @@ int xalm_cuda_forward_async(xalm_cuda_model* m, int token, int pos, int mode) {
 	sp.kv_sink = pos >= c.max_seq_len ? 2 : 0;
 	sp.kv_pos = sp.kv_sink + (pos - sp.kv_sink) % (c.max_seq_len - sp.kv_sink);
 	sp.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
+	sp.kv_fresh = sp.kv_pos;
 	sp.mode = mode;
 	sp.ar_base = m->token_serial * 1024u; // 2 x n_layers <= 1024 exchanges per token; wraps consistently on every rank
 	m->token_serial++;
@@ -1794,24 +1795,38 @@ static int ensure_bgraph(xalm_cuda_model* m, int mode, int n) {
 	return XALM_OK;
 }
 
-int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode) {
+// One step of n entries: entry i drives slot seqs[i] with tokens[i] at pos[i].  spans = false (forward_batch): every slot at most
+// once.  spans = true (forward_spans): a slot may take several consecutive positions, all inside the window; the attention of
+// each such entry re-reads, after its dependency wait, every row the step writes for its slot up to its own (kv_fresh .. kv_pos).
+// Everything is validated before anything is enqueued, so a refusal leaves every cache untouched.
+static int forward_step_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, bool spans) {
+	const char* fn = spans ? "forward_spans" : "forward_batch";
 	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
-	if (!m->finalized) return set_error(XALM_ERR_STATE, "forward_batch before finalize");
-	if (!m->batched) return set_error(XALM_ERR_STATE, "forward_batch on a handle without xalm_cuda_set_batch");
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "%s before finalize", fn);
+	if (!m->batched) return set_error(XALM_ERR_STATE, "%s on a handle without xalm_cuda_set_batch", fn);
 	if (mode != XALM_HYDRATE_KV_CACHE && mode != XALM_OUTPUT_LOGITS) return set_error(XALM_ERR_INVALID, "bad mode %d", mode);
-	if (n < 1 || n > m->max_seqs) return set_error(XALM_ERR_INVALID, "forward_batch: n = %d not in [1, %d]", n, m->max_seqs);
+	if (n < 1 || n > m->max_seqs) return set_error(XALM_ERR_INVALID, "%s: n = %d not in [1, %d]", fn, n, m->max_seqs);
 	if (!seqs || !tokens || !pos) return set_error(XALM_ERR_INVALID, "NULL argument");
 	const xalm_config& c = m->c;
-	unsigned int seen = 0;
+	int first[MMB_MAX_SEQS], last[MMB_MAX_SEQS]; // per slot: its first and latest entry so far (-1: none)
+	for (int s = 0; s < MMB_MAX_SEQS; s++) first[s] = last[s] = -1;
 	for (int i = 0; i < n; i++) {
-		if (seqs[i] < 0 || seqs[i] >= m->max_seqs) return set_error(XALM_ERR_INVALID, "forward_batch: slot %d not in [0, %d)", seqs[i], m->max_seqs);
-		if (seen & (1u << seqs[i])) return set_error(XALM_ERR_INVALID, "forward_batch: slot %d named twice", seqs[i]);
-		seen |= 1u << seqs[i];
+		const int s = seqs[i];
+		if (s < 0 || s >= m->max_seqs) return set_error(XALM_ERR_INVALID, "%s: slot %d not in [0, %d)", fn, s, m->max_seqs);
+		if (last[s] >= 0 && !spans) return set_error(XALM_ERR_INVALID, "forward_batch: slot %d named twice", s);
+		if (last[s] >= 0 && (long long) pos[i] != (long long) pos[last[s]] + 1)
+			return set_error(XALM_ERR_INVALID, "forward_spans: slot %d takes position %d after %d (a span's positions are consecutive)", s, pos[i], pos[last[s]]);
+		if (first[s] < 0) first[s] = i;
+		last[s] = i;
 		if (tokens[i] < 0 || tokens[i] >= c.vocab_size) return set_error(XALM_ERR_INVALID, "token %d out of range [0,%d)", tokens[i], c.vocab_size);
 		if (pos[i] < 0) return set_error(XALM_ERR_INVALID, "negative position");
 	}
+	for (int s = 0; s < m->max_seqs; s++) // positions of a span increase, so its last one is its largest
+		if (first[s] != last[s] && pos[last[s]] >= c.max_seq_len)
+			return set_error(XALM_ERR_INVALID, "forward_spans: the span of slot %d reaches position %d, spans stay below max_seq_len %d", s,
+			                 pos[last[s]], c.max_seq_len);
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	cudaStream_t s = m->stream;
+	cudaStream_t st = m->stream;
 	const int slot = m->step_slot;
 	m->step_slot = (slot + 1) % 64;
 	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
@@ -1823,24 +1838,25 @@ int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, co
 		p.kv_sink = pos[i] >= c.max_seq_len ? 2 : 0;
 		p.kv_pos = p.kv_sink + (pos[i] - p.kv_sink) % (c.max_seq_len - p.kv_sink);
 		p.kv_len = pos[i] >= c.max_seq_len ? c.max_seq_len : pos[i] + 1;
+		p.kv_fresh = sp[first[seqs[i]]].kv_pos; // == kv_pos unless an earlier entry of this step drives the same slot
 		p.mode = mode;
 		p.ar_base = 0;
 		p.slot = seqs[i];
 	}
-	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, sp, (size_t) n * sizeof(StepParams), cudaMemcpyHostToDevice, s));
-	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], s));
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, sp, (size_t) n * sizeof(StepParams), cudaMemcpyHostToDevice, st));
+	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], st));
 	if (tune("graph")) {
 		XALM_TRY(ensure_bgraph(m, mode, n));
-		XALM_CUDA_CHECK(cudaGraphLaunch(m->bgraph[mode * 16 + n], s));
+		XALM_CUDA_CHECK(cudaGraphLaunch(m->bgraph[mode * 16 + n], st));
 		m->last_launches = m->bgraph_launches[mode * 16 + n];
 	} else {
-		XALM_TRY(enqueue_batch(m, mode, n, s, &m->last_launches));
+		XALM_TRY(enqueue_batch(m, mode, n, st, &m->last_launches));
 	}
 	return XALM_OK;
 }
 
-int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, float* logits_host) {
-	XALM_TRY(xalm_cuda_forward_batch_async(m, n, seqs, tokens, pos, mode));
+// after a step of n entries: copy their logits back (logits_host may be NULL) and wait
+static int finish_step(xalm_cuda_model* m, int n, int mode, float* logits_host) {
 	const size_t bytes = (size_t) n * m->c.vocab_size * sizeof(float);
 	if (mode == XALM_OUTPUT_LOGITS && logits_host) {
 		XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_logits, m->logits, bytes, cudaMemcpyDeviceToHost, m->stream));
@@ -1852,15 +1868,40 @@ int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const in
 	return XALM_OK;
 }
 
-int xalm_cuda_forward_batch_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens) {
-	if (!next_tokens) return set_error(XALM_ERR_INVALID, "next_tokens is NULL");
-	XALM_TRY(xalm_cuda_forward_batch_async(m, n, seqs, tokens, pos, XALM_OUTPUT_LOGITS));
+// after a step of n entries with logits: Sampler::sample_argmax of every row on the device, next_tokens[i] for entry i
+static int finish_step_argmax(xalm_cuda_model* m, int n, int* next_tokens) {
 	argmax_rows_kernel<<<n, 1024, 0, m->stream>>>(m->logits, m->c.vocab_size, m->d_argmax);
 	XALM_CUDA_CHECK(cudaGetLastError());
 	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, (size_t) n * sizeof(int), cudaMemcpyDeviceToHost, m->stream));
 	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
 	memcpy(next_tokens, m->h_argmax, (size_t) n * sizeof(int));
 	return XALM_OK;
+}
+
+int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode) {
+	return forward_step_async(m, n, seqs, tokens, pos, mode, false);
+}
+
+int xalm_cuda_forward_batch(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, float* logits_host) {
+	XALM_TRY(forward_step_async(m, n, seqs, tokens, pos, mode, false));
+	return finish_step(m, n, mode, logits_host);
+}
+
+int xalm_cuda_forward_batch_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens) {
+	if (!next_tokens) return set_error(XALM_ERR_INVALID, "next_tokens is NULL");
+	XALM_TRY(forward_step_async(m, n, seqs, tokens, pos, XALM_OUTPUT_LOGITS, false));
+	return finish_step_argmax(m, n, next_tokens);
+}
+
+int xalm_cuda_forward_spans(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, float* logits_host) {
+	XALM_TRY(forward_step_async(m, n, seqs, tokens, pos, XALM_OUTPUT_LOGITS, true));
+	return finish_step(m, n, XALM_OUTPUT_LOGITS, logits_host);
+}
+
+int xalm_cuda_forward_spans_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens) {
+	if (!next_tokens) return set_error(XALM_ERR_INVALID, "next_tokens is NULL");
+	XALM_TRY(forward_step_async(m, n, seqs, tokens, pos, XALM_OUTPUT_LOGITS, true));
+	return finish_step_argmax(m, n, next_tokens);
 }
 
 float* xalm_cuda_logits_host(xalm_cuda_model* m) { return m ? m->h_logits : nullptr; }

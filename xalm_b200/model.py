@@ -200,6 +200,22 @@ class Model:
         arrs, ptrs = self._batch_args(seqs, tokens, pos)
         capi.check(capi.lib().xalm_cuda_forward_batch_async(self._h, arrs[0].size, *ptrs, mode))
 
+    def forward_spans(self, seqs, tokens, pos):
+        """forward_batch where a slot may take several consecutive positions in one step (a span, e.g. drafted tokens to
+        verify): entry i is slot seqs[i], tokens[i] at pos[i].  Returns the (n, vocab) logits, row i for entry i."""
+        arrs, ptrs = self._batch_args(seqs, tokens, pos)
+        n = arrs[0].size
+        lg = np.empty((n, self.config["vocab_size"]), dtype=np.float32)
+        capi.check(capi.lib().xalm_cuda_forward_spans(self._h, n, *ptrs, lg.ctypes.data_as(C.c_void_p)))
+        return lg
+
+    def forward_spans_argmax(self, seqs, tokens, pos) -> list:
+        """forward_spans + Sampler.sample_argmax of each row on the device."""
+        arrs, ptrs = self._batch_args(seqs, tokens, pos)
+        out = np.empty(arrs[0].size, dtype=np.int32)
+        capi.check(capi.lib().xalm_cuda_forward_spans_argmax(self._h, arrs[0].size, *ptrs, out.ctypes.data_as(C.c_void_p)))
+        return [int(v) for v in out]
+
     def select_seq(self, seq: int) -> None:
         """The slot forward*, prefill*, read_kv and read_state work on (default 0)."""
         capi.check(capi.lib().xalm_cuda_select_seq(self._h, seq))
