@@ -42,6 +42,8 @@ def test_bench_matvec_batch_validates_arguments():
     ]
     for args in bad:
         assert L.xalm_cuda_bench_matvec_batch(*args, C.byref(ms)) == 1, args
+        if 1 <= args[5] <= 8:   # the batch-1 bench takes the same arguments without n_seqs, and checks them before the device
+            assert L.xalm_cuda_bench_matvec(*args[:5], *args[6:], C.byref(ms)) == 1, args
     # formats the tensor-core kernel does not take are refused, not run another way
     for t in (T.F16, T.BF16, T.F32, T.TQ1_0, T.QI8):
         assert L.xalm_cuda_bench_matvec_batch(t.id, 4096, 4096, 0, 0, 2, 1, 1, C.byref(ms)) == 2, t.name

@@ -545,18 +545,10 @@ static int launch_matvec(MatvecArgs a, cudaStream_t s, bool pdl) {
 // ---------------------------------------------------------------------------------------------------------
 // small kernels
 // ---------------------------------------------------------------------------------------------------------
-// _copy_embedding (infer.cpp:553-602) from the ON-DISK layout of the table (block formats: extension)
-__global__ void embed_kernel(int type, const uint8_t* __restrict__ table, size_t row_bytes, int dim, const StepParams* step,
-                             float* __restrict__ x) {
-	pdl_launch_dependents();
-	pdl_wait();
-	const uint8_t* row = table + (size_t) step->token * row_bytes;
-	for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < dim; i += gridDim.x * blockDim.x) x[i] = decode_disk_elem(type, row, i);
-}
-
-// batched decode: one row per sequence (blockIdx.y), x is (nseq, dim)
-__global__ void embed_batch_kernel(int type, const uint8_t* __restrict__ table, size_t row_bytes, int dim, const StepParams* steps,
-                                   float* __restrict__ x) {
+// _copy_embedding (infer.cpp:553-602) from the ON-DISK layout of the table (block formats: extension); one row per step entry
+// (blockIdx.y), x is (entries, dim)
+__global__ void embed_rows_kernel(int type, const uint8_t* __restrict__ table, size_t row_bytes, int dim, const StepParams* steps,
+                                  float* __restrict__ x) {
 	pdl_launch_dependents();
 	pdl_wait();
 	const uint8_t* row = table + (size_t) steps[blockIdx.y].token * row_bytes;
@@ -602,8 +594,7 @@ __device__ __forceinline__ void argmax_row(const float* __restrict__ logits, int
 		if (threadIdx.x == 0) *out = bi >= n ? 0 : bi;
 	}
 }
-__global__ void argmax_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) { argmax_row(logits, n, out); }
-// batched decode: row b of (rows, n) logits -> out[b]
+// row b of (rows, n) logits -> out[b]
 __global__ void argmax_rows_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) {
 	argmax_row(logits + (size_t) blockIdx.x * n, n, out + blockIdx.x);
 }
@@ -913,6 +904,11 @@ struct LayerDev {
 };
 enum { P_ATT_NORM = 0, P_FFN_NORM, P_Q, P_K, P_V, P_O, P_GATE, P_DOWN, P_UP };
 
+struct StepGraph {
+	cudaGraphExec_t exec;
+	int launches;
+};
+
 struct xalm_cuda_model {
 	xalm_config c;
 	int device = 0, tp_rank = 0, tp_size = 1;
@@ -924,8 +920,8 @@ struct xalm_cuda_model {
 	size_t kv_slot = 0;
 	uint8_t* ximg = nullptr;          // activation image of the batched matvec
 	float* nscale = nullptr;          // (max_seqs,) 1/rms of the batched matvec's norm prologue
-	std::map<int, cudaGraphExec_t> bgraph; // (mode, n) -> captured batched step
-	std::map<int, int> bgraph_launches;
+	// (mode, n) -> captured step; n = 0: the single-sequence kernel sequence, else a batched step of n entries (run_step)
+	std::map<std::pair<int, int>, StepGraph> graphs;
 	// local (per-rank) sizes
 	int q_dim = 0, kv_dim = 0, q_dim_l = 0, kv_dim_l = 0, n_heads_l = 0, n_kv_heads_l = 0, hidden_l = 0, vocab_l = 0;
 	DevAlloc da;
@@ -952,9 +948,7 @@ struct xalm_cuda_model {
 	int step_slot = 0;
 	float* h_logits = nullptr; // pinned
 	cudaStream_t own_stream = nullptr, stream = nullptr;
-	cudaGraphExec_t graph[2] = {nullptr, nullptr};
 	bool finalized = false;
-	int launches_per_token[2] = {0, 0};
 	int last_launches = 0;
 	ncclComm_t comm = nullptr;
 	// peer-memory allreduce
@@ -1067,9 +1061,7 @@ void xalm_cuda_destroy(xalm_cuda_model* m) {
 	m->prefill = nullptr;
 	cudaSetDevice(m->device);
 	cudaStreamSynchronize(m->stream);
-	for (int i = 0; i < 2; i++)
-		if (m->graph[i]) cudaGraphExecDestroy(m->graph[i]);
-	for (auto& kv : m->bgraph) cudaGraphExecDestroy(kv.second);
+	for (auto& kv : m->graphs) cudaGraphExecDestroy(kv.second.exec);
 	if (m->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(m->comm);
 	for (int i = 0; i < 64; i++)
 		if (m->h_step_ev_used[i]) cudaEventDestroy(m->h_step_ev[i]);
@@ -1353,12 +1345,14 @@ static int upload_impl(xalm_cuda_model* m, const char* name, int type_id, const 
 
 } // extern "C" (templates below)
 
-static void fill_layer_args(xalm_cuda_model* m, int l, MatvecArgs* qkv, AttnArgs* at, MatvecArgs* wo, MatvecArgs* w13, MatvecArgs* w2) {
+// kv_seq: the slot whose K/V cache the arguments point at (the batched kernels add step[i].slot * kv_slot to slot 0's)
+static void fill_layer_args(xalm_cuda_model* m, int l, int kv_seq, MatvecArgs* qkv, AttnArgs* at, MatvecArgs* wo, MatvecArgs* w13,
+                            MatvecArgs* w2) {
 	const xalm_config& c = m->c;
 	LayerDev& L = m->layers[l];
 	const bool tp = m->tp_size > 1;
-	__half* k_cache = L.k_cache + (size_t) m->cur_seq * m->kv_slot;
-	__half* v_cache = L.v_cache + (size_t) m->cur_seq * m->kv_slot;
+	__half* k_cache = L.k_cache + (size_t) kv_seq * m->kv_slot;
+	__half* v_cache = L.v_cache + (size_t) kv_seq * m->kv_slot;
 	{ // attention pre-norm + q,k,v + clip + rope + KV write (+ sinks)
 		MatvecArgs a = {};
 		a.w = L.wqkv.m; a.x = m->x; a.n = c.dim; a.d = m->q_dim_l + 2 * m->kv_dim_l; a.epi = EPI_QKV;
@@ -1394,6 +1388,30 @@ static void fill_layer_args(xalm_cuda_model* m, int l, MatvecArgs* qkv, AttnArgs
 	}
 }
 
+// bytes of a matrix's first plane: in fragment layout s0 bytes hold a tile row of 16 matrix rows (alloc_wmat), else one row
+static size_t plane0_bytes(const WMat& w) { return w.s0 * (size_t) (w.layout_frag ? w.rows / MMA_RC : w.rows); }
+
+// the tail-prefetch chain of layer l: every kernel warms L2 with the first pf_mb MB of the next kernel's weights
+static void chain_tail_prefetch(xalm_cuda_model* m, int l, int mode, int pf_mb, AttnArgs* at, MatvecArgs* wo, MatvecArgs* w13, MatvecArgs* w2) {
+	auto head = [&](const WMat& w, const uint8_t** ptr, unsigned long long* bytes) {
+		*ptr = w.p0;
+		*bytes = std::min<unsigned long long>(plane0_bytes(w), (unsigned long long) pf_mb << 20);
+	};
+	head(wo->w, &at->pf_ptr, &at->pf_bytes);
+	head(w13->w, &wo->pf_ptr, &wo->pf_bytes);
+	head(w2->w, &w13->pf_ptr, &w13->pf_bytes);
+	if (l + 1 < m->c.n_layers) head(m->layers[l + 1].wqkv.m, &w2->pf_ptr, &w2->pf_bytes);
+	else if (mode == XALM_OUTPUT_LOGITS) head(m->wcls.m, &w2->pf_ptr, &w2->pf_bytes);
+}
+
+// a step's first kernel: one embedding row per entry, launched without PDL, so it starts only after the previous step has completed
+static int launch_embed(xalm_cuda_model* m, int n, cudaStream_t s) {
+	cudaError_t e = launch(embed_rows_kernel, dim3(4, n), dim3(256), s, false, m->embed_type, (const uint8_t*) m->embed_raw, m->embed_row_bytes,
+	                       m->c.dim, (const StepParams*) m->d_step, m->x);
+	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "embed launch failed: %s", cudaGetErrorString(e));
+	return XALM_OK;
+}
+
 extern "C" {
 
 // ---- the per-token kernel sequence ---------------------------------------------------------------------------
@@ -1403,9 +1421,7 @@ static int enqueue_token(xalm_cuda_model* m, int mode, cudaStream_t s, int* n_la
 	const bool tp = m->tp_size > 1;
 	int nl = 0;
 	cudaError_t e;
-	e = launch(embed_kernel, dim3(4), dim3(256), s, false, m->embed_type, (const uint8_t*) m->embed_raw, m->embed_row_bytes,
-	                       c.dim, (const StepParams*) m->d_step, m->x);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "embed launch failed: %s", cudaGetErrorString(e));
+	XALM_TRY(launch_embed(m, 1, s));
 	nl++;
 	const int G = c.n_heads / c.n_kv_heads;
 	// fused tensor-parallel exchange: Wo / W2 push their partial rows to every rank, the next norm-prologue kernel receives
@@ -1427,29 +1443,38 @@ static int enqueue_token(xalm_cuda_model* m, int mode, cudaStream_t s, int* n_la
 		a.x = X[cur]; a.x_out = X[cur ^ 1];
 		cur ^= 1;
 	};
+	// Wo / W2 + residual; idx: the exchange (2l, 2l + 1) under tensor parallelism
+	auto residual = [&](MatvecArgs a, int idx) -> int {
+		if (tp && m->peer_ready && !fused) a.out = m->xchg + (size_t) (idx & 1) * c.dim;
+		XALM_TRY(launch_matvec(a, s, pdl));
+		nl++;
+		if (fused) {
+		} else if (tp && m->peer_ready) {
+			e = launch(peer_allreduce_residual_kernel, dim3(4), dim3(256), s, pdl, m->peer, m->x, c.dim, idx, (const StepParams*) m->d_step);
+			if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "peer allreduce launch failed: %s", cudaGetErrorString(e));
+			nl++;
+		} else if (tp) {
+			XALM_NCCL_CHECK(g_nccl.AllReduce(m->part, m->part, c.dim, ncclFloat32, ncclSum, m->comm, s));
+			e = launch(residual_add_kernel, dim3(8), dim3(256), s, false, m->x, (const float*) m->part, c.dim);
+			if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "residual launch failed: %s", cudaGetErrorString(e));
+			nl += 2;
+		}
+		return XALM_OK;
+	};
 	for (int l = 0; l < c.n_layers; l++) {
 		LayerDev& L = m->layers[l];
 		MatvecArgs a_qkv, a_wo, a_w13, a_w2;
 		AttnArgs a_at;
-		fill_layer_args(m, l, &a_qkv, &a_at, &a_wo, &a_w13, &a_w2);
-		(void) L;
+		fill_layer_args(m, l, m->cur_seq, &a_qkv, &a_at, &a_wo, &a_w13, &a_w2);
 		if (fused) {
 			if (l > 0) set_recv(a_qkv, 2 * l - 1);
 			set_push(a_wo, 2 * l);
 			set_recv(a_w13, 2 * l);
 			set_push(a_w2, 2 * l + 1);
 		}
-		if (const int pf_mb = tune("tail_prefetch_mb")) { // chain: every kernel warms L2 with the head of the next kernel's stream
-			auto head = [&](const WMat& w, const uint8_t** ptr, unsigned long long* bytes) {
-				*ptr = w.p0;
-				*bytes = std::min<unsigned long long>((unsigned long long) w.s0 * w.rows, (unsigned long long) pf_mb << 20);
-			};
+		if (const int pf_mb = tune("tail_prefetch_mb")) {
 			a_qkv.pf_kv = 1;
-			head(a_wo.w, &a_at.pf_ptr, &a_at.pf_bytes);
-			head(a_w13.w, &a_wo.pf_ptr, &a_wo.pf_bytes);
-			head(a_w2.w, &a_w13.pf_ptr, &a_w13.pf_bytes);
-			if (l + 1 < c.n_layers) head(m->layers[l + 1].wqkv.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
-			else if (mode == XALM_OUTPUT_LOGITS) head(m->wcls.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
+			chain_tail_prefetch(m, l, mode, pf_mb, &a_at, &a_wo, &a_w13, &a_w2);
 			// ... and with the rmsnorm weights the next norm-fused kernel asks for before its dependency wait
 			auto norm_bytes = [&](int type) { return (unsigned int) ((size_t) c.dim * (type == XALM_F32 ? 4 : 2)); };
 			a_wo.pf_norm_ptr = (const uint8_t*) L.rms_ffn; a_wo.pf_norm_bytes = norm_bytes(L.rms_ffn_type);
@@ -1459,52 +1484,13 @@ static int enqueue_token(xalm_cuda_model* m, int mode, cudaStream_t s, int* n_la
 				a_w2.pf_norm_ptr = (const uint8_t*) m->rms_final; a_w2.pf_norm_bytes = norm_bytes(m->rms_final_type);
 			}
 		}
-		{ // attention pre-norm + q,k,v + clip + rope + KV write (+ sinks)
-			XALM_TRY(launch_matvec(a_qkv, s, pdl));
-			nl++;
-		}
-		{
-			XALM_TRY(launch_attn(a_at, c.head_dim, G, s, pdl));
-			nl++;
-		}
-		{ // Wo + residual
-			MatvecArgs a = a_wo;
-			if (tp && m->peer_ready && !fused) a.out = m->xchg + (size_t) ((2 * l) & 1) * c.dim;
-			XALM_TRY(launch_matvec(a, s, pdl));
-			nl++;
-			if (fused) {
-			} else if (tp && m->peer_ready) {
-				e = launch(peer_allreduce_residual_kernel, dim3(4), dim3(256), s, pdl, m->peer, m->x, c.dim, 2 * l, (const StepParams*) m->d_step);
-				if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "peer allreduce launch failed: %s", cudaGetErrorString(e));
-				nl++;
-			} else if (tp) {
-				XALM_NCCL_CHECK(g_nccl.AllReduce(m->part, m->part, c.dim, ncclFloat32, ncclSum, m->comm, s));
-				e = launch(residual_add_kernel, dim3(8), dim3(256), s, false, m->x, (const float*) m->part, c.dim);
-				if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "residual launch failed: %s", cudaGetErrorString(e));
-				nl += 2;
-			}
-		}
-		{ // ffn pre-norm + W1,W3 + act*gate
-			XALM_TRY(launch_matvec(a_w13, s, pdl && (!tp || m->peer_ready)));
-			nl++;
-		}
-		{ // W2 + residual
-			MatvecArgs a = a_w2;
-			if (tp && m->peer_ready && !fused) a.out = m->xchg + (size_t) ((2 * l + 1) & 1) * c.dim;
-			XALM_TRY(launch_matvec(a, s, pdl));
-			nl++;
-			if (fused) {
-			} else if (tp && m->peer_ready) {
-				e = launch(peer_allreduce_residual_kernel, dim3(4), dim3(256), s, pdl, m->peer, m->x, c.dim, 2 * l + 1, (const StepParams*) m->d_step);
-				if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "peer allreduce launch failed: %s", cudaGetErrorString(e));
-				nl++;
-			} else if (tp) {
-				XALM_NCCL_CHECK(g_nccl.AllReduce(m->part, m->part, c.dim, ncclFloat32, ncclSum, m->comm, s));
-				e = launch(residual_add_kernel, dim3(8), dim3(256), s, false, m->x, (const float*) m->part, c.dim);
-				if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "residual launch failed: %s", cudaGetErrorString(e));
-				nl += 2;
-			}
-		}
+		XALM_TRY(launch_matvec(a_qkv, s, pdl)); // attention pre-norm + q,k,v + clip + rope + KV write (+ sinks)
+		XALM_TRY(launch_attn(a_at, c.head_dim, G, s, pdl));
+		nl += 2;
+		XALM_TRY(residual(a_wo, 2 * l));
+		XALM_TRY(launch_matvec(a_w13, s, pdl && (!tp || m->peer_ready))); // ffn pre-norm + W1,W3 + act*gate
+		nl++;
+		XALM_TRY(residual(a_w2, 2 * l + 1));
 	}
 	if (fused && mode != XALM_OUTPUT_LOGITS && c.n_layers > 0) { // nobody else receives the token's last exchange: drain it
 		const int idx = 2 * c.n_layers - 1;
@@ -1614,20 +1600,90 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 	return XALM_OK;
 }
 
-static int ensure_graph(xalm_cuda_model* m, int mode) {
-	if (m->graph[mode]) return XALM_OK;
-	cudaStream_t s = m->stream;
-	cudaGraph_t g = nullptr;
-	XALM_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+// the batched kernel sequence: n entries (several sequence slots, or consecutive positions of one), one pass over the weights
+static int enqueue_batch(xalm_cuda_model* m, int mode, int n, cudaStream_t s, int* n_launches) {
+	const xalm_config& c = m->c;
+	const bool pdl = tune("pdl") != 0;
+	const int G = c.n_heads / c.n_kv_heads;
 	int nl = 0;
-	int rc = enqueue_token(m, mode, s, &nl);
-	cudaError_t e = cudaStreamEndCapture(s, &g);
-	if (rc != XALM_OK) { if (g) cudaGraphDestroy(g); return rc; }
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(e));
-	e = cudaGraphInstantiate(&m->graph[mode], g, 0);
-	cudaGraphDestroy(g);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
-	m->launches_per_token[mode] = nl;
+	XALM_TRY(launch_embed(m, n, s));
+	nl++;
+	auto io = [&](int x_stride, int out_stride) { return BatchIo{n, x_stride, out_stride, m->ximg, m->nscale, m->kv_slot}; };
+	for (int l = 0; l < c.n_layers; l++) {
+		MatvecArgs a_qkv, a_wo, a_w13, a_w2;
+		AttnArgs a_at;
+		fill_layer_args(m, l, 0, &a_qkv, &a_at, &a_wo, &a_w13, &a_w2);
+		a_at.q_stride = m->q_dim_l; a_at.kv_slot = m->kv_slot;
+		if (const int pf_mb = tune("tail_prefetch_mb")) chain_tail_prefetch(m, l, mode, pf_mb, &a_at, &a_wo, &a_w13, &a_w2);
+		XALM_TRY(launch_matvec_batch(a_qkv, io(c.dim, m->q_dim_l), s, pdl));
+		XALM_TRY(launch_attn(a_at, c.head_dim, G, s, pdl, n));
+		XALM_TRY(launch_matvec_batch(a_wo, io(m->q_dim_l, c.dim), s, pdl));
+		XALM_TRY(launch_matvec_batch(a_w13, io(c.dim, m->hidden_l), s, pdl));
+		XALM_TRY(launch_matvec_batch(a_w2, io(m->hidden_l, c.dim), s, pdl));
+		nl += 9;
+	}
+	if (mode == XALM_OUTPUT_LOGITS) {
+		MatvecArgs a = {};
+		a.w = m->wcls.m; a.x = m->x; a.n = c.dim; a.d = m->vocab_l; a.epi = EPI_STORE;
+		a.norm_w = m->rms_final; a.norm_type = m->rms_final_type; a.norm_eps = c.norm_eps; a.out = m->logits;
+		XALM_TRY(launch_matvec_batch(a, io(c.dim, m->vocab_l), s, pdl));
+		nl += 2;
+	}
+	if (n_launches) *n_launches = nl;
+	return XALM_OK;
+}
+
+// Enqueue the kernels of one step: n = 0 the single-sequence sequence, else a batched step of n entries.  With the graph knob on
+// the step is captured into a CUDA graph on first use and replayed after that.
+static int run_step(xalm_cuda_model* m, int mode, int n) {
+	cudaStream_t s = m->stream;
+	auto enqueue = [&](int* nl) { return n ? enqueue_batch(m, mode, n, s, nl) : enqueue_token(m, mode, s, nl); };
+	if (!tune("graph")) return enqueue(&m->last_launches);
+	const std::pair<int, int> key(mode, n);
+	auto it = m->graphs.find(key);
+	if (it == m->graphs.end()) {
+		cudaGraph_t g = nullptr;
+		XALM_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+		int nl = 0;
+		int rc = enqueue(&nl);
+		cudaError_t e = cudaStreamEndCapture(s, &g);
+		if (rc != XALM_OK) { if (g) cudaGraphDestroy(g); return rc; }
+		if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(e));
+		cudaGraphExec_t ge = nullptr;
+		e = cudaGraphInstantiate(&ge, g, 0);
+		cudaGraphDestroy(g);
+		if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
+		it = m->graphs.emplace(key, StepGraph{ge, nl}).first;
+	}
+	XALM_CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
+	m->last_launches = it->second.launches;
+	return XALM_OK;
+}
+
+// the next row group of the pinned StepParams ring, once the copy that last read it has run
+static int claim_step_rows(xalm_cuda_model* m, StepParams** rows) {
+	const int slot = m->step_slot;
+	m->step_slot = (slot + 1) % 64;
+	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
+	else { XALM_CUDA_CHECK(cudaEventCreateWithFlags(&m->h_step_ev[slot], cudaEventDisableTiming)); m->h_step_ev_used[slot] = true; }
+	*rows = m->h_step + (size_t) slot * m->max_seqs;
+	return XALM_OK;
+}
+
+// an entry's token, position and mode, and its ring / sink indices: infer.cpp:611-613, KV_SINKS = 2 (model.h:10)
+static void fill_step_entry(const xalm_config& c, StepParams& p, int token, int pos, int mode) {
+	p.token = token; p.pos = pos;
+	p.kv_sink = pos >= c.max_seq_len ? 2 : 0;
+	p.kv_pos = p.kv_sink + (pos - p.kv_sink) % (c.max_seq_len - p.kv_sink);
+	p.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
+	p.mode = mode;
+}
+
+// copy the first n rows of a claimed row group to the device, and mark the group free again once the copy has run
+static int upload_step_rows(xalm_cuda_model* m, const StepParams* rows, int n) {
+	const int slot = (int) ((rows - m->h_step) / m->max_seqs);
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, rows, (size_t) n * sizeof(StepParams), cudaMemcpyHostToDevice, m->stream));
+	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], m->stream));
 	return XALM_OK;
 }
 
@@ -1639,31 +1695,14 @@ int xalm_cuda_forward_async(xalm_cuda_model* m, int token, int pos, int mode) {
 	if (token < 0 || token >= c.vocab_size) return set_error(XALM_ERR_INVALID, "token %d out of range [0,%d)", token, c.vocab_size);
 	if (pos < 0) return set_error(XALM_ERR_INVALID, "negative position");
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	cudaStream_t s = m->stream;
-	// ring / sink index math: infer.cpp:611-613, KV_SINKS = 2 (model.h:10)
-	const int slot = m->step_slot;
-	m->step_slot = (slot + 1) % 64;
-	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
-	else { XALM_CUDA_CHECK(cudaEventCreateWithFlags(&m->h_step_ev[slot], cudaEventDisableTiming)); m->h_step_ev_used[slot] = true; }
-	StepParams& sp = m->h_step[(size_t) slot * m->max_seqs];
-	sp.token = token; sp.pos = pos;
-	sp.kv_sink = pos >= c.max_seq_len ? 2 : 0;
-	sp.kv_pos = sp.kv_sink + (pos - sp.kv_sink) % (c.max_seq_len - sp.kv_sink);
-	sp.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
-	sp.kv_fresh = sp.kv_pos;
-	sp.mode = mode;
-	sp.ar_base = m->token_serial * 1024u; // 2 x n_layers <= 1024 exchanges per token; wraps consistently on every rank
-	m->token_serial++;
-	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, &sp, sizeof sp, cudaMemcpyHostToDevice, s));
-	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], s));
-	if (tune("graph")) {
-		XALM_TRY(ensure_graph(m, mode));
-		XALM_CUDA_CHECK(cudaGraphLaunch(m->graph[mode], s));
-		m->last_launches = m->launches_per_token[mode];
-	} else {
-		XALM_TRY(enqueue_token(m, mode, s, &m->last_launches));
-	}
-	return XALM_OK;
+	StepParams* sp = nullptr;
+	XALM_TRY(claim_step_rows(m, &sp));
+	fill_step_entry(c, *sp, token, pos, mode);
+	sp->kv_fresh = sp->kv_pos;
+	sp->ar_base = m->token_serial++ * 1024u; // 2 x n_layers <= 1024 exchanges per token; wraps consistently on every rank
+	sp->slot = 0;                            // the single-sequence kernels address the cache of cur_seq directly
+	XALM_TRY(upload_step_rows(m, sp, 1));
+	return run_step(m, mode, 0);
 }
 
 // a tensor-parallel wait that timed out inside a kernel (a peer died): report it instead of hanging
@@ -1679,30 +1718,41 @@ int xalm_cuda_sync(xalm_cuda_model* m) {
 	return check_tp_error(m);
 }
 
-int xalm_cuda_forward(xalm_cuda_model* m, int token, int pos, int mode, float* logits_host) {
-	XALM_TRY(xalm_cuda_forward_async(m, token, pos, mode));
+// after a step of n entries (1 for the single-sequence calls): copy their logits back (logits_host may be NULL) and wait
+static int finish_step(xalm_cuda_model* m, int n, int mode, float* logits_host) {
+	const size_t bytes = (size_t) n * m->c.vocab_size * sizeof(float);
 	if (mode == XALM_OUTPUT_LOGITS && logits_host) {
-		XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_logits, m->logits_full, (size_t) m->c.vocab_size * sizeof(float), cudaMemcpyDeviceToHost, m->stream));
+		XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_logits, m->logits_full, bytes, cudaMemcpyDeviceToHost, m->stream));
 		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-		if (logits_host != m->h_logits) memcpy(logits_host, m->h_logits, (size_t) m->c.vocab_size * sizeof(float));
+		if (logits_host != m->h_logits) memcpy(logits_host, m->h_logits, bytes);
 	} else {
 		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
 	}
 	return check_tp_error(m);
 }
 
+// after a step of n entries with logits: Sampler::sample_argmax of every row on the device, next_tokens[i] for entry i
+static int finish_step_argmax(xalm_cuda_model* m, int n, int* next_tokens) {
+	argmax_rows_kernel<<<n, 1024, 0, m->stream>>>(m->logits_full, m->c.vocab_size, m->d_argmax);
+	XALM_CUDA_CHECK(cudaGetLastError());
+	// a pinned buffer of its own: the host logits buffer (InferenceState::_logits alias) stays untouched
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, (size_t) n * sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+	XALM_TRY(check_tp_error(m));
+	memcpy(next_tokens, m->h_argmax, (size_t) n * sizeof(int));
+	return XALM_OK;
+}
+
+int xalm_cuda_forward(xalm_cuda_model* m, int token, int pos, int mode, float* logits_host) {
+	XALM_TRY(xalm_cuda_forward_async(m, token, pos, mode));
+	return finish_step(m, 1, mode, logits_host);
+}
+
 // Model::forward + Sampler::sample_argmax with the sampler on the device: 4 bytes come back instead of vocab * 4
 int xalm_cuda_forward_argmax(xalm_cuda_model* m, int token, int pos, int* next_token) {
 	if (!next_token) return set_error(XALM_ERR_INVALID, "next_token is NULL");
 	XALM_TRY(xalm_cuda_forward_async(m, token, pos, XALM_OUTPUT_LOGITS));
-	argmax_kernel<<<1, 1024, 0, m->stream>>>(m->logits_full, m->c.vocab_size, m->d_argmax);
-	XALM_CUDA_CHECK(cudaGetLastError());
-	// a pinned word of its own: the host logits buffer (InferenceState::_logits alias) stays untouched
-	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-	XALM_TRY(check_tp_error(m));
-	*next_token = *m->h_argmax;
-	return XALM_OK;
+	return finish_step_argmax(m, 1, next_token);
 }
 
 // ---- batched decode: several sequence slots, one pass over the weights per step ------------------------------------------
@@ -1722,76 +1772,10 @@ int xalm_cuda_select_seq(xalm_cuda_model* m, int seq) {
 	if (seq == m->cur_seq) return XALM_OK;
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
 	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-	for (int i = 0; i < 2; i++) // the single-sequence graphs hold the previous slot's cache pointers
-		if (m->graph[i]) { cudaGraphExecDestroy(m->graph[i]); m->graph[i] = nullptr; }
+	for (auto it = m->graphs.begin(); it != m->graphs.end();) // the single-sequence graphs hold the previous slot's cache pointers
+		if (it->first.second == 0) { cudaGraphExecDestroy(it->second.exec); it = m->graphs.erase(it); }
+		else ++it;
 	m->cur_seq = seq;
-	return XALM_OK;
-}
-
-static int enqueue_batch(xalm_cuda_model* m, int mode, int n, cudaStream_t s, int* n_launches) {
-	const xalm_config& c = m->c;
-	const bool pdl = tune("pdl") != 0;
-	const int G = c.n_heads / c.n_kv_heads;
-	int nl = 0;
-	cudaError_t e = launch(embed_batch_kernel, dim3(4, n), dim3(256), s, false, m->embed_type, (const uint8_t*) m->embed_raw, m->embed_row_bytes,
-	                       c.dim, (const StepParams*) m->d_step, m->x);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "embed launch failed: %s", cudaGetErrorString(e));
-	nl++;
-	auto io = [&](int x_stride, int out_stride) { return BatchIo{n, x_stride, out_stride, m->ximg, m->nscale, m->kv_slot}; };
-	for (int l = 0; l < c.n_layers; l++) {
-		LayerDev& L = m->layers[l];
-		MatvecArgs a_qkv, a_wo, a_w13, a_w2;
-		AttnArgs a_at;
-		fill_layer_args(m, l, &a_qkv, &a_at, &a_wo, &a_w13, &a_w2);
-		a_qkv.k_cache = L.k_cache; a_qkv.v_cache = L.v_cache; // slot 0: the kernels add step[i].slot * kv_slot
-		a_at.k_cache = L.k_cache; a_at.v_cache = L.v_cache;
-		a_at.q_stride = m->q_dim_l; a_at.kv_slot = m->kv_slot;
-		if (const int pf_mb = tune("tail_prefetch_mb")) {
-			auto head = [&](const WMat& w, const uint8_t** ptr, unsigned long long* bytes) {
-				*ptr = w.p0;
-				*bytes = std::min<unsigned long long>((unsigned long long) w.s0 * (w.rows / MMA_RC), (unsigned long long) pf_mb << 20);
-			};
-			head(a_wo.w, &a_at.pf_ptr, &a_at.pf_bytes);
-			head(a_w13.w, &a_wo.pf_ptr, &a_wo.pf_bytes);
-			head(a_w2.w, &a_w13.pf_ptr, &a_w13.pf_bytes);
-			if (l + 1 < c.n_layers) head(m->layers[l + 1].wqkv.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
-			else if (mode == XALM_OUTPUT_LOGITS) head(m->wcls.m, &a_w2.pf_ptr, &a_w2.pf_bytes);
-		}
-		XALM_TRY(launch_matvec_batch(a_qkv, io(c.dim, m->q_dim_l), s, pdl));
-		XALM_TRY(launch_attn(a_at, c.head_dim, G, s, pdl, n));
-		XALM_TRY(launch_matvec_batch(a_wo, io(m->q_dim_l, c.dim), s, pdl));
-		XALM_TRY(launch_matvec_batch(a_w13, io(c.dim, m->hidden_l), s, pdl));
-		XALM_TRY(launch_matvec_batch(a_w2, io(m->hidden_l, c.dim), s, pdl));
-		nl += 9;
-	}
-	if (mode == XALM_OUTPUT_LOGITS) {
-		MatvecArgs a = {};
-		a.w = m->wcls.m; a.x = m->x; a.n = c.dim; a.d = m->vocab_l; a.epi = EPI_STORE;
-		a.norm_w = m->rms_final; a.norm_type = m->rms_final_type; a.norm_eps = c.norm_eps; a.out = m->logits;
-		XALM_TRY(launch_matvec_batch(a, io(c.dim, m->vocab_l), s, pdl));
-		nl += 2;
-	}
-	if (n_launches) *n_launches = nl;
-	return XALM_OK;
-}
-
-static int ensure_bgraph(xalm_cuda_model* m, int mode, int n) {
-	const int key = mode * 16 + n;
-	if (m->bgraph.count(key)) return XALM_OK;
-	cudaStream_t s = m->stream;
-	cudaGraph_t g = nullptr;
-	XALM_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-	int nl = 0;
-	int rc = enqueue_batch(m, mode, n, s, &nl);
-	cudaError_t e = cudaStreamEndCapture(s, &g);
-	if (rc != XALM_OK) { if (g) cudaGraphDestroy(g); return rc; }
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph capture failed: %s", cudaGetErrorString(e));
-	cudaGraphExec_t ge = nullptr;
-	e = cudaGraphInstantiate(&ge, g, 0);
-	cudaGraphDestroy(g);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "graph instantiate failed: %s", cudaGetErrorString(e));
-	m->bgraph[key] = ge;
-	m->bgraph_launches[key] = nl;
 	return XALM_OK;
 }
 
@@ -1826,56 +1810,16 @@ static int forward_step_async(xalm_cuda_model* m, int n, const int* seqs, const 
 			return set_error(XALM_ERR_INVALID, "forward_spans: the span of slot %d reaches position %d, spans stay below max_seq_len %d", s,
 			                 pos[last[s]], c.max_seq_len);
 	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	cudaStream_t st = m->stream;
-	const int slot = m->step_slot;
-	m->step_slot = (slot + 1) % 64;
-	if (m->h_step_ev_used[slot]) XALM_CUDA_CHECK(cudaEventSynchronize(m->h_step_ev[slot]));
-	else { XALM_CUDA_CHECK(cudaEventCreateWithFlags(&m->h_step_ev[slot], cudaEventDisableTiming)); m->h_step_ev_used[slot] = true; }
-	StepParams* sp = m->h_step + (size_t) slot * m->max_seqs;
-	for (int i = 0; i < n; i++) { // ring / sink index math per sequence: infer.cpp:611-613, KV_SINKS = 2 (model.h:10)
-		StepParams& p = sp[i];
-		p.token = tokens[i]; p.pos = pos[i];
-		p.kv_sink = pos[i] >= c.max_seq_len ? 2 : 0;
-		p.kv_pos = p.kv_sink + (pos[i] - p.kv_sink) % (c.max_seq_len - p.kv_sink);
-		p.kv_len = pos[i] >= c.max_seq_len ? c.max_seq_len : pos[i] + 1;
-		p.kv_fresh = sp[first[seqs[i]]].kv_pos; // == kv_pos unless an earlier entry of this step drives the same slot
-		p.mode = mode;
-		p.ar_base = 0;
-		p.slot = seqs[i];
+	StepParams* sp = nullptr;
+	XALM_TRY(claim_step_rows(m, &sp));
+	for (int i = 0; i < n; i++) {
+		fill_step_entry(c, sp[i], tokens[i], pos[i], mode);
+		sp[i].kv_fresh = sp[first[seqs[i]]].kv_pos; // == kv_pos unless an earlier entry of this step drives the same slot
+		sp[i].ar_base = 0;
+		sp[i].slot = seqs[i];
 	}
-	XALM_CUDA_CHECK(cudaMemcpyAsync(m->d_step, sp, (size_t) n * sizeof(StepParams), cudaMemcpyHostToDevice, st));
-	XALM_CUDA_CHECK(cudaEventRecord(m->h_step_ev[slot], st));
-	if (tune("graph")) {
-		XALM_TRY(ensure_bgraph(m, mode, n));
-		XALM_CUDA_CHECK(cudaGraphLaunch(m->bgraph[mode * 16 + n], st));
-		m->last_launches = m->bgraph_launches[mode * 16 + n];
-	} else {
-		XALM_TRY(enqueue_batch(m, mode, n, st, &m->last_launches));
-	}
-	return XALM_OK;
-}
-
-// after a step of n entries: copy their logits back (logits_host may be NULL) and wait
-static int finish_step(xalm_cuda_model* m, int n, int mode, float* logits_host) {
-	const size_t bytes = (size_t) n * m->c.vocab_size * sizeof(float);
-	if (mode == XALM_OUTPUT_LOGITS && logits_host) {
-		XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_logits, m->logits, bytes, cudaMemcpyDeviceToHost, m->stream));
-		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-		memcpy(logits_host, m->h_logits, bytes);
-	} else {
-		XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-	}
-	return XALM_OK;
-}
-
-// after a step of n entries with logits: Sampler::sample_argmax of every row on the device, next_tokens[i] for entry i
-static int finish_step_argmax(xalm_cuda_model* m, int n, int* next_tokens) {
-	argmax_rows_kernel<<<n, 1024, 0, m->stream>>>(m->logits, m->c.vocab_size, m->d_argmax);
-	XALM_CUDA_CHECK(cudaGetLastError());
-	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, (size_t) n * sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
-	memcpy(next_tokens, m->h_argmax, (size_t) n * sizeof(int));
-	return XALM_OK;
+	XALM_TRY(upload_step_rows(m, sp, n));
+	return run_step(m, mode, n);
 }
 
 int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode) {
@@ -2170,49 +2114,39 @@ static void fill_prefill_model(xalm_cuda_model* m, PrefillModel& pm) {
 }
 
 // ---- batched prefill / perplexity on the tensor-core path (prefill.cu); a collective under tensor parallelism --------------
+// fn names the entry point in error messages; window: past the context window (prefill_run's ring regime); sync: wait for the
+// stream (the synchronous calls also check want_logits up front, the async one leaves that to prefill_run)
+static int prefill_call(const char* fn, xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host,
+                        const int* targets, float* probs_host, bool window, bool sync) {
+	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
+	if (sync && (want_logits < 0 || want_logits > 2)) return set_error(XALM_ERR_INVALID, "%s: want_logits = %d", fn, want_logits);
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	PrefillModel pm;
+	fill_prefill_model(m, pm);
+	XALM_TRY(prefill_run(pm, &m->prefill, tokens, n, pos0, want_logits, logits_host, targets, probs_host, tune("prefill_split"),
+	                     &m->last_prefill_launches, window));
+	if (sync) {
+		cudaError_t e = cudaStreamSynchronize(m->stream);
+		if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "%s failed: %s", fn, cudaGetErrorString(e));
+	}
+	m->last_launches = m->last_prefill_launches;
+	return XALM_OK;
+}
+
 int xalm_cuda_prefill(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host, const int* targets,
                       float* probs_host) {
-	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
-	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill: want_logits = %d", want_logits);
-	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	PrefillModel pm;
-	fill_prefill_model(m, pm);
-	const int split = tune("prefill_split");
-	XALM_TRY(prefill_run(pm, &m->prefill, tokens, n, pos0, want_logits, logits_host, targets, probs_host, split, &m->last_prefill_launches));
-	cudaError_t e = cudaStreamSynchronize(m->stream);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "prefill failed: %s", cudaGetErrorString(e));
-	m->last_launches = m->last_prefill_launches;
-	return XALM_OK;
+	return prefill_call("prefill", m, tokens, n, pos0, want_logits, logits_host, targets, probs_host, false, true);
 }
 
-// past the context window: the ring regime (prefill_run's window mode)
 int xalm_cuda_prefill_window(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits, float* logits_host, const int* targets,
                              float* probs_host) {
-	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
-	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	if (want_logits < 0 || want_logits > 2) return set_error(XALM_ERR_INVALID, "prefill_window: want_logits = %d", want_logits);
-	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	PrefillModel pm;
-	fill_prefill_model(m, pm);
-	const int split = tune("prefill_split");
-	XALM_TRY(prefill_run(pm, &m->prefill, tokens, n, pos0, want_logits, logits_host, targets, probs_host, split, &m->last_prefill_launches, true));
-	cudaError_t e = cudaStreamSynchronize(m->stream);
-	if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "prefill_window failed: %s", cudaGetErrorString(e));
-	m->last_launches = m->last_prefill_launches;
-	return XALM_OK;
+	return prefill_call("prefill_window", m, tokens, n, pos0, want_logits, logits_host, targets, probs_host, true, true);
 }
 
+// same as xalm_cuda_prefill without the host synchronisation and read-back (bench.py's device-timed leg)
 int xalm_cuda_prefill_async(xalm_cuda_model* m, const int* tokens, int n, int pos0, int want_logits) {
-	if (!m || !tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
-	// same as xalm_cuda_prefill without the host synchronisation and read-back (bench.py's device-timed leg)
-	if (!m->finalized) return set_error(XALM_ERR_STATE, "prefill before finalize");
-	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	PrefillModel pm;
-	fill_prefill_model(m, pm);
-	XALM_TRY(prefill_run(pm, &m->prefill, tokens, n, pos0, want_logits, nullptr, nullptr, nullptr, tune("prefill_split"), &m->last_prefill_launches));
-	m->last_launches = m->last_prefill_launches;
-	return XALM_OK;
+	return prefill_call("prefill", m, tokens, n, pos0, want_logits, nullptr, nullptr, nullptr, false, false);
 }
 
 // out(T,N) = a(T,K) . W(N,K)^T — the batched form of matmul (model.h:315) on the tcgen05 path, host pointers in and out
@@ -2268,131 +2202,88 @@ int xalm_cuda_timeline(int n_records, unsigned long long* out, int* n_out) {
 	return XALM_OK;
 }
 
-int xalm_cuda_bench_matvec(int type_id, int n, int d, int epi, int with_norm, int n_buffers, int iters, float* ms_per_launch) {
+// Times one matvec over n_buffers rotating copies of a random weight matrix.  n_seqs = 0: the kernel the single-sequence path
+// picks for the matrix; 1..8: the batched tensor-core matvec (activation quantiser + matvec) at that many sequences.
+static int bench_matvec_run(int type_id, int n, int d, int epi, int with_norm, int n_seqs, int n_buffers, int iters, float* ms_per_launch) {
 	if (!ms_per_launch || n <= 0 || d <= 0 || n % 32 || d % 32 || n_buffers <= 0 || iters <= 0) return set_error(XALM_ERR_INVALID, "bad argument");
-	XALM_TRY(need_device());
+	if (epi != EPI_STORE && epi != EPI_GLU && epi != EPI_RESIDUAL) return set_error(XALM_ERR_INVALID, "bench epi must be 0 (store), 1 (residual) or 2 (glu)");
 	TypeInfo ti;
 	if (!type_info(type_id, &ti)) return set_error(XALM_ERR_INVALID, "invalid type: %d", type_id);
 	if (n % ti.block) return set_error(XALM_ERR_INVALID, "n %% block");
-	if (epi != EPI_STORE && epi != EPI_GLU && epi != EPI_RESIDUAL) return set_error(XALM_ERR_INVALID, "bench epi must be 0 (store), 1 (residual) or 2 (glu)");
 	const int rows = epi == EPI_GLU ? 2 * d : d;
+	if (n_seqs && !mma_takes(type_id, rows, n, epi == EPI_GLU ? d : 0))
+		return set_error(XALM_ERR_UNSUPPORTED, "the batched matvec cannot take type %d, %d x %d", type_id, rows, n);
+	XALM_TRY(need_device());
+	const int nx = n_seqs ? n_seqs : 1; // activation rows
 	DevAlloc da;
-	std::vector<WMat> ws(n_buffers);
-	const size_t raw_bytes = (size_t) rows * n / ti.block * ti.bytes;
-	// random but decodable bytes: scales must be finite f16 -> build on host once
-	std::vector<uint8_t> host(raw_bytes);
-	uint32_t st = 12345;
-	for (size_t i = 0; i < raw_bytes; i++) { st = st * 1664525u + 1013904223u; host[i] = (uint8_t) ((st >> 24) & 0x3F); }
-	int rc = XALM_OK;
 	Staging sg;
-	for (int b = 0; b < n_buffers && rc == XALM_OK; b++) {
-		rc = alloc_wmat(da, ws[b], type_id, rows, n, epi == EPI_GLU ? d : 0);
-		if (rc == XALM_OK) rc = upload_piece(ws[b], 0, type_id, host.data(), n, 0, rows, 0, n, sg, 0);
-	}
-	float *dx = nullptr, *dy = nullptr, *dg = nullptr;
-	if (rc == XALM_OK && with_norm) {
-		rc = da.alloc((void**) &dg, (size_t) n * sizeof(float));
-		if (rc == XALM_OK) {
-			std::vector<float> hg(n, 1.0f);
-			cudaMemcpy(dg, hg.data(), (size_t) n * sizeof(float), cudaMemcpyHostToDevice);
+	cudaEvent_t e0 = nullptr, e1 = nullptr;
+	cudaStream_t s = nullptr;
+	auto run = [&]() -> int {
+		std::vector<WMat> ws(n_buffers);
+		const size_t raw_bytes = (size_t) rows * n / ti.block * ti.bytes;
+		// random but decodable bytes: scales must be finite f16 -> build on host once
+		std::vector<uint8_t> host(raw_bytes);
+		uint32_t st = 12345;
+		for (size_t i = 0; i < raw_bytes; i++) { st = st * 1664525u + 1013904223u; host[i] = (uint8_t) ((st >> 24) & 0x3F); }
+		for (WMat& w : ws) {
+			XALM_TRY(alloc_wmat(da, w, type_id, rows, n, epi == EPI_GLU ? d : 0, false, n_seqs > 0));
+			XALM_TRY(upload_piece(w, 0, type_id, host.data(), n, 0, rows, 0, n, sg, 0));
 		}
-	}
-	if (rc == XALM_OK) rc = da.alloc((void**) &dx, (size_t) n * sizeof(float));
-	if (rc == XALM_OK) rc = da.alloc((void**) &dy, (size_t) d * sizeof(float));
-	if (rc == XALM_OK) {
-		std::vector<float> hx(n, 0.01f);
-		cudaMemcpy(dx, hx.data(), (size_t) n * sizeof(float), cudaMemcpyHostToDevice);
-		cudaEvent_t e0, e1;
-		cudaEventCreate(&e0); cudaEventCreate(&e1);
-		cudaStream_t s;
-		cudaStreamCreate(&s);
+		float *dx = nullptr, *dy = nullptr, *dg = nullptr, *dsc = nullptr;
+		uint8_t* img = nullptr;
+		if (with_norm) {
+			const std::vector<float> hg(n, 1.0f);
+			XALM_TRY(da.alloc((void**) &dg, (size_t) n * sizeof(float)));
+			XALM_CUDA_CHECK(cudaMemcpy(dg, hg.data(), (size_t) n * sizeof(float), cudaMemcpyHostToDevice));
+		}
+		const std::vector<float> hx((size_t) nx * n, 0.01f);
+		XALM_TRY(da.alloc((void**) &dx, hx.size() * sizeof(float)));
+		XALM_CUDA_CHECK(cudaMemcpy(dx, hx.data(), hx.size() * sizeof(float), cudaMemcpyHostToDevice));
+		XALM_TRY(da.alloc((void**) &dy, (size_t) nx * d * sizeof(float)));
+		XALM_CUDA_CHECK(cudaMemset(dy, 0, (size_t) nx * d * sizeof(float)));
+		if (n_seqs) {
+			XALM_TRY(da.alloc((void**) &dsc, (size_t) n_seqs * sizeof(float)));
+			XALM_TRY(da.alloc((void**) &img, (size_t) n / 32 * ((n_seqs + 1) / 2) * MMB_PAIR));
+		}
+		XALM_CUDA_CHECK(cudaEventCreate(&e0));
+		XALM_CUDA_CHECK(cudaEventCreate(&e1));
+		XALM_CUDA_CHECK(cudaStreamCreate(&s));
 		const bool pdl = tune("pdl") != 0;
-		for (int it = -3 * n_buffers; it < iters && rc == XALM_OK; it++) {
-			if (it == 0) cudaEventRecord(e0, s);
+		const BatchIo io = {n_seqs, n, d, img, dsc, 0};
+		for (int it = -3 * n_buffers; it < iters; it++) {
+			if (it == 0) XALM_CUDA_CHECK(cudaEventRecord(e0, s));
 			MatvecArgs a = {};
 			a.w = ws[((it % n_buffers) + n_buffers) % n_buffers]; a.x = dx; a.n = n; a.d = d; a.epi = epi; a.out = dy;
 			a.glu_off = d; a.act = XALM_SILU;
 			if (with_norm) { a.norm_w = (const uint8_t*) dg; a.norm_type = XALM_F32; a.norm_eps = 1e-5f; }
-			rc = launch_matvec(a, s, pdl);
+			XALM_TRY(n_seqs ? launch_matvec_batch(a, io, s, pdl) : launch_matvec(a, s, pdl));
 		}
-		cudaEventRecord(e1, s);
+		XALM_CUDA_CHECK(cudaEventRecord(e1, s));
 		cudaError_t e = cudaStreamSynchronize(s);
-		if (rc == XALM_OK && e != cudaSuccess) rc = set_error(XALM_ERR_CUDA, "bench failed: %s", cudaGetErrorString(e));
+		if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "bench failed: %s", cudaGetErrorString(e));
 		float ms = 0.f;
-		cudaEventElapsedTime(&ms, e0, e1);
+		XALM_CUDA_CHECK(cudaEventElapsedTime(&ms, e0, e1));
 		*ms_per_launch = ms / iters;
-		cudaEventDestroy(e0); cudaEventDestroy(e1); cudaStreamDestroy(s);
-	}
+		return XALM_OK;
+	};
+	const int rc = run();
+	if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); } // a failed launch may leave earlier ones in flight on the buffers freed below
+	if (e0) cudaEventDestroy(e0);
+	if (e1) cudaEventDestroy(e1);
 	if (sg.p) cudaFree(sg.p);
 	if (sg.flag) cudaFree(sg.flag);
 	da.free_all();
 	return rc;
 }
 
+int xalm_cuda_bench_matvec(int type_id, int n, int d, int epi, int with_norm, int n_buffers, int iters, float* ms_per_launch) {
+	return bench_matvec_run(type_id, n, d, epi, with_norm, 0, n_buffers, iters, ms_per_launch);
+}
+
 int xalm_cuda_bench_matvec_batch(int type_id, int n, int d, int epi, int with_norm, int n_seqs, int n_buffers, int iters, float* ms_per_launch) {
-	if (!ms_per_launch || n <= 0 || d <= 0 || n % 32 || d % 32 || n_buffers <= 0 || iters <= 0 || n_seqs < 1 || n_seqs > MMB_MAX_SEQS)
-		return set_error(XALM_ERR_INVALID, "bad argument");
-	if (epi != EPI_STORE && epi != EPI_GLU && epi != EPI_RESIDUAL) return set_error(XALM_ERR_INVALID, "bench epi must be 0 (store), 1 (residual) or 2 (glu)");
-	TypeInfo ti;
-	if (!type_info(type_id, &ti)) return set_error(XALM_ERR_INVALID, "invalid type: %d", type_id);
-	const int rows = epi == EPI_GLU ? 2 * d : d;
-	if (!mma_takes(type_id, rows, n, epi == EPI_GLU ? d : 0)) return set_error(XALM_ERR_UNSUPPORTED, "the batched matvec cannot take type %d, %d x %d", type_id, rows, n);
-	XALM_TRY(need_device());
-	DevAlloc da;
-	std::vector<WMat> ws(n_buffers);
-	const size_t raw_bytes = (size_t) rows * n / ti.block * ti.bytes;
-	std::vector<uint8_t> host(raw_bytes);
-	uint32_t st = 12345;
-	for (size_t i = 0; i < raw_bytes; i++) { st = st * 1664525u + 1013904223u; host[i] = (uint8_t) ((st >> 24) & 0x3F); }
-	int rc = XALM_OK;
-	Staging sg;
-	for (int b = 0; b < n_buffers && rc == XALM_OK; b++) {
-		rc = alloc_wmat(da, ws[b], type_id, rows, n, epi == EPI_GLU ? d : 0, false, true);
-		if (rc == XALM_OK) rc = upload_piece(ws[b], 0, type_id, host.data(), n, 0, rows, 0, n, sg, 0);
-	}
-	float *dx = nullptr, *dy = nullptr, *dg = nullptr, *dsc = nullptr;
-	uint8_t* img = nullptr;
-	if (rc == XALM_OK && with_norm) {
-		rc = da.alloc((void**) &dg, (size_t) n * sizeof(float));
-		if (rc == XALM_OK) {
-			std::vector<float> hg(n, 1.0f);
-			cudaMemcpy(dg, hg.data(), (size_t) n * sizeof(float), cudaMemcpyHostToDevice);
-		}
-	}
-	if (rc == XALM_OK) rc = da.alloc((void**) &dx, (size_t) n_seqs * n * sizeof(float));
-	if (rc == XALM_OK) rc = da.alloc((void**) &dy, (size_t) n_seqs * d * sizeof(float));
-	if (rc == XALM_OK) rc = da.alloc((void**) &dsc, (size_t) n_seqs * sizeof(float));
-	if (rc == XALM_OK) rc = da.alloc((void**) &img, (size_t) n / 32 * ((n_seqs + 1) / 2) * MMB_PAIR);
-	if (rc == XALM_OK) {
-		std::vector<float> hx((size_t) n_seqs * n, 0.01f);
-		cudaMemcpy(dx, hx.data(), hx.size() * sizeof(float), cudaMemcpyHostToDevice);
-		cudaMemset(dy, 0, (size_t) n_seqs * d * sizeof(float));
-		cudaEvent_t e0, e1;
-		cudaEventCreate(&e0); cudaEventCreate(&e1);
-		cudaStream_t s;
-		cudaStreamCreate(&s);
-		const bool pdl = tune("pdl") != 0;
-		const BatchIo io = {n_seqs, n, d, img, dsc, 0};
-		for (int it = -3 * n_buffers; it < iters && rc == XALM_OK; it++) {
-			if (it == 0) cudaEventRecord(e0, s);
-			MatvecArgs a = {};
-			a.w = ws[((it % n_buffers) + n_buffers) % n_buffers]; a.x = dx; a.n = n; a.d = d; a.epi = epi; a.out = dy;
-			a.glu_off = d; a.act = XALM_SILU;
-			if (with_norm) { a.norm_w = (const uint8_t*) dg; a.norm_type = XALM_F32; a.norm_eps = 1e-5f; }
-			rc = launch_matvec_batch(a, io, s, pdl);
-		}
-		cudaEventRecord(e1, s);
-		cudaError_t e = cudaStreamSynchronize(s);
-		if (rc == XALM_OK && e != cudaSuccess) rc = set_error(XALM_ERR_CUDA, "bench failed: %s", cudaGetErrorString(e));
-		float ms = 0.f;
-		cudaEventElapsedTime(&ms, e0, e1);
-		*ms_per_launch = ms / iters;
-		cudaEventDestroy(e0); cudaEventDestroy(e1); cudaStreamDestroy(s);
-	}
-	if (sg.p) cudaFree(sg.p);
-	if (sg.flag) cudaFree(sg.flag);
-	da.free_all();
-	return rc;
+	if (n_seqs < 1 || n_seqs > MMB_MAX_SEQS) return set_error(XALM_ERR_INVALID, "bad argument");
+	return bench_matvec_run(type_id, n, d, epi, with_norm, n_seqs, n_buffers, iters, ms_per_launch);
 }
 
 } // extern "C"
