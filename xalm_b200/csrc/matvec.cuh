@@ -60,10 +60,10 @@ struct MatvecArgs {
 	// activation loads issued after them return in order behind them (profiles/r2_decode_timeline.md)
 	const uint8_t* pf_norm_ptr;
 	unsigned int pf_norm_bytes;
-	// tensor-parallel exchange fused into the matvec kernels (matvec_tma.cuh), LL style: the row-split matvecs (Wo, W2) PUSH every
-	// partial row as an 8-byte {value, sequence tag} word straight into every rank's receive slot over NVLink (posted stores, no
-	// fence, no flag, no extra kernel); the next kernel's rmsnorm prologue polls the tags of the words it needs and adds the
-	// partials (fixed rank order) to the residual stream.
+	// tensor-parallel exchange fused into the matvec kernels, LL style: the row-split matvecs (Wo, W2) PUSH every partial row as
+	// an 8-byte {value, sequence tag} word straight into every rank's receive slot over NVLink (posted stores, no fence, no flag,
+	// no extra kernel); the next kernel's rmsnorm prologue polls the tags of the words it needs and adds the partials (fixed rank
+	// order) to the residual stream (tp_receive).
 	uint2* push_dst[8];          // per destination rank: its receive slot for THIS rank's partial, (dim,) {float bits, tag}
 	int n_push;                  // 0 = off
 	int push_idx;                // exchange index inside the token: tag = step->ar_base + push_idx + 1
@@ -73,9 +73,6 @@ struct MatvecArgs {
 	float* x_out;                // the first CTAs store x + sum(partials) here: the residual stream after the exchange
 	unsigned int* err_flag;      // set to 1 when a wait for a peer's words times out (the host turns it into XALM_ERR_COMM)
 	uint2* xl;                   // local (dim,) {value, tag} words: the reducing CTAs publish the summed stream here, every CTA polls it
-	// L2 prefetcher hand-shake (prefetch.cuh): block 0 publishes "kernel #prog_idx of this token has started"
-	unsigned int* progress;
-	int prog_idx;
 };
 
 __device__ __forceinline__ float act_gelu(float x) { return 0.5f * x * (1.0f + tanhf(0.797885f * (x + 0.044715f * x * x * x))); }
@@ -93,15 +90,38 @@ __device__ __forceinline__ void rope_pair(float& v0, float& v1, int j_head, int 
 	v1 = a * fci + b * fcr;
 }
 
-// Re-rotate the kv_sink attention-sink keys by one position, through fp16 (infer.cpp:421-431).
-__device__ inline void rotate_sinks(const MatvecArgs& a, int kv_sink) {
+// Re-rotate the kv_sink attention-sink keys of k_cache by one position, through fp16 (infer.cpp:421-431).  Threads tid = 0 .. nt-1
+// of the block share the work: in the warp-specialised kernels nt is the consumer thread count, not blockDim.x, because their
+// producer warp has returned by then.
+__device__ __forceinline__ void rotate_sinks(const MatvecArgs& a, __half* k_cache, int kv_sink, int tid, int nt) {
 	const int pairs = a.kv_dim / 2;
-	for (int i = threadIdx.x; i < kv_sink * pairs; i += blockDim.x) {
+	for (int i = tid; i < kv_sink * pairs; i += nt) {
 		const int r = i / pairs, p = i % pairs;
-		__half2* kp = reinterpret_cast<__half2*>(a.k_cache + (size_t) r * a.kv_dim) + p;
+		__half2* kp = reinterpret_cast<__half2*>(k_cache + (size_t) r * a.kv_dim) + p;
 		float2 v = __half22float2(*kp);
 		rope_pair(v.x, v.y, (2 * p) % a.head_dim, 1, a.rope_freq);
 		*kp = __floats2half2_rn(v.x, v.y);
+	}
+}
+
+// One QKV output pair (row, row + 1) of the sequence sp, row even: clip -> RoPE(q, k) -> q fp32 into out, k / v fp16 into the KV
+// ring of slot sp.slot at sp.kv_pos (infer.cpp:388-420).  kv_slot = elements between two slots' caches (0: one cache).
+__device__ __forceinline__ void qkv_pair(const MatvecArgs& a, const StepParams& sp, size_t kv_slot, float* out, int row, float y0, float y1) {
+	const int pos = sp.pos, kv_pos = sp.kv_pos;
+	float v0 = clipf(y0, a.qkv_clip), v1 = clipf(y1, a.qkv_clip);
+	if (row < a.q_dim) {
+		rope_pair(v0, v1, row % a.head_dim, pos, a.rope_freq);
+		out[row] = v0;
+		out[row + 1] = v1;
+	} else if (row < a.q_dim + a.kv_dim) {
+		const int i = row - a.q_dim;
+		rope_pair(v0, v1, i % a.head_dim, pos, a.rope_freq);
+		__half* kc = a.k_cache + (size_t) sp.slot * kv_slot;
+		*reinterpret_cast<__half2*>(kc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
+	} else {
+		const int i = row - a.q_dim - a.kv_dim;
+		__half* vc = a.v_cache + (size_t) sp.slot * kv_slot;
+		*reinterpret_cast<__half2*>(vc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
 	}
 }
 
@@ -127,24 +147,137 @@ __device__ __forceinline__ void epilogue(const MatvecArgs& a, int row0, const fl
 			}
 		}
 	} else { // EPI_QKV
-		const int pos = a.step->pos, kv_pos = a.step->kv_pos;
+		const StepParams sp = *a.step;
 #pragma unroll
 		for (int r = 0; r < R; r += 2) {
 			const int row = row0 + r;
 			if (row >= a.d) break;
-			float v0 = clipf(y[r], a.qkv_clip), v1 = clipf(y[r + 1], a.qkv_clip);
-			if (row < a.q_dim) {
-				rope_pair(v0, v1, row % a.head_dim, pos, a.rope_freq);
-				a.out[row] = v0;
-				a.out[row + 1] = v1;
-			} else if (row < a.q_dim + a.kv_dim) {
-				const int i = row - a.q_dim;
-				rope_pair(v0, v1, i % a.head_dim, pos, a.rope_freq);
-				*reinterpret_cast<__half2*>(a.k_cache + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
-			} else {
-				const int i = row - a.q_dim - a.kv_dim;
-				*reinterpret_cast<__half2*>(a.v_cache + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
-			}
+			qkv_pair(a, sp, 0, a.out, row, y[r], y[r + 1]);
+		}
+	}
+}
+
+// ---- shared by the warp-specialised kernels (matvec_tma.cuh, matvec_idp.cuh, matvec_mma.cuh) ---------------------------------------
+
+constexpr unsigned int XALM_SPIN_LIMIT = 1u << 23; // polls of a tagged word (~1 us each) before a tensor-parallel wait gives up
+
+// Four consecutive {value, tag} words: poll until all carry the exchange's tag seq and return the values.  A peer that never
+// writes them has died: after XALM_SPIN_LIMIT polls set *err_flag (the host turns it into XALM_ERR_COMM) instead of hanging the GPU.
+__device__ __forceinline__ float4 poll_tagged4(const uint2* src, unsigned int seq, unsigned int* err_flag) {
+	uint4 w0, w1;
+	unsigned int spins = 0;
+	do {
+		asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src));
+		asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 2));
+		if (++spins > XALM_SPIN_LIMIT) { if (err_flag) *err_flag = 1u; break; }
+	} while (w0.y != seq || w0.w != seq || w1.y != seq || w1.w != seq);
+	return make_float4(__uint_as_float(w0.x), __uint_as_float(w0.z), __uint_as_float(w1.x), __uint_as_float(w1.z));
+}
+
+// Tensor-parallel receive (LL style), run by the nt consumer threads of a norm-fused kernel with n_recv set: the first min(grid, 8)
+// CTAs each reduce a slice of the stream — x += sum over ranks of the partial rows the previous row-split matvec pushed here (rank
+// order: identical bits on every rank; infer.cpp:450-452 / :492-494) — store it to x_out and publish it locally as {value, tag}
+// words, so every other CTA reads dim words instead of n_ranks x dim.
+__device__ __forceinline__ void tp_receive(const MatvecArgs& a, int tid, int nt) {
+	const int n_red = min((int) gridDim.x, 8);
+	if ((int) blockIdx.x >= n_red) return;
+	const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
+	const int chunk = ((a.n / 4 + n_red - 1) / n_red) * 4;
+	const int i0 = (int) blockIdx.x * chunk, i1 = min(a.n, i0 + chunk);
+	for (int i = i0 + tid * 4; i < i1; i += nt * 4) {
+		float4 v = ld_act4(a.x + i);
+		float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
+		for (int p = 0; p < a.n_recv; p++) {
+			const float4 w = poll_tagged4(a.recv + (size_t) p * a.n + i, seq, a.err_flag);
+			sum.x += w.x; sum.y += w.y; sum.z += w.z; sum.w += w.w;
+		}
+		v.x += sum.x; v.y += sum.y; v.z += sum.z; v.w += sum.w;
+		*reinterpret_cast<float4*>(a.x_out + i) = v;
+		*reinterpret_cast<uint4*>(a.xl + i) = make_uint4(__float_as_uint(v.x), seq, __float_as_uint(v.y), seq);
+		*reinterpret_cast<uint4*>(a.xl + i + 2) = make_uint4(__float_as_uint(v.z), seq, __float_as_uint(v.w), seq);
+	}
+}
+
+// The staging input x[8 grp .. 8 grp + 8): with recv, the summed stream the reducing CTAs publish as {value, tag} words (poll this
+// exchange's tag), else x itself
+__device__ __forceinline__ void load_x8(const MatvecArgs& a, int grp, bool recv, float (&v)[8]) {
+	float4 q0, q1;
+	if (recv) {
+		const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
+		q0 = poll_tagged4(a.xl + grp * 8, seq, a.err_flag);
+		q1 = poll_tagged4(a.xl + grp * 8 + 4, seq, a.err_flag);
+	} else {
+		q0 = ld_act4(a.x + grp * 8);
+		q1 = ld_act4(a.x + grp * 8 + 4);
+	}
+	v[0] = q0.x; v[1] = q0.y; v[2] = q0.z; v[3] = q0.w;
+	v[4] = q1.x; v[5] = q1.y; v[6] = q1.z; v[7] = q1.w;
+}
+
+// rmsnorm weights of the 8-element group grp, raw: two uint4 of F32, or one of BF16
+__device__ __forceinline__ void load_norm8(const uint8_t* norm_w, int norm_type, int grp, uint4 (&gw)[2]) {
+	if (norm_type == XALM_F32) {
+		gw[0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(norm_w) + grp * 8);
+		gw[1] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(norm_w) + grp * 8 + 4);
+	} else {
+		gw[0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(norm_w) + grp * 8);
+	}
+}
+// element e of a group load_norm8 fetched
+__device__ __forceinline__ float norm_weight(const uint4 (&gw)[2], int norm_type, int e) {
+	if (norm_type == XALM_F32) {
+		const uint4 q = gw[e >> 2];
+		return __uint_as_float((e & 3) == 0 ? q.x : (e & 3) == 1 ? q.y : (e & 3) == 2 ? q.z : q.w);
+	}
+	const uint4 q = gw[0];
+	const int h = e >> 1;
+	const uint32_t u = h == 0 ? q.x : h == 1 ? q.y : h == 2 ? q.z : q.w;
+	return __uint_as_float((e & 1) ? (u & 0xFFFF0000u) : (u << 16));
+}
+
+// Producer warp, at entry: CTA 0 pulls the next norm-fused kernel's rmsnorm weights into L2 (pf_norm_ptr)
+__device__ __forceinline__ void prefetch_next_norm(const MatvecArgs& a) {
+	if (blockIdx.x == 0 && a.pf_norm_ptr && a.pf_norm_bytes >= 16)
+		asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.pf_norm_ptr), "r"(a.pf_norm_bytes & ~15u) : "memory");
+}
+// Producer warp, after its last weight load: this CTA's slice of the next kernel's weights and, with kv and pf_kv set, of the K/V
+// rows the attention kernel after QKV reads
+__device__ __forceinline__ void prefetch_tail(const MatvecArgs& a, bool kv) {
+	l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
+	if (kv && a.pf_kv) {
+		const unsigned long long kvb = (unsigned long long) a.step->kv_len * a.kv_dim * sizeof(__half);
+		l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.k_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
+		l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.v_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
+	}
+}
+
+// Epilogue of a finished tile of RC rows, run by one whole warp: lane i < RC holds the sum yv of row row0 + i and, for EPI_RESIDUAL,
+// the old activation xold of that row.  GLU pairs the W1 row of lane i with the W3 row RC/2 lanes up; otherwise even lanes hand a
+// row pair to epilogue<2> (RoPE needs both) or, tensor parallel, push it to every rank.
+template <int RC>
+__device__ __forceinline__ void row_epilogue(const MatvecArgs& a, int row0, int lane, float yv, float xold) {
+	const float ynext = __shfl_down_sync(0xffffffffu, yv, 1);
+	if (a.epi == EPI_GLU) {
+		const float ypart = __shfl_down_sync(0xffffffffu, yv, RC / 2); // W3 value for the W1 row in this lane
+		const int o = row0 / 2 + lane;
+		if (lane < RC / 2 && o < a.d) {
+			const float g = a.act == XALM_SILU ? act_silu(yv) : act_gelu(yv);
+			a.out[o] = g * ypart;
+		}
+		return;
+	}
+	const int row = row0 + lane;
+	if (lane >= RC || row >= a.d) return;
+	if (a.epi == EPI_RESIDUAL) {
+		a.out[row] = xold + yv;
+	} else if ((lane & 1) == 0) {
+		if (a.epi == EPI_STORE && a.n_push) { // tensor parallel: this rank's partial rows go to every rank (NVLink stores)
+			const unsigned int seq = a.step->ar_base + (unsigned int) a.push_idx + 1u;
+			const uint4 w = make_uint4(__float_as_uint(yv), seq, __float_as_uint(ynext), seq);
+			for (int p = 0; p < a.n_push; p++) *reinterpret_cast<uint4*>(a.push_dst[p] + row) = w;
+		} else {
+			const float y2[2] = {yv, ynext};
+			epilogue<2>(a, row, y2);
 		}
 	}
 }
@@ -181,10 +314,7 @@ __global__ void __launch_bounds__(NW * 32) matvec_kernel(const MatvecArgs a) {
 
 	pdl_launch_dependents();
 	int tl = -1;
-	if (blockIdx.x == 0 && threadIdx.x == 0) {
-		tl = tl_begin(200 + a.epi);
-		if (a.progress) *reinterpret_cast<volatile unsigned int*>(a.progress) = (unsigned int) a.prog_idx;
-	}
+	if (blockIdx.x == 0 && threadIdx.x == 0) tl = tl_begin(200 + a.epi);
 
 	RowPtr rp[R];
 #pragma unroll
@@ -209,7 +339,7 @@ __global__ void __launch_bounds__(NW * 32) matvec_kernel(const MatvecArgs a) {
 	pdl_wait(); // activations (and the KV ring) written by earlier kernels are visible from here on
 	tl_mark(tl, 2);
 
-	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.step->kv_sink);
+	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.k_cache, a.step->kv_sink, threadIdx.x, blockDim.x);
 
 	// ---- rmsnorm prologue: every CTA recomputes the scale (n floats from L1/L2, hidden under the weight fetch) ----
 	float scale = 1.0f;
@@ -322,9 +452,8 @@ __global__ void __launch_bounds__(NW * 32) matvec_tq1_kernel(const MatvecArgs a)
 	const int row0 = (blockIdx.x * NW + warp) * R;
 	const bool active = row0 < vrows;
 	pdl_launch_dependents();
-	if (blockIdx.x == 0 && threadIdx.x == 0 && a.progress) *reinterpret_cast<volatile unsigned int*>(a.progress) = (unsigned int) a.prog_idx;
 	pdl_wait();
-	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.step->kv_sink);
+	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.k_cache, a.step->kv_sink, threadIdx.x, blockDim.x);
 	float scale = 1.0f;
 	if (NORM) {
 		float ss = 0.f;

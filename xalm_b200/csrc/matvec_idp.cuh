@@ -54,7 +54,7 @@ __global__ void __maxnreg__(96) matvec_idp_kernel(const IdpArgs ta) {
 	constexpr int SLOT = RC * ROW_STAGE;
 	const MatvecArgs& a = ta.a;
 	const int NS = ta.NS, PB = idp_pb(ta.NS);
-	const int n = a.n, nu = n / 256, nb_row = n / 32;
+	const int n = a.n, nu = n / 256;
 	const int kranges = (nu + U - 1) / U;
 
 	extern __shared__ __align__(128) uint8_t smem[];
@@ -85,8 +85,7 @@ __global__ void __maxnreg__(96) matvec_idp_kernel(const IdpArgs ta) {
 	if (warp == NCW) {
 		// ===================== producer: weights only — runs ahead of griddepcontrol.wait =====================
 		if (lane == 0) {
-			if (blockIdx.x == 0 && a.pf_norm_ptr && a.pf_norm_bytes >= 16)
-				asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.pf_norm_ptr), "r"(a.pf_norm_bytes & ~15u) : "memory");
+			prefetch_next_norm(a);
 			int slot = 0, phase = 0;
 			for (int tt = 0; tt < my_tiles; tt++) {
 				const int row0 = ((int) blockIdx.x + tt * (int) gridDim.x) * RC;
@@ -118,12 +117,7 @@ __global__ void __maxnreg__(96) matvec_idp_kernel(const IdpArgs ta) {
 					if (++slot == NS) { slot = 0; phase ^= 1; }
 				}
 			}
-			l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
-			if (a.pf_kv) {
-				const unsigned long long kvb = (unsigned long long) a.step->kv_len * a.kv_dim * sizeof(__half);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.k_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.v_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-			}
+			prefetch_tail(a, true);
 		}
 		return;
 	}
@@ -139,141 +133,62 @@ __global__ void __maxnreg__(96) matvec_idp_kernel(const IdpArgs ta) {
 #pragma unroll
 		for (int p = 0; p < MP; p++) {
 			const int grp = p * NT + tid;
-			if (grp < ngrp) {
-				if (a.norm_type == XALM_F32) {
-					gw[p][0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(a.norm_w) + grp * 8);
-					gw[p][1] = *reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(a.norm_w) + grp * 8 + 4);
-				} else {
-					gw[p][0] = *reinterpret_cast<const uint4*>(reinterpret_cast<const uint16_t*>(a.norm_w) + grp * 8);
-				}
-			}
+			if (grp < ngrp) load_norm8(a.norm_w, a.norm_type, grp, gw[p]);
 		}
 	}
 	pdl_wait(); // activations / KV ring of earlier kernels are visible from here on
 	tl_mark(tl, 2);
-	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) {
-		const int pairs = a.kv_dim / 2;
-		for (int i = threadIdx.x; i < a.step->kv_sink * pairs; i += NT) {
-			const int r = i / pairs, p = i % pairs;
-			__half2* kp = reinterpret_cast<__half2*>(a.k_cache + (size_t) r * a.kv_dim) + p;
-			float2 v = __half22float2(*kp);
-			rope_pair(v.x, v.y, (2 * p) % a.head_dim, 1, a.rope_freq);
-			*kp = __floats2half2_rn(v.x, v.y);
-		}
-	}
-	// ---- tensor-parallel receive (LL style), as in matvec_tma_kernel: the first CTAs each reduce a slice of the stream and publish
-	//      it locally as {value, tag} words ----
-	if (NORM && a.n_recv) {
-		const int n_red = min((int) gridDim.x, 8);
-		if ((int) blockIdx.x < n_red) {
-			const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
-			const int chunk = ((n / 4 + n_red - 1) / n_red) * 4;
-			const int i0 = (int) blockIdx.x * chunk, i1 = min(n, i0 + chunk);
-			for (int i = i0 + (int) threadIdx.x * 4; i < i1; i += NT * 4) {
-				float4 v = ld_act4(a.x + i);
-				float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
-				for (int p = 0; p < a.n_recv; p++) {
-					const uint2* src = a.recv + (size_t) p * n + i; // four {value, tag} words; poll until all carry this exchange's tag
-					uint4 w0, w1;
-					unsigned int spins = 0;
-					do {
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src));
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 2));
-						if (++spins > XALM_SPIN_LIMIT) { if (a.err_flag) *a.err_flag = 1u; break; } // a peer died: report, do not hang the GPU
-					} while (w0.y != seq || w0.w != seq || w1.y != seq || w1.w != seq);
-					sum.x += __uint_as_float(w0.x); sum.y += __uint_as_float(w0.z); sum.z += __uint_as_float(w1.x); sum.w += __uint_as_float(w1.z);
-				}
-				v.x += sum.x; v.y += sum.y; v.z += sum.z; v.w += sum.w;
-				*reinterpret_cast<float4*>(a.x_out + i) = v;
-				*reinterpret_cast<uint4*>(a.xl + i) = make_uint4(__float_as_uint(v.x), seq, __float_as_uint(v.y), seq);
-				*reinterpret_cast<uint4*>(a.xl + i + 2) = make_uint4(__float_as_uint(v.z), seq, __float_as_uint(v.w), seq);
-			}
-		}
-	}
+	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.k_cache, a.step->kv_sink, tid, NT);
+	if (NORM && a.n_recv) tp_receive(a, tid, NT);
 	// ---- stage activations: xq = quantise(NORM ? x * scale * g : x) ----
 	const XqView xv = xq_view(xq_base, n);
-	{
-		auto load_group = [&](int grp, float (&v)[8]) {
-			if (NORM && a.n_recv) { // the summed stream, published by the reducing CTAs as {value, tag} words: poll this exchange's tag
-				const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
+	if (NORM) {
+		float xr[MP][8];
+		float ss = 0.f;
 #pragma unroll
-				for (int c = 0; c < 2; c++) {
-					const uint2* src = a.xl + grp * 8 + 4 * c;
-					uint4 w0, w1;
-					unsigned int spins = 0;
-					do {
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src));
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 2));
-						if (++spins > XALM_SPIN_LIMIT) { if (a.err_flag) *a.err_flag = 1u; break; }
-					} while (w0.y != seq || w0.w != seq || w1.y != seq || w1.w != seq);
-					v[4 * c] = __uint_as_float(w0.x); v[4 * c + 1] = __uint_as_float(w0.z); v[4 * c + 2] = __uint_as_float(w1.x); v[4 * c + 3] = __uint_as_float(w1.z);
-				}
-			} else {
-				const float4 q0 = ld_act4(a.x + grp * 8), q1 = ld_act4(a.x + grp * 8 + 4);
-				v[0] = q0.x; v[1] = q0.y; v[2] = q0.z; v[3] = q0.w;
-				v[4] = q1.x; v[5] = q1.y; v[6] = q1.z; v[7] = q1.w;
-			}
-		};
-		if (NORM) {
-			float xr[MP][8];
-			float ss = 0.f;
+		for (int p = 0; p < MP; p++) {
+			const int grp = p * NT + tid;
+			if (grp < ngrp) load_x8(a, grp, NORM && a.n_recv, xr[p]);
+		}
 #pragma unroll
-			for (int p = 0; p < MP; p++) {
-				const int grp = p * NT + tid;
-				if (grp < ngrp) load_group(grp, xr[p]);
-			}
+		for (int p = 0; p < MP; p++) {
+			const int grp = p * NT + tid;
+			if (grp < ngrp) {
 #pragma unroll
-			for (int p = 0; p < MP; p++) {
-				const int grp = p * NT + tid;
-				if (grp < ngrp) {
-#pragma unroll
-					for (int e = 0; e < 8; e++) ss += xr[p][e] * xr[p][e];
-				}
-			}
-			ss = warp_sum(ss);
-			if (tl >= 0) tl_begin(600 + a.epi); // event: x arrived
-			if (lane == 0) s_red[warp] = ss;
-			// The staged vector is x * g; the scalar 1/rms is applied to the row sums in the epilogue (y = scale * sum w * (x * g)), so
-			// the staging does not wait for the CTA-wide sum of squares: one barrier instead of two between x arriving and the first tile
-#pragma unroll
-			for (int p = 0; p < MP; p++) {
-				const int grp = p * NT + tid;
-				if (grp < ngrp) { // (warp-uniform: n % 256 == 0)
-#pragma unroll
-					for (int e = 0; e < 8; e++) {
-						float g;
-						if (a.norm_type == XALM_F32) {
-							const uint4 q = gw[p][e >> 2];
-							g = __uint_as_float((e & 3) == 0 ? q.x : (e & 3) == 1 ? q.y : (e & 3) == 2 ? q.z : q.w);
-						} else {
-							const uint4 q = gw[p][0];
-							const int h = e >> 1;
-							const uint32_t u = h == 0 ? q.x : h == 1 ? q.y : h == 2 ? q.z : q.w;
-							g = __uint_as_float((e & 1) ? (u & 0xFFFF0000u) : (u << 16));
-						}
-						xr[p][e] = xr[p][e] * g; // infer.cpp:233-235 without the scalar
-					}
-					xq_store_group8(xv, grp, xr[p]);
-				}
-			}
-		} else {
-			constexpr int UNR = 4; // groups in flight per lane (n = 14336 on 512 threads: one round of loads)
-			for (int base = 0; base < ngrp; base += UNR * NT) {
-				float xr[UNR][8];
-#pragma unroll
-				for (int p = 0; p < UNR; p++) {
-					const int grp = base + p * NT + tid;
-					if (grp < ngrp) load_group(grp, xr[p]);
-				}
-#pragma unroll
-				for (int p = 0; p < UNR; p++) {
-					const int grp = base + p * NT + tid;
-					if (grp < ngrp) xq_store_group8(xv, grp, xr[p]);
-				}
+				for (int e = 0; e < 8; e++) ss += xr[p][e] * xr[p][e];
 			}
 		}
-		cbar();
+		ss = warp_sum(ss);
+		if (tl >= 0) tl_begin(600 + a.epi); // event: x arrived
+		if (lane == 0) s_red[warp] = ss;
+		// The staged vector is x * g; the scalar 1/rms is applied to the row sums in the epilogue (y = scale * sum w * (x * g)), so
+		// the staging does not wait for the CTA-wide sum of squares: one barrier instead of two between x arriving and the first tile
+#pragma unroll
+		for (int p = 0; p < MP; p++) {
+			const int grp = p * NT + tid;
+			if (grp < ngrp) { // (warp-uniform: n % 256 == 0)
+#pragma unroll
+				for (int e = 0; e < 8; e++) xr[p][e] = xr[p][e] * norm_weight(gw[p], a.norm_type, e); // infer.cpp:233-235 without the scalar
+				xq_store_group8(xv, grp, xr[p]);
+			}
+		}
+	} else {
+		constexpr int UNR = 4; // groups in flight per lane (n = 14336 on 512 threads: one round of loads)
+		for (int base = 0; base < ngrp; base += UNR * NT) {
+			float xr[UNR][8];
+#pragma unroll
+			for (int p = 0; p < UNR; p++) {
+				const int grp = base + p * NT + tid;
+				if (grp < ngrp) load_x8(a, grp, NORM && a.n_recv, xr[p]);
+			}
+#pragma unroll
+			for (int p = 0; p < UNR; p++) {
+				const int grp = base + p * NT + tid;
+				if (grp < ngrp) xq_store_group8(xv, grp, xr[p]);
+			}
+		}
 	}
+	cbar();
 	float nscale = 1.f; // 1/rms of the input (infer.cpp:229-232), applied to the row sums
 	if (NORM) {
 		float tot = 0.f;
@@ -351,29 +266,7 @@ __global__ void __maxnreg__(96) matvec_idp_kernel(const IdpArgs ta) {
 				}
 			}
 			if (NORM) yv *= nscale;
-			const float ynext = __shfl_down_sync(0xffffffffu, yv, 1);
-			if (a.epi == EPI_RESIDUAL) {
-				if (lane < RC && row0 + lane < a.d) a.out[row0 + lane] = xold + yv;
-			} else if (a.epi == EPI_STORE && a.n_push) { // tensor parallel: this rank's partial rows go to every rank (NVLink stores)
-				if (lane < RC && (lane & 1) == 0 && row0 + lane < a.d) {
-					const unsigned int seq = a.step->ar_base + (unsigned int) a.push_idx + 1u;
-					const uint4 w = make_uint4(__float_as_uint(yv), seq, __float_as_uint(ynext), seq);
-					for (int p = 0; p < a.n_push; p++) *reinterpret_cast<uint4*>(a.push_dst[p] + row0 + lane) = w;
-				}
-			} else if (lane < RC && (lane & 1) == 0 && a.epi != EPI_GLU) { // GLU below (partner rows RC/2 apart)
-				const float y2[2] = {yv, ynext};
-				epilogue<2>(a, row0 + lane, y2);
-			}
-			if (a.epi == EPI_GLU) {
-				const float ypart = __shfl_down_sync(0xffffffffu, yv, RC / 2); // W3 value for the W1 row in this lane
-				if (lane < RC / 2) {
-					const int o = row0 / 2 + lane;
-					if (o < a.d) {
-						const float g = a.act == XALM_SILU ? act_silu(yv) : act_gelu(yv);
-						a.out[o] = g * ypart;
-					}
-				}
-			}
+			row_epilogue<RC>(a, row0, lane, yv, xold);
 		}
 	}
 	tl_mark(tl, 3);

@@ -260,8 +260,7 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_kernel(const
 	if (warp == NCW) {
 		// ===================== producer: weights only — runs ahead of griddepcontrol.wait =====================
 		if (lane == 0) {
-			if (blockIdx.x == 0 && a.pf_norm_ptr && a.pf_norm_bytes >= 16)
-				asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.pf_norm_ptr), "r"(a.pf_norm_bytes & ~15u) : "memory");
+			prefetch_next_norm(a);
 			int slot = 0, phase = 0;
 			for (int tt = 0; tt < my_tiles; tt++) {
 				const uint8_t* tile = a.w.p0 + (size_t) ((int) blockIdx.x + tt * (int) gridDim.x) * a.w.s0;
@@ -273,12 +272,7 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_kernel(const
 					if (++slot == NS) { slot = 0; phase ^= 1; }
 				}
 			}
-			l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
-			if (a.pf_kv) {
-				const unsigned long long kvb = (unsigned long long) a.step->kv_len * a.kv_dim * sizeof(__half);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.k_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.v_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-			}
+			prefetch_tail(a, true);
 		}
 		return;
 	}
@@ -751,7 +745,7 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_batch_kernel
 				bulk_g2s(ring + (size_t) slot * STAGE, src, wb, &full[slot]);
 				bulk_g2s(ring + (size_t) slot * STAGE + WB, ta.img + xo, xb, &full[slot]);
 			}
-			l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
+			prefetch_tail(a, false); // (K/V prefetch is off for batched steps)
 		}
 		return;
 	}
@@ -797,24 +791,8 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_batch_kernel
 						const float gt = a.act == XALM_SILU ? act_silu(yv) : act_gelu(yv);
 						out[o] = gt * ypart;
 					}
-				} else if ((r & 1) == 0 && row < a.d) { // EPI_QKV, as epilogue<2>: clip -> RoPE -> q fp32 / k, v fp16 into this slot's ring
-					const StepParams& sp = a.step[s];
-					const int pos = sp.pos, kv_pos = sp.kv_pos;
-					float v0 = clipf(yv, a.qkv_clip), v1 = clipf(ynext, a.qkv_clip);
-					if (row < a.q_dim) {
-						rope_pair(v0, v1, row % a.head_dim, pos, a.rope_freq);
-						out[row] = v0;
-						out[row + 1] = v1;
-					} else if (row < a.q_dim + a.kv_dim) {
-						const int i = row - a.q_dim;
-						rope_pair(v0, v1, i % a.head_dim, pos, a.rope_freq);
-						__half* kc = a.k_cache + (size_t) sp.slot * ta.kv_slot;
-						*reinterpret_cast<__half2*>(kc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
-					} else {
-						const int i = row - a.q_dim - a.kv_dim;
-						__half* vc = a.v_cache + (size_t) sp.slot * ta.kv_slot;
-						*reinterpret_cast<__half2*>(vc + (size_t) kv_pos * a.kv_dim + i) = __floats2half2_rn(v0, v1);
-					}
+				} else if ((r & 1) == 0 && row < a.d) { // EPI_QKV into this slot's ring
+					qkv_pair(a, a.step[s], ta.kv_slot, out, row, yv, ynext);
 				}
 			}
 			__syncwarp();
@@ -826,19 +804,8 @@ __global__ void __launch_bounds__((MMA_NCW + 2) * 32, 1) matvec_mma_batch_kernel
 
 	// ===================== consumers =====================
 	pdl_wait();
-	if (a.epi == EPI_QKV && blockIdx.x == 0) { // re-rotate the attention sinks of every sequence past its window (infer.cpp:393-399)
-		const int pairs = a.kv_dim / 2;
-		for (int s = 0; s < nseq; s++) {
-			const int kv_sink = a.step[s].kv_sink;
-			__half* kc = a.k_cache + (size_t) a.step[s].slot * ta.kv_slot;
-			for (int i = threadIdx.x; i < kv_sink * pairs; i += NT) {
-				const int rr = i / pairs, p = i % pairs;
-				__half2* kp = reinterpret_cast<__half2*>(kc + (size_t) rr * a.kv_dim) + p;
-				float2 v = __half22float2(*kp);
-				rope_pair(v.x, v.y, (2 * p) % a.head_dim, 1, a.rope_freq);
-				*kp = __floats2half2_rn(v.x, v.y);
-			}
-		}
+	if (a.epi == EPI_QKV && blockIdx.x == 0) { // re-rotate the attention sinks of every sequence past its window
+		for (int s = 0; s < nseq; s++) rotate_sinks(a, a.k_cache + (size_t) a.step[s].slot * ta.kv_slot, a.step[s].kv_sink, threadIdx.x, NT);
 	}
 
 	// this lane's place in the mma fragments: column g of the B operand is limb plane (2 - g) of sequence 2p (g < 3), the ones column

@@ -139,7 +139,6 @@ struct TmaArgs {
 };
 
 constexpr int TMA_NW = 8; // consumer warps
-constexpr unsigned int XALM_SPIN_LIMIT = 1u << 23; // polls of a tagged word (~1 us each) before a tensor-parallel wait gives up
 
 __host__ __device__ inline size_t tma_smem_bytes(int type, int n, int RC, int U, int NS) {
 	size_t s = 0;
@@ -189,18 +188,14 @@ __global__ void __launch_bounds__((TMA_NW + 1) * 32, 1) matvec_tma_kernel(const 
 	__syncthreads();
 	pdl_launch_dependents();
 	int tl = -1;
-	if (blockIdx.x == 0 && threadIdx.x == 0) {
-		tl = tl_begin(100 + a.epi);
-		if (a.progress) *reinterpret_cast<volatile unsigned int*>(a.progress) = (unsigned int) a.prog_idx;
-	}
+	if (blockIdx.x == 0 && threadIdx.x == 0) tl = tl_begin(100 + a.epi);
 
 	const int my_tiles = ((int) blockIdx.x < ta.n_tiles) ? (ta.n_tiles - 1 - (int) blockIdx.x) / (int) gridDim.x + 1 : 0;
 
 	if (warp == TMA_NW) {
 		// ===================== producer: weights only — runs ahead of griddepcontrol.wait =====================
 		if (lane == 0) {
-			if (blockIdx.x == 0 && a.pf_norm_ptr && a.pf_norm_bytes >= 16) // the next norm-fused kernel's rmsnorm weights -> L2 (matvec.cuh)
-				asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.pf_norm_ptr), "r"(a.pf_norm_bytes & ~15u) : "memory");
+			prefetch_next_norm(a);
 			int slot = 0, phase = 0;
 			for (int tt = 0; tt < my_tiles; tt++) {
 				const int row0 = ((int) blockIdx.x + tt * (int) gridDim.x) * RC;
@@ -219,12 +214,7 @@ __global__ void __launch_bounds__((TMA_NW + 1) * 32, 1) matvec_tma_kernel(const 
 					if (++slot == NS) { slot = 0; phase ^= 1; }
 				}
 			}
-			l2_prefetch_slice(a.pf_ptr, a.pf_bytes, (int) blockIdx.x, (int) gridDim.x);
-			if (a.pf_kv) {
-				const unsigned long long kvb = (unsigned long long) a.step->kv_len * a.kv_dim * sizeof(__half);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.k_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-				l2_prefetch_slice(reinterpret_cast<const uint8_t*>(a.v_cache), kvb, (int) blockIdx.x, (int) gridDim.x);
-			}
+			prefetch_tail(a, true);
 		}
 		return;
 	}
@@ -250,46 +240,8 @@ __global__ void __launch_bounds__((TMA_NW + 1) * 32, 1) matvec_tma_kernel(const 
 	}
 	pdl_wait(); // activations / KV ring of earlier kernels are visible from here on
 	tl_mark(tl, 2);
-	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) {
-		const int pairs = a.kv_dim / 2;
-		for (int i = threadIdx.x; i < a.step->kv_sink * pairs; i += TMA_NW * 32) {
-			const int r = i / pairs, p = i % pairs;
-			__half2* kp = reinterpret_cast<__half2*>(a.k_cache + (size_t) r * a.kv_dim) + p;
-			float2 v = __half22float2(*kp);
-			rope_pair(v.x, v.y, (2 * p) % a.head_dim, 1, a.rope_freq);
-			*kp = __floats2half2_rn(v.x, v.y);
-		}
-	}
-	// ---- tensor-parallel receive (LL style): the first CTAs each reduce a slice of the stream — x += sum over ranks of the partial
-	//      rows the previous row-split matvec pushed here (rank order: identical bits on every rank; infer.cpp:450-452 / :492-494) —
-	//      and publish it locally as {value, tag} words, so every other CTA reads dim words instead of n_ranks x dim ----
-	if (NORM && a.n_recv) {
-		const int n_red = min((int) gridDim.x, 8);
-		if ((int) blockIdx.x < n_red) {
-			const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
-			const int chunk = ((a.n / 4 + n_red - 1) / n_red) * 4;
-			const int i0 = (int) blockIdx.x * chunk, i1 = min(a.n, i0 + chunk);
-			for (int i = i0 + (int) threadIdx.x * 4; i < i1; i += TMA_NW * 32 * 4) {
-				float4 v = ld_act4(a.x + i);
-				float4 sum = make_float4(0.f, 0.f, 0.f, 0.f);
-				for (int p = 0; p < a.n_recv; p++) {
-					const uint2* src = a.recv + (size_t) p * a.n + i; // four {value, tag} words; poll until all carry this exchange's tag
-					uint4 w0, w1;
-					unsigned int spins = 0;
-					do {
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src));
-						asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 2));
-						if (++spins > XALM_SPIN_LIMIT) { if (a.err_flag) *a.err_flag = 1u; break; } // a peer died: report, do not hang the GPU
-					} while (w0.y != seq || w0.w != seq || w1.y != seq || w1.w != seq);
-					sum.x += __uint_as_float(w0.x); sum.y += __uint_as_float(w0.z); sum.z += __uint_as_float(w1.x); sum.w += __uint_as_float(w1.z);
-				}
-				v.x += sum.x; v.y += sum.y; v.z += sum.z; v.w += sum.w;
-				*reinterpret_cast<float4*>(a.x_out + i) = v;
-				*reinterpret_cast<uint4*>(a.xl + i) = make_uint4(__float_as_uint(v.x), seq, __float_as_uint(v.y), seq);
-				*reinterpret_cast<uint4*>(a.xl + i + 2) = make_uint4(__float_as_uint(v.z), seq, __float_as_uint(v.w), seq);
-			}
-		}
-	}
+	if (a.epi == EPI_QKV && blockIdx.x == 0 && a.step->kv_sink > 0) rotate_sinks(a, a.k_cache, a.step->kv_sink, threadIdx.x, TMA_NW * 32);
+	if (NORM && a.n_recv) tp_receive(a, threadIdx.x, TMA_NW * 32);
 	// ---- stage activations: xb = NORM ? x * scale * g : x ----
 	if (!xg) {
 		// xb is stored permuted inside each 256-element unit: the E floats a lane needs for one piece are split into
@@ -302,17 +254,8 @@ __global__ void __launch_bounds__((TMA_NW + 1) * 32, 1) matvec_tma_kernel(const 
 		float ss = 0.f;
 		for (int i = threadIdx.x * 4; i < a.n; i += TMA_NW * 32 * 4) {
 			float4 v;
-			if (NORM && a.n_recv) { // the summed stream, published by the reducing CTAs below as {value, tag} words: poll this exchange's tag
-				const unsigned int seq = a.step->ar_base + (unsigned int) a.recv_idx + 1u;
-				const uint2* src = a.xl + i;
-				uint4 w0, w1;
-				unsigned int spins = 0;
-				do {
-					asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w0.x), "=r"(w0.y), "=r"(w0.z), "=r"(w0.w) : "l"(src));
-					asm volatile("ld.volatile.global.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(w1.x), "=r"(w1.y), "=r"(w1.z), "=r"(w1.w) : "l"(src + 2));
-					if (++spins > XALM_SPIN_LIMIT) { if (a.err_flag) *a.err_flag = 1u; break; }
-				} while (w0.y != seq || w0.w != seq || w1.y != seq || w1.w != seq);
-				v = make_float4(__uint_as_float(w0.x), __uint_as_float(w0.z), __uint_as_float(w1.x), __uint_as_float(w1.z));
+			if (NORM && a.n_recv) { // the summed stream, published by the reducing CTAs above as {value, tag} words: poll this exchange's tag
+				v = poll_tagged4(a.xl + i, a.step->ar_base + (unsigned int) a.recv_idx + 1u, a.err_flag);
 			} else {
 				v = ld_act4(a.x + i);
 			}
@@ -417,31 +360,7 @@ __global__ void __launch_bounds__((TMA_NW + 1) * 32, 1) matvec_tma_kernel(const 
 #pragma unroll
 				for (int k = 0; k < KW; k++) yv += pt[k * 16 + lane];
 			}
-			// gather the RC sums into lane 0 .. (pairs stay adjacent for RoPE): each even lane takes its neighbour's value
-			const float ynext = __shfl_down_sync(0xffffffffu, yv, 1);
-			const int row0 = ((int) blockIdx.x + tt * (int) gridDim.x) * RC;
-			if (a.epi == EPI_RESIDUAL) {
-				if (lane < RC && row0 + lane < a.d) a.out[row0 + lane] = xold + yv;
-			} else if (a.epi == EPI_STORE && a.n_push) { // tensor parallel: this rank's partial rows go to every rank (NVLink stores)
-				if (lane < RC && (lane & 1) == 0 && row0 + lane < a.d) {
-					const unsigned int seq = a.step->ar_base + (unsigned int) a.push_idx + 1u;
-					const uint4 w = make_uint4(__float_as_uint(yv), seq, __float_as_uint(ynext), seq);
-					for (int p = 0; p < a.n_push; p++) *reinterpret_cast<uint4*>(a.push_dst[p] + row0 + lane) = w;
-				}
-			} else if (lane < RC && (lane & 1) == 0 && a.epi != EPI_GLU) { // GLU below (partner rows RC/2 apart)
-				const float y2[2] = {yv, ynext};
-				epilogue<2>(a, row0 + lane, y2);
-			}
-			if (a.epi == EPI_GLU) {
-				const float ypart = __shfl_down_sync(0xffffffffu, yv, RC / 2); // W3 value for the W1 row in this lane
-				if (lane < RC / 2) {
-					const int o = row0 / 2 + lane;
-					if (o < a.d) {
-						const float g = a.act == XALM_SILU ? act_silu(yv) : act_gelu(yv);
-						a.out[o] = g * ypart;
-					}
-				}
-			}
+			row_epilogue<RC>(a, ((int) blockIdx.x + tt * (int) gridDim.x) * RC, lane, yv, xold);
 		}
 	}
 	tl_mark(tl, 3);

@@ -659,9 +659,9 @@ __global__ void tp_drain_kernel(const uint2* __restrict__ recv, int n_ranks, int
 	pdl_wait();
 	const unsigned int seq = step->ar_base + (unsigned int) idx + 1u;
 	for (int i = threadIdx.x; i < n_ranks * dim; i += blockDim.x) {
-		unsigned int tag, val, spins = 0;
+		unsigned int tag, spins = 0;
 		do {
-			asm volatile("ld.volatile.global.v2.u32 {%0,%1}, [%2];" : "=r"(val), "=r"(tag) : "l"(recv + i));
+			asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(tag) : "l"(&recv[i].y));
 			if (++spins > xalm::XALM_SPIN_LIMIT) { if (err_flag) *err_flag = 1u; break; }
 		} while (tag != seq);
 	}
@@ -1256,7 +1256,6 @@ static int upload_impl(xalm_cuda_model* m, const char* name, int type_id, const 
 	auto put = [&](WMat& w, int dst_row, int r0, int r1, int c0, int c1) -> int {
 		return upload_piece(w, dst_row, type_id, host, sc1 - sc0, r0 - sr0, r1 - sr0, c0 - sc0, c1 - sc0, m->staging, m->stream);
 	};
-	cudaStream_t s = m->stream;
 	const int P = m->tp_size, R = m->tp_rank;
 
 	if (is_norm) {
