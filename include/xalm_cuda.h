@@ -124,6 +124,18 @@ int xalm_cuda_forward(xalm_cuda_model* m, int token, int pos, int mode, float* l
 /* forward(OUTPUT_LOGITS) followed by Sampler::sample_argmax (sampler.cpp:3-16, FLT_MIN-seeded running maximum, first
  * maximum wins) on the device: only the 4-byte token id crosses PCIe.  Leaves the host logits buffer untouched. */
 int xalm_cuda_forward_argmax(xalm_cuda_model* m, int token, int pos, int* next_token);
+/* Greedy chain, as a draft model drafts: exactly the loop
+ *     for j in 0 .. n_in-2:   forward(tokens[j], pos+j, XALM_HYDRATE_KV_CACHE)
+ *     t = forward_argmax(tokens[n_in-1], pos+n_in-1);        out_tokens[0] = t
+ *     for i in 1 .. n_out-1:  t = forward_argmax(t, pos+n_in-1+i);  out_tokens[i] = t
+ * on the same handle, with one host synchronisation instead of one per token: each step's greedy token is written into the next
+ * step's parameters on the device.  The KV cache, the logits left on the device (read_state XALM_S_LOGITS) and out_tokens are
+ * bit-identical to that loop, past the context window too (ring slots and re-rotated sinks); the host logits buffer is untouched.
+ * Runs the kernels xalm_cuda_forward runs, for every weight format; on a batched handle it drives the slot of select_seq.
+ * 1 <= n_in <= 8 and 1 <= n_out <= 16.  Limits out of range, a NULL pointer, a token out of range or a negative position are
+ * XALM_ERR_INVALID before anything is enqueued (the cache is untouched); XALM_ERR_UNSUPPORTED on a tensor-parallel handle, whose
+ * exchange tags are assigned per token on the host. */
+int xalm_cuda_forward_greedy(xalm_cuda_model* m, int n_in, const int* tokens, int pos, int n_out, int* out_tokens);
 /* Enqueue only (no host sync, logits stay on the device): the device-timed leg of bench.py. */
 int xalm_cuda_forward_async(xalm_cuda_model* m, int token, int pos, int mode);
 int xalm_cuda_sync(xalm_cuda_model* m);

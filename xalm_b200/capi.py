@@ -60,6 +60,7 @@ SYMBOLS = {
     "xalm_cuda_forward": (_i, [_vp, _i, _i, _i, _vp]),
     "xalm_cuda_forward_async": (_i, [_vp, _i, _i, _i]),
     "xalm_cuda_forward_argmax": (_i, [_vp, _i, _i, C.POINTER(_i)]),
+    "xalm_cuda_forward_greedy": (_i, [_vp, _i, _vp, _i, _i, _vp]),
     "xalm_cuda_sync": (_i, [_vp]),
     "xalm_cuda_logits_host": (_fp, [_vp]),
     "xalm_cuda_active_bytes": (_i, [_vp, C.c_longlong, C.POINTER(C.c_longlong)]),

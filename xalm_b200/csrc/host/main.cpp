@@ -1,7 +1,7 @@
 // main.cpp — the reference's CLI surface (src/main.cpp:417-547) on top of the CUDA backend.
 //
 //   xalm_main <checkpoint.xalm> [-d cuda] [-m completion|passkey|perplexity|batch] [-T ctx] [-i prompt | -f file] [-n steps] [-l pos] [-g gpus] [-b seqs]
-//             [-s draft]
+//             [-s draft] [-D draft.xalm]
 //
 // Same flags, same prefix matching for -m/-d, same defaults (mode completion, -n 128, the default prompt), same stats
 // block, plus the roofline fraction.  Differences, on purpose:
@@ -24,6 +24,7 @@
 #include <cstring>
 #include <fstream>
 #include <iostream>
+#include <optional>
 #include <sstream>
 #include <string>
 
@@ -45,6 +46,8 @@ namespace {
 	fprintf(stderr, "Completion mode options:\n  -n <int>    number of steps to run for in completion mode, default 128. 0 = max_seq_len, -1 = infinite\n");
 	fprintf(stderr, "  -s <int>    speculative decoding: verify up to this many prompt-lookup draft tokens per pass (1..7; one GPU,\n"
 	                "              integer block formats; same output as without -s)\n");
+	fprintf(stderr, "  -D <filepath> with -s: draft the tokens with this model (same tokenizer, any weight format, same GPU) instead of\n"
+	                "              prompt lookup\n");
 	fprintf(stderr, "  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
 	fprintf(stderr, "Batch mode options (one GPU; integer block formats):\n  -f <filepath> prompts, one per non-empty line\n"
 	                "  -b <int>    sequences decoded together (1..8, default 8)\n  -n <int>    tokens per prompt, default 128. 0 = max_seq_len\n");
@@ -120,14 +123,42 @@ struct SpecStats {
 	size_t passes = 0, drafted = 0, accepted = 0, decoded = 0; // decoded: tokens the passes produced (accepted + one per pass)
 };
 
+// Where the drafts of -m completion -s k come from: prompt lookup, or a draft model (-D) decoding greedily on its own handle.
+struct Drafter {
+	const Model* model = nullptr; // the draft model; nullptr: prompt lookup
+	size_t valid = 0;             // draft model: its KV rows 0 .. valid-1 hold the accepted sequence
+	size_t steps = 0, calls = 0;  // draft model: forward steps run, and forward_greedy calls that ran them
+	double seconds = 0.0;
+
+	// up to k tokens to follow seq; P = seq.size() - 1 is the target's next position and P + k stays inside the window.  The draft
+	// model catches up on the accepted tokens it has not decoded (seq[valid .. P]) and drafts k tokens in one greedy chain.
+	std::vector<int> draft(const std::vector<int>& seq, int k) {
+		if (!model) return draft_lookup(seq, k);
+		const size_t P = seq.size() - 1;
+		std::vector<int> out(k);
+		const double t0 = now_s();
+		model->forward_greedy(seq.data() + valid, (int) (P + 1 - valid), (int) valid, k, out.data());
+		seconds += now_s() - t0;
+		steps += P + 1 - valid + k - 1;
+		calls++;
+		return out;
+	}
+	// a of the drafts of a round at P were accepted.  The chain wrote draft rows P+1 .. P+n-1 for its first n-1 drafts, and those
+	// of the accepted ones hold accepted tokens; rows of rejected drafts are rewritten before they are read, as a span's are
+	// (xalm_cuda.h).  So the next round feeds one token, or two when every draft was accepted.
+	void accepted(size_t P, int a, int n) {
+		if (model) valid = P + std::min(a, n - 1) + 1;
+	}
+};
+
 // The generation loop of -m completion -s k: the same greedy tokens, fewer passes over the weights.  Each step drafts up to k
-// tokens by prompt lookup and verifies them with the last token in ONE span (Model::forward_spans_argmax): entry j's greedy
+// tokens (Drafter) and verifies them with the last token in ONE span (Model::forward_spans_argmax): entry j's greedy
 // token is what a plain step would produce after the entries before it, so the longest prefix of the draft that matches those
 // tokens is accepted, plus the model's own token after it.  Rows written for rejected drafts need no cleanup (xalm_cuda.h).
 // Without a draft, or past the context window where spans are refused, the step is a plain forward on slot 0.  Prints the tokens
 // as run_completion does; returns the bytes read.
 size_t generate_speculative(const Model& model, const InferenceState& state, const Sampler& sampler, const Tokenizer& tokenizer,
-                            std::vector<int>& encoding, int num_steps, int k, SpecStats& st) {
+                            std::vector<int>& encoding, int num_steps, int k, Drafter& drafter, SpecStats& st) {
 	const size_t W = (size_t) model.config.max_seq_len;
 	const size_t kv_row = W > 1 ? model.active_bytes(1) - model.active_bytes(0) : 0, weights = model.active_bytes(0) - kv_row;
 	size_t read_bytes = 0;
@@ -145,7 +176,7 @@ size_t generate_speculative(const Model& model, const InferenceState& state, con
 		if (stop || !(i < num_steps || num_steps == -1)) break;
 		const size_t P = encoding.size() - 1;            // position of the last token, not yet decoded
 		const size_t room = P + 1 < W ? W - 1 - P : 0;    // draft positions P+1 .. P+len stay inside the window
-		const std::vector<int> draft = room ? draft_lookup(encoding, (int) std::min(room, (size_t) k)) : std::vector<int>{};
+		const std::vector<int> draft = room ? drafter.draft(encoding, (int) std::min(room, (size_t) k)) : std::vector<int>{};
 		st.passes++;
 		if (draft.empty()) {
 			model.forward(state, encoding.back(), (int) P);
@@ -166,6 +197,7 @@ size_t generate_speculative(const Model& model, const InferenceState& state, con
 		for (int j = 0; j < n; j++) read_bytes += (P + j + 1) * kv_row;
 		int a = 0;
 		while (a < n - 1 && out[a] == draft[a]) a++;
+		drafter.accepted(P, a, (int) draft.size());
 		pending.assign(draft.begin(), draft.begin() + a);
 		pending.push_back(out[a]);
 		st.drafted += draft.size();
@@ -175,10 +207,24 @@ size_t generate_speculative(const Model& model, const InferenceState& state, con
 	return read_bytes;
 }
 
-void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps, int spec) {
+void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps, int spec,
+                    const std::string& draft_path) {
 	auto model_data = Xalm::load(checkpoint_path);
 	std::cout << "loading model " << checkpoint_path << std::endl;
 	Model model = Model::from_xalm(model_data, context, /*defer_load=*/true); // weights go disk -> pinned -> device in model.cuda()
+	// -D: the draft model must speak the target's tokens: the same vocabulary size and tokenizer, checked before any device work
+	std::optional<Xalm::file_info> draft_data;
+	std::optional<Model> draft;
+	if (!draft_path.empty()) {
+		draft_data.emplace(Xalm::load(draft_path));
+		draft.emplace(Model::from_xalm(*draft_data, context, /*defer_load=*/true));
+		if (draft->config.vocab_size != model.config.vocab_size)
+			throw std::invalid_argument("draft model " + draft_path + ": vocab_size " + std::to_string(draft->config.vocab_size) + " differs from the target's " +
+			                            std::to_string(model.config.vocab_size));
+		const Tensor a = model_data.load_tensor("tokenizer.tokens"), b = draft_data->load_tensor("tokenizer.tokens");
+		if (a.size != b.size || std::memcmp(a.bytes(), b.bytes(), a.size) != 0)
+			throw std::invalid_argument("draft model " + draft_path + ": tokenizer.tokens differ from the target's");
+	}
 	printf("Model active bytes(m): %zu\n", model.active_bytes(model.config.max_seq_len) / (1024 * 1024));
 	std::cout << "Using CUDA" << std::endl;
 	if (spec) model.cuda(0, 0, 1, nullptr, {}, spec + 1); // -s k: a batched handle wide enough for a span of k drafts + the last token
@@ -190,6 +236,15 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	if (num_steps == 0) num_steps = model.config.max_seq_len; // `-n 0` = full context (main.cpp:67-70)
 	model.forward(state, 0, 0);                               // warm-up (main.cpp:72): captures the CUDA graph
 	const int launches = model.last_launch_count();
+	std::optional<InferenceState> draft_state;
+	Drafter drafter;
+	if (draft) { // the same GPU, a plain batch-1 handle: any weight format
+		draft->cuda();
+		draft_state.emplace(draft->config);
+		draft_state->cuda();
+		draft->forward(*draft_state, 0, 0);
+		drafter.model = &*draft;
+	}
 
 	double t0 = now_s();
 	std::vector<int> encoding = tokenizer.encode(prompt, true);
@@ -200,9 +255,13 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 
 	t0 = now_s();
 	size_t read_bytes = hydrate(model, state, encoding);
+	if (draft) {
+		hydrate(*draft, *draft_state, encoding);
+		drafter.valid = encoding.size();
+	}
 	const double hydrate_s = now_s() - t0;
 	SpecStats spec_stats;
-	if (spec) read_bytes += generate_speculative(model, state, sampler, tokenizer, encoding, num_steps, spec, spec_stats);
+	if (spec) read_bytes += generate_speculative(model, state, sampler, tokenizer, encoding, num_steps, spec, drafter, spec_stats);
 	else for (int i = 0; i < num_steps || num_steps == -1; i++) { // main.cpp:105-115
 		// the logits are all-gathered under -g, so every rank picks the same token and stops at the same step
 		const int token_id = sampler.sample_argmax(state);
@@ -223,6 +282,7 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	if (spec)
 		printf("  speculative: %zu passes, %zu drafted, %zu accepted, %.3g tokens/pass\n", spec_stats.passes, spec_stats.drafted, spec_stats.accepted,
 		       spec_stats.passes ? (double) spec_stats.decoded / spec_stats.passes : 0.0);
+	if (draft) printf("  draft: %s, %zu steps in %zu calls, %.5gs\n", draft_path.c_str(), drafter.steps, drafter.calls, drafter.seconds);
 }
 
 // -m batch: every non-empty line of the prompt file is one prompt; up to `max_batch` of them decode together on one batched handle,
@@ -451,7 +511,7 @@ int main(int argc, char* argv[]) {
 	std::string checkpoint_path, device = "cuda", mode = "completion";
 	std::string prompt = "Q: What is the meaning of life? A:"; // main.cpp:421
 	std::string prompt_path;
-	std::string convert_type;
+	std::string convert_type, draft_path;
 	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8, spec = 0;
 	if (argc >= 2) checkpoint_path = argv[1];
 	else error_usage();
@@ -484,12 +544,17 @@ int main(int argc, char* argv[]) {
 			spec = parse_gpus(v);
 			if (spec > 7) error_usage();
 		}
+		else if (f == 'D') draft_path = v;
 		else if (f == 'n') { num_steps = std::stoi(v); n_junk = num_steps; }
 		else error_usage();
 		i += 2;
 	}
 	if (spec && (mode != "completion" || gpus != 1)) {
 		fprintf(stderr, "Error: -s runs -m completion on one GPU (no -g)\n");
+		error_usage();
+	}
+	if (!draft_path.empty() && !spec) {
+		fprintf(stderr, "Error: -D drafts for -s (speculative -m completion on one GPU)\n");
 		error_usage();
 	}
 	if (mode == "verify") {
@@ -541,7 +606,7 @@ int main(int argc, char* argv[]) {
 	}
 	auto run = [&](const TpRank& tp) {
 		try {
-			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps, spec);
+			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps, spec, draft_path);
 			else if (mode == "passkey") run_passkey(tp, checkpoint_path, context, n_junk, passkey_pos);
 			else run_perplexity(tp, checkpoint_path, prompt, context);
 		} catch (const std::exception& e) {

@@ -269,7 +269,9 @@ xalm_config Config::to_c() const {
 InferenceState::InferenceState(const Config& config) : own_logits_((size_t) config.vocab_size, 0.f) {}
 
 // ---- Model -------------------------------------------------------------------------------------------------------
-Model::Model(Model&& o) noexcept : config(o.config), device(o.device), host_(std::move(o.host_)), types_(std::move(o.types_)), handle_(o.handle_) {
+Model::Model(Model&& o) noexcept : config(o.config), device(o.device), host_(std::move(o.host_)), types_(std::move(o.types_)),
+                                   deferred_(o.deferred_), handle_(o.handle_) {
+	o.deferred_ = nullptr;
 	o.handle_ = nullptr;
 }
 Model::~Model() {
@@ -454,6 +456,11 @@ void Model::forward_batch_argmax(const int n, const int* seqs, const int* tokens
 void Model::forward_spans_argmax(const int n, const int* seqs, const int* tokens, const int* pos, int* next) const {
 	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_spans_argmax: model is not on a CUDA device (call model.cuda())");
 	if (xalm_cuda_forward_spans_argmax(handle_, n, seqs, tokens, pos, next) != XALM_OK) xalm_throw_last("Model::forward_spans_argmax");
+}
+
+void Model::forward_greedy(const int* tokens, const int n_in, const int pos, const int n_out, int* out) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_greedy: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_forward_greedy(handle_, n_in, tokens, pos, n_out, out) != XALM_OK) xalm_throw_last("Model::forward_greedy");
 }
 
 void Model::select_seq(const int seq) const {

@@ -186,6 +186,10 @@ struct Model {
 	// forward_batch_argmax where a slot may take several consecutive positions in one step (xalm_cuda_forward_spans_argmax):
 	// how drafted tokens are verified in one pass over the weights.  next[i] is the greedy token after entry i.  A refused call throws.
 	void forward_spans_argmax(int n, const int* seqs, const int* tokens, const int* pos, int* next) const;
+	// Greedy chain (xalm_cuda_forward_greedy): tokens[0 .. n_in-2] hydrate positions pos .. pos+n_in-2, tokens[n_in-1] decodes at
+	// pos+n_in-1, and each of the n_out - 1 further steps decodes the previous step's greedy token; out[i] is step i's token.  One
+	// host synchronisation per call, as a draft model drafts.  1 <= n_in <= 8, 1 <= n_out <= 16.  A refused call throws.
+	void forward_greedy(const int* tokens, int n_in, int pos, int n_out, int* out) const;
 	// The slot forward / prefill / prefill_window work on (default 0): how a prompt is hydrated into a slot.
 	void select_seq(int seq) const;
 

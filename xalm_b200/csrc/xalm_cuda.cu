@@ -12,6 +12,7 @@
 //   matvec[norm -> classifier]              logits                         (skipped in HYDRATE_KV_CACHE mode)
 #include <cuda_runtime.h>
 #include <dlfcn.h>
+#include <limits.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -597,6 +598,34 @@ __device__ __forceinline__ void argmax_row(const float* __restrict__ logits, int
 // row b of (rows, n) logits -> out[b]
 __global__ void argmax_rows_kernel(const float* __restrict__ logits, int n, int* __restrict__ out) {
 	argmax_row(logits + (size_t) blockIdx.x * n, n, out + blockIdx.x);
+}
+
+// an entry's token, position and mode, and its ring / sink indices: infer.cpp:611-613, KV_SINKS = 2 (model.h:10).  On the host for
+// every step the host sets up, on the device for the steps of a greedy chain (argmax_next_step_kernel).
+static __host__ __device__ void fill_step_entry(const xalm_config& c, StepParams& p, int token, int pos, int mode) {
+	p.token = token; p.pos = pos;
+	p.kv_sink = pos >= c.max_seq_len ? 2 : 0;
+	p.kv_pos = p.kv_sink + (pos - p.kv_sink) % (c.max_seq_len - p.kv_sink);
+	p.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
+	p.mode = mode;
+}
+
+// One link of a greedy chain (xalm_cuda_forward_greedy): Sampler::sample_argmax of the single-sequence logits into *out and, unless
+// `next` is NULL (the chain's last step), the single-sequence StepParams row of the next step, which decodes that token at next_pos.
+// Freshness: every kernel of a step reads StepParams from d_step, some of them before their PDL dependency wait.  This kernel is
+// therefore launched WITHOUT the PDL attribute: it starts only once the step that read the row has completed, and the next step's
+// first kernel (the embedding, also launched without PDL) starts only once this one has completed.
+__global__ void argmax_next_step_kernel(const float* __restrict__ logits, int n, int* __restrict__ out, StepParams* __restrict__ next,
+                                        xalm_config c, int next_pos, unsigned int ar_base) {
+	argmax_row(logits, n, out);
+	if (next && threadIdx.x == 0) { // the thread that wrote *out
+		StepParams p;
+		fill_step_entry(c, p, *out, next_pos, XALM_OUTPUT_LOGITS);
+		p.kv_fresh = p.kv_pos;
+		p.ar_base = ar_base;
+		p.slot = 0;
+		*next = p;
+	}
 }
 
 __global__ void residual_add_kernel(float* __restrict__ x, const float* __restrict__ y, int n) {
@@ -1669,15 +1698,6 @@ static int claim_step_rows(xalm_cuda_model* m, StepParams** rows) {
 	return XALM_OK;
 }
 
-// an entry's token, position and mode, and its ring / sink indices: infer.cpp:611-613, KV_SINKS = 2 (model.h:10)
-static void fill_step_entry(const xalm_config& c, StepParams& p, int token, int pos, int mode) {
-	p.token = token; p.pos = pos;
-	p.kv_sink = pos >= c.max_seq_len ? 2 : 0;
-	p.kv_pos = p.kv_sink + (pos - p.kv_sink) % (c.max_seq_len - p.kv_sink);
-	p.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
-	p.mode = mode;
-}
-
 // copy the first n rows of a claimed row group to the device, and mark the group free again once the copy has run
 static int upload_step_rows(xalm_cuda_model* m, const StepParams* rows, int n) {
 	const int slot = (int) ((rows - m->h_step) / m->max_seqs);
@@ -1752,6 +1772,42 @@ int xalm_cuda_forward_argmax(xalm_cuda_model* m, int token, int pos, int* next_t
 	if (!next_token) return set_error(XALM_ERR_INVALID, "next_token is NULL");
 	XALM_TRY(xalm_cuda_forward_async(m, token, pos, XALM_OUTPUT_LOGITS));
 	return finish_step_argmax(m, 1, next_token);
+}
+
+// The loop forward(HYDRATE) x (n_in - 1), forward_argmax, then forward_argmax of each result, with one host synchronisation.  The
+// steps fed from `tokens` are set up by the host as xalm_cuda_forward_async sets them up; after every logits step
+// argmax_next_step_kernel writes the greedy token to d_argmax[i] and, but for the last, the next step's row of d_step, and that
+// step's graph (the single-sequence logits graph) is replayed without an upload.  The n_out tokens come back in one copy.
+int xalm_cuda_forward_greedy(xalm_cuda_model* m, int n_in, const int* tokens, int pos, int n_out, int* out_tokens) {
+	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
+	if (m->tp_size > 1)
+		return set_error(XALM_ERR_UNSUPPORTED, "forward_greedy: tensor-parallel exchange tags are assigned per token on the host (tp_size %d)", m->tp_size);
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "forward_greedy before finalize");
+	if (n_in < 1 || n_in > 8) return set_error(XALM_ERR_INVALID, "forward_greedy: n_in = %d not in [1, 8]", n_in);
+	if (n_out < 1 || n_out > 16) return set_error(XALM_ERR_INVALID, "forward_greedy: n_out = %d not in [1, 16]", n_out); // d_argmax holds 16
+	if (!tokens || !out_tokens) return set_error(XALM_ERR_INVALID, "NULL argument");
+	const xalm_config& c = m->c;
+	for (int j = 0; j < n_in; j++)
+		if (tokens[j] < 0 || tokens[j] >= c.vocab_size) return set_error(XALM_ERR_INVALID, "token %d out of range [0,%d)", tokens[j], c.vocab_size);
+	if (pos < 0) return set_error(XALM_ERR_INVALID, "negative position");
+	if (pos > INT_MAX - n_in - n_out) return set_error(XALM_ERR_INVALID, "forward_greedy: position %d overflows", pos);
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	for (int j = 0; j < n_in; j++) XALM_TRY(xalm_cuda_forward_async(m, tokens[j], pos + j, j + 1 < n_in ? XALM_HYDRATE_KV_CACHE : XALM_OUTPUT_LOGITS));
+	for (int i = 0; i < n_out; i++) {
+		const bool last = i + 1 == n_out;
+		StepParams* next = last ? nullptr : m->d_step;
+		cudaError_t e = launch(argmax_next_step_kernel, dim3(1), dim3(1024), m->stream, false, (const float*) m->logits_full, c.vocab_size,
+		                       m->d_argmax + i, next, c, pos + n_in + i, m->token_serial * 1024u);
+		if (e != cudaSuccess) return set_error(XALM_ERR_CUDA, "argmax launch failed: %s", cudaGetErrorString(e));
+		if (last) break;
+		m->token_serial++; // the step's ar_base, as xalm_cuda_forward_async counts them
+		XALM_TRY(run_step(m, XALM_OUTPUT_LOGITS, 0));
+	}
+	XALM_CUDA_CHECK(cudaMemcpyAsync(m->h_argmax, m->d_argmax, (size_t) n_out * sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+	XALM_CUDA_CHECK(cudaStreamSynchronize(m->stream));
+	XALM_TRY(check_tp_error(m));
+	memcpy(out_tokens, m->h_argmax, (size_t) n_out * sizeof(int));
+	return XALM_OK;
 }
 
 // ---- batched decode: several sequence slots, one pass over the weights per step ------------------------------------------

@@ -167,6 +167,29 @@ class Model:
         capi.check(capi.lib().xalm_cuda_forward_argmax(self._h, token, pos, C.byref(out)))
         return out.value
 
+    GREEDY_MAX_IN, GREEDY_MAX_OUT = 8, 16   # xalm_cuda_forward_greedy's limits on n_in and n_out
+
+    def forward_greedy(self, tokens, pos: int, n_out: int) -> list:
+        """tokens[0..n-2] hydrate positions pos..pos+n-2, tokens[-1] decodes at pos+n-1, then n_out - 1 more greedy steps each
+        feed the previous step's token: the n_out greedy tokens, with one host synchronisation (the tokens never leave the
+        device in between).  The cache and the logits left on the device are those of the equivalent forward / forward_argmax
+        loop.  1 <= len(tokens) <= 8, 1 <= n_out <= 16."""
+        tok = np.ascontiguousarray(tokens, dtype=np.int32).reshape(-1)
+        if not 1 <= tok.size <= self.GREEDY_MAX_IN:
+            raise ValueError(f"forward_greedy: {tok.size} input tokens, expected 1..{self.GREEDY_MAX_IN}")
+        if not 1 <= int(n_out) <= self.GREEDY_MAX_OUT:
+            raise ValueError(f"forward_greedy: n_out {n_out} not in 1..{self.GREEDY_MAX_OUT}")
+        if tok.min() < 0 or tok.max() >= self.config["vocab_size"]:
+            raise ValueError(f"forward_greedy: a token is out of range [0, {self.config['vocab_size']})")
+        if int(pos) < 0:
+            raise ValueError("forward_greedy: negative position")
+        if self._h is None:
+            raise RuntimeError("Model.forward_greedy: the model is not on a CUDA device (call model.cuda()); this backend has no CPU path")
+        out = np.zeros(int(n_out), dtype=np.int32)
+        capi.check(capi.lib().xalm_cuda_forward_greedy(self._h, int(tok.size), tok.ctypes.data_as(C.c_void_p), int(pos), int(n_out),
+                                                      out.ctypes.data_as(C.c_void_p)))
+        return [int(v) for v in out]
+
     def forward_async(self, token: int, pos: int, mode: int = InferenceMode.OUTPUT_LOGITS) -> None:
         capi.check(capi.lib().xalm_cuda_forward_async(self._h, token, pos, mode))
 

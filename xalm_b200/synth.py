@@ -30,6 +30,10 @@ SHAPES = {
     # Llama-3-70B style (config 5)
     "l70": dict(dim=8192, hidden_dim=28672, head_dim=128, n_layers=80, n_heads=64, n_kv_heads=8, vocab_size=128256,
                 max_seq_len=8192, rope_theta=500000.0, arch="LlamaForCausalLM"),
+    # TinyLlama-1.1B, a draft model for m7 (same vocabulary size); context 4096 rather than 2048 so that it drafts across m7's
+    # default window
+    "d1": dict(dim=2048, hidden_dim=5632, head_dim=64, n_layers=22, n_heads=32, n_kv_heads=4, vocab_size=32000,
+               max_seq_len=4096, rope_theta=10000.0, arch="LlamaForCausalLM"),
     # small shapes for tests / smoke
     "tiny": dict(dim=256, hidden_dim=512, head_dim=64, n_layers=2, n_heads=4, n_kv_heads=2, vocab_size=512,
                  max_seq_len=128, rope_theta=10000.0, arch="MistralForCausalLM"),
