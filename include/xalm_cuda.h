@@ -205,6 +205,27 @@ int xalm_cuda_select_seq(xalm_cuda_model* m, int seq);
  * xalm_cuda_forward_spans_argmax: the same + Sampler::sample_argmax per row on the device; next_tokens[i] for entry i.  Synchronous. */
 int xalm_cuda_forward_spans(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, float* logits_host);
 int xalm_cuda_forward_spans_argmax(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int* next_tokens);
+/* ---- trees: several drafted continuations of one sequence in one step (tree verification) --------------------------------
+ * xalm_cuda_forward_tree: one step of n tree nodes on slot `slot` of a batched handle, always with logits.  Node 0 is the root,
+ * the last accepted token at position pos; parents[0] == -1 and 0 <= parents[i] < i for i >= 1 (nodes in topological order).  Node
+ * i has depth d(i) = d(parents[i]) + 1, decodes tokens[i] at position pos + d(i) and writes its K/V to row pos + i of the slot.  It
+ * attends to the slot's rows 0 .. pos-1, then the rows of its ancestors, root first, then its own row, so its logits
+ * (logits_host row i, may be NULL) and the rows it writes are bit-identical to decoding the root-to-i branch one token at a time on
+ * a batch-1 handle with the tensor-core matvec (xalm_cuda_tune("mma", 1)).  1 <= n <= max_seqs and pos + n <= max_seq_len (a tree
+ * never touches the ring or the attention sinks).  A bad parents array, a token out of range, a negative position, a slot out of
+ * range, a tree reaching max_seq_len and NULL arrays are XALM_ERR_INVALID before anything is enqueued, with every cache untouched;
+ * XALM_ERR_STATE on a handle without xalm_cuda_set_batch or before finalize.  Other slots are untouched.  Synchronous.
+ * xalm_cuda_forward_tree_argmax: the same + Sampler::sample_argmax per node on the device; next_tokens[i] for node i.  Synchronous.
+ * xalm_cuda_tree_accept: makes rows pos .. pos+n-1 of the slot hold an accepted branch of the tree last verified at pos on that
+ * slot.  nodes is the root-to-node path: nodes[0] == 0, strictly increasing.  For every j with nodes[j] != j, K and V row
+ * pos + nodes[j] of every layer is copied to row pos + j, in increasing j; that is safe in place, since nodes[k] > nodes[j] >= j
+ * for every later k, so no row is overwritten before it is read.  Enqueue only: stream order puts the copy before the next step.
+ * When every nodes[j] == j (a chain, or the leftmost path) nothing is enqueued.  Rows past pos+n-1 keep stale contents, which a
+ * later step rewrites before any entry reads them, as for spans.  nodes[0] != 0, nodes not increasing or reaching max_seqs, a row
+ * reaching max_seq_len, a slot out of range, n outside [1, max_seqs] and NULL nodes are XALM_ERR_INVALID with nothing enqueued. */
+int xalm_cuda_forward_tree(xalm_cuda_model* m, int slot, int n, const int* tokens, const int* parents, int pos, float* logits_host);
+int xalm_cuda_forward_tree_argmax(xalm_cuda_model* m, int slot, int n, const int* tokens, const int* parents, int pos, int* next_tokens);
+int xalm_cuda_tree_accept(xalm_cuda_model* m, int slot, int pos, int n, const int* nodes);
 /* Pinned host buffer the logits are copied into by xalm_cuda_forward (alias it as InferenceState::_logits). */
 float* xalm_cuda_logits_host(xalm_cuda_model* m);
 /* Model::active_bytes(pos) (model.cpp:12-35), 64-bit, per-format bytes; this rank's shard only. */

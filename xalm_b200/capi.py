@@ -87,6 +87,9 @@ SYMBOLS = {
     "xalm_cuda_forward_batch_async": (_i, [_vp, _i, _vp, _vp, _vp, _i]),
     "xalm_cuda_forward_spans": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "xalm_cuda_forward_spans_argmax": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "xalm_cuda_forward_tree": (_i, [_vp, _i, _i, _vp, _vp, _i, _vp]),
+    "xalm_cuda_forward_tree_argmax": (_i, [_vp, _i, _i, _vp, _vp, _i, _vp]),
+    "xalm_cuda_tree_accept": (_i, [_vp, _i, _i, _i, _vp]),
     "xalm_cuda_select_seq": (_i, [_vp, _i]),
     "xalm_cuda_bench_matvec_batch": (_i, [_i, _i, _i, _i, _i, _i, _i, _i, _fp]),
 }

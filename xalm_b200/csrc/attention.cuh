@@ -95,13 +95,27 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 	const float inv_sqrt = 1.0f / sqrtf((float) HD);
 	const __half* kbase = a.k_cache + kv_off + (size_t) kvh * HD + li * 8;
 	const __half* vbase = a.v_cache + kv_off + (size_t) kvh * HD + li * 8;
+	// Batched steps read row t of the sequence where the entry's row map puts it (StepParams::tree).  A tree node i at depth d
+	// (xalm_cuda_forward_tree) has kv_fresh = the root's row, kv_pos = kv_fresh + i and kv_len = kv_fresh + d + 1; rows kv_fresh ..
+	// kv_len-1 map to its ancestors' rows, root first, then its own.  Since i >= d, kv_pos >= kv_len - 1: every row of this step it
+	// reads maps from a t in [kv_fresh, kv_pos], so the re-fetch after the dependency wait below (tested on t) covers all of them.
+	// The map is loaded where it is used (read-only path: StepParams rows are written before the step starts) rather than held in a
+	// register: that way no BATCH instance spills.
+	auto row = [&](int t) -> int {
+		if constexpr (!BATCH) {
+			return t;
+		} else {
+			const unsigned int d = (unsigned int) (t - kv_fresh);
+			return d < 8u ? kv_fresh + (int) ((__ldg(&step->tree) >> (3u * d)) & 7u) : t;
+		}
+	};
 
 	uint4 kn[TB], vn[TB]; // next batch, requested one iteration ahead
 	auto fetch = [&](int tb) {
 #pragma unroll
 		for (int j = 0; j < TB; j++) {
 			const int t = tb + j * RPW + sub;
-			const int tc = t < t1 ? t : t0;
+			const int tc = row(t < t1 ? t : t0);
 			kn[j] = ld_kv16(kbase + (size_t) tc * kv_stride);
 			vn[j] = ld_kv16(vbase + (size_t) tc * kv_stride);
 		}
@@ -135,8 +149,8 @@ __global__ void __launch_bounds__(NW * 32) attn_decode_kernel(const AttnArgs a) 
 		for (int j = 0; j < TB; j++) {
 			const int t = tb_first + j * RPW + sub;
 			if (t < t1 && ((t >= kv_fresh && t <= kv_pos) || t < kv_sink)) {
-				kn[j] = ld_kv16(kbase + (size_t) t * kv_stride);
-				vn[j] = ld_kv16(vbase + (size_t) t * kv_stride);
+				kn[j] = ld_kv16(kbase + (size_t) row(t) * kv_stride);
+				vn[j] = ld_kv16(vbase + (size_t) row(t) * kv_stride);
 			}
 		}
 	} else if (tb_first < t1) fetch(tb_first);

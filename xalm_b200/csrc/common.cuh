@@ -40,7 +40,11 @@ struct StepParams {
 	int slot;    // batched decode: the sequence slot (KV cache) this entry drives
 	int kv_fresh; // first ring row of this entry's slot written in this step: kv_pos, or the span's first row when the slot has
 	              // several entries (consecutive positions, xalm_cuda_forward_spans); rows kv_fresh .. kv_pos are written by the QKV kernel
+	uint32_t tree; // batched attention's row map (xalm_cuda_forward_tree): for 0 <= t - kv_fresh <= 7, row t of the entry's sequence is
+	               // read from row kv_fresh + ((tree >> 3 * (t - kv_fresh)) & 7); every other row is read where it is.  TREE_IDENTITY
+	               // everywhere but in a tree step.
 };
+constexpr uint32_t TREE_IDENTITY = 0xFAC688u; // 3-bit fields 0, 1, .., 7: row t is read from row t
 
 // ---- loads ---------------------------------------------------------------------------------------------
 // Weights are streamed exactly once per token: read-only path, do not allocate in L1 (activations live there).

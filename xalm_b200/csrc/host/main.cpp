@@ -1,7 +1,7 @@
 // main.cpp — the reference's CLI surface (src/main.cpp:417-547) on top of the CUDA backend.
 //
 //   xalm_main <checkpoint.xalm> [-d cuda] [-m completion|passkey|perplexity|batch] [-T ctx] [-i prompt | -f file] [-n steps] [-l pos] [-g gpus] [-b seqs]
-//             [-s draft] [-D draft.xalm]
+//             [-s draft] [-w branches] [-D draft.xalm]
 //
 // Same flags, same prefix matching for -m/-d, same defaults (mode completion, -n 128, the default prompt), same stats
 // block, plus the roofline fraction.  Differences, on purpose:
@@ -46,6 +46,8 @@ namespace {
 	fprintf(stderr, "Completion mode options:\n  -n <int>    number of steps to run for in completion mode, default 128. 0 = max_seq_len, -1 = infinite\n");
 	fprintf(stderr, "  -s <int>    speculative decoding: verify up to this many prompt-lookup draft tokens per pass (1..7; one GPU,\n"
 	                "              integer block formats; same output as without -s)\n");
+	fprintf(stderr, "  -w <int>    with -s k: verify up to this many prompt-lookup continuations per pass as one tree (1..k,\n"
+	                "              default 1; not with -D)\n");
 	fprintf(stderr, "  -D <filepath> with -s: draft the tokens with this model (same tokenizer, any weight format, same GPU) instead of\n"
 	                "              prompt lookup\n");
 	fprintf(stderr, "  Choose one:\n    -i <string> input prompt\n    -f <filepath> input file with prompt\n");
@@ -104,23 +106,59 @@ size_t hydrate(const Model& model, const InferenceState& state, const std::vecto
 	return read_bytes;
 }
 
-// Prompt lookup: up to k tokens that followed the most recent earlier occurrence of the sequence's last 3 tokens (else its last 2;
-// a single token is too weak a match to be worth a wider pass).  Empty when neither suffix occurred before.
-std::vector<int> draft_lookup(const std::vector<int>& seq, int k) {
+// Drafted tokens to verify in one pass, as a tree under the sequence's last token (node 0, not stored here): drafted node i + 1
+// decodes tokens[i] after node parents[i] (0: the last token itself).  Nodes are numbered in insertion order, so parents[i] <= i.
+struct DraftTree {
+	std::vector<int> tokens, parents;
+};
+
+// Prompt lookup: the continuations after earlier occurrences of the sequence's last 3 tokens, most recent first, then after those
+// of its last 2 (a single token is too weak a match to be worth a wider pass), up to k tokens each.  The first b that each add a
+// token the ones before do not already propose are merged into a trie under the last token, which grows level by level (every
+// candidate's first token, then every candidate's second, ...) in candidate order until it holds k drafted nodes.  With b = 1 this
+// is the chain after the most recent occurrence.  Empty when neither suffix occurred before.
+DraftTree draft_lookup(const std::vector<int>& seq, int k, int b) {
 	const size_t N = seq.size();
-	for (size_t n = 3; n >= 2; n--) {
+	std::vector<std::vector<int>> cand;
+	auto adds_nothing = [&](const std::vector<int>& c) {
+		for (const auto& o : cand)
+			if (o.size() >= c.size() && std::equal(c.begin(), c.end(), o.begin())) return true;
+		return false;
+	};
+	for (size_t n = 3; n >= 2 && (int) cand.size() < b; n--) {
 		if (N <= n) continue;
-		for (size_t s = N - n; s-- > 0;) // occurrences starting before the suffix itself, latest first
+		for (size_t s = N - n; s-- > 0 && (int) cand.size() < b;) // occurrences starting before the suffix itself, latest first
 			if (std::equal(seq.begin() + s, seq.begin() + s + n, seq.end() - n)) {
 				const size_t from = s + n, len = std::min((size_t) k, N - from);
-				return std::vector<int>(seq.begin() + from, seq.begin() + from + len);
+				std::vector<int> c(seq.begin() + from, seq.begin() + from + len);
+				if (!adds_nothing(c)) cand.push_back(std::move(c));
 			}
 	}
-	return {};
+	DraftTree t;
+	std::vector<int> at(cand.size(), 0); // the node each candidate has reached
+	for (size_t d = 0; (int) t.tokens.size() < k; d++) {
+		bool any = false;
+		for (size_t c = 0; c < cand.size() && (int) t.tokens.size() < k; c++) {
+			if (d >= cand[c].size()) continue;
+			any = true;
+			int child = -1;
+			for (size_t i = 0; i < t.tokens.size() && child < 0; i++)
+				if (t.parents[i] == at[c] && t.tokens[i] == cand[c][d]) child = (int) i + 1;
+			if (child < 0) {
+				t.tokens.push_back(cand[c][d]);
+				t.parents.push_back(at[c]);
+				child = (int) t.tokens.size();
+			}
+			at[c] = child;
+		}
+		if (!any) break;
+	}
+	return t;
 }
 
 struct SpecStats {
 	size_t passes = 0, drafted = 0, accepted = 0, decoded = 0; // decoded: tokens the passes produced (accepted + one per pass)
+	size_t branched = 0;                                       // passes whose tree had more than one branch
 };
 
 // Where the drafts of -m completion -s k come from: prompt lookup, or a draft model (-D) decoding greedily on its own handle.
@@ -132,16 +170,19 @@ struct Drafter {
 
 	// up to k tokens to follow seq; P = seq.size() - 1 is the target's next position and P + k stays inside the window.  The draft
 	// model catches up on the accepted tokens it has not decoded (seq[valid .. P]) and drafts k tokens in one greedy chain.
-	std::vector<int> draft(const std::vector<int>& seq, int k) {
-		if (!model) return draft_lookup(seq, k);
+	// b: prompt lookup's candidates per pass (-w); the draft model gives one, a chain.
+	DraftTree draft(const std::vector<int>& seq, int k, int b) {
+		if (!model) return draft_lookup(seq, k, b);
 		const size_t P = seq.size() - 1;
-		std::vector<int> out(k);
+		DraftTree t;
+		t.tokens.resize(k);
 		const double t0 = now_s();
-		model->forward_greedy(seq.data() + valid, (int) (P + 1 - valid), (int) valid, k, out.data());
+		model->forward_greedy(seq.data() + valid, (int) (P + 1 - valid), (int) valid, k, t.tokens.data());
 		seconds += now_s() - t0;
 		steps += P + 1 - valid + k - 1;
 		calls++;
-		return out;
+		for (int i = 0; i < k; i++) t.parents.push_back(i);
+		return t;
 	}
 	// a of the drafts of a round at P were accepted.  The chain wrote draft rows P+1 .. P+n-1 for its first n-1 drafts, and those
 	// of the accepted ones hold accepted tokens; rows of rejected drafts are rewritten before they are read, as a span's are
@@ -151,19 +192,21 @@ struct Drafter {
 	}
 };
 
-// The generation loop of -m completion -s k: the same greedy tokens, fewer passes over the weights.  Each step drafts up to k
-// tokens (Drafter) and verifies them with the last token in ONE span (Model::forward_spans_argmax): entry j's greedy
-// token is what a plain step would produce after the entries before it, so the longest prefix of the draft that matches those
-// tokens is accepted, plus the model's own token after it.  Rows written for rejected drafts need no cleanup (xalm_cuda.h).
-// Without a draft, or past the context window where spans are refused, the step is a plain forward on slot 0.  Prints the tokens
+// The generation loop of -m completion -s k [-w b]: the same greedy tokens, fewer passes over the weights.  Each step drafts a tree
+// of up to k tokens (Drafter; a chain unless prompt lookup has several candidates) and verifies it with the last token as its
+// root in ONE pass (Model::forward_tree_argmax): node i's greedy token is what a plain step would produce after the branch from
+// the root to i.  So starting at the root, the walk moves to the child whose token is the current node's greedy token while there
+// is one; the drafts it passes are accepted, plus the model's own token after the last.  Model::tree_accept moves that branch's
+// rows into place (nothing for a chain, or the lowest-numbered branch); rows of rejected drafts need no cleanup (xalm_cuda.h).
+// Without a draft, or past the context window where trees are refused, the step is a plain forward on slot 0.  Prints the tokens
 // as run_completion does; returns the bytes read.
 size_t generate_speculative(const Model& model, const InferenceState& state, const Sampler& sampler, const Tokenizer& tokenizer,
-                            std::vector<int>& encoding, int num_steps, int k, Drafter& drafter, SpecStats& st) {
+                            std::vector<int>& encoding, int num_steps, int k, int b, Drafter& drafter, SpecStats& st) {
 	const size_t W = (size_t) model.config.max_seq_len;
 	const size_t kv_row = W > 1 ? model.active_bytes(1) - model.active_bytes(0) : 0, weights = model.active_bytes(0) - kv_row;
 	size_t read_bytes = 0;
 	std::vector<int> pending = {sampler.sample_argmax(state)}; // greedy tokens known but not printed yet
-	std::vector<int> seqs, toks, pos, out;
+	std::vector<int> toks, parents, depth, out, path;
 	for (int i = 0;;) {
 		bool stop = false;
 		for (const int token_id : pending) {
@@ -176,39 +219,45 @@ size_t generate_speculative(const Model& model, const InferenceState& state, con
 		if (stop || !(i < num_steps || num_steps == -1)) break;
 		const size_t P = encoding.size() - 1;            // position of the last token, not yet decoded
 		const size_t room = P + 1 < W ? W - 1 - P : 0;    // draft positions P+1 .. P+len stay inside the window
-		const std::vector<int> draft = room ? drafter.draft(encoding, (int) std::min(room, (size_t) k)) : std::vector<int>{};
+		const DraftTree draft = room ? drafter.draft(encoding, (int) std::min(room, (size_t) k), b) : DraftTree{};
 		st.passes++;
-		if (draft.empty()) {
+		if (draft.tokens.empty()) {
 			model.forward(state, encoding.back(), (int) P);
 			read_bytes += model.active_bytes(P);
 			pending = {sampler.sample_argmax(state)};
 			st.decoded++;
 			continue;
 		}
-		const int n = (int) draft.size() + 1;
-		seqs.assign(n, 0);
+		const int n = (int) draft.tokens.size() + 1;
 		toks.assign(1, encoding.back());
-		toks.insert(toks.end(), draft.begin(), draft.end());
-		pos.resize(n);
+		toks.insert(toks.end(), draft.tokens.begin(), draft.tokens.end());
+		parents.assign(1, -1);
+		parents.insert(parents.end(), draft.parents.begin(), draft.parents.end());
+		depth.assign(1, 0);
+		for (int i = 1; i < n; i++) depth.push_back(depth[parents[i]] + 1);
 		out.resize(n);
-		for (int j = 0; j < n; j++) pos[j] = (int) P + j;
-		model.forward_spans_argmax(n, seqs.data(), toks.data(), pos.data(), out.data());
+		model.forward_tree_argmax(0, n, toks.data(), parents.data(), (int) P, out.data());
 		read_bytes += weights;
-		for (int j = 0; j < n; j++) read_bytes += (P + j + 1) * kv_row;
-		int a = 0;
-		while (a < n - 1 && out[a] == draft[a]) a++;
-		drafter.accepted(P, a, (int) draft.size());
-		pending.assign(draft.begin(), draft.begin() + a);
-		pending.push_back(out[a]);
-		st.drafted += draft.size();
+		for (int i = 0; i < n; i++) read_bytes += (P + depth[i] + 1) * kv_row;
+		path.assign(1, 0);
+		for (int i = 1; i < n; i++) // children come after their parent: one scan finds the accepted branch
+			if (parents[i] == path.back() && toks[i] == out[path.back()]) path.push_back(i);
+		model.tree_accept(0, (int) P, (int) path.size(), path.data());
+		const int a = (int) path.size() - 1;
+		drafter.accepted(P, a, n - 1);
+		pending.clear();
+		for (int j = 1; j <= a; j++) pending.push_back(toks[path[j]]);
+		pending.push_back(out[path.back()]);
+		st.drafted += n - 1;
 		st.accepted += a;
 		st.decoded += a + 1;
+		if (*std::max_element(depth.begin(), depth.end()) < n - 1) st.branched++;
 	}
 	return read_bytes;
 }
 
 void run_completion(const TpRank& tp, const std::string& checkpoint_path, const std::string& prompt, int context, int num_steps, int spec,
-                    const std::string& draft_path) {
+                    int width, const std::string& draft_path) {
 	auto model_data = Xalm::load(checkpoint_path);
 	std::cout << "loading model " << checkpoint_path << std::endl;
 	Model model = Model::from_xalm(model_data, context, /*defer_load=*/true); // weights go disk -> pinned -> device in model.cuda()
@@ -261,7 +310,7 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	}
 	const double hydrate_s = now_s() - t0;
 	SpecStats spec_stats;
-	if (spec) read_bytes += generate_speculative(model, state, sampler, tokenizer, encoding, num_steps, spec, drafter, spec_stats);
+	if (spec) read_bytes += generate_speculative(model, state, sampler, tokenizer, encoding, num_steps, spec, width, drafter, spec_stats);
 	else for (int i = 0; i < num_steps || num_steps == -1; i++) { // main.cpp:105-115
 		// the logits are all-gathered under -g, so every rank picks the same token and stops at the same step
 		const int token_id = sampler.sample_argmax(state);
@@ -282,6 +331,7 @@ void run_completion(const TpRank& tp, const std::string& checkpoint_path, const 
 	if (spec)
 		printf("  speculative: %zu passes, %zu drafted, %zu accepted, %.3g tokens/pass\n", spec_stats.passes, spec_stats.drafted, spec_stats.accepted,
 		       spec_stats.passes ? (double) spec_stats.decoded / spec_stats.passes : 0.0);
+	if (width > 1) printf("  tree: up to %d branches, %zu passes verified more than one\n", width, spec_stats.branched);
 	if (draft) printf("  draft: %s, %zu steps in %zu calls, %.5gs\n", draft_path.c_str(), drafter.steps, drafter.calls, drafter.seconds);
 }
 
@@ -512,7 +562,7 @@ int main(int argc, char* argv[]) {
 	std::string prompt = "Q: What is the meaning of life? A:"; // main.cpp:421
 	std::string prompt_path;
 	std::string convert_type, draft_path;
-	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8, spec = 0;
+	int context = 0, num_steps = 128, n_junk = 250, passkey_pos = -1, gpus = 1, max_batch = 8, spec = 0, width = 0;
 	if (argc >= 2) checkpoint_path = argv[1];
 	else error_usage();
 	for (int i = 2; i < argc;) { // main.cpp:435-512
@@ -544,6 +594,7 @@ int main(int argc, char* argv[]) {
 			spec = parse_gpus(v);
 			if (spec > 7) error_usage();
 		}
+		else if (f == 'w') width = parse_gpus(v);
 		else if (f == 'D') draft_path = v;
 		else if (f == 'n') { num_steps = std::stoi(v); n_junk = num_steps; }
 		else error_usage();
@@ -557,6 +608,11 @@ int main(int argc, char* argv[]) {
 		fprintf(stderr, "Error: -D drafts for -s (speculative -m completion on one GPU)\n");
 		error_usage();
 	}
+	if (width && (!spec || width > spec || !draft_path.empty())) {
+		fprintf(stderr, "Error: -w b widens -s k's prompt-lookup drafts to a tree of up to b branches, 1 <= b <= k (not with -D)\n");
+		error_usage();
+	}
+	if (!width) width = 1;
 	if (mode == "verify") {
 		if (gpus != 1) {
 			fprintf(stderr, "Error: -m verify runs on the host only and takes no -g\n");
@@ -606,7 +662,7 @@ int main(int argc, char* argv[]) {
 	}
 	auto run = [&](const TpRank& tp) {
 		try {
-			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps, spec, draft_path);
+			if (mode == "completion") run_completion(tp, checkpoint_path, prompt, context, num_steps, spec, width, draft_path);
 			else if (mode == "passkey") run_passkey(tp, checkpoint_path, context, n_junk, passkey_pos);
 			else run_perplexity(tp, checkpoint_path, prompt, context);
 		} catch (const std::exception& e) {

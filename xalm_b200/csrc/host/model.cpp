@@ -458,6 +458,16 @@ void Model::forward_spans_argmax(const int n, const int* seqs, const int* tokens
 	if (xalm_cuda_forward_spans_argmax(handle_, n, seqs, tokens, pos, next) != XALM_OK) xalm_throw_last("Model::forward_spans_argmax");
 }
 
+void Model::forward_tree_argmax(const int slot, const int n, const int* tokens, const int* parents, const int pos, int* next) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_tree_argmax: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_forward_tree_argmax(handle_, slot, n, tokens, parents, pos, next) != XALM_OK) xalm_throw_last("Model::forward_tree_argmax");
+}
+
+void Model::tree_accept(const int slot, const int pos, const int n, const int* nodes) const {
+	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::tree_accept: model is not on a CUDA device (call model.cuda())");
+	if (xalm_cuda_tree_accept(handle_, slot, pos, n, nodes) != XALM_OK) xalm_throw_last("Model::tree_accept");
+}
+
 void Model::forward_greedy(const int* tokens, const int n_in, const int pos, const int n_out, int* out) const {
 	if (device != Device::CUDA || !handle_) throw std::runtime_error("Model::forward_greedy: model is not on a CUDA device (call model.cuda())");
 	if (xalm_cuda_forward_greedy(handle_, n_in, tokens, pos, n_out, out) != XALM_OK) xalm_throw_last("Model::forward_greedy");

@@ -186,6 +186,12 @@ struct Model {
 	// forward_batch_argmax where a slot may take several consecutive positions in one step (xalm_cuda_forward_spans_argmax):
 	// how drafted tokens are verified in one pass over the weights.  next[i] is the greedy token after entry i.  A refused call throws.
 	void forward_spans_argmax(int n, const int* seqs, const int* tokens, const int* pos, int* next) const;
+	// Tree verification on one slot (xalm_cuda_forward_tree_argmax): node i decodes tokens[i] after its ancestors (parents[0] == -1,
+	// 0 <= parents[i] < i) at position pos + depth(i); next[i] is the greedy token after node i.  A refused call throws.
+	void forward_tree_argmax(int slot, int n, const int* tokens, const int* parents, int pos, int* next) const;
+	// Move the accepted root-to-node path nodes[0 .. n-1] of the tree last verified at pos into rows pos .. pos+n-1 of the slot
+	// (xalm_cuda_tree_accept; enqueue only, nothing for a chain).  A refused call throws.
+	void tree_accept(int slot, int pos, int n, const int* nodes) const;
 	// Greedy chain (xalm_cuda_forward_greedy): tokens[0 .. n_in-2] hydrate positions pos .. pos+n_in-2, tokens[n_in-1] decodes at
 	// pos+n_in-1, and each of the n_out - 1 further steps decodes the previous step's greedy token; out[i] is step i's token.  One
 	// host synchronisation per call, as a draft model drafts.  1 <= n_in <= 8, 1 <= n_out <= 16.  A refused call throws.

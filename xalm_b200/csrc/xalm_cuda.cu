@@ -608,6 +608,7 @@ static __host__ __device__ void fill_step_entry(const xalm_config& c, StepParams
 	p.kv_pos = p.kv_sink + (pos - p.kv_sink) % (c.max_seq_len - p.kv_sink);
 	p.kv_len = pos >= c.max_seq_len ? c.max_seq_len : pos + 1;
 	p.mode = mode;
+	p.tree = TREE_IDENTITY;
 }
 
 // One link of a greedy chain (xalm_cuda_forward_greedy): Sampler::sample_argmax of the single-sequence logits into *out and, unless
@@ -625,6 +626,26 @@ __global__ void argmax_next_step_kernel(const float* __restrict__ logits, int n,
 		p.ar_base = ar_base;
 		p.slot = 0;
 		*next = p;
+	}
+}
+
+// xalm_cuda_tree_accept: move j copies row src[j] to row dst[j] of one K or V cache, for j = 0 .. n-1 in that order, each once
+// the one before has landed.  The order matters: a move may write the row an earlier move read (never one a later move reads,
+// because sources lie above every earlier destination; xalm_cuda.h).  One CTA per cache: caches[2 l] / caches[2 l + 1] are layer l's
+// K / V caches, offset is the slot's first element, a row is kv_dim halves.  Launched without PDL, like argmax_next_step_kernel: it
+// starts once the verifying step has completed, and the next step's embedding (also launched without PDL) once it has.
+struct TreeMoves {
+	int n;
+	int src[MMB_MAX_SEQS], dst[MMB_MAX_SEQS]; // rows within the slot
+};
+__global__ void tree_accept_kernel(__half* const* __restrict__ caches, size_t offset, int kv_dim, const TreeMoves mv) {
+	__half* base = caches[blockIdx.x] + offset;
+	const int n16 = kv_dim / 8; // uint4 per row
+	for (int j = 0; j < mv.n; j++) {
+		const uint4* src = reinterpret_cast<const uint4*>(base + (size_t) mv.src[j] * kv_dim);
+		uint4* dst = reinterpret_cast<uint4*>(base + (size_t) mv.dst[j] * kv_dim);
+		for (int i = threadIdx.x; i < n16; i += blockDim.x) dst[i] = src[i];
+		__syncthreads();
 	}
 }
 
@@ -990,6 +1011,7 @@ struct xalm_cuda_model {
 	xalm::PeerArgs peer = {};
 	std::vector<void*> peer_opened;
 	unsigned int token_serial = 0;
+	__half** kv_table = nullptr;      // device: every layer's K and V cache (tree_accept_kernel)
 	int* d_argmax = nullptr;          // device-side sampler result
 	int* h_argmax = nullptr;          // pinned
 	// batched prefill (prefill.cu)
@@ -1603,6 +1625,12 @@ int xalm_cuda_finalize(xalm_cuda_model* m) {
 		XALM_CUDA_CHECK(cudaMemset(L.k_cache, 0, kv_elems * sizeof(__half)));
 		XALM_CUDA_CHECK(cudaMemset(L.v_cache, 0, kv_elems * sizeof(__half)));
 	}
+	if (m->batched) {
+		std::vector<__half*> table;
+		for (auto& L : m->layers) { table.push_back(L.k_cache); table.push_back(L.v_cache); }
+		XALM_TRY(m->da.alloc((void**) &m->kv_table, table.size() * sizeof(__half*)));
+		XALM_CUDA_CHECK(cudaMemcpy(m->kv_table, table.data(), table.size() * sizeof(__half*), cudaMemcpyHostToDevice));
+	}
 	const std::vector<float> freq = rope_freq_table(c.head_dim, c.rotary_dim, c.rope_theta);
 	XALM_TRY(m->da.alloc((void**) &m->rope_freq, freq.size() * sizeof(float)));
 	XALM_CUDA_CHECK(cudaMemcpy(m->rope_freq, freq.data(), freq.size() * sizeof(float), cudaMemcpyHostToDevice));
@@ -1834,17 +1862,36 @@ int xalm_cuda_select_seq(xalm_cuda_model* m, int seq) {
 	return XALM_OK;
 }
 
+// The checks every call on a batched handle's slots starts with: a finalized batched handle, 1 <= n <= max_seqs.
+static int check_batched(xalm_cuda_model* m, const char* fn, int n) {
+	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
+	if (!m->finalized) return set_error(XALM_ERR_STATE, "%s before finalize", fn);
+	if (!m->batched) return set_error(XALM_ERR_STATE, "%s on a handle without xalm_cuda_set_batch", fn);
+	if (n < 1 || n > m->max_seqs) return set_error(XALM_ERR_INVALID, "%s: n = %d not in [1, %d]", fn, n, m->max_seqs);
+	return XALM_OK;
+}
+
+// Claim a row group of the StepParams ring, let fill(rows) write its n entries, upload them and run the batched step of n entries.
+extern "C++" {
+template <class Fill>
+static int run_batched_rows(xalm_cuda_model* m, int n, int mode, Fill fill) {
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	StepParams* sp = nullptr;
+	XALM_TRY(claim_step_rows(m, &sp));
+	fill(sp);
+	XALM_TRY(upload_step_rows(m, sp, n));
+	return run_step(m, mode, n);
+}
+}
+
 // One step of n entries: entry i drives slot seqs[i] with tokens[i] at pos[i].  spans = false (forward_batch): every slot at most
 // once.  spans = true (forward_spans): a slot may take several consecutive positions, all inside the window; the attention of
 // each such entry re-reads, after its dependency wait, every row the step writes for its slot up to its own (kv_fresh .. kv_pos).
 // Everything is validated before anything is enqueued, so a refusal leaves every cache untouched.
 static int forward_step_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode, bool spans) {
 	const char* fn = spans ? "forward_spans" : "forward_batch";
-	if (!m) return set_error(XALM_ERR_INVALID, "model is NULL");
-	if (!m->finalized) return set_error(XALM_ERR_STATE, "%s before finalize", fn);
-	if (!m->batched) return set_error(XALM_ERR_STATE, "%s on a handle without xalm_cuda_set_batch", fn);
+	XALM_TRY(check_batched(m, fn, n));
 	if (mode != XALM_HYDRATE_KV_CACHE && mode != XALM_OUTPUT_LOGITS) return set_error(XALM_ERR_INVALID, "bad mode %d", mode);
-	if (n < 1 || n > m->max_seqs) return set_error(XALM_ERR_INVALID, "%s: n = %d not in [1, %d]", fn, n, m->max_seqs);
 	if (!seqs || !tokens || !pos) return set_error(XALM_ERR_INVALID, "NULL argument");
 	const xalm_config& c = m->c;
 	int first[MMB_MAX_SEQS], last[MMB_MAX_SEQS]; // per slot: its first and latest entry so far (-1: none)
@@ -1864,17 +1911,80 @@ static int forward_step_async(xalm_cuda_model* m, int n, const int* seqs, const 
 		if (first[s] != last[s] && pos[last[s]] >= c.max_seq_len)
 			return set_error(XALM_ERR_INVALID, "forward_spans: the span of slot %d reaches position %d, spans stay below max_seq_len %d", s,
 			                 pos[last[s]], c.max_seq_len);
-	XALM_CUDA_CHECK(cudaSetDevice(m->device));
-	StepParams* sp = nullptr;
-	XALM_TRY(claim_step_rows(m, &sp));
+	return run_batched_rows(m, n, mode, [&](StepParams* sp) {
+		for (int i = 0; i < n; i++) {
+			fill_step_entry(c, sp[i], tokens[i], pos[i], mode);
+			sp[i].kv_fresh = sp[first[seqs[i]]].kv_pos; // == kv_pos unless an earlier entry of this step drives the same slot
+			sp[i].ar_base = 0;
+			sp[i].slot = seqs[i];
+		}
+	});
+}
+
+// One step of a tree of n drafted nodes of one slot (xalm_cuda_forward_tree): node i decodes tokens[i] at position pos + depth(i),
+// writes its K/V to row pos + i, and its attention reads rows pos .. pos + depth(i) through the row map (StepParams::tree), which
+// sends depth e to the row of its ancestor at depth e.  Everything is validated before anything is enqueued.
+static int forward_tree_async(xalm_cuda_model* m, int slot, int n, const int* tokens, const int* parents, int pos) {
+	XALM_TRY(check_batched(m, "forward_tree", n));
+	if (!tokens || !parents) return set_error(XALM_ERR_INVALID, "NULL argument");
+	const xalm_config& c = m->c;
+	if (slot < 0 || slot >= m->max_seqs) return set_error(XALM_ERR_INVALID, "forward_tree: slot %d not in [0, %d)", slot, m->max_seqs);
+	if (pos < 0) return set_error(XALM_ERR_INVALID, "negative position");
+	if (pos > c.max_seq_len - n)
+		return set_error(XALM_ERR_INVALID, "forward_tree: rows %d .. %d reach max_seq_len %d, trees stay below the window", pos, pos + n - 1,
+		                 c.max_seq_len);
+	int depth[MMB_MAX_SEQS];
 	for (int i = 0; i < n; i++) {
-		fill_step_entry(c, sp[i], tokens[i], pos[i], mode);
-		sp[i].kv_fresh = sp[first[seqs[i]]].kv_pos; // == kv_pos unless an earlier entry of this step drives the same slot
-		sp[i].ar_base = 0;
-		sp[i].slot = seqs[i];
+		if (tokens[i] < 0 || tokens[i] >= c.vocab_size) return set_error(XALM_ERR_INVALID, "token %d out of range [0,%d)", tokens[i], c.vocab_size);
+		if (i == 0 ? parents[0] != -1 : parents[i] < 0 || parents[i] >= i)
+			return set_error(XALM_ERR_INVALID, "forward_tree: parents[%d] = %d (the root's is -1, node i's lies in [0, i))", i, parents[i]);
+		depth[i] = i == 0 ? 0 : depth[parents[i]] + 1;
 	}
-	XALM_TRY(upload_step_rows(m, sp, n));
-	return run_step(m, mode, n);
+	return run_batched_rows(m, n, XALM_OUTPUT_LOGITS, [&](StepParams* sp) {
+		for (int i = 0; i < n; i++) {
+			fill_step_entry(c, sp[i], tokens[i], pos + depth[i], XALM_OUTPUT_LOGITS); // kv_len = pos + depth + 1: the branch's length
+			sp[i].kv_pos = pos + i;
+			sp[i].kv_fresh = pos;
+			sp[i].ar_base = 0;
+			sp[i].slot = slot;
+			for (int v = i; v >= 0; v = parents[v])
+				sp[i].tree = (sp[i].tree & ~(7u << 3 * depth[v])) | (uint32_t) v << 3 * depth[v];
+		}
+	});
+}
+
+int xalm_cuda_forward_tree(xalm_cuda_model* m, int slot, int n, const int* tokens, const int* parents, int pos, float* logits_host) {
+	XALM_TRY(forward_tree_async(m, slot, n, tokens, parents, pos));
+	return finish_step(m, n, XALM_OUTPUT_LOGITS, logits_host);
+}
+
+int xalm_cuda_forward_tree_argmax(xalm_cuda_model* m, int slot, int n, const int* tokens, const int* parents, int pos, int* next_tokens) {
+	if (!next_tokens) return set_error(XALM_ERR_INVALID, "next_tokens is NULL");
+	XALM_TRY(forward_tree_async(m, slot, n, tokens, parents, pos));
+	return finish_step_argmax(m, n, next_tokens);
+}
+
+int xalm_cuda_tree_accept(xalm_cuda_model* m, int slot, int pos, int n, const int* nodes) {
+	XALM_TRY(check_batched(m, "tree_accept", n));
+	if (!nodes) return set_error(XALM_ERR_INVALID, "NULL argument");
+	if (slot < 0 || slot >= m->max_seqs) return set_error(XALM_ERR_INVALID, "tree_accept: slot %d not in [0, %d)", slot, m->max_seqs);
+	if (pos < 0) return set_error(XALM_ERR_INVALID, "negative position");
+	if (nodes[0] != 0) return set_error(XALM_ERR_INVALID, "tree_accept: nodes[0] = %d, a path starts at the root (0)", nodes[0]);
+	for (int j = 1; j < n; j++)
+		if (nodes[j] <= nodes[j - 1] || nodes[j] >= m->max_seqs)
+			return set_error(XALM_ERR_INVALID, "tree_accept: nodes[%d] = %d after %d (a path's nodes increase and stay below %d)", j, nodes[j],
+			                 nodes[j - 1], m->max_seqs);
+	if (pos > m->c.max_seq_len - 1 - nodes[n - 1])
+		return set_error(XALM_ERR_INVALID, "tree_accept: row %d reaches max_seq_len %d, trees stay below the window", pos + nodes[n - 1],
+		                 m->c.max_seq_len);
+	TreeMoves mv = {};
+	for (int j = 0; j < n; j++)
+		if (nodes[j] != j) { mv.src[mv.n] = pos + nodes[j]; mv.dst[mv.n] = pos + j; mv.n++; }
+	if (!mv.n) return XALM_OK;
+	XALM_CUDA_CHECK(cudaSetDevice(m->device));
+	XALM_CUDA_CHECK(launch(tree_accept_kernel, dim3(2 * m->c.n_layers), dim3(128), m->stream, false, (__half* const*) m->kv_table,
+	                       (size_t) slot * m->kv_slot, m->kv_dim_l, mv));
+	return XALM_OK;
 }
 
 int xalm_cuda_forward_batch_async(xalm_cuda_model* m, int n, const int* seqs, const int* tokens, const int* pos, int mode) {

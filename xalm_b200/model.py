@@ -239,6 +239,37 @@ class Model:
         capi.check(capi.lib().xalm_cuda_forward_spans_argmax(self._h, arrs[0].size, *ptrs, out.ctypes.data_as(C.c_void_p)))
         return [int(v) for v in out]
 
+    @staticmethod
+    def _tree_args(tokens, parents):
+        arrs = [np.ascontiguousarray(v, dtype=np.int32).reshape(-1) for v in (tokens, parents)]
+        if arrs[0].size == 0 or arrs[0].size != arrs[1].size:
+            raise ValueError("tokens and parents must have the same, non-zero length")
+        return arrs, [a.ctypes.data_as(C.c_void_p) for a in arrs]
+
+    def forward_tree(self, slot: int, tokens, parents, pos: int):
+        """One step of a tree of drafted tokens on one slot (tree verification): node i decodes tokens[i] after its ancestors
+        (parents[0] == -1, 0 <= parents[i] < i), at position pos + depth(i).  Returns the (n, vocab) logits, row i for node i."""
+        arrs, ptrs = self._tree_args(tokens, parents)
+        n = arrs[0].size
+        lg = np.empty((n, self.config["vocab_size"]), dtype=np.float32)
+        capi.check(capi.lib().xalm_cuda_forward_tree(self._h, int(slot), n, *ptrs, int(pos), lg.ctypes.data_as(C.c_void_p)))
+        return lg
+
+    def forward_tree_argmax(self, slot: int, tokens, parents, pos: int) -> list:
+        """forward_tree + Sampler.sample_argmax of each node's row on the device."""
+        arrs, ptrs = self._tree_args(tokens, parents)
+        out = np.empty(arrs[0].size, dtype=np.int32)
+        capi.check(capi.lib().xalm_cuda_forward_tree_argmax(self._h, int(slot), arrs[0].size, *ptrs, int(pos), out.ctypes.data_as(C.c_void_p)))
+        return [int(v) for v in out]
+
+    def tree_accept(self, slot: int, pos: int, nodes) -> None:
+        """Move the accepted root-to-node path `nodes` (nodes[0] == 0, increasing) of the tree last verified at pos on this slot
+        into rows pos .. pos + len(nodes) - 1.  Enqueue only; nothing when nodes[j] == j for every j."""
+        arr = np.ascontiguousarray(nodes, dtype=np.int32).reshape(-1)
+        if arr.size == 0:
+            raise ValueError("tree_accept: nodes must not be empty")
+        capi.check(capi.lib().xalm_cuda_tree_accept(self._h, int(slot), int(pos), arr.size, arr.ctypes.data_as(C.c_void_p)))
+
     def select_seq(self, seq: int) -> None:
         """The slot forward*, prefill*, read_kv and read_state work on (default 0)."""
         capi.check(capi.lib().xalm_cuda_select_seq(self._h, seq))
